@@ -18,6 +18,9 @@ N > 1    : one process per GPU (torchrun), each rank piles up its own sample (th
            with the pileup in one enqueue (tc_pileup_counts_allreduce, NCCL) inside the timed region — strong scaling, checked bit for bit
            against the single-GPU table.  `configs` (N = 1): tc_pileup_counts on the other configs.
            `parity_checked`: the GPU table over the cpu_baseline prefix equals the oracle's.
+`--dump-outputs DIR`: after the timed steps, the last step's count table, call table and insertion calls go to DIR/<name>.npy
+           (float64).  The sample is generated from a fixed seed, so two builds run with the same arguments can be compared
+           output for output.
 `--impl reference` times the CPU oracle port of the reference path (oracle/, all host threads) on a
 bounded sample of the same workload; the reference itself is pure Python on pysam, which is not
 installable here (DESIGN.md), so oracle/_ref does not exist.
@@ -141,6 +144,35 @@ def make_sample(scale: float, sample: int):
     w.params.seed = w.params.seed * 1000 + sample
     batch = synth.generate_reads(w.params, w.ref)
     return w, batch
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def step_outputs(counts, table, calls) -> dict:
+    """What a caller of the hot path receives from one step, as float64 host arrays (exact for every value here): the count
+    table, the call table's columns and the insertion calls (strings as character codes, zero-padded; a call without
+    entries is a row of zeros)."""
+    names = ("call_char", "flags", "xrun", "rank_letter", "rank_count", "ambig_char")
+    out = {"counts": counts.cpu().numpy()}
+    out.update({n: t.cpu().numpy() for n, t in zip(names, table)})
+    width = max([len(c["string"] or "") for c in calls], default=0)
+    strings = np.zeros((len(calls), width))
+    for i, c in enumerate(calls):
+        strings[i, :len(c["string"] or "")] = [ord(ch) for ch in c["string"] or ""]
+    for k in ("pos", "n_entries", "mode_count", "first_read"):
+        out[f"insert_{k}"] = np.array([c[k] for c in calls])
+    out["insert_string"] = strings
+    return {k: v.astype(np.float64) for k, v in out.items()}
+
+
+def dump_outputs(directory: str, arrays: dict) -> None:
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"bench.py: {total} bytes of outputs exceed the {DUMP_LIMIT_BYTES}-byte dump limit")
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, f"{name}.npy"), a)
 
 
 def hot_path(ctx, reads, L, mincov, counts_dev, table, flags_dev, stream, params=None, chained=True):
@@ -550,6 +582,13 @@ def run_ours(args):
     sampler.close_window()
     launches = ctx.launches - launches0
     ms_total = ev0.elapsed_time(ev1)
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        # the chained loop alternates two sets of tables: step s wrote the second set when s is even; the end-to-end loop
+        # below writes into both count tables, so the last step's outputs are read back here
+        last = (counts_dev2, out2) if args.steps % 2 == 0 and not args.unchained else \
+            (counts_dev, (call_char, flags_dev, xrun, rank_letter, rank_count, ambig))
+        dumped = step_outputs(*last, calls)
     # ---------------- end to end through the C-ABI with host buffers: `e2e`
     # Two samples travel at a time: two host threads, each with a context, a stream and output buffers of its own, so one
     # sample's upload overlaps the other's kernels and read-backs (every call below blocks its own thread only; the C-ABI
@@ -678,6 +717,8 @@ def run_ours(args):
         if ceiling is not None:
             line["e2e"]["h2d_ceiling"] = ceiling
             line["e2e"]["h2d_frac_of_ceiling"] = (h2d / (e2e_ms / args.steps * 1e-3) / 1e9) / ceiling["gb_per_s_per_rank"]
+        if dumped is not None:
+            dump_outputs(args.dump_outputs, dumped)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -701,7 +742,11 @@ def main():
     ap.add_argument("--h2d-ceiling", action="store_true", help="also measure the concurrent pinned H2D ceiling at N = 1")
     ap.add_argument("--cpu-reads", type=float, default=1_000_000, help="reads in the cpu_baseline sample (1 M reads = 400 M aligned bases, 10-15 s on one core)")
     ap.add_argument("--ref-reads", type=float, default=400_000, help="reads per step of the --impl reference arm")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs (rank 0's sample) to DIR/<name>.npy "
+                                                         "as float64: count table, call table, insertion calls")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -13,7 +13,6 @@ GOLD = os.path.join(ROOT, "tests", "golden")
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "reference: needs /root/reference (only present in the build container)")
 
 
 def _has_cuda() -> bool:
@@ -33,8 +32,6 @@ def pytest_collection_modifyitems(config, items):
                 has = _has_cuda()
             if not has:
                 item.add_marker(pytest.mark.skip(reason="no CUDA device"))
-        if "reference" in item.keywords and not os.path.isdir("/root/reference/TrueConsense"):
-            item.add_marker(pytest.mark.skip(reason="/root/reference not present"))
 
 
 @pytest.fixture(scope="session")

@@ -1416,3 +1416,49 @@ def test_bam_file_on_device_long_header_and_unplaced_records(ctx, tmp_path):
     assert dev.info["n_records"] == len(out) and dev.info["n_dropped_unplaced"] == len(out) - len(recs)
     _assert_device_reads_equal_host(ctx, dev, host)
     assert bamio.read_bam_header(path) == (host.ref_names, host.ref_lens)
+
+
+# ---------------------------------------------------------------------------- (7) bench.py --dump-outputs
+def test_bench_dump_outputs_are_the_last_steps_results(orc, tmp_path):
+    """`bench.py --dump-outputs DIR`: the last timed step's count table, call table and insertion calls as float64 arrays —
+    the same from run to run (an odd and an even number of steps read back the two different sets of tables the chained
+    loop alternates between) and equal to the oracle's on the benchmarked sample."""
+    import importlib.util
+    import re
+    import subprocess
+    import sys
+
+    from conftest import ROOT
+
+    pileup, call = orc
+    dumps = []
+    for steps in (1, 2):
+        d = tmp_path / f"steps{steps}"
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", str(steps), "--warmup", "1",
+                              "--scale", "0.01", "--spinup", "0", "--no-read-range", "--no-configs", "--cpu-reads", "2000",
+                              "--e2e-lanes", "1", "--dump-outputs", str(d)], capture_output=True, text=True, timeout=900)
+        assert out.returncode == 0, out.stderr[-2000:]
+        assert json.loads(out.stdout.strip().splitlines()[-1])["steps"] == steps
+        dumps.append({p.stem: np.load(p) for p in d.glob("*.npy")})
+    a, b = dumps
+    assert sorted(a) == sorted(b) and all(np.array_equal(a[k], b[k]) for k in a)
+    assert all(v.dtype == np.float64 for v in a.values()) and sum(v.nbytes for v in a.values()) <= 64 << 20
+
+    spec = importlib.util.spec_from_file_location("tc_bench", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    w, batch = bench.make_sample(0.01, 0)
+    L = len(w.ref)
+    exp = pileup.pileup_counts(batch, L).astype(np.int64)
+    assert np.array_equal(a["counts"], exp)
+    ref = call.call_table(exp, w.mincov, True)
+    for k in ("call_char", "flags", "xrun", "ambig_char"):
+        assert np.array_equal(a[k], ref[k]), k
+    cands = call.insert_candidates(exp, w.mincov)
+    assert len(cands) > 0 and a["insert_pos"].tolist() == cands
+    for i, p in enumerate(cands):
+        cols = pileup.pileup_columns(batch, region=(p - 1, p), **pileup.EXTRACTINSERTS)
+        exp_bases = call.extract_insert(cols[0][1] if cols else "")
+        s = "".join(chr(int(c)) for c in a["insert_string"][i] if c)
+        m = re.search(r"(\d)([a-zA-Z]+)", s)
+        assert ((m.group(2), m.group(1)) if m else (None, None)) == exp_bases, (p, s)
