@@ -23,6 +23,9 @@
  * (TrueConsense/TrueConsense.py:225-226), so every entry point sets the CUDA
  * device of its context itself.
  *
+ * A pass covers one reference (contig); a BAM with several is called in one pass by placing its references side by side
+ * (tc_bam_contig_ranges, tc_reads_to_contig_coords, tc_call_contigs below).
+ *
  * There is no CPU fallback anywhere behind this ABI: without a CUDA device
  * tc_ctx_create fails with TC_ERR_NO_DEVICE.
  */
@@ -58,7 +61,8 @@ enum {
 };
 
 /* ---- flat read arrays (what the BAM decoder produces; BAM field names) ----
- * Reads are in file order and must be sorted by `pos` (coordinate-sorted BAM, one contig).
+ * Reads are in file order and must be sorted by `pos` (coordinate-sorted BAM, one contig — or several references moved
+ * side by side by tc_reads_to_contig_coords).
  * seq4 uses BAM's own packing (high nibble first, codes "=ACMGRSVTWYHKDBN"), but every
  * read starts on a 32-bit word boundary: read i occupies words seq_off[i] .. seq_off[i+1]-1,
  * the byte stream inside those words is the BAM byte stream.  QUAL shares the same
@@ -254,6 +258,38 @@ int  tc_depth(tc_ctx_t* ctx, const tc_reads_t* reads, int32_t ref_len,
  * counts as produced by tc_pileup_counts (or an overridden index).  Any member of *table may be NULL. */
 int  tc_call(tc_ctx_t* ctx, const int32_t* counts, int32_t ref_len,
              const tc_call_params_t* params, const tc_call_table_t* table, void* stream);
+
+/* ---- several references side by side (a segmented genome, a panel of references) ----
+ * In a multi-reference pass reference k occupies the global columns [contig_start[k], contig_start[k+1]) of one count table
+ * of total_len columns (contig_start: the exclusive prefix sum of the references' lengths, contig_start[n] = total_len).
+ * tc_pileup_counts, tc_list_insert_candidates and tc_extract_inserts run over total_len as they are; these three entry
+ * points are what such a pass needs besides them (every column of reference k then holds what a pass over reference k
+ * alone computes for it).
+ *
+ * tc_bam_contig_ranges: first_read[n_ref + 1] (host or device) from the records tc_bam_records_to_reads parses (payload and
+ * rec_off as it takes them, host or device): the reads of reference k are first_read[k] .. first_read[k+1]-1.  One thread
+ * per record reads its refID.  TC_ERR_UNSORTED when the refIDs decrease, TC_ERR_RANGE for a refID outside [0, n_ref).
+ * Synchronises the stream. */
+int  tc_bam_contig_ranges(tc_ctx_t* ctx, const uint8_t* payload, int64_t n_bytes, const int64_t* rec_off, int64_t n_reads,
+                          int32_t n_ref, int32_t* first_read, void* stream);
+
+/* tc_reads_to_contig_coords: moves device-resident reads (tc_reads_upload, tc_bam_records_to_reads) to the global columns
+ * IN PLACE: pos += contig_start[k] for the reads of reference k (first_read as above, ref_len[n_ref]: the lengths the
+ * pileup of each reference takes, host or device), and mpos likewise when it is >= 0 (-1 and -2 stay).  A mapped read
+ * with pos < 0, pos >= ref_len[k] or pos + reference span > ref_len[k] is TC_ERR_RANGE (what tc_pileup_counts over that
+ * reference alone says; the message names the read and the reference's index) — the reads before it are moved by then,
+ * so the batch must be decoded again.  Unmapped reads (FLAG 0x4, dropped by every pass) are kept inside their
+ * reference.  TC_ERR_ARG when the lengths add up to more than INT32_MAX.  contig_start[n_ref + 1] (host or device, may
+ * be NULL) receives the boundaries.  Calling it twice on the same arrays moves them twice: the caller keeps track.
+ * Synchronises the stream. */
+int  tc_reads_to_contig_coords(tc_ctx_t* ctx, const tc_reads_t* reads, int32_t n_ref, const int32_t* ref_len,
+                               const int32_t* first_read, int32_t* contig_start, void* stream);
+
+/* tc_call_contigs: tc_call over a count table of total_len columns holding n references (contig_start[n + 1], host or
+ * device): every column as tc_call computes it, except that a run of X positions (xrun) never crosses into the next
+ * reference and TC_CF_XRUN_OFF_END marks the runs that reach their own reference's end.  tc_call is the case n == 1. */
+int  tc_call_contigs(tc_ctx_t* ctx, const int32_t* counts, int32_t total_len, int32_t n, const int32_t* contig_start,
+                     const tc_call_params_t* params, const tc_call_table_t* table, void* stream);
 
 /* IsAmbiguous on n independent columns given already-ranked (letter,count) tuples
  * (Ambig.py:179): letters uint8[4][n], cnts int32[4][n], cov int32[n] -> out_char uint8[n] (0 = not ambiguous). */

@@ -19,6 +19,14 @@ def BuildCoverage(iDict, output):
             outfile.write(str(i + 1) + "\t" + str(cov) + "\n")
 
 
+def BuildCoverageContigs(indexes, output):
+    """``reference<TAB>pos<TAB>coverage`` (the usual three-column depth format), positions 1-based per reference, for
+    ``{reference: index dict}`` in its order."""
+    with open(output, "w") as outfile:
+        for name, iDict in indexes.items():
+            outfile.write("".join(f"{name}\t{i + 1}\t{iDict[i + 1].get('coverage')}\n" for i in range(len(iDict))))
+
+
 def GetCoverage(iDict, position):
     """Coverage.py:19-34."""
     return iDict[position].get("coverage")

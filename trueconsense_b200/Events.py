@@ -100,6 +100,42 @@ def ListInserts(iDict, mincov, bam):
     return out
 
 
+def ListInsertsContigs(indexes, mincov, bam):
+    """``ListInserts`` for every reference of the BAM in one pass: ``{reference: (True, {pos: {size: bases}}) | (False, None)}``
+    in header order, each equal to ``ListInserts`` over that reference alone.  ``indexes``: ``{reference: index dict}``
+    (``BuildIndexContigs``' frames as dicts).  One segmented call (``tc_call_contigs``), one candidate list and one
+    ExtractInserts call cover all references; positions come back per reference, 1-based."""
+    h = _bam_handle(bam)
+    names = list(h.references)
+    missing = [n for n in names if n not in indexes]
+    if missing:
+        raise ValueError(f"no index for reference {missing[0]!r}")
+    parts = [_counts_from_index(indexes[n]) for n in names]
+    out = {n: (False, None) for n in names}
+    lens = [c.shape[1] for c in parts]
+    if sum(lens) == 0:
+        return out
+    d, lay = h.device_reads_contigs(names, lens)
+    ctx = gpu.default_context()
+    table = ctx.call_contigs(np.concatenate(parts, axis=1), lay.start, mincov, False)
+    cands = ctx.list_insert_candidates(table.flags, lay.total)
+    if not len(cands):
+        return out
+    k, local = lay.locate(cands)
+    bam_lens = np.asarray(h.lengths, dtype=np.int64)
+    keep = local <= bam_lens[k]                 # as ListInserts keeps the columns inside the BAM's reference
+    res = ctx.extract_inserts(d, lay.total, cands[keep]) if keep.any() else []
+    found: dict[str, dict] = {}
+    for r, kk, pos in zip(res, k[keep].tolist(), local[keep].tolist()):
+        bases, size = _parse_modal(r["string"])
+        if bases is None or size is None:
+            continue
+        found.setdefault(names[kk], {})[int(pos)] = {size: bases}
+    for n, positions in found.items():
+        out[n] = (True, positions)
+    return out
+
+
 def MinorityDel(index, p):
     """``(X / cov) * 100 >= 15`` — Events.py:85-106 (ZeroDivisionError when cov == 0)."""
     row = index[p]

@@ -13,6 +13,8 @@ from __future__ import annotations
 import sys
 from datetime import date
 
+import numpy as np
+
 from .Coverage import GetCoverage
 from .Events import ListInserts
 from .indexing import Readbam
@@ -37,6 +39,27 @@ def _first_fasta_record(path):
     if not seen:
         raise UnboundLocalError("cannot access local variable 'reflist' where it is not associated with a value")
     return rec_id, list("".join(chunks))
+
+
+def _fasta_records(path):
+    """{id: list of residues} of every record, the first of an id winning — _first_fasta_record for each reference."""
+    out: dict[str, list] = {}
+    rec_id, chunks = None, []
+
+    def close():
+        if rec_id is not None and rec_id not in out:
+            out[rec_id] = list("".join(chunks))
+
+    with open(path) as fh:
+        for line in fh:
+            if line.startswith(">"):
+                close()
+                words = line[1:].split(None, 1)
+                rec_id, chunks = (words[0] if words else ""), []
+            elif rec_id is not None:
+                chunks.append("".join(line.split()))
+    close()
+    return out
 
 
 def _gff_line(feature: dict) -> str:
@@ -83,6 +106,12 @@ VCF_HEADER = ("##fileformat=VCFv4.3\n"
               '##INFO=<ID=DP,Number=1,Type=Integer,Description="Read Depth">\n'
               '##INFO=<ID=INDEL,Number=0,Type=Flag,Description="Indicates that the variant is an INDEL.">\n'
               "#CHROM\tPOS\tID\tREF\tALT\tQUAL\tFILTER\tINFO\n")
+
+
+def vcf_header(ref, contigs) -> str:
+    """The VCF header with one ``##contig`` line per reference."""
+    head = VCF_HEADER.format(today=date.today().strftime("%Y%m%d"), argv=" ".join(sys.argv[1:]), ref=ref, contig="\0")
+    return head.replace("##contig=<ID=\0>\n", "".join(f"##contig=<ID={c}>\n" for c in contigs))
 
 
 def _vcf_records(contig, reference, called, index, mincov, inserts):
@@ -138,4 +167,53 @@ def WriteOutputs(mincov, iDict, uGffDict, inputbam, IncludeAmbig, output_vcf, na
 
     with open(output_consensus, "w") as out:
         out.write(f">{name} mincov={mincov}\n{with_inserts}\n")
+    return None, None
+
+
+def WriteOutputsContigs(mincov, indexes, gffdicts, inputbam, IncludeAmbig, output_vcf, name, ref, output_gff, gffheader,
+                        output_consensus):
+    """``WriteOutputs`` for every reference of the BAM (``indexes`` / ``gffdicts``: ``{reference: index dict}`` and
+    ``{reference: that reference's GFF rows as a dict}``, header order).  Both walks of every reference are computed first —
+    one segmented call table and one insertion pass for all of them — then the files are written in the usual order:
+    the GFF header once and each reference's corrected features; one VCF header with a ``##contig`` line per reference
+    and each reference's records with CHROM = the reference; one FASTA record ``>{name}_{reference}`` per reference.  An
+    exception of any reference aborts the run before a file is written (the VCF writer's own, part-way, as usual); the
+    FASTA then does not exist."""
+    from . import gpu
+    from .Events import ListInsertsContigs, _counts_from_index
+    from .Sequences import complement_index, consensus_from_inserts
+
+    bam = Readbam(inputbam)
+    names = list(bam.references)
+    for n in names:
+        complement_index(indexes[n], gffdicts[n], [])
+    inserts = ListInsertsContigs(indexes, mincov, bam)
+    parts = [_counts_from_index(indexes[n]) for n in names]
+    start = np.concatenate(([0], np.cumsum([c.shape[1] for c in parts]))).astype(np.int64)
+    table = gpu.default_context().call_contigs(np.concatenate(parts, axis=1), start, mincov, IncludeAmbig is True)
+    walks = {}
+    for k, n in enumerate(names):
+        t = table.slice(int(start[k]), int(start[k + 1]))
+        with_inserts, corrected_gff = consensus_from_inserts(mincov, parts[k], gffdicts[n], IncludeAmbig, inserts[n], True, table=t)
+        without_inserts = consensus_from_inserts(mincov, parts[k], gffdicts[n], IncludeAmbig, inserts[n], False, table=t)[0]
+        walks[n] = (with_inserts, corrected_gff, without_inserts)
+
+    if output_gff is not None:
+        with open(output_gff, "w") as out:
+            out.write(gffheader.raw_text)
+            for n in names:
+                for feature in walks[n][1].values():
+                    out.write(_gff_line(feature))
+
+    if output_vcf is not None:
+        residues = _fasta_records(ref)
+        with open(output_vcf, "w") as out:
+            out.write(vcf_header(ref, names))
+            for n in names:
+                for line in _vcf_records(n, residues[n], list(walks[n][2].upper()), indexes[n], mincov, inserts[n]):
+                    out.write(line)
+
+    with open(output_consensus, "w") as out:
+        for n in names:
+            out.write(f">{name}_{n} mincov={mincov}\n{walks[n][0]}\n")
     return None, None

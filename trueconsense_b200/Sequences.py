@@ -148,12 +148,20 @@ def _call_table(counts: np.ndarray, L: int, mincov: int, include_ambig: bool):
     return cols
 
 
-def consensus_from_inserts(mincov, counts, GFFdict, IncludeAmbig, inserts, includeINS):
-    """The walk of Sequences.py:175-322 over a count table [8][L] given ListInserts' result."""
+def consensus_from_inserts(mincov, counts, GFFdict, IncludeAmbig, inserts, includeINS, table=None):
+    """The walk of Sequences.py:175-322 over a count table [8][L] given ListInserts' result.  ``table``: the call table of
+    exactly these columns computed with the same mincov and IncludeAmbig (a ``gpu.CallResult``, e.g. one reference's
+    slice of a ``tc_call_contigs`` table); None: ``tc_call`` here."""
     hasinserts, insertpositions = inserts
     counts = np.ascontiguousarray(counts, dtype=np.int32)
     L = counts.shape[1]
-    cov_l, flags, xrun, chars = _call_table(counts, L, mincov, bool(IncludeAmbig is True))
+    if table is None:
+        cov_l, flags, xrun, chars = _call_table(counts, L, mincov, bool(IncludeAmbig is True))
+    else:
+        if table.flags.shape[0] != L:
+            raise ValueError(f"the call table holds {table.flags.shape[0]} columns, the count table {L}")
+        cov_l, flags, xrun, chars = (counts[0].tolist(), table.flags.tolist(), table.xrun.tolist(),
+                                     table.call_char.tobytes().decode("ascii"))
 
     LOWCOV, PRIMX, MDEL, OFFEND, ZEROCOV = gpu.CF_LOWCOV, gpu.CF_PRIMARY_X, gpu.CF_MINORITY_DEL, gpu.CF_XRUN_OFF_END, gpu.CF_ZERO_COV
 

@@ -2,6 +2,7 @@
 validators and exit behaviour, same order of work — on top of the GPU hot path.
 
     python -m trueconsense_b200.TrueConsense -i x.bam -ref ref.fasta -gff f.gff -cov 30 -name S -o cons.fasta
+    python -m trueconsense_b200.TrueConsense --all-contigs -i flu.bam -ref flu.fasta -gff flu.gff -cov 30 -name S -o S.fasta
 
 ``main(args)`` is the console-script entry point of the reference (pyproject.toml:38-40).
 """
@@ -14,10 +15,11 @@ import os
 import pathlib
 import sys
 
-from .Coverage import BuildCoverage
+from .Coverage import BuildCoverage, BuildCoverageContigs
 from .func import MyHelpFormatter, color
-from .indexing import BuildIndex, Gffindex, Override_index_positions, Readbam, read_override_index
-from .Outputs import WriteOutputs
+from .indexing import (BuildIndex, BuildIndexContigs, Gffindex, Override_index_positions, Readbam, gff_by_contig,
+                       read_override_index)
+from .Outputs import WriteOutputs, WriteOutputsContigs
 from .version import __version__
 
 
@@ -81,10 +83,17 @@ def GetArgs(givenargs):
                      help="Override the positional index of certain genome positions with 'known' information if the given "
                           "alignment is not sufficient for these positions\nMust be a compressed csv.\nPlease use with caution "
                           "as this will overwrite the generated index at the given positions!\n")
+    opt.add_argument("--all-contigs", action="store_true",
+                     help="Call every reference of a multi-contig BAM (a segmented genome, a panel of references) in one "
+                          "pass: one FASTA record '{samplename}_{reference}' per reference, the GFF rows matched by seqid, "
+                          "one VCF and one depth file for all references")
     opt.add_argument("--version", "-v", action="version", version=__version__,
                      help="Show the TrueConsense version and exit")
     opt.add_argument("--help", "-h", action="help", default=argparse.SUPPRESS, help="Show this help message and exit")
-    return parser.parse_args(givenargs)
+    opts = parser.parse_args(givenargs)
+    if opts.all_contigs and opts.index_override:
+        parser.error("--index-override cannot be combined with --all-contigs: its positions name no reference")
+    return opts
 
 
 def _index_and_features(opts, bam):
@@ -98,6 +107,23 @@ def _index_and_features(opts, bam):
     return frame, gff
 
 
+def _main_all_contigs(opts, bam):
+    """--all-contigs: every reference of the BAM header through one device pass, the outputs assembled per reference."""
+    with cf.ThreadPoolExecutor(max_workers=opts.threads) as pool:
+        jobs = (pool.submit(BuildIndexContigs, bam, opts.reference), pool.submit(Gffindex, opts.features))
+        frames, gff = (j.result() for j in jobs)
+    indexes = {n: f.to_dict("index") for n, f in frames.items()}
+    gffdicts = {}
+    for n, rows in gff_by_contig(gff.df, list(frames)).items():
+        rows["seqid"] = f"{opts.samplename}_{n}"
+        gffdicts[n] = rows.to_dict("index")
+    if opts.depth_of_coverage is not None:
+        with cf.ThreadPoolExecutor(max_workers=opts.threads) as pool:
+            pool.submit(BuildCoverageContigs, indexes, opts.depth_of_coverage)
+    WriteOutputsContigs(opts.coverage_level, indexes, gffdicts, bam, opts.noambiguity is False, opts.variants, opts.samplename,
+                        opts.reference, opts.output_gff, gff.header, opts.output)
+
+
 def main(args: list[str] | None = None):
     """The reference's command line (TrueConsense.py:212-264): same flags, same files."""
     argv = args or sys.argv[1:]
@@ -107,6 +133,8 @@ def main(args: list[str] | None = None):
         sys.exit(1)
     opts = GetArgs(argv)
     bam = Readbam(opts.input)        # one decoded copy of the BAM serves the index and the insertion columns
+    if opts.all_contigs:
+        return _main_all_contigs(opts, bam)
     frame, gff = _index_and_features(opts, bam)
     index = frame.to_dict("index")
     features = gff.df

@@ -14,6 +14,8 @@
 // keep ptxas from contracting anything (the file is also built with --fmad=false).  Integer
 // cross-multiplication gives different answers at the thresholds (SURVEY.md §4.3: 55/45 at
 // coverage 100 is not ambiguous, 6/5 at coverage 10 is).
+#include <stdlib.h>
+
 #include "tc_common.cuh"
 
 __device__ __forceinline__ double pct(int c, int cov) { return __dmul_rn(__ddiv_rn((double)c, (double)cov), 100.0); }
@@ -116,6 +118,9 @@ __global__ void __launch_bounds__(256) call_kernel(call_args a) {
 // nn is a reverse min-scan.  xrun_local_kernel scans inside blocks of XR_BLOCK positions (coalesced, warp
 // shuffles) and leaves every block's first non-X position; xrun_apply_kernel looks up the blocks to the
 // right for runs that leave their block.  Both are ordinary multi-CTA kernels: no serial pass over L.
+// Several references side by side (tc_call_contigs): a run stops at the end of its own reference, so xrun_apply_kernel
+// clamps nn to that end — the first non-X position at or after k, if it lies beyond the end, means every position from
+// k to the end is X.  The local scan needs no boundaries.
 constexpr int XR_BLOCK = 256;
 
 __global__ void __launch_bounds__(XR_BLOCK) xrun_local_kernel(const uint8_t* __restrict__ flags, int32_t* __restrict__ nn_local,
@@ -137,8 +142,20 @@ __global__ void __launch_bounds__(XR_BLOCK) xrun_local_kernel(const uint8_t* __r
     if (threadIdx.x == 0) block_first[blockIdx.x] = v;
 }
 
+// the end (exclusive) of the reference holding position j: contig_start[n] = L, references may be empty
+__device__ __forceinline__ int contig_end(const int32_t* __restrict__ contig_start, int n, int j) {
+    int lo = 0, hi = n - 1;                     // the last reference k with contig_start[k] <= j
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (__ldg(contig_start + mid) <= j) lo = mid; else hi = mid - 1;
+    }
+    return __ldg(contig_start + lo + 1);
+}
+
+// contig_start: NULL (one reference) or the n_contigs + 1 boundaries of the references
 __global__ void __launch_bounds__(XR_BLOCK) xrun_apply_kernel(uint8_t* __restrict__ flags, const int32_t* __restrict__ nn_local,
-                                                              const int32_t* __restrict__ block_first, int32_t* __restrict__ xrun, int L, int n_blocks) {
+                                                              const int32_t* __restrict__ block_first, int32_t* __restrict__ xrun, int L, int n_blocks,
+                                                              const int32_t* __restrict__ contig_start, int n_contigs) {
     __shared__ int right_s;
     const int INF = 0x7fffffff;
     const int lane = threadIdx.x & 31;
@@ -166,8 +183,10 @@ __global__ void __launch_bounds__(XR_BLOCK) xrun_apply_kernel(uint8_t* __restric
             for (int b2 = blockIdx.x + 2; b2 < n_blocks; ++b2) { const int w = block_first[b2]; if (w != INF) { nn = w; break; } }
         }
     }
+    const int end = contig_start ? contig_end(contig_start, n_contigs, j) : L;
+    nn = min(nn, end);
     xrun[j] = nn - k;
-    if (nn == L) flags[j] |= TC_CF_XRUN_OFF_END;
+    if (nn == end) flags[j] |= TC_CF_XRUN_OFF_END;
 }
 
 __global__ void is_ambiguous_kernel(const uint8_t* __restrict__ letters, const int32_t* __restrict__ cnts,
@@ -201,13 +220,9 @@ __global__ void rank_sort_kernel(const int32_t* __restrict__ in, const int32_t* 
 }
 
 // ---------------------------------------------------------------- C-ABI
-TC_API int tc_call(tc_ctx_t* ctx, const int32_t* counts, int32_t ref_len, const tc_call_params_t* p,
-                   const tc_call_table_t* t, void* stream) {
-    if (!ctx) return TC_ERR_ARG;
-    if (!counts || !p || !t) return tc_fail(ctx, TC_ERR_ARG, "NULL argument");
-    if (ref_len <= 0) return tc_fail(ctx, TC_ERR_ARG, "ref_len must be positive");
-    cudaStream_t s = (cudaStream_t)stream;
-    TC_CUDA(cudaSetDevice(ctx->device));
+// tc_call and tc_call_contigs: d_contig_start is NULL (one reference) or the n_contigs + 1 boundaries in device memory
+static int call_table(tc_ctx_t* ctx, const int32_t* counts, int32_t ref_len, const int32_t* d_contig_start, int32_t n_contigs,
+                      const tc_call_params_t* p, const tc_call_table_t* t, cudaStream_t s) {
     const size_t L = (size_t)ref_len;
     int rc;
     call_args a;
@@ -236,7 +251,7 @@ TC_API int tc_call(tc_ctx_t* ctx, const int32_t* counts, int32_t ref_len, const 
         int32_t* block_first = nn_local + L;
         xrun_local_kernel<<<n_blocks, XR_BLOCK, 0, s>>>(a.flags, nn_local, block_first, ref_len);
         TC_LAUNCH_CHECK();
-        xrun_apply_kernel<<<n_blocks, XR_BLOCK, 0, s>>>(a.flags, nn_local, block_first, a.xrun, ref_len, n_blocks);
+        xrun_apply_kernel<<<n_blocks, XR_BLOCK, 0, s>>>(a.flags, nn_local, block_first, a.xrun, ref_len, n_blocks, d_contig_start, n_contigs);
         TC_LAUNCH_CHECK();
     }
     bool any_host = false;
@@ -248,6 +263,46 @@ TC_API int tc_call(tc_ctx_t* ctx, const int32_t* counts, int32_t ref_len, const 
     }
     if (any_host) TC_CUDA(cudaStreamSynchronize(s));
     return TC_OK;
+}
+
+TC_API int tc_call(tc_ctx_t* ctx, const int32_t* counts, int32_t ref_len, const tc_call_params_t* p,
+                   const tc_call_table_t* t, void* stream) {
+    if (!ctx) return TC_ERR_ARG;
+    if (!counts || !p || !t) return tc_fail(ctx, TC_ERR_ARG, "NULL argument");
+    if (ref_len <= 0) return tc_fail(ctx, TC_ERR_ARG, "ref_len must be positive");
+    TC_CUDA(cudaSetDevice(ctx->device));
+    return call_table(ctx, counts, ref_len, nullptr, 0, p, t, (cudaStream_t)stream);
+}
+
+TC_API int tc_call_contigs(tc_ctx_t* ctx, const int32_t* counts, int32_t total_len, int32_t n, const int32_t* contig_start,
+                           const tc_call_params_t* p, const tc_call_table_t* t, void* stream) {
+    if (!ctx) return TC_ERR_ARG;
+    if (!counts || !p || !t || !contig_start) return tc_fail(ctx, TC_ERR_ARG, "NULL argument");
+    if (total_len <= 0 || n <= 0) return tc_fail(ctx, TC_ERR_ARG, "total_len and the number of references must be positive");
+    cudaStream_t s = (cudaStream_t)stream;
+    TC_CUDA(cudaSetDevice(ctx->device));
+    // the boundaries are checked on the host (a device array is read back: n + 1 integers) and kept on the device
+    const size_t bytes = 4 * ((size_t)n + 1);
+    const bool on_dev = tc_is_device_ptr(contig_start);
+    const int32_t* h = contig_start;
+    int32_t* tmp = nullptr;
+    if (on_dev) {
+        tmp = (int32_t*)malloc(bytes);
+        if (!tmp) return tc_fail(ctx, TC_ERR_NOMEM, "host memory for %d boundaries", n + 1);
+        cudaError_t e = cudaMemcpyAsync(tmp, contig_start, bytes, cudaMemcpyDeviceToHost, s);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+        if (e != cudaSuccess) { free(tmp); return tc_cuda_fail(ctx, e, "reading contig_start"); }
+        ctx->d2h_bytes += (int64_t)bytes;
+        h = tmp;
+    }
+    int bad = h[0] != 0 || h[n] != total_len;
+    for (int32_t k = 0; k < n && !bad; ++k) bad = h[k + 1] < h[k];
+    free(tmp);
+    if (bad) return tc_fail(ctx, TC_ERR_ARG, "contig_start must rise from 0 to total_len (%d) in %d steps", total_len, n);
+    int rc;
+    const int32_t* d_cs = (const int32_t*)tc_stage_in(ctx, SLOT_CONTIG_A, contig_start, bytes, s, &rc);
+    if (rc) return rc;
+    return call_table(ctx, counts, total_len, d_cs, n, p, t, s);
 }
 
 TC_API int tc_is_ambiguous(tc_ctx_t* ctx, const uint8_t* letters, const int32_t* cnts, const int32_t* cov, int64_t n,

@@ -130,6 +130,10 @@ def lib() -> C.CDLL:
                                             C.POINTER(PileupParams), vp, C.POINTER(CallTable), vp, C.POINTER(i32)]
             l.tc_sample_finish.argtypes = [vp, i32, C.POINTER(InsertCall), i32, C.POINTER(i32), vp, i64]
             l.tc_sample_enqueue.restype = l.tc_sample_finish.restype = C.c_int
+            l.tc_bam_contig_ranges.argtypes = [vp, vp, i64, vp, i64, i32, vp, vp]
+            l.tc_reads_to_contig_coords.argtypes = [vp, C.POINTER(TcReads), i32, vp, vp, vp, vp]
+            l.tc_call_contigs.argtypes = [vp, vp, i32, i32, vp, C.POINTER(CallParams), C.POINTER(CallTable), vp]
+            l.tc_bam_contig_ranges.restype = l.tc_reads_to_contig_coords.restype = l.tc_call_contigs.restype = C.c_int
             for name in ("tc_ctx_create", "tc_ctx_destroy", "tc_reads_upload", "tc_pileup_counts", "tc_depth", "tc_call",
                          "tc_is_ambiguous", "tc_extract_inserts", "tc_list_insert_candidates", "tc_allreduce_counts", "tc_pileup_call_inserts"):
                 getattr(l, name).restype = C.c_int
@@ -163,6 +167,24 @@ class CallResult:
     rank_count: np.ndarray
     ambig_char: np.ndarray
 
+    def slice(self, a: int, b: int) -> "CallResult":
+        """Columns [a, b) of the table (views): one reference's part of a multi-reference table."""
+        return CallResult(self.call_char[a:b], self.flags[a:b], self.xrun[a:b], self.rank_letter[:, a:b], self.rank_count[:, a:b],
+                          self.ambig_char[a:b])
+
+
+def _call_buffers(counts, L: int):
+    """Host outputs of a call table of L columns, the CallTable pointing at them, and ``counts`` checked (numpy: [8][L])."""
+    res = CallResult(np.empty(L, np.uint8), np.empty(L, np.uint8), np.empty(L, np.int32), np.empty((4, L), np.uint8),
+                     np.empty((4, L), np.int32), np.empty(L, np.uint8))
+    t = CallTable(_ptr(res.call_char), _ptr(res.flags), _ptr(res.xrun), _ptr(res.rank_letter), _ptr(res.rank_count),
+                  _ptr(res.ambig_char))
+    if isinstance(counts, np.ndarray):
+        counts = np.ascontiguousarray(counts, dtype=np.int32)
+        if counts.shape != (TC_NROWS, L):
+            raise ValueError(f"counts must be [{TC_NROWS}][{L}]")
+    return res, t, counts
+
 
 class DeviceReads:
     """A read batch resident in context-owned device memory (see tc_reads_upload)."""
@@ -174,6 +196,8 @@ class DeviceReads:
         self.ctx = ctx
         self.generation = generation
         self.stats = None
+        self.first_read = None      # [n_ref + 1]: where each reference's reads begin (bam_file_to_device(contig_ranges=True))
+        self.contig_start = None    # set once the reads sit in the global columns of a multi-reference pass
 
     def with_host_qual(self) -> "DeviceReads":
         """The same device arrays plus the batch's HOST quality and mate arrays (QNAME hash, PNEXT, TLEN):
@@ -266,7 +290,12 @@ class Context:
         self._check(self._lib.tc_download(self._h, _ptr(out), dev_ptr, out.nbytes, stream))
         return out
 
-    def bam_to_device(self, payload, stream: int = 0) -> DeviceReads:
+    def _contig_ranges(self, payload_ptr, n_bytes: int, rec_ptr, n_reads: int, n_ref: int, stream: int) -> np.ndarray:
+        first = np.zeros(n_ref + 1, np.int32)
+        self._check(self._lib.tc_bam_contig_ranges(self._h, payload_ptr, n_bytes, rec_ptr, n_reads, n_ref, _ptr(first), stream))
+        return first
+
+    def bam_to_device(self, payload, stream: int = 0, contig_ranges: bool = False) -> DeviceReads:
         """GPU-side record parsing (tc_bam_records_to_reads): a ``bamio.BamPayload`` (the BAM inflated on the host, its records
         indexed) becomes the flat read arrays in the context's device buffers — the CPU never touches a record's body.
         ``.stats`` of the result: aligned bases, longest span, sortedness, whether more than one reference occurs."""
@@ -277,14 +306,19 @@ class Context:
                                                       payload.n_reads, C.byref(dev), C.byref(st), stream))
         d = DeviceReads(dev, None, self, self._generation)
         d.stats = st
+        if contig_ranges and payload.ref_names and not st.unsorted:
+            d.first_read = self._contig_ranges(payload.payload_ptr, payload.n_bytes, payload.rec_off_ptr, payload.n_reads,
+                                               len(payload.ref_names), stream)
         return d
 
-    def bam_file_to_device(self, path: str, stream: int = 0) -> DeviceReads:
+    def bam_file_to_device(self, path: str, stream: int = 0, contig_ranges: bool = False) -> DeviceReads:
         """A BAM file to the flat read arrays in device memory with the GPU doing all of it: the host maps the file and walks
         the BGZF member headers (``bamio.map_bgzf``); the device inflates every member and checks its CRC-32
         (``tc_bgzf_inflate``), finds and proves the record offsets (``tc_bam_index_records``) and parses the records
         (``tc_bam_records_to_reads``).  The result carries ``.ref_names``, ``.ref_lens``, ``.stats`` and ``.info``
-        (records, unplaced records dropped, timings).  ``TcError`` / ``OSError`` for a file that does not decode."""
+        (records, unplaced records dropped, timings).  ``TcError`` / ``OSError`` for a file that does not decode.
+        ``contig_ranges``: also ``.first_read``, where each reference's reads begin (``tc_bam_contig_ranges``, taken while the
+        payload and the record offsets are still in the context's buffers); left None for an unsorted file."""
         import time
 
         from . import bamio
@@ -321,10 +355,40 @@ class Context:
         d = DeviceReads(dev, None, self, self._generation)
         d.stats = st
         d.ref_names, d.ref_lens = names, lens
+        if contig_ranges and lens and not st.unsorted:
+            d.first_read = self._contig_ranges(payload, n_bytes, rec, n_placed.value, len(lens), stream)
         info.update(n_records=int(n_records.value), n_dropped_unplaced=int(n_records.value - n_placed.value), t_map_s=t1 - t0,
                     t_inflate_s=t2 - t1, t_index_s=t3 - t2, t_parse_s=t4 - t3)
         d.info = info
         return d
+
+    def reads_to_contig_coords(self, reads: DeviceReads, ref_lens, first_read, names=None, stream: int = 0) -> np.ndarray:
+        """Move device-resident reads to the global columns of a multi-reference pass, in place (``tc_reads_to_contig_coords``):
+        reference k's reads (``first_read[k]`` .. ``first_read[k+1]-1``) shift by the sum of the lengths before it.  Returns
+        those boundaries (int32[n_ref + 1]).  A batch moves once: a second call on it raises.  A read outside its reference
+        is ``TcError`` (TC_ERR_RANGE) naming the reference (``names``); the batch is unusable afterwards."""
+        if not isinstance(reads, DeviceReads) or reads.ctx is not self:
+            raise TypeError("reads_to_contig_coords moves the device reads of this context (upload / bam_file_to_device)")
+        if reads.contig_start is not None:
+            raise RuntimeError("these device reads sit in contig coordinates already")
+        rs = self._reads_struct(reads)
+        lens = np.ascontiguousarray(ref_lens, dtype=np.int32) if not hasattr(ref_lens, "data_ptr") else ref_lens
+        first = np.ascontiguousarray(first_read, dtype=np.int32) if not hasattr(first_read, "data_ptr") else first_read
+        n_ref = int(lens.shape[0])
+        start = np.zeros(n_ref + 1, np.int32)
+        rc = self._lib.tc_reads_to_contig_coords(self._h, C.byref(rs), n_ref, _ptr(lens), _ptr(first), _ptr(start), stream)
+        if rc != 0:
+            msg = self._lib.tc_last_error(self._h).decode()
+            if rc == -7:
+                reads.generation = -1           # partly moved: stale from now on
+                import re
+
+                m = re.search(r"reference (\d+)", msg)
+                if m and names is not None and int(m.group(1)) < len(names):
+                    msg = msg.replace(m.group(0), f"{m.group(0)} ({names[int(m.group(1))]!r})", 1)
+            raise TcError(rc, msg)
+        reads.contig_start = start
+        return start
 
     # ------------------------------------------------------------------ (1) pileup
     def pileup_counts(self, reads, ref_len: int, params: PileupParams | None = None, out=None, stream: int = 0):
@@ -378,15 +442,8 @@ class Context:
     def call(self, counts, ref_len: int, mincov: int, include_ambig: bool, stream: int = 0, maxdist: float = 10.0,
              minority_del_pct: float = 15.0, insert_pct: float = 55.0) -> CallResult:
         L = int(ref_len)
-        res = CallResult(np.empty(L, np.uint8), np.empty(L, np.uint8), np.empty(L, np.int32), np.empty((4, L), np.uint8),
-                         np.empty((4, L), np.int32), np.empty(L, np.uint8))
-        t = CallTable(_ptr(res.call_char), _ptr(res.flags), _ptr(res.xrun), _ptr(res.rank_letter), _ptr(res.rank_count),
-                      _ptr(res.ambig_char))
+        res, t, counts = _call_buffers(counts, L)
         p = CallParams(int(mincov), int(bool(include_ambig)), maxdist, minority_del_pct, insert_pct)
-        if isinstance(counts, np.ndarray):
-            counts = np.ascontiguousarray(counts, dtype=np.int32)
-            if counts.shape != (TC_NROWS, L):
-                raise ValueError(f"counts must be [{TC_NROWS}][{L}]")
         self._check(self._lib.tc_call(self._h, _ptr(counts), L, C.byref(p), C.byref(t), stream))
         return res
 
@@ -395,6 +452,17 @@ class Context:
         """tc_call with caller-provided (device) output pointers; asynchronous."""
         p = CallParams(int(mincov), int(bool(include_ambig)), maxdist, minority_del_pct, insert_pct)
         self._check(self._lib.tc_call(self._h, _ptr(counts), int(ref_len), C.byref(p), C.byref(table), stream))
+
+    def call_contigs(self, counts, contig_start, mincov: int, include_ambig: bool, stream: int = 0, maxdist: float = 10.0,
+                     minority_del_pct: float = 15.0, insert_pct: float = 55.0) -> CallResult:
+        """``tc_call_contigs``: the call table of a multi-reference count table [8][total] whose references start at
+        ``contig_start`` (n + 1 boundaries): X-runs stop at their reference's end."""
+        cs = np.ascontiguousarray(contig_start, dtype=np.int32)
+        n, L = int(cs.shape[0]) - 1, int(cs[-1])
+        res, t, counts = _call_buffers(counts, L)
+        p = CallParams(int(mincov), int(bool(include_ambig)), maxdist, minority_del_pct, insert_pct)
+        self._check(self._lib.tc_call_contigs(self._h, _ptr(counts), L, n, _ptr(cs), C.byref(p), C.byref(t), stream))
+        return res
 
     def is_ambiguous(self, letters: np.ndarray, cnts: np.ndarray, cov: np.ndarray, maxdist: float = 10.0, stream: int = 0) -> np.ndarray:
         letters = np.ascontiguousarray(letters, dtype=np.uint8)

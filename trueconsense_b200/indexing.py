@@ -9,6 +9,7 @@ BAM is inflated on the host (csrc/host/bamio.c), its records are parsed on the G
 from __future__ import annotations
 
 import threading
+from dataclasses import dataclass
 
 import numpy as np
 import pandas as pd
@@ -31,6 +32,7 @@ class BamHandle:
         self._payload = None
         self._hdr = None
         self._dev = None
+        self._dev_contigs = None        # (key, DeviceReads, ContigLayout): the reads moved to a multi-reference layout
         self._lock = threading.Lock()
         self._insert_cache: dict = {}
 
@@ -107,12 +109,105 @@ class BamHandle:
                 self._dev = d
             return d.with_host_qual() if with_host_qual else d
 
+    def device_reads_contigs(self, names, lens):
+        """The reads in device memory moved to the global columns of a multi-reference pass, and that layout
+        (``ContigLayout``): every reference of the header (``names``, in header order) side by side with the lengths
+        ``lens`` (from the FASTA).  Kept apart from :meth:`device_reads` — the two share the context's buffers, so making one
+        makes the other stale, and each is made again when asked for."""
+        ctx = gpu.default_context()
+        key = (tuple(names), tuple(int(x) for x in lens))
+        with self._lock:
+            c = self._dev_contigs
+            if c is not None and c[0] == key and c[1].ctx is ctx and c[1].generation == ctx._generation:
+                return c[1], c[2]
+            self._dev_contigs = None
+            if self._reads is not None:
+                b = self._reads
+                if not b.sorted:
+                    raise ValueError("Unsorted input. Pileup aborts")
+                first_read = contig_ranges_from_tid(b.tid, len(names), b.n_reads)
+                d = ctx.upload(b)       # QUAL and mate fields too: the move shifts PNEXT on the device
+            else:
+                try:
+                    d = ctx.bam_file_to_device(self.filename, contig_ranges=True)
+                    self._hdr = (d.ref_names, d.ref_lens)
+                except gpu.TcError:
+                    self._payload = bamio.read_bam_payload(self.filename)
+                    d = ctx.bam_to_device(self._payload, contig_ranges=True)
+                    self._payload.release()
+                if d.stats.unsorted:
+                    raise ValueError("Unsorted input. Pileup aborts")
+                first_read = d.first_read
+            if len(first_read) != len(names) + 1:
+                raise ValueError(f"the BAM header holds {len(first_read) - 1} references, {len(names)} were given")
+            start = ctx.reads_to_contig_coords(d, key[1], first_read, names)
+            layout = ContigLayout(list(names), list(key[1]), start.astype(np.int64), np.asarray(first_read, np.int64))
+            self._dev_contigs = (key, d, layout)
+            return d, layout
+
     def pileup(self, *args, **kwargs):
         raise NotImplementedError("column iteration is not part of this implementation; "
                                   "use Events.ExtractInserts / indexing.BuildIndex")
 
     def close(self):
         pass
+
+
+@dataclass
+class ContigLayout:
+    """Every reference of a BAM side by side: reference k (``names[k]``, ``lens[k]`` columns) occupies the global columns
+    ``start[k]`` .. ``start[k+1]-1``; its reads are ``first_read[k]`` .. ``first_read[k+1]-1``."""
+
+    names: list
+    lens: list
+    start: np.ndarray
+    first_read: np.ndarray
+
+    @property
+    def total(self) -> int:
+        return int(self.start[-1])
+
+    def locate(self, positions) -> tuple[np.ndarray, np.ndarray]:
+        """1-based global positions -> (reference index, 1-based position on that reference)."""
+        p = np.asarray(positions, dtype=np.int64)
+        k = np.searchsorted(self.start, p - 1, side="right") - 1
+        return k, p - self.start[k]
+
+
+def contig_ranges_from_tid(tid, n_ref: int, n_reads: int) -> np.ndarray:
+    """``first_read[n_ref + 1]`` of a host-decoded batch (``ReadBatch.tid``, sorted): what ``tc_bam_contig_ranges`` computes
+    on the device from the records."""
+    t = np.zeros(n_reads, np.int32) if tid is None else np.asarray(tid)
+    if t.size and (int(t.min()) < 0 or int(t.max()) >= n_ref):
+        raise ValueError(f"a read's reference index lies outside the header's {n_ref} references")
+    if t.size and np.any(np.diff(t.astype(np.int64)) < 0):
+        raise ValueError("Unsorted input. Pileup aborts")
+    return np.searchsorted(t, np.arange(n_ref + 1), side="left").astype(np.int32)
+
+
+def fasta_lengths_by_name(names, ref) -> list[int]:
+    """The lengths of the FASTA records named like the BAM's references (the first record of a name counts), in the
+    order of ``names``.  A reference without a record is a ValueError that names it."""
+    fnames, flens = bamio.read_fasta_lengths(ref)
+    by_name: dict[str, int] = {}
+    for n, l in zip(fnames, flens):
+        by_name.setdefault(n, int(l))
+    missing = [n for n in names if n not in by_name]
+    if missing:
+        raise ValueError(f"reference {missing[0]!r} of the BAM header has no record in {ref}"
+                         + (f" (nor have {len(missing) - 1} more)" if len(missing) > 1 else ""))
+    return [by_name[n] for n in names]
+
+
+def gff_by_contig(df: pd.DataFrame, names) -> dict:
+    """The GFF rows of every reference (by ``seqid``), in the order of ``names``, each frame indexed 0.. like a GFF file
+    holding only that reference's rows.  A row whose seqid names no reference is a ValueError: dropping it would lose
+    that feature's ORF corrections."""
+    known = set(names)
+    unknown = sorted(set(df["seqid"]) - known)
+    if unknown:
+        raise ValueError(f"GFF rows with seqid {unknown[0]!r} name no reference of the BAM ({len(names)} references)")
+    return {n: df[df["seqid"] == n].reset_index(drop=True) for n in names}
 
 
 def Readbam(f):
@@ -189,3 +284,16 @@ def BuildIndex(bamfile, ref):
     ref_length = int(lens[0])
     counts = gpu.default_context().pileup_counts(handle.device_reads(), ref_length)
     return frame_from_counts(counts)
+
+
+def BuildIndexContigs(bamfile, ref):
+    """``BuildIndex`` for every reference of the BAM header in one device pass: ``{reference: frame}`` in header order, each
+    frame equal to ``BuildIndex`` over a BAM holding only that reference's records and the FASTA record of its name."""
+    handle = bamfile if isinstance(bamfile, BamHandle) else BamHandle(bamfile)
+    names = list(handle.references)
+    if not names:
+        raise ValueError(f"{handle.filename}: the BAM header lists no reference")
+    lens = fasta_lengths_by_name(names, ref)
+    d, lay = handle.device_reads_contigs(names, lens)
+    counts = gpu.default_context().pileup_counts(d, lay.total)
+    return {n: frame_from_counts(counts[:, lay.start[k]:lay.start[k + 1]]) for k, n in enumerate(names)}
