@@ -56,7 +56,7 @@ struct tc_rr_slot {
     cudaEvent_t done;
     tc_reads_t reads; int32_t ref_len; tc_pileup_params_t p; int32_t* counts; void* comm; void* stream;
     tc_pileup_pending pend;         // of the run that was enqueued eagerly or captured: a replay is that run again
-    cudaGraphExec_t exec; unsigned char key[256]; int key_len, seen; int64_t g_launches, g_d2h;
+    tc_graph_cache graph;
 };
 
 static int rr_slots(tc_ctx* ctx) {
@@ -77,7 +77,7 @@ void tc_rr_slots_free(tc_ctx* ctx) {
     for (int i = 0; i < 2; ++i) {
         if (ctx->rr[i].host) cudaFreeHost(ctx->rr[i].host);
         if (ctx->rr[i].done) cudaEventDestroy(ctx->rr[i].done);
-        if (ctx->rr[i].exec) cudaGraphExecDestroy(ctx->rr[i].exec);
+        tc_graph_destroy(ctx->rr[i].graph);
     }
     free(ctx->rr);
     ctx->rr = nullptr;
@@ -124,43 +124,8 @@ TC_API int tc_pileup_counts_allreduce_enqueue(tc_ctx_t* ctx, const tc_reads_t* r
     put(reads, sizeof(*reads)); put(&ref_len, 4); put(p, sizeof(*p)); put(&counts, sizeof(counts)); put(&comm, sizeof(comm));
     put(&ctx->buf_epoch, 8); put(&ctx->timing, 4);
     static_assert(sizeof(tc_reads_t) + 4 + sizeof(tc_pileup_params_t) + 16 + 12 <= 256, "shard key");
-    const bool same = sl.key_len == kn && memcmp(sl.key, key, (size_t)kn) == 0;
-    if (!same) {
-        if (sl.exec) { cudaGraphExecDestroy(sl.exec); sl.exec = nullptr; }
-        memcpy(sl.key, key, (size_t)kn); sl.key_len = kn; sl.seen = 0;
-    }
-    if (same && sl.exec) {
-        TC_CUDA(cudaGraphLaunch(sl.exec, s));
-        ctx->launches += sl.g_launches; ctx->d2h_bytes += sl.g_d2h;
-    } else if (same && sl.seen >= 1 && tc_reads_all_device(reads) && !getenv("TC_NO_GRAPH")) {
-        if (!ctx->cap_stream) TC_CUDA(cudaStreamCreateWithFlags(&ctx->cap_stream, cudaStreamNonBlocking));
-        const int64_t l0 = ctx->launches, d0 = ctx->d2h_bytes, epoch0 = ctx->buf_epoch;
-        TC_CUDA(cudaStreamBeginCapture(ctx->cap_stream, cudaStreamCaptureModeRelaxed));
-        ctx->in_capture = 1;
-        rc = rr_chain(ctx, sl, ctx->cap_stream);
-        ctx->in_capture = 0;
-        cudaGraph_t graph = nullptr;
-        const cudaError_t ce = cudaStreamEndCapture(ctx->cap_stream, &graph);
-        if (rc == TC_OK && ce == cudaSuccess && graph && ctx->buf_epoch == epoch0) {
-            const cudaError_t ie = cudaGraphInstantiate(&sl.exec, graph, 0);
-            cudaGraphDestroy(graph);
-            if (ie != cudaSuccess) { sl.exec = nullptr; return tc_cuda_fail(ctx, ie, "cudaGraphInstantiate"); }
-            sl.g_launches = ctx->launches - l0; sl.g_d2h = ctx->d2h_bytes - d0;
-            TC_CUDA(cudaGraphLaunch(sl.exec, s));
-        } else {
-            if (graph) cudaGraphDestroy(graph);
-            cudaGetLastError();
-            ctx->launches = l0; ctx->d2h_bytes = d0;
-            if (rc && rc != TC_ERR_CUDA) return rc;
-            sl.key_len = 0;
-            rc = rr_chain(ctx, sl, s);
-            if (rc) return rc;
-        }
-    } else {
-        rc = rr_chain(ctx, sl, s);
-        if (rc) return rc;
-        sl.seen++;
-    }
+    rc = tc_graph_run(ctx, sl.graph, key, kn, tc_reads_all_device(reads), [&](cudaStream_t cs) { return rr_chain(ctx, sl, cs); }, s);
+    if (rc) return rc;
     TC_CUDA(cudaEventRecord(sl.done, s));
     sl.state = 1;
     ctx->rr_next = slot ^ 1;
@@ -182,7 +147,7 @@ TC_API int tc_pileup_counts_allreduce_finish(tc_ctx_t* ctx, int32_t ticket) {
     if (h.any_err != 0) {
         // some rank's shard did not go through: every rank takes the separate calls (which handle the kernel variants) and
         // makes the same collective call whatever its own outcome, so nobody waits for a rank that failed
-        sl.key_len = 0;
+        sl.graph.key_len = 0;
         const int prc = tc_pileup_counts(ctx, &sl.reads, L, &sl.p, sl.counts, sl.stream);
         if (prc) TC_CUDA(cudaMemsetAsync(sl.counts, 0, sizeof(int32_t) * TC_NROWS * (size_t)L, s));
         char keep[sizeof(ctx->err)];

@@ -32,6 +32,9 @@
 //            admitted entries are counted.
 #include <cub/device/device_segmented_radix_sort.cuh>
 
+#include <memory>
+#include <new>
+
 #include "tc_common.cuh"
 
 constexpr int INS_TILE = 256;               // reads per tile == threads per CTA of the select / admit kernels
@@ -166,9 +169,9 @@ __global__ void __launch_bounds__(256) ins_layout_kernel(ins_args a, int64_t* __
     const int n_cand = ins_ncand(a);
     // device-side candidates: their number and positions, and the pileup's status block, travel back with the results
     if (rb_extra) {
-        if (threadIdx.x == 0) rb_extra[0] = *a.n_cand_dev;
-        if (threadIdx.x < 16) rb_extra[16 + threadIdx.x] = pileup_status ? reinterpret_cast<const int32_t*>(pileup_status)[threadIdx.x] : 0;
-        for (int i = threadIdx.x; i < n_cand; i += blockDim.x) rb_extra[32 + i] = a.cand[i];
+        if (threadIdx.x == 0) rb_extra[TC_RB_EXTRA_NCAND] = *a.n_cand_dev;
+        if (threadIdx.x < 16) rb_extra[TC_RB_EXTRA_STATUS + threadIdx.x] = pileup_status ? reinterpret_cast<const int32_t*>(pileup_status)[threadIdx.x] : 0;
+        for (int i = threadIdx.x; i < n_cand; i += blockDim.x) rb_extra[TC_RB_EXTRA_CAND + i] = a.cand[i];
     }
     if (threadIdx.x == 0) {
         int64_t off = 0; int64_t tiles = 0;
@@ -727,16 +730,143 @@ __global__ void ins_bases_kernel(ins_args a, const tc_insert_call_t* __restrict_
     for (int j = threadIdx.x; j < c.indel; j += blockDim.x) bases[c.bases_off + j] = (uint8_t)ins_char(a, r, a.ent_qpos[e], j + 1, rev);
 }
 
-static int launch_pair(tc_ctx* ctx, const ins_args& a, int grid, cudaStream_t s) {
-    const size_t smem = (size_t)PAIR_TBL * 10;
-    if (!(ctx->ins_attr_set & 2)) {
-        TC_CUDA(cudaFuncSetAttribute(ins_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        ctx->ins_attr_set |= 2;
-    }
-    ins_pair_kernel<<<grid, 1024, smem, s>>>(a);
+// ---------------------------------------------------------------- host side, shared by both drivers
+// The results block: status, device-built layout, overflow flags, pair-scratch bump; with_extra (the chained form) the
+// candidate count, the pileup's status and the candidates; then seg_count / pair_any, the calls and their inserted
+// characters.  n_cand: the candidates, or the capacity the chained form enqueues for.
+static ins_block ins_block_of(int n_cand, bool with_extra) {
+    static_assert(sizeof(tc_status) <= 64, "tc_status outgrew its place in the results block");
+    ins_block b;
+    b.layout = 64; b.over = 80; b.bump = 88;
+    b.extra = with_extra ? 128 : 0;
+    b.seg = with_extra ? b.extra + 4 * (TC_RB_EXTRA_CAND + (size_t)n_cand) : 96;
+    b.calls = b.seg + ((4 * (2 * (size_t)n_cand + 2) + 15) & ~(size_t)15);
+    b.fixed = b.calls + sizeof(tc_insert_call_t) * (size_t)n_cand;
+    b.bytes = b.fixed + (size_t)n_cand * INS_BASES_FIXED;
+    return b;
+}
+
+// One slab (SLOT_INS_D) for T entry slots and NT tiles: keys, indel, qpos, head, sel, quality per slot; tile tables;
+// per-candidate offsets.  The pair scratch, the per-candidate words of the results block and p's filter fields.
+static int ins_bind(tc_ctx* ctx, ins_args& a, uint8_t* d_rb, const ins_block& rb, size_t T, size_t NT, int n_cand, const tc_pileup_params_t* p) {
+    const size_t bytes = T * (8 + 4 + 4 + 1 + 1 + 1) + NT * 12 + ((size_t)n_cand + 1) * 16 + 256 + 16;
+    uint8_t* slab = (uint8_t*)tc_dev_buf(ctx, SLOT_INS_D, bytes);
+    if (!slab) return TC_ERR_NOMEM;
+    a.ent_key = (uint64_t*)slab;
+    int64_t* d_off = (int64_t*)(a.ent_key + T);
+    a.seg_off = d_off;
+    a.ent_indel = (int32_t*)(d_off + n_cand + 1); a.ent_qpos = a.ent_indel + T;
+    int32_t* d_tcand = a.ent_qpos + T; int32_t* d_tfirst = d_tcand + NT;
+    a.tile_cand = d_tcand; a.tile_first = d_tfirst;
+    a.tile_sel = d_tfirst + n_cand + 1; a.tile_last = a.tile_sel + NT;
+    a.ent_head = (uint8_t*)(a.tile_last + NT); a.ent_sel = a.ent_head + T; a.ent_q = a.ent_sel + T;
+    a.seg_count = (int32_t*)(d_rb + rb.seg); a.pair_any = a.seg_count + n_cand + 1; a.overflow = (int32_t*)(d_rb + rb.over);
+    a.bases_fixed = d_rb + rb.fixed;
+    if (ctx->pair_cap <= 0) ctx->pair_cap = 1 << 22;
+    a.pair_bump = (unsigned long long*)(d_rb + rb.bump); a.pair_cap = (unsigned long long)ctx->pair_cap;
+    a.pair_q = (uint8_t*)tc_dev_buf(ctx, SLOT_INS_F, (size_t)ctx->pair_cap);
+    if (!a.pair_q) return TC_ERR_NOMEM;
+    a.flag_filter = p->flag_filter; a.min_mapq = p->min_mapq; a.min_bq = p->min_base_quality; a.ignore_orphans = p->ignore_orphans;
+    a.olap_mode = (p->reserved >> 8) & 3;
+    a.max_depth = p->max_depth > 0 ? p->max_depth : (1ll << 62);
+    return TC_OK;
+}
+
+// the slot / tile layout built on the device into the bound buffers (T slots, NT tiles); rb.extra: the chained form's extra section
+static int ins_layout_dev(tc_ctx* ctx, ins_args& a, uint8_t* d_rb, const ins_block& rb, size_t T, size_t NT, const tc_status* pileup_status,
+                          cudaStream_t s) {
+    int32_t* d_layout = (int32_t*)(d_rb + rb.layout);
+    a.layout = d_layout;
+    ins_layout_kernel<<<1, 256, 0, s>>>(a, const_cast<int64_t*>(a.seg_off), const_cast<int32_t*>(a.tile_first), const_cast<int32_t*>(a.tile_cand),
+                                        d_layout, (int64_t)T, (int)NT, pileup_status, rb.extra ? (int32_t*)(d_rb + rb.extra) : nullptr);
     TC_LAUNCH_CHECK();
     return TC_OK;
 }
+
+// select and admit over `tiles` tiles, the mate-overlap pass when a base-quality filter applies, then (d_calls not NULL) the
+// hash count; the last two over `grid` candidates
+static int ins_enqueue_count(tc_ctx* ctx, const ins_args& a, unsigned tiles, int grid, tc_insert_call_t* d_calls, cudaStream_t s) {
+    if (tiles) {
+        ins_select_kernel<<<tiles, INS_TILE, 0, s>>>(a);
+        TC_LAUNCH_CHECK();
+        ins_admit_kernel<<<tiles, INS_TILE, 0, s>>>(a);
+        TC_LAUNCH_CHECK();
+    }
+    if (a.min_bq > 0) {
+        const size_t smem = (size_t)PAIR_TBL * 10;
+        if (!(ctx->ins_attr_set & 2)) {
+            TC_CUDA(cudaFuncSetAttribute(ins_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            ctx->ins_attr_set |= 2;
+        }
+        ins_pair_kernel<<<grid, 1024, smem, s>>>(a);
+        TC_LAUNCH_CHECK();
+    }
+    if (d_calls) {
+        const size_t smem = (size_t)INS_TBL * 16;
+        if (!(ctx->ins_attr_set & 1)) {
+            TC_CUDA(cudaFuncSetAttribute(ins_count_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            ctx->ins_attr_set |= 1;
+        }
+        ins_count_kernel<<<grid, 1024, smem, s>>>(a, d_calls);
+        TC_LAUNCH_CHECK();
+    }
+    return TC_OK;
+}
+
+static int ins_check_status(tc_ctx* ctx, const tc_status& st) {
+    if (st.err == TC_ERR_UNSORTED) return tc_fail(ctx, TC_ERR_UNSORTED, "Unsorted input. Pileup aborts");
+    if (st.err) return tc_fail(ctx, st.err, "insertion key collision or device-side failure %d", st.err);
+    return TC_OK;
+}
+
+// Every call's offset into the caller's `bases` (-1 without inserted characters), and the winners' inserted characters
+// placed there from `fixed` ([n][INS_BASES_FIXED]); an insertion longer than INS_BASES_FIXED gets its offset only.  *need_out:
+// the bytes all insertions take.
+static int ins_place_bases(tc_ctx* ctx, tc_insert_call_t* calls, int n, const uint8_t* fixed, uint8_t* bases, int64_t bases_cap,
+                           int64_t* need_out = nullptr) {
+    int64_t need = 0;
+    for (int i = 0; i < n; ++i) {
+        if (calls[i].indel > 0) { calls[i].bases_off = need; need += calls[i].indel; } else calls[i].bases_off = -1;
+    }
+    if (need_out) *need_out = need;
+    if (need > 0 && (!bases || need > bases_cap)) return tc_fail(ctx, TC_ERR_CAPACITY, "bases buffer too small: need %lld bytes", (long long)need);
+    for (int i = 0; i < n; ++i)
+        if (calls[i].indel > 0 && calls[i].indel <= INS_BASES_FIXED)
+            memcpy(bases + calls[i].bases_off, fixed + (size_t)i * INS_BASES_FIXED, (size_t)calls[i].indel);
+    return TC_OK;
+}
+
+// Ranges [r[stride * i], r[stride * i + 1]) of ascending candidates ascend too: merge the overlapping ones and hand every
+// stretch to copy(first, length) once.
+template <class T, class F>
+static int ins_stage_merged(const T* r, int stride, int n, F copy) {
+    int i = 0;
+    while (i < n) {
+        const T b0 = r[stride * i];
+        T b1 = r[stride * i + 1];
+        int j = i + 1;
+        while (j < n && r[stride * j] <= b1) { if (r[stride * j + 1] > b1) b1 = r[stride * j + 1]; ++j; }
+        if (b1 != b0) {
+            const int rc = copy((size_t)b0, (size_t)(b1 - b0));
+            if (rc) return rc;
+        }
+        i = j;
+    }
+    return TC_OK;
+}
+
+static int ins_copy(tc_ctx* ctx, const void* dst, const void* src, size_t bytes, cudaMemcpyKind kind, cudaStream_t s, const char* what) {
+    const cudaError_t e = cudaMemcpyAsync(const_cast<void*>(dst), src, bytes, kind, s);
+    return e == cudaSuccess ? TC_OK : tc_cuda_fail(ctx, e, what);
+}
+
+static int ins_sync(tc_ctx* ctx, cudaStream_t s, const char* what) {
+    const cudaError_t e = cudaStreamSynchronize(s);
+    return e == cudaSuccess ? TC_OK : tc_cuda_fail(ctx, e, what);
+}
+
+template <class T>
+static std::unique_ptr<T[]> host_array(size_t n) { return std::unique_ptr<T[]>(new (std::nothrow) T[n > 0 ? n : 1]); }
 
 TC_API int tc_extract_inserts(tc_ctx_t* ctx, const tc_reads_t* reads, int32_t ref_len, const int32_t* cand_pos, int32_t n_cand,
                               const tc_pileup_params_t* p, tc_insert_call_t* calls, uint8_t* bases, int64_t bases_cap, void* stream) {
@@ -749,288 +879,207 @@ TC_API int tc_extract_inserts(tc_ctx_t* ctx, const tc_reads_t* reads, int32_t re
         if (cand_pos[i] < 1 || cand_pos[i] > ref_len) return tc_fail(ctx, TC_ERR_ARG, "candidate position %d outside 1..%d", cand_pos[i], ref_len);
     cudaStream_t s = (cudaStream_t)stream;
     TC_CUDA(cudaSetDevice(ctx->device));
-    ins_args a;
-    memset(&a, 0, sizeof(a));
-    // Host-resident SEQ / QUAL / CIGAR are staged range by range once the candidate ranges are known: this pass
-    // reads them only for the reads over the candidate columns, and QUAL alone is 8x the packed bases.  (Without a
-    // span bound the CIGARs of all reads are needed first, so they are staged in full.)
-    // the caller's span bound is only trusted when tc_pileup_counts has verified it for these very arrays; a bound that is too
-    // small would silently narrow the range of reads fetched for a column
-    const bool bounded = reads->max_ref_span > 0 && ctx->span_ok_bound == reads->max_ref_span && ctx->span_ok_cigar == reads->cigar &&
-                         ctx->span_ok_off == reads->cigar_off && ctx->span_ok_n == reads->n_reads && ctx->span_ok_ops == reads->n_cigar_ops;
-    const int stage = NEED_QUAL | NEED_MATE | DEFER_SEQ | DEFER_QUAL | DEFER_MATE | (bounded ? DEFER_CIGAR : 0);
-    const bool host_seq = reads->seq4 && !tc_is_device_ptr(reads->seq4);
-    const bool host_qual = reads->qual && !tc_is_device_ptr(reads->qual);
-    const bool host_cig = bounded && reads->cigar && !tc_is_device_ptr(reads->cigar);
-    const bool host_mate = reads->qname_hash && reads->mpos && reads->isize && !tc_is_device_ptr(reads->qname_hash);
-    int rc = tc_resolve_reads(ctx, reads, &a.r, stage, s);
-    if (rc) return rc;
-    const int64_t n = a.r.n;
-    for (int i = 0; i < n_cand; ++i) { calls[i].pos = cand_pos[i]; calls[i].n_entries = 0; calls[i].mode_count = 0; calls[i].first_read = -1; calls[i].head = 0; calls[i].indel = 0; calls[i].bases_off = -1; }
-    if (n == 0) return TC_OK;
-    // results block: status, layout, overflow flag, admitted counts, the calls and their inserted characters — one
-    // memset in front, one copy back
-    const size_t RB_LAYOUT = 64, RB_OVER = 80, RB_BUMP = 88, RB_SEG = 96;
-    const size_t rb_calls = RB_SEG + ((4 * (2 * (size_t)n_cand + 2) + 15) & ~(size_t)15);     // seg_count, then pair_any
-    const size_t rb_fixed = rb_calls + sizeof(tc_insert_call_t) * (size_t)n_cand;
-    const size_t rb_bytes = rb_fixed + (size_t)n_cand * INS_BASES_FIXED;
-    static_assert(sizeof(tc_status) <= 64, "tc_status outgrew its place in the results block");
-    uint8_t* d_rb = (uint8_t*)tc_dev_buf(ctx, SLOT_INS_E, rb_bytes + 16);
-    tc_status* d_status = (tc_status*)d_rb;
-    int32_t* d_cand = (int32_t*)tc_dev_buf(ctx, SLOT_INS_A, 4 * (size_t)n_cand);
-    int32_t* d_range = (int32_t*)tc_dev_buf(ctx, SLOT_INS_B, 24 * (size_t)n_cand);       // [n_cand][2] ranges, then [n_cand][4] offsets
-    if (!d_status || !d_cand || !d_range) return TC_ERR_NOMEM;
-    TC_CUDA(cudaMemsetAsync(d_rb, 0, rb_calls, s));
-    TC_CUDA(cudaMemcpyAsync(d_cand, cand_pos, 4 * (size_t)n_cand, cudaMemcpyHostToDevice, s));
-    ctx->h2d_bytes += 4 * (int64_t)n_cand;
-    a.span_hint = bounded ? reads->max_ref_span : 0;
-    if (a.span_hint == 0) {
-        max_span_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(a.r, d_status);
+    auto upload = [&](const void* d, const void* h, size_t bytes, const char* what) {
+        const int rc = ins_copy(ctx, d, h, bytes, cudaMemcpyHostToDevice, s, what);
+        if (rc == TC_OK) ctx->h2d_bytes += (int64_t)bytes;
+        return rc;
+    };
+    // Every pass runs from the start.  A pass runs again when the pair scratch overflowed (sized from its bump), or when the
+    // speculative layout did not fit (sized for next time) or a column needs the sorted form: then with the layout built on
+    // the host (reserved bit 0).
+    tc_pileup_params_t q = *p;
+    for (;;) {
+        ins_args a;
+        memset(&a, 0, sizeof(a));
+        // Host-resident SEQ / QUAL / CIGAR are staged range by range once the candidate ranges are known: this pass
+        // reads them only for the reads over the candidate columns, and QUAL alone is 8x the packed bases.  (Without a
+        // span bound the CIGARs of all reads are needed first, so they are staged in full.)
+        // the caller's span bound is only trusted when tc_pileup_counts has verified it for these very arrays; a bound that is too
+        // small would silently narrow the range of reads fetched for a column
+        const bool bounded = reads->max_ref_span > 0 && ctx->span_ok_bound == reads->max_ref_span && ctx->span_ok_cigar == reads->cigar &&
+                             ctx->span_ok_off == reads->cigar_off && ctx->span_ok_n == reads->n_reads && ctx->span_ok_ops == reads->n_cigar_ops;
+        const int stage = NEED_QUAL | NEED_MATE | DEFER_SEQ | DEFER_QUAL | DEFER_MATE | (bounded ? DEFER_CIGAR : 0);
+        const bool host_seq = reads->seq4 && !tc_is_device_ptr(reads->seq4);
+        const bool host_qual = reads->qual && !tc_is_device_ptr(reads->qual);
+        const bool host_cig = bounded && reads->cigar && !tc_is_device_ptr(reads->cigar);
+        const bool host_mate = reads->qname_hash && reads->mpos && reads->isize && !tc_is_device_ptr(reads->qname_hash);
+        int rc = tc_resolve_reads(ctx, reads, &a.r, stage, s);
+        if (rc) return rc;
+        const int64_t n = a.r.n;
+        for (int i = 0; i < n_cand; ++i) { calls[i].pos = cand_pos[i]; calls[i].n_entries = 0; calls[i].mode_count = 0; calls[i].first_read = -1; calls[i].head = 0; calls[i].indel = 0; calls[i].bases_off = -1; }
+        if (n == 0) return TC_OK;
+        const ins_block rb = ins_block_of(n_cand, false);
+        uint8_t* d_rb = (uint8_t*)tc_dev_buf(ctx, SLOT_INS_E, rb.bytes + 16);
+        int32_t* d_cand = (int32_t*)tc_dev_buf(ctx, SLOT_INS_A, 4 * (size_t)n_cand);
+        int32_t* d_range = (int32_t*)tc_dev_buf(ctx, SLOT_INS_B, 24 * (size_t)n_cand);       // [n_cand][2] ranges, then [n_cand][4] offsets
+        if (!d_rb || !d_cand || !d_range) return TC_ERR_NOMEM;
+        a.status = (tc_status*)d_rb;
+        TC_CUDA(cudaMemsetAsync(d_rb, 0, rb.calls, s));
+        TC_CUDA(cudaMemcpyAsync(d_cand, cand_pos, 4 * (size_t)n_cand, cudaMemcpyHostToDevice, s));
+        ctx->h2d_bytes += 4 * (int64_t)n_cand;
+        a.span_hint = bounded ? reads->max_ref_span : 0;
+        if (a.span_hint == 0) {
+            max_span_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(a.r, a.status);
+            TC_LAUNCH_CHECK();
+        }
+        a.cand = d_cand; a.n_cand = n_cand; a.range = d_range; a.range_off = (uint32_t*)(d_range + 2 * (size_t)n_cand);
+        cand_range_kernel<<<(n_cand + 3) / 4, 128, 0, s>>>(a);
         TC_LAUNCH_CHECK();
-    }
-    a.cand = d_cand; a.n_cand = n_cand; a.range = d_range; a.range_off = (uint32_t*)(d_range + 2 * (size_t)n_cand); a.status = d_status;
-    a.flag_filter = p->flag_filter; a.min_mapq = p->min_mapq; a.min_bq = p->min_base_quality; a.ignore_orphans = p->ignore_orphans;
-    a.olap_mode = (p->reserved >> 8) & 3;
-    a.max_depth = p->max_depth > 0 ? p->max_depth : (1ll << 62);
-    cand_range_kernel<<<(n_cand + 3) / 4, 128, 0, s>>>(a);
-    TC_LAUNCH_CHECK();
-    // Layout of the entry slots.  With everything resident on the device and the hash count, the layout is built
-    // on the device into buffers sized from the last calls (no read-back of the ranges, one synchronisation per
-    // call); otherwise — host arrays to stage range by range, the sorted form, or a layout that did not fit — on
-    // the host from the ranges.
-    const bool spec = !(host_seq || host_qual || host_cig || host_mate) && p->kernel != 2 && !(p->reserved & 1);
-    if (ctx->ins_slot_cap <= 0) ctx->ins_slot_cap = 1 << 16;     // grows to twice the largest layout seen
-    int32_t* h_range = (int32_t*)malloc(24 * (size_t)n_cand);
-    int64_t* h_off = (int64_t*)malloc(8 * ((size_t)n_cand + 1));
-    int32_t* h_tfirst = (int32_t*)malloc(4 * ((size_t)n_cand + 1));
-    int32_t* h_tcand = NULL;
-    int64_t* h_entry = NULL;
-    uint8_t* h_fixed = (uint8_t*)malloc((size_t)n_cand * INS_BASES_FIXED);
-    if (!h_range || !h_off || !h_tfirst || !h_fixed) { free(h_range); free(h_off); free(h_tfirst); free(h_fixed); return tc_fail(ctx, TC_ERR_NOMEM, "out of host memory"); }
-#define INS_FREE() do { free(h_range); free(h_off); free(h_tfirst); free(h_tcand); free(h_entry); free(h_fixed); } while (0)
-#define INS_CUDA(call, what) do { cudaError_t e__ = (call); if (e__ != cudaSuccess) { INS_FREE(); return tc_cuda_fail(ctx, e__, what); } } while (0)
-    int64_t total = 0;
-    int n_tiles = 0;
-    if (!spec) {
-    INS_CUDA(cudaMemcpyAsync(h_range, d_range, 24 * (size_t)n_cand, cudaMemcpyDeviceToHost, s), "range readback");
-    INS_CUDA(cudaStreamSynchronize(s), "range readback");
-    ctx->d2h_bytes += 24 * (int64_t)n_cand;
-    if (host_mate) {
-        // QNAME hash, PNEXT, TLEN of the reads over the candidate columns (read index ranges; candidates ascend, so do their ranges)
-        int i = 0;
-        while (i < n_cand) {
-            int64_t b0 = h_range[2 * i], b1 = h_range[2 * i + 1];
-            int j = i + 1;
-            while (j < n_cand && h_range[2 * j] <= b1) { if (h_range[2 * j + 1] > b1) b1 = h_range[2 * j + 1]; ++j; }
-            const size_t len = (size_t)(b1 - b0);
-            if (len) {
-                INS_CUDA(cudaMemcpyAsync((uint64_t*)a.r.qname_hash + b0, reads->qname_hash + b0, 8 * len, cudaMemcpyHostToDevice, s), "QNAME hash range upload");
-                INS_CUDA(cudaMemcpyAsync((int32_t*)a.r.mpos + b0, reads->mpos + b0, 4 * len, cudaMemcpyHostToDevice, s), "PNEXT range upload");
-                INS_CUDA(cudaMemcpyAsync((int32_t*)a.r.isize + b0, reads->isize + b0, 4 * len, cudaMemcpyHostToDevice, s), "TLEN range upload");
-                ctx->h2d_bytes += 16 * (int64_t)len;
+        // Layout of the entry slots.  With everything resident on the device and the hash count, the layout is built
+        // on the device into buffers sized from the last calls (no read-back of the ranges, one synchronisation per
+        // call); otherwise — host arrays to stage range by range, the sorted form, or a layout that did not fit — on
+        // the host from the ranges.
+        const bool spec = !(host_seq || host_qual || host_cig || host_mate) && q.kernel != 2 && !(q.reserved & 1);
+        if (ctx->ins_slot_cap <= 0) ctx->ins_slot_cap = 1 << 16;     // grows to twice the largest layout seen
+        std::unique_ptr<int64_t[]> h_off;
+        std::unique_ptr<int32_t[]> h_tfirst, h_tcand;
+        int64_t total = ctx->ins_slot_cap;
+        int n_tiles = (int)(total / INS_TILE) + n_cand + 1;
+        if (!spec) {
+            auto h_range = host_array<int32_t>(6 * (size_t)n_cand);
+            h_off = host_array<int64_t>((size_t)n_cand + 1);
+            h_tfirst = host_array<int32_t>((size_t)n_cand + 1);
+            if (!h_range || !h_off || !h_tfirst) return tc_fail(ctx, TC_ERR_NOMEM, "out of host memory");
+            if ((rc = ins_copy(ctx, h_range.get(), d_range, 24 * (size_t)n_cand, cudaMemcpyDeviceToHost, s, "range readback")) ||
+                (rc = ins_sync(ctx, s, "range readback")))
+                return rc;
+            ctx->d2h_bytes += 24 * (int64_t)n_cand;
+            // QNAME hash, PNEXT, TLEN of the reads over the candidate columns (read index ranges); SEQ + QUAL word ranges; CIGAR op ranges
+            if (host_mate)
+                rc = ins_stage_merged(h_range.get(), 2, n_cand, [&](size_t b0, size_t len) {
+                    int e = upload(a.r.qname_hash + b0, reads->qname_hash + b0, 8 * len, "QNAME hash range upload");
+                    if (!e) e = upload(a.r.mpos + b0, reads->mpos + b0, 4 * len, "PNEXT range upload");
+                    if (!e) e = upload(a.r.isize + b0, reads->isize + b0, 4 * len, "TLEN range upload");
+                    return e;
+                });
+            const uint32_t* ho = (const uint32_t*)(h_range.get() + 2 * (size_t)n_cand);
+            if (!rc && (host_seq || host_qual))
+                rc = ins_stage_merged(ho, 4, n_cand, [&](size_t b0, size_t len) {
+                    int e = host_seq ? upload(a.r.seq4 + b0, reads->seq4 + b0, 4 * len, "SEQ range upload") : TC_OK;
+                    if (!e && host_qual) e = upload(a.r.qual + 8 * b0, reads->qual + 8 * b0, 8 * len, "QUAL range upload");
+                    return e;
+                });
+            if (!rc && host_cig)
+                rc = ins_stage_merged(ho + 2, 4, n_cand,
+                                      [&](size_t b0, size_t len) { return upload(a.r.cigar + b0, reads->cigar + b0, 4 * len, "CIGAR range upload"); });
+            if (rc) return rc;
+            h_off[0] = 0; h_tfirst[0] = 0;
+            for (int i = 0; i < n_cand; ++i) {
+                const int64_t len = h_range[2 * i + 1] - h_range[2 * i];
+                h_off[i + 1] = h_off[i] + len;
+                h_tfirst[i + 1] = h_tfirst[i] + (int32_t)((len + INS_TILE - 1) / INS_TILE);
             }
-            i = j;
+            total = h_off[n_cand];
+            n_tiles = h_tfirst[n_cand];
+            if (total >= 0x7fffffffll) return tc_fail(ctx, TC_ERR_CAPACITY, "too many candidate column entries (%lld)", (long long)total);
+            h_tcand = host_array<int32_t>((size_t)n_tiles);
+            if (!h_tcand) return tc_fail(ctx, TC_ERR_NOMEM, "out of host memory");
+            for (int i = 0; i < n_cand; ++i) for (int t = h_tfirst[i]; t < h_tfirst[i + 1]; ++t) h_tcand[t] = i;
         }
-    }
-    if (host_seq || host_qual || host_cig) {
-        // candidates ascend, so do their ranges: merge the overlapping ones and copy every stretch once
-        const uint32_t* ho = (const uint32_t*)(h_range + 2 * (size_t)n_cand);
-        for (int k = 0; k < 2; ++k) {           // k = 0: SEQ + QUAL word ranges, k = 1: CIGAR op ranges
-            if (k == 0 ? !(host_seq || host_qual) : !host_cig) continue;
-            int i = 0;
-            while (i < n_cand) {
-                uint32_t b0 = ho[4 * i + 2 * k], b1 = ho[4 * i + 2 * k + 1];
-                int j = i + 1;
-                while (j < n_cand && ho[4 * j + 2 * k] <= b1) { if (ho[4 * j + 2 * k + 1] > b1) b1 = ho[4 * j + 2 * k + 1]; ++j; }
-                const size_t len = (size_t)(b1 - b0);
-                if (len) {
-                    if (k == 0 && host_seq) { INS_CUDA(cudaMemcpyAsync((uint32_t*)a.r.seq4 + b0, reads->seq4 + b0, 4 * len, cudaMemcpyHostToDevice, s), "SEQ range upload"); ctx->h2d_bytes += 4 * (int64_t)len; }
-                    if (k == 0 && host_qual) { INS_CUDA(cudaMemcpyAsync((uint8_t*)a.r.qual + 8 * (size_t)b0, reads->qual + 8 * (size_t)b0, 8 * len, cudaMemcpyHostToDevice, s), "QUAL range upload"); ctx->h2d_bytes += 8 * (int64_t)len; }
-                    if (k == 1) { INS_CUDA(cudaMemcpyAsync((uint32_t*)a.r.cigar + b0, reads->cigar + b0, 4 * len, cudaMemcpyHostToDevice, s), "CIGAR range upload"); ctx->h2d_bytes += 4 * (int64_t)len; }
-                }
-                i = j;
+        const size_t T = (size_t)(total > 0 ? total : 1), NT = (size_t)(n_tiles > 0 ? n_tiles : 1);
+        if ((rc = ins_bind(ctx, a, d_rb, rb, T, NT, n_cand, &q))) return rc;
+        tc_insert_call_t* d_calls = (tc_insert_call_t*)(d_rb + rb.calls);
+        if (spec) rc = ins_layout_dev(ctx, a, d_rb, rb, T, NT, nullptr, s);
+        else if (!(rc = upload(a.seg_off, h_off.get(), 8 * ((size_t)n_cand + 1), "offset upload")) &&
+                 !(rc = upload(a.tile_first, h_tfirst.get(), 4 * ((size_t)n_cand + 1), "tile table upload")) && n_tiles)
+            rc = upload(a.tile_cand, h_tcand.get(), 4 * (size_t)n_tiles, "tile table upload");
+        if (rc) return rc;
+        const bool sorted_form = q.kernel == 2;
+        if ((rc = ins_enqueue_count(ctx, a, (unsigned)n_tiles, n_cand, sorted_form ? nullptr : d_calls, s))) return rc;
+        int32_t h_over = 0;
+        unsigned long long h_bump = 0;
+        int32_t h_layout[3] = {0, 0, 0};
+        const size_t calls_bytes = sizeof(tc_insert_call_t) * (size_t)n_cand, fixed_bytes = (size_t)n_cand * INS_BASES_FIXED;
+        auto h_fixed = host_array<uint8_t>(fixed_bytes);
+        if (!h_fixed) return tc_fail(ctx, TC_ERR_NOMEM, "out of host memory");
+        // the results block comes back in one copy through pinned memory (copies into the caller's pageable buffers
+        // would each wait for the stream)
+        if (rb.bytes <= TC_HOST_SCRATCH) {
+            const uint8_t* pin = (const uint8_t*)ctx->host_scratch;
+            if ((rc = ins_copy(ctx, pin, d_rb, rb.bytes, cudaMemcpyDeviceToHost, s, "results readback")) || (rc = ins_sync(ctx, s, "results readback")))
+                return rc;
+            memcpy(ctx->host_status, pin, sizeof(tc_status));
+            memcpy(h_layout, pin + rb.layout, 12); memcpy(&h_over, pin + rb.over, 4); memcpy(&h_bump, pin + rb.bump, 8);
+            memcpy(calls, pin + rb.calls, calls_bytes); memcpy(h_fixed.get(), pin + rb.fixed, fixed_bytes);
+        } else if ((rc = ins_copy(ctx, &h_over, a.overflow, 4, cudaMemcpyDeviceToHost, s, "overflow readback")) ||
+                   (rc = ins_copy(ctx, &h_bump, a.pair_bump, 8, cudaMemcpyDeviceToHost, s, "overflow readback")) ||
+                   (spec && (rc = ins_copy(ctx, h_layout, a.layout, 12, cudaMemcpyDeviceToHost, s, "layout readback"))) ||
+                   (rc = ins_copy(ctx, calls, d_calls, calls_bytes, cudaMemcpyDeviceToHost, s, "insert calls readback")) ||
+                   (rc = ins_copy(ctx, h_fixed.get(), a.bases_fixed, fixed_bytes, cudaMemcpyDeviceToHost, s, "inserted bases readback")) ||
+                   (rc = ins_copy(ctx, ctx->host_status, a.status, sizeof(tc_status), cudaMemcpyDeviceToHost, s, "status readback")) ||
+                   (rc = ins_sync(ctx, s, "insert calls readback"))) {
+            return rc;
+        }
+        ctx->d2h_bytes += (int64_t)(sizeof(tc_insert_call_t) + INS_BASES_FIXED) * n_cand + (int64_t)sizeof(tc_status) + 4;
+        if (sorted_form) h_over &= 2;
+        if (h_over & 2) {
+            // the scratch for the rewritten quality strings of overlapping mates was too small: size it and run again
+            ctx->pair_cap = 2 * (int64_t)h_bump + 4096;
+            continue;
+        }
+        if (spec) {
+            if (h_layout[2] || h_over) {
+                // the layout did not fit the speculative buffers (size them for next time), or a column needs the sorted
+                // form: run again with the layout built on the host
+                if (h_layout[2]) ctx->ins_slot_cap = 2 * (int64_t)h_layout[1] + 4096;
+                q.reserved |= 1;
+                continue;
             }
+            total = h_layout[1];
         }
-    }
-    h_off[0] = 0; h_tfirst[0] = 0;
-    for (int i = 0; i < n_cand; ++i) {
-        const int64_t len = h_range[2 * i + 1] - h_range[2 * i];
-        h_off[i + 1] = h_off[i] + len;
-        h_tfirst[i + 1] = h_tfirst[i] + (int32_t)((len + INS_TILE - 1) / INS_TILE);
-    }
-    total = h_off[n_cand];
-    n_tiles = h_tfirst[n_cand];
-    if (total >= 0x7fffffffll) { INS_FREE(); return tc_fail(ctx, TC_ERR_CAPACITY, "too many candidate column entries (%lld)", (long long)total); }
-    h_tcand = (int32_t*)malloc(4 * (size_t)(n_tiles > 0 ? n_tiles : 1));
-    if (!h_tcand) { INS_FREE(); return tc_fail(ctx, TC_ERR_NOMEM, "out of host memory"); }
-    for (int i = 0; i < n_cand; ++i) for (int t = h_tfirst[i]; t < h_tfirst[i + 1]; ++t) h_tcand[t] = i;
-    } else {
-        total = ctx->ins_slot_cap;
-        n_tiles = (int)(total / INS_TILE) + n_cand + 1;
-    }
-    const size_t T = (size_t)(total > 0 ? total : 1), NT = (size_t)(n_tiles > 0 ? n_tiles : 1);
-    // one slab: keys, indel, qpos, head, sel per slot; tile tables; per-candidate offsets, counts
-    const size_t bytes = T * (8 + 4 + 4 + 1 + 1 + 1) + NT * 12 + ((size_t)n_cand + 1) * 16 + (size_t)n_cand * INS_BASES_FIXED + 256 + 16;
-    uint8_t* slab = (uint8_t*)tc_dev_buf(ctx, SLOT_INS_D, bytes);
-    tc_insert_call_t* d_calls = (tc_insert_call_t*)(d_rb + rb_calls);
-    if (!slab) { INS_FREE(); return TC_ERR_NOMEM; }
-    uint64_t* d_key = (uint64_t*)slab;
-    int64_t* d_off = (int64_t*)(d_key + T);
-    a.ent_indel = (int32_t*)(d_off + n_cand + 1); a.ent_qpos = a.ent_indel + T;
-    int32_t* d_tcand = a.ent_qpos + T; int32_t* d_tfirst = d_tcand + NT;
-    a.tile_sel = d_tfirst + n_cand + 1; a.tile_last = a.tile_sel + NT;
-    a.seg_count = (int32_t*)(d_rb + RB_SEG); a.pair_any = a.seg_count + n_cand + 1; a.overflow = (int32_t*)(d_rb + RB_OVER);
-    if (ctx->pair_cap <= 0) ctx->pair_cap = 1 << 22;
-    a.pair_bump = (unsigned long long*)(d_rb + RB_BUMP); a.pair_cap = (unsigned long long)ctx->pair_cap;
-    a.pair_q = (uint8_t*)tc_dev_buf(ctx, SLOT_INS_F, (size_t)ctx->pair_cap);
-    if (!a.pair_q) { INS_FREE(); return TC_ERR_NOMEM; }
-    int32_t* d_layout = (int32_t*)(d_rb + RB_LAYOUT);         // [3], speculative layout only
-    a.ent_head = (uint8_t*)(a.tile_last + NT); a.ent_sel = a.ent_head + T; a.ent_q = a.ent_sel + T; a.bases_fixed = d_rb + rb_fixed;
-    a.ent_key = d_key; a.seg_off = d_off; a.tile_cand = d_tcand; a.tile_first = d_tfirst;
-    if (spec) {
-        a.layout = d_layout;
-        ins_layout_kernel<<<1, 256, 0, s>>>(a, d_off, d_tfirst, d_tcand, d_layout, (int64_t)T, (int)NT, nullptr, nullptr);
-        ctx->launches++;
-    } else {
-        a.layout = nullptr;
-        INS_CUDA(cudaMemcpyAsync(d_off, h_off, 8 * ((size_t)n_cand + 1), cudaMemcpyHostToDevice, s), "offset upload");
-        INS_CUDA(cudaMemcpyAsync(d_tfirst, h_tfirst, 4 * ((size_t)n_cand + 1), cudaMemcpyHostToDevice, s), "tile table upload");
-        if (n_tiles) INS_CUDA(cudaMemcpyAsync(d_tcand, h_tcand, 4 * (size_t)n_tiles, cudaMemcpyHostToDevice, s), "tile table upload");
-        ctx->h2d_bytes += 12 * ((int64_t)n_cand + 1) + 4 * (int64_t)n_tiles;
-    }
-    if (n_tiles) {
-        ins_select_kernel<<<n_tiles, INS_TILE, 0, s>>>(a);
-        ctx->launches++;
-        ins_admit_kernel<<<n_tiles, INS_TILE, 0, s>>>(a);
-        ctx->launches++;
-    }
-    if (a.min_bq > 0) {
-        rc = launch_pair(ctx, a, n_cand, s);
-        if (rc) { INS_FREE(); return rc; }
-    }
-    bool sorted_form = p->kernel == 2;
-    const size_t tbl_smem = (size_t)INS_TBL * 16;
-    int32_t h_over = 0;
-    unsigned long long h_bump = 0;
-    int32_t h_layout[3] = {0, 0, 0};
-    // the results block comes back in one copy through pinned memory (copies into the caller's pageable buffers
-    // would each wait for the stream)
-    const size_t calls_bytes = sizeof(tc_insert_call_t) * (size_t)n_cand, fixed_bytes = (size_t)n_cand * INS_BASES_FIXED;
-    const bool via_pinned = rb_bytes <= TC_HOST_SCRATCH;
-    if (!sorted_form) {
-        if (!(ctx->ins_attr_set & 1)) {
-            INS_CUDA(cudaFuncSetAttribute(ins_count_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tbl_smem), "smem attribute");
-            ctx->ins_attr_set |= 1;
+        if (sorted_form || h_over) {
+            // radix sort + run-length encoding over the same slots
+            uint8_t* slab2 = (uint8_t*)tc_dev_buf(ctx, SLOT_INS_C, T * (8 + 4 + 4) + 64);
+            if (!slab2) return TC_ERR_NOMEM;
+            uint64_t* d_skey = (uint64_t*)slab2; uint32_t* d_idx = (uint32_t*)(d_skey + T); uint32_t* d_sidx = d_idx + T;
+            int64_t* d_off = const_cast<int64_t*>(a.seg_off);
+            iota_kernel<<<(unsigned)((T + 255) / 256), 256, 0, s>>>(d_idx, (int64_t)total);
+            TC_LAUNCH_CHECK();
+            size_t tmp_bytes = 0;
+            cudaError_t e = cub::DeviceSegmentedRadixSort::SortPairs(nullptr, tmp_bytes, a.ent_key, d_skey, d_idx, d_sidx, (int64_t)total, n_cand,
+                                                                     d_off, d_off + 1, 0, 64, s);
+            if (e != cudaSuccess) return tc_cuda_fail(ctx, e, "cub sort sizing");
+            void* d_tmp = tc_dev_buf(ctx, SLOT_INS_G, tmp_bytes + 16);
+            if (!d_tmp) return TC_ERR_NOMEM;
+            e = cub::DeviceSegmentedRadixSort::SortPairs(d_tmp, tmp_bytes, a.ent_key, d_skey, d_idx, d_sidx, (int64_t)total, n_cand, d_off,
+                                                         d_off + 1, 0, 64, s);
+            if (e != cudaSuccess) return tc_cuda_fail(ctx, e, "cub segmented radix sort");
+            ctx->launches++;
+            ins_mode_kernel<<<n_cand, 1024, 0, s>>>(a, d_skey, d_sidx, d_calls);
+            TC_LAUNCH_CHECK();
+            if ((rc = ins_copy(ctx, calls, d_calls, calls_bytes, cudaMemcpyDeviceToHost, s, "insert calls readback")) ||
+                (rc = ins_copy(ctx, h_fixed.get(), a.bases_fixed, fixed_bytes, cudaMemcpyDeviceToHost, s, "inserted bases readback")) ||
+                (rc = ins_copy(ctx, ctx->host_status, a.status, sizeof(tc_status), cudaMemcpyDeviceToHost, s, "status readback")) ||
+                (rc = ins_sync(ctx, s, "insert calls readback")))
+                return rc;
         }
-        ins_count_kernel<<<n_cand, 1024, tbl_smem, s>>>(a, d_calls);
-        ctx->launches++;
+        tc_status st; memcpy(&st, ctx->host_status, sizeof(st));
+        if ((rc = ins_check_status(ctx, st))) return rc;
+        // lay the winners' inserted characters out in the caller's buffer: up to INS_BASES_FIXED characters came back
+        // with the call; longer insertions (rare) are fetched by one more small kernel
+        auto h_entry = host_array<int64_t>((size_t)n_cand);
+        if (!h_entry) return tc_fail(ctx, TC_ERR_NOMEM, "out of host memory");
+        int64_t n_long = 0;
+        for (int i = 0; i < n_cand; ++i) { h_entry[i] = calls[i].bases_off; n_long += calls[i].indel > INS_BASES_FIXED; }
+        int64_t need = 0;
+        if ((rc = ins_place_bases(ctx, calls, n_cand, h_fixed.get(), bases, bases_cap, &need)) || n_long == 0) return rc;
+        uint8_t* d_bases = (uint8_t*)tc_dev_buf(ctx, SLOT_TMP_A, (size_t)need);
+        int64_t* d_entry = (int64_t*)tc_dev_buf(ctx, SLOT_TMP_B, 8 * (size_t)n_cand);
+        auto h_long = host_array<uint8_t>((size_t)need);
+        if (!d_bases || !d_entry || !h_long) return TC_ERR_NOMEM;
+        const char* what = "inserted bases readback";
+        if ((rc = ins_copy(ctx, d_entry, h_entry.get(), 8 * (size_t)n_cand, cudaMemcpyHostToDevice, s, what)) ||
+            (rc = ins_copy(ctx, d_calls, calls, calls_bytes, cudaMemcpyHostToDevice, s, what)))
+            return rc;
+        ins_bases_kernel<<<n_cand, 128, 0, s>>>(a, d_calls, d_entry, d_bases);
+        TC_LAUNCH_CHECK();
+        if (!(rc = ins_copy(ctx, h_long.get(), d_bases, (size_t)need, cudaMemcpyDeviceToHost, s, what))) rc = ins_sync(ctx, s, what);
+        ctx->d2h_bytes += need;
+        if (rc) return rc;
+        for (int i = 0; i < n_cand; ++i)
+            if (calls[i].indel > INS_BASES_FIXED) memcpy(bases + calls[i].bases_off, h_long.get() + calls[i].bases_off, (size_t)calls[i].indel);
+        return TC_OK;
     }
-    if (via_pinned) {
-        uint8_t* pin = (uint8_t*)ctx->host_scratch;
-        INS_CUDA(cudaMemcpyAsync(pin, d_rb, rb_bytes, cudaMemcpyDeviceToHost, s), "results readback");
-        INS_CUDA(cudaStreamSynchronize(s), "results readback");
-        memcpy(ctx->host_status, pin, sizeof(tc_status));
-        memcpy(h_layout, pin + RB_LAYOUT, 12); memcpy(&h_over, pin + RB_OVER, 4); memcpy(&h_bump, pin + RB_BUMP, 8);
-        memcpy(calls, pin + rb_calls, calls_bytes); memcpy(h_fixed, pin + rb_fixed, fixed_bytes);
-        if (sorted_form) { h_over &= 2; }
-        if (!spec) { h_layout[0] = h_layout[1] = h_layout[2] = 0; }
-    } else {
-        INS_CUDA(cudaMemcpyAsync(&h_over, a.overflow, 4, cudaMemcpyDeviceToHost, s), "overflow readback");
-        INS_CUDA(cudaMemcpyAsync(&h_bump, a.pair_bump, 8, cudaMemcpyDeviceToHost, s), "overflow readback");
-        if (!sorted_form && spec) INS_CUDA(cudaMemcpyAsync(h_layout, d_layout, 12, cudaMemcpyDeviceToHost, s), "layout readback");
-        INS_CUDA(cudaMemcpyAsync(calls, d_calls, calls_bytes, cudaMemcpyDeviceToHost, s), "insert calls readback");
-        INS_CUDA(cudaMemcpyAsync(h_fixed, a.bases_fixed, fixed_bytes, cudaMemcpyDeviceToHost, s), "inserted bases readback");
-        INS_CUDA(cudaMemcpyAsync(ctx->host_status, d_status, sizeof(tc_status), cudaMemcpyDeviceToHost, s), "status readback");
-        INS_CUDA(cudaStreamSynchronize(s), "insert calls readback");
-    }
-    ctx->d2h_bytes += (int64_t)(sizeof(tc_insert_call_t) + INS_BASES_FIXED) * n_cand + (int64_t)sizeof(tc_status) + 4;
-    if (!via_pinned && sorted_form) h_over &= 2;
-    if (h_over & 2) {
-        // the scratch for the rewritten quality strings of overlapping mates was too small: size it and run again
-        ctx->pair_cap = 2 * (int64_t)h_bump + 4096;
-        INS_FREE();
-        return tc_extract_inserts(ctx, reads, ref_len, cand_pos, n_cand, p, calls, bases, bases_cap, stream);
-    }
-    if (spec) {
-        if (h_layout[2] || h_over) {
-            // the layout did not fit the speculative buffers (size them for next time), or a column needs the sorted
-            // form: run again with the layout built on the host
-            if (h_layout[2]) ctx->ins_slot_cap = 2 * (int64_t)h_layout[1] + 4096;
-            INS_FREE();
-            tc_pileup_params_t q = *p;
-            q.reserved |= 1;
-            return tc_extract_inserts(ctx, reads, ref_len, cand_pos, n_cand, &q, calls, bases, bases_cap, stream);
-        }
-        total = h_layout[1];
-    }
-    if (sorted_form || h_over) {
-        // radix sort + run-length encoding over the same slots
-        uint8_t* slab2 = (uint8_t*)tc_dev_buf(ctx, SLOT_INS_C, T * (8 + 4 + 4) + 64);
-        if (!slab2) { INS_FREE(); return TC_ERR_NOMEM; }
-        uint64_t* d_skey = (uint64_t*)slab2; uint32_t* d_idx = (uint32_t*)(d_skey + T); uint32_t* d_sidx = d_idx + T;
-        iota_kernel<<<(unsigned)((T + 255) / 256), 256, 0, s>>>(d_idx, (int64_t)total);
-        ctx->launches++;
-        size_t tmp_bytes = 0;
-        INS_CUDA(cub::DeviceSegmentedRadixSort::SortPairs(nullptr, tmp_bytes, d_key, d_skey, d_idx, d_sidx, (int64_t)total, n_cand, d_off, d_off + 1, 0, 64, s), "cub sort sizing");
-        void* d_tmp = tc_dev_buf(ctx, SLOT_INS_G, tmp_bytes + 16);
-        if (!d_tmp) { INS_FREE(); return TC_ERR_NOMEM; }
-        INS_CUDA(cub::DeviceSegmentedRadixSort::SortPairs(d_tmp, tmp_bytes, d_key, d_skey, d_idx, d_sidx, (int64_t)total, n_cand, d_off, d_off + 1, 0, 64, s), "cub segmented radix sort");
-        ctx->launches++;
-        ins_mode_kernel<<<n_cand, 1024, 0, s>>>(a, d_skey, d_sidx, d_calls);
-        ctx->launches++;
-        INS_CUDA(cudaMemcpyAsync(calls, d_calls, sizeof(tc_insert_call_t) * (size_t)n_cand, cudaMemcpyDeviceToHost, s), "insert calls readback");
-        INS_CUDA(cudaMemcpyAsync(h_fixed, a.bases_fixed, (size_t)n_cand * INS_BASES_FIXED, cudaMemcpyDeviceToHost, s), "inserted bases readback");
-        INS_CUDA(cudaMemcpyAsync(ctx->host_status, d_status, sizeof(tc_status), cudaMemcpyDeviceToHost, s), "status readback");
-        INS_CUDA(cudaStreamSynchronize(s), "insert calls readback");
-    }
-    tc_status st; memcpy(&st, ctx->host_status, sizeof(st));
-    if (st.err == TC_ERR_UNSORTED) { INS_FREE(); return tc_fail(ctx, TC_ERR_UNSORTED, "Unsorted input. Pileup aborts"); }
-    if (st.err) { INS_FREE(); return tc_fail(ctx, st.err, "insertion key collision or device-side failure %d", st.err); }
-    // lay the winners' inserted characters out in the caller's buffer: up to INS_BASES_FIXED characters came back
-    // with the call; longer insertions (rare) are fetched by one more small kernel
-    int64_t need = 0, n_long = 0;
-    h_entry = (int64_t*)malloc(8 * (size_t)n_cand);
-    if (!h_entry) { INS_FREE(); return tc_fail(ctx, TC_ERR_NOMEM, "out of host memory"); }
-    for (int i = 0; i < n_cand; ++i) {
-        h_entry[i] = calls[i].bases_off;
-        if (calls[i].indel > 0) { calls[i].bases_off = need; need += calls[i].indel; n_long += calls[i].indel > INS_BASES_FIXED; } else calls[i].bases_off = -1;
-    }
-    rc = TC_OK;
-    if (need > 0) {
-        if (!bases || need > bases_cap) rc = tc_fail(ctx, TC_ERR_CAPACITY, "bases buffer too small: need %lld bytes", (long long)need);
-        else {
-            for (int i = 0; i < n_cand; ++i)
-                if (calls[i].indel > 0 && calls[i].indel <= INS_BASES_FIXED)
-                    memcpy(bases + calls[i].bases_off, h_fixed + (size_t)i * INS_BASES_FIXED, (size_t)calls[i].indel);
-            if (n_long > 0) {
-                uint8_t* d_bases = (uint8_t*)tc_dev_buf(ctx, SLOT_TMP_A, (size_t)need);
-                int64_t* d_entry = (int64_t*)tc_dev_buf(ctx, SLOT_TMP_B, 8 * (size_t)n_cand);
-                uint8_t* h_long = (uint8_t*)malloc((size_t)need);
-                if (!d_bases || !d_entry || !h_long) rc = TC_ERR_NOMEM;
-                else {
-                    cudaError_t e = cudaMemcpyAsync(d_entry, h_entry, 8 * (size_t)n_cand, cudaMemcpyHostToDevice, s);
-                    if (e == cudaSuccess) e = cudaMemcpyAsync(d_calls, calls, sizeof(tc_insert_call_t) * (size_t)n_cand, cudaMemcpyHostToDevice, s);
-                    if (e == cudaSuccess) {
-                        ins_bases_kernel<<<n_cand, 128, 0, s>>>(a, d_calls, d_entry, d_bases);
-                        ctx->launches++;
-                        e = cudaMemcpyAsync(h_long, d_bases, (size_t)need, cudaMemcpyDeviceToHost, s);
-                    }
-                    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-                    if (e != cudaSuccess) rc = tc_cuda_fail(ctx, e, "inserted bases readback");
-                    else
-                        for (int i = 0; i < n_cand; ++i)
-                            if (calls[i].indel > INS_BASES_FIXED) memcpy(bases + calls[i].bases_off, h_long + calls[i].bases_off, (size_t)calls[i].indel);
-                    ctx->d2h_bytes += need;
-                }
-                free(h_long);
-            }
-        }
-    }
-    INS_FREE();
-#undef INS_FREE
-#undef INS_CUDA
-    if (rc == TC_OK) { cudaError_t le = cudaGetLastError(); if (le != cudaSuccess) rc = tc_cuda_fail(ctx, le, "insert kernels"); }
-    return rc;
 }
 
 
@@ -1049,16 +1098,12 @@ int tc_inserts_enqueue_dev(tc_ctx* ctx, const tc_reads_t* reads, const int32_t* 
     int rc = tc_resolve_reads(ctx, reads, &a.r, NEED_QUAL | NEED_MATE, s);       // every array is a device pointer already: nothing is copied
     if (rc) return rc;
     const int64_t n = a.r.n;
-    const size_t RB_LAYOUT = 64, RB_OVER = 80, RB_EXTRA = 128;      // extra: [0] n_cand, [16..32) pileup status, [32..32+cap) candidates
-    const size_t rb_seg = RB_EXTRA + 4 * (32 + (size_t)cap);
-    const size_t rb_calls = rb_seg + ((4 * (2 * (size_t)cap + 2) + 15) & ~(size_t)15);         // seg_count, then pair_any
-    const size_t rb_fixed = rb_calls + sizeof(tc_insert_call_t) * (size_t)cap;
-    const size_t rb_bytes = rb_fixed + (size_t)cap * INS_BASES_FIXED;
-    if (rb_bytes > TC_HOST_SCRATCH) return tc_fail(ctx, TC_ERR_ARG, "candidate capacity %d too large for the pinned results block", cap);
-    uint8_t* d_rb = (uint8_t*)tc_dev_buf(ctx, SLOT_INS_E, rb_bytes + 16);
+    const ins_block rb = ins_block_of(cap, true);
+    if (rb.bytes > TC_HOST_SCRATCH) return tc_fail(ctx, TC_ERR_ARG, "candidate capacity %d too large for the pinned results block", cap);
+    uint8_t* d_rb = (uint8_t*)tc_dev_buf(ctx, SLOT_INS_E, rb.bytes + 16);
     int32_t* d_range = (int32_t*)tc_dev_buf(ctx, SLOT_INS_B, 24 * (size_t)cap);
     if (!d_rb || !d_range) return TC_ERR_NOMEM;
-    TC_CUDA(cudaMemsetAsync(d_rb, 0, rb_calls, s));
+    TC_CUDA(cudaMemsetAsync(d_rb, 0, rb.calls, s));
     a.span_hint = reads->max_ref_span > 0 ? reads->max_ref_span : 0;
     a.status = (tc_status*)d_rb;
     if (a.span_hint == 0 && n > 0) {
@@ -1066,49 +1111,15 @@ int tc_inserts_enqueue_dev(tc_ctx* ctx, const tc_reads_t* reads, const int32_t* 
         TC_LAUNCH_CHECK();
     }
     a.cand = d_cand; a.n_cand = cap; a.n_cand_dev = d_ncand; a.range = d_range; a.range_off = (uint32_t*)(d_range + 2 * (size_t)cap);
-    a.flag_filter = p->flag_filter; a.min_mapq = p->min_mapq; a.min_bq = p->min_base_quality; a.ignore_orphans = p->ignore_orphans;
-    a.olap_mode = (p->reserved >> 8) & 3;
-    a.max_depth = p->max_depth > 0 ? p->max_depth : (1ll << 62);
     cand_range_kernel<<<(cap + 3) / 4, 128, 0, s>>>(a);
     TC_LAUNCH_CHECK();
     if (ctx->ins_slot_cap <= 0) ctx->ins_slot_cap = 1 << 16;
     const size_t T = (size_t)ctx->ins_slot_cap, NT = T / INS_TILE + (size_t)cap + 1;
-    const size_t bytes = T * (8 + 4 + 4 + 1 + 1 + 1) + NT * 12 + ((size_t)cap + 1) * 16 + 256 + 16;
-    uint8_t* slab = (uint8_t*)tc_dev_buf(ctx, SLOT_INS_D, bytes);
-    if (!slab) return TC_ERR_NOMEM;
-    uint64_t* d_key = (uint64_t*)slab;
-    int64_t* d_off = (int64_t*)(d_key + T);
-    a.ent_indel = (int32_t*)(d_off + cap + 1); a.ent_qpos = a.ent_indel + T;
-    int32_t* d_tcand = a.ent_qpos + T; int32_t* d_tfirst = d_tcand + NT;
-    a.tile_sel = d_tfirst + cap + 1; a.tile_last = a.tile_sel + NT;
-    a.seg_count = (int32_t*)(d_rb + rb_seg); a.pair_any = a.seg_count + cap + 1; a.overflow = (int32_t*)(d_rb + RB_OVER);
-    if (ctx->pair_cap <= 0) ctx->pair_cap = 1 << 22;
-    a.pair_bump = (unsigned long long*)(d_rb + 88); a.pair_cap = (unsigned long long)ctx->pair_cap;
-    a.pair_q = (uint8_t*)tc_dev_buf(ctx, SLOT_INS_F, (size_t)ctx->pair_cap);
-    if (!a.pair_q) return TC_ERR_NOMEM;
-    int32_t* d_layout = (int32_t*)(d_rb + RB_LAYOUT);
-    a.ent_head = (uint8_t*)(a.tile_last + NT); a.ent_sel = a.ent_head + T; a.ent_q = a.ent_sel + T; a.bases_fixed = d_rb + rb_fixed;
-    a.ent_key = d_key; a.seg_off = d_off; a.tile_cand = d_tcand; a.tile_first = d_tfirst; a.layout = d_layout;
-    ins_layout_kernel<<<1, 256, 0, s>>>(a, d_off, d_tfirst, d_tcand, d_layout, (int64_t)T, (int)NT, d_pileup_status, (int32_t*)(d_rb + RB_EXTRA));
-    TC_LAUNCH_CHECK();
-    if (n > 0) {
-        ins_select_kernel<<<(unsigned)NT, INS_TILE, 0, s>>>(a);
-        TC_LAUNCH_CHECK();
-        ins_admit_kernel<<<(unsigned)NT, INS_TILE, 0, s>>>(a);
-        TC_LAUNCH_CHECK();
-        if (a.min_bq > 0) { rc = launch_pair(ctx, a, cap, s); if (rc) return rc; }
-        const size_t tbl_smem = (size_t)INS_TBL * 16;
-        if (!(ctx->ins_attr_set & 1)) {
-            TC_CUDA(cudaFuncSetAttribute(ins_count_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tbl_smem));
-            ctx->ins_attr_set |= 1;
-        }
-        ins_count_kernel<<<cap, 1024, tbl_smem, s>>>(a, (tc_insert_call_t*)(d_rb + rb_calls));
-        TC_LAUNCH_CHECK();
-    }
-    TC_CUDA(cudaMemcpyAsync(host_block, d_rb, rb_bytes, cudaMemcpyDeviceToHost, s));
-    ctx->d2h_bytes += (int64_t)rb_bytes;
-    pend->rb_extra = RB_EXTRA; pend->rb_layout = RB_LAYOUT; pend->rb_over = RB_OVER; pend->rb_calls = rb_calls; pend->rb_fixed = rb_fixed;
-    pend->cap = cap; pend->n_reads = n;
+    if ((rc = ins_bind(ctx, a, d_rb, rb, T, NT, cap, p)) || (rc = ins_layout_dev(ctx, a, d_rb, rb, T, NT, d_pileup_status, s))) return rc;
+    if (n > 0 && (rc = ins_enqueue_count(ctx, a, (unsigned)NT, cap, (tc_insert_call_t*)(d_rb + rb.calls), s))) return rc;
+    TC_CUDA(cudaMemcpyAsync(host_block, d_rb, rb.bytes, cudaMemcpyDeviceToHost, s));
+    ctx->d2h_bytes += (int64_t)rb.bytes;
+    pend->rb = rb; pend->cap = cap; pend->n_reads = n;
     return TC_OK;
 }
 
@@ -1117,32 +1128,25 @@ int tc_inserts_enqueue_dev(tc_ctx* ctx, const tc_reads_t* reads, const int32_t* 
 int tc_inserts_finish_dev(tc_ctx* ctx, const tc_ins_pending* pend, const void* host_block, tc_status* pileup_status, int32_t* cands, int32_t* n_cand,
                           tc_insert_call_t* calls, uint8_t* bases, int64_t bases_cap, int* fit) {
     const uint8_t* pin = (const uint8_t*)host_block;
-    const int32_t* extra = (const int32_t*)(pin + pend->rb_extra);
+    const ins_block& rb = pend->rb;
+    const int32_t* extra = (const int32_t*)(pin + rb.extra);
     tc_status st; memcpy(&st, pin, sizeof(st));
-    memcpy(pileup_status, extra + 16, sizeof(tc_status));
-    int32_t layout[3]; memcpy(layout, pin + pend->rb_layout, 12);
-    int32_t over; memcpy(&over, pin + pend->rb_over, 4);
-    const int n = extra[0];
+    memcpy(pileup_status, extra + TC_RB_EXTRA_STATUS, sizeof(tc_status));
+    int32_t layout[3]; memcpy(layout, pin + rb.layout, 12);
+    int32_t over; memcpy(&over, pin + rb.over, 4);
+    const int n = extra[TC_RB_EXTRA_NCAND];
     *n_cand = n;
     *fit = 1;
     if (n > pend->cap) { *fit = 0; return TC_OK; }
-    memcpy(cands, extra + 32, 4 * (size_t)n);
+    memcpy(cands, extra + TC_RB_EXTRA_CAND, 4 * (size_t)n);
     if (layout[2]) { ctx->ins_slot_cap = 2 * (int64_t)layout[1] + 4096; *fit = 0; return TC_OK; }
-    if (over & 2) { unsigned long long bump; memcpy(&bump, pin + 88, 8); ctx->pair_cap = 2 * (int64_t)bump + 4096; }
+    if (over & 2) { unsigned long long bump; memcpy(&bump, pin + rb.bump, 8); ctx->pair_cap = 2 * (int64_t)bump + 4096; }
     if (over) { *fit = 0; return TC_OK; }
-    if (st.err == TC_ERR_UNSORTED) return tc_fail(ctx, TC_ERR_UNSORTED, "Unsorted input. Pileup aborts");
-    if (st.err) return tc_fail(ctx, st.err, "insertion key collision or device-side failure %d", st.err);
-    memcpy(calls, pin + pend->rb_calls, sizeof(tc_insert_call_t) * (size_t)n);
-    int64_t need = 0;
+    if (const int rc = ins_check_status(ctx, st)) return rc;
+    memcpy(calls, pin + rb.calls, sizeof(tc_insert_call_t) * (size_t)n);
     for (int i = 0; i < n; ++i) {
         if (pend->n_reads == 0) { calls[i].pos = cands[i]; calls[i].n_entries = 0; calls[i].mode_count = 0; calls[i].first_read = -1; calls[i].head = 0; calls[i].indel = 0; }
         if (calls[i].indel > INS_BASES_FIXED) { *fit = 0; return TC_OK; }       // rare: the separate call fetches long insertions
-        if (calls[i].indel > 0) { calls[i].bases_off = need; need += calls[i].indel; } else calls[i].bases_off = -1;
     }
-    if (need > 0) {
-        if (!bases || need > bases_cap) return tc_fail(ctx, TC_ERR_CAPACITY, "bases buffer too small: need %lld bytes", (long long)need);
-        for (int i = 0; i < n; ++i)
-            if (calls[i].indel > 0) memcpy(bases + calls[i].bases_off, pin + pend->rb_fixed + (size_t)i * INS_BASES_FIXED, (size_t)calls[i].indel);
-    }
-    return TC_OK;
+    return ins_place_bases(ctx, calls, n, pin + rb.fixed, bases, bases_cap);
 }

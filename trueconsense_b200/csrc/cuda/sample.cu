@@ -21,6 +21,56 @@ bool tc_reads_all_device(const tc_reads_t* r) {
            (!r->n_cigar_ops || tc_is_device_ptr(r->cigar)) && (!r->mapq || tc_is_device_ptr(r->mapq));
 }
 
+void tc_graph_destroy(tc_graph_cache& g) {
+    if (g.exec) cudaGraphExecDestroy(g.exec);
+    g.exec = nullptr;
+}
+
+int tc_graph_run(tc_ctx* ctx, tc_graph_cache& g, const unsigned char* key, int key_len, bool can_capture,
+                 const std::function<int(cudaStream_t)>& chain, cudaStream_t s) {
+    const bool same = g.key_len == key_len && memcmp(g.key, key, (size_t)key_len) == 0;
+    if (!same) {
+        tc_graph_destroy(g);
+        memcpy(g.key, key, (size_t)key_len); g.key_len = key_len; g.seen = 0;
+    }
+    if (same && g.exec) {
+        // the same chain with the same buffers again: replay
+        TC_CUDA(cudaGraphLaunch(g.exec, s));
+        ctx->launches += g.g_launches; ctx->d2h_bytes += g.g_d2h;
+        return TC_OK;
+    }
+    if (!same || g.seen < 1 || !can_capture || getenv("TC_NO_GRAPH")) {
+        const int rc = chain(s);
+        if (rc) return rc;
+        g.seen++;
+        return TC_OK;
+    }
+    // second time: every buffer exists (the eager run allocated them) — capture the chain and launch it as a graph
+    if (!ctx->cap_stream) TC_CUDA(cudaStreamCreateWithFlags(&ctx->cap_stream, cudaStreamNonBlocking));
+    const int64_t l0 = ctx->launches, d0 = ctx->d2h_bytes, epoch0 = ctx->buf_epoch;
+    TC_CUDA(cudaStreamBeginCapture(ctx->cap_stream, cudaStreamCaptureModeRelaxed));
+    ctx->in_capture = 1;
+    int rc = chain(ctx->cap_stream);
+    ctx->in_capture = 0;
+    cudaGraph_t graph = nullptr;
+    const cudaError_t ce = cudaStreamEndCapture(ctx->cap_stream, &graph);
+    if (rc == TC_OK && ce == cudaSuccess && graph && ctx->buf_epoch == epoch0) {
+        const cudaError_t ie = cudaGraphInstantiate(&g.exec, graph, 0);
+        cudaGraphDestroy(graph);
+        if (ie != cudaSuccess) { g.exec = nullptr; return tc_cuda_fail(ctx, ie, "cudaGraphInstantiate"); }
+        g.g_launches = ctx->launches - l0; g.g_d2h = ctx->d2h_bytes - d0;
+        TC_CUDA(cudaGraphLaunch(g.exec, s));
+        return TC_OK;
+    }
+    // something in the chain could not be captured (or a buffer grew): run it eagerly, try again next time
+    if (graph) cudaGraphDestroy(graph);
+    cudaGetLastError();
+    ctx->launches = l0; ctx->d2h_bytes = d0;
+    if (rc && rc != TC_ERR_CUDA) return rc;
+    g.key_len = 0;
+    return chain(s);
+}
+
 // the separate entry points in sequence (any input the chained form does not take)
 static int sample_unchained(tc_ctx* ctx, const tc_reads_t* reads, int32_t L, const tc_pileup_params_t* pp, const tc_call_params_t* cp,
                             const tc_pileup_params_t* ip, int32_t* counts, const tc_call_table_t* table, bool pileup_done,
@@ -57,7 +107,7 @@ void tc_sample_slots_free(tc_ctx* ctx) {
     for (int i = 0; i < 2; ++i) {
         if (ctx->samples[i].host_block) cudaFreeHost(ctx->samples[i].host_block);
         if (ctx->samples[i].done) { cudaEventDestroy(ctx->samples[i].done); cudaEventDestroy(ctx->samples[i].t0); cudaEventDestroy(ctx->samples[i].t1); }
-        if (ctx->samples[i].exec) cudaGraphExecDestroy(ctx->samples[i].exec);
+        tc_graph_destroy(ctx->samples[i].graph);
     }
     free(ctx->samples);
     ctx->samples = nullptr;
@@ -116,46 +166,8 @@ TC_API int tc_sample_enqueue(tc_ctx_t* ctx, const tc_reads_t* reads, int32_t ref
     } else {
         unsigned char key[512];
         const int key_len = sample_key(ctx, reads, ref_len, pp, cp, ip, counts, table, key);
-        const bool same = sl.key_len == key_len && memcmp(sl.key, key, (size_t)key_len) == 0;
-        if (!same) {
-            if (sl.exec) { cudaGraphExecDestroy(sl.exec); sl.exec = nullptr; }
-            memcpy(sl.key, key, (size_t)key_len); sl.key_len = key_len; sl.key_seen = 0;
-        }
-        if (same && sl.exec) {
-            // the same sample shape with the same buffers again: replay
-            TC_CUDA(cudaGraphLaunch(sl.exec, s));
-            ctx->launches += sl.g_launches; ctx->d2h_bytes += sl.g_d2h;
-        } else if (same && sl.key_seen >= 1 && !getenv("TC_NO_GRAPH")) {
-            // second time: every buffer exists (the eager run allocated them) — capture the chain and launch it as a graph
-            if (!ctx->cap_stream) TC_CUDA(cudaStreamCreateWithFlags(&ctx->cap_stream, cudaStreamNonBlocking));
-            const int64_t l0 = ctx->launches, d0 = ctx->d2h_bytes, epoch0 = ctx->buf_epoch;
-            TC_CUDA(cudaStreamBeginCapture(ctx->cap_stream, cudaStreamCaptureModeRelaxed));
-            ctx->in_capture = 1;
-            rc = sample_enqueue_chain(ctx, sl, ctx->cap_stream);
-            ctx->in_capture = 0;
-            cudaGraph_t graph = nullptr;
-            const cudaError_t ce = cudaStreamEndCapture(ctx->cap_stream, &graph);
-            if (rc == TC_OK && ce == cudaSuccess && graph && ctx->buf_epoch == epoch0) {
-                const cudaError_t ie = cudaGraphInstantiate(&sl.exec, graph, 0);
-                cudaGraphDestroy(graph);
-                if (ie != cudaSuccess) { sl.exec = nullptr; return tc_cuda_fail(ctx, ie, "cudaGraphInstantiate"); }
-                sl.g_launches = ctx->launches - l0; sl.g_d2h = ctx->d2h_bytes - d0;
-                TC_CUDA(cudaGraphLaunch(sl.exec, s));
-            } else {
-                // something in the chain could not be captured (or a buffer grew): run it eagerly, try again next time
-                if (graph) cudaGraphDestroy(graph);
-                cudaGetLastError();
-                ctx->launches = l0; ctx->d2h_bytes = d0;
-                if (rc && rc != TC_ERR_CUDA) return rc;
-                sl.key_len = 0;
-                rc = sample_enqueue_chain(ctx, sl, s);
-                if (rc) return rc;
-            }
-        } else {
-            rc = sample_enqueue_chain(ctx, sl, s);
-            if (rc) return rc;
-            sl.key_seen++;
-        }
+        rc = tc_graph_run(ctx, sl.graph, key, key_len, true, [&](cudaStream_t cs) { return sample_enqueue_chain(ctx, sl, cs); }, s);
+        if (rc) return rc;
         TC_CUDA(cudaEventRecord(sl.done, s));
         sl.state = 1;
     }

@@ -7,6 +7,8 @@
 #include <stdio.h>
 #include <string.h>
 
+#include <functional>
+
 #include "trueconsense_b200.h"
 
 #define TC_API extern "C" __attribute__((visibility("default")))
@@ -126,11 +128,34 @@ int tc_pileup_finish(tc_ctx* ctx, const tc_status& st, const tc_pileup_pending* 
 int tc_h2d(tc_ctx* ctx, void* d, const void* p, size_t bytes, cudaStream_t s);
 bool tc_reads_all_device(const tc_reads_t* r);     // every array of the batch already in device memory
 int tc_candidates_enqueue(tc_ctx* ctx, const uint8_t* d_flags, int32_t ref_len, int32_t cap, int32_t** d_count, int32_t** d_sorted, cudaStream_t s);
-struct tc_ins_pending { size_t rb_extra, rb_layout, rb_over, rb_calls, rb_fixed; int cap; int64_t n_reads; };
+// ExtractInserts' results block: one memset in front, one copy back.  Offsets in bytes; ins_block_of (inserts.cu) lays it out.
+struct ins_block {
+    size_t layout;      // int32[3] device-built layout: tiles, slots, 1 = did not fit
+    size_t over;        // int32 overflow flags: 1 a column needs the sorted form, 2 the pair scratch was too small
+    size_t bump;        // uint64 pair-scratch bump
+    size_t extra;       // chained form only (else 0): candidate count, pileup status, candidates (TC_RB_EXTRA_*)
+    size_t seg;         // int32 seg_count[n_cand + 1], then pair_any[n_cand + 1]
+    size_t calls;       // tc_insert_call_t[n_cand]
+    size_t fixed;       // uint8[n_cand][INS_BASES_FIXED] inserted characters of each winner
+    size_t bytes;       // the whole block
+};
+// int32 words of the chained form's extra section
+constexpr int TC_RB_EXTRA_NCAND = 0, TC_RB_EXTRA_STATUS = 16, TC_RB_EXTRA_CAND = 32;
+struct tc_ins_pending { ins_block rb; int cap; int64_t n_reads; };
 int tc_inserts_enqueue_dev(tc_ctx* ctx, const tc_reads_t* reads, const int32_t* d_cand, const int32_t* d_ncand, int cap,
                            const tc_pileup_params_t* p, const tc_status* d_pileup_status, void* host_block, cudaStream_t s, tc_ins_pending* pend);
 int tc_inserts_finish_dev(tc_ctx* ctx, const tc_ins_pending* pend, const void* host_block, tc_status* pileup_status, int32_t* cands, int32_t* n_cand,
                           tc_insert_call_t* calls, uint8_t* bases, int64_t bases_cap, int* fit);
+// A chain of enqueues as a CUDA graph, keyed by everything it depends on: the first run with a key is eager (and
+// allocates), the second is captured (when can_capture and TC_NO_GRAPH is unset), later ones replay.  A failed capture
+// runs the chain eagerly and tries again next time.
+struct tc_graph_cache {
+    unsigned char key[512]; int key_len, seen;
+    cudaGraphExec_t exec; int64_t g_launches, g_d2h;        // what one replay adds to the context's counters
+};
+int tc_graph_run(tc_ctx* ctx, tc_graph_cache& g, const unsigned char* key, int key_len, bool can_capture,
+                 const std::function<int(cudaStream_t)>& chain, cudaStream_t s);
+void tc_graph_destroy(tc_graph_cache& g);
 // a sample in flight
 struct tc_sample_slot {
     int state;                      // 0 free, 1 chained and enqueued, 2 to be run through the separate calls at finish time
@@ -139,10 +164,7 @@ struct tc_sample_slot {
     int timed;
     tc_reads_t reads; int32_t ref_len; tc_pileup_params_t pp, ip; tc_call_params_t cp; int32_t* counts; tc_call_table_t table; void* stream;
     tc_pileup_pending pend; tc_ins_pending ipend;
-    // the sample's enqueue as a CUDA graph: the first enqueue with a key runs eagerly (and allocates), the second is captured,
-    // later ones replay — one launch per sample instead of ~25 (kernels, memsets, the results copy)
-    unsigned char key[512]; int key_len; int key_seen;
-    cudaGraphExec_t exec; int64_t g_launches, g_d2h;
+    tc_graph_cache graph;           // one launch per sample instead of ~25 (kernels, memsets, the results copy)
 };
 
 // ---------------------------------------------------------------- device helpers

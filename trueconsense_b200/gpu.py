@@ -576,20 +576,7 @@ class Context:
                 cap *= 16
                 continue
             self._check(rc)
-            break
-        out = []
-        for c in calls:
-            if c.n_entries == 0:
-                out.append({"pos": c.pos, "n_entries": 0, "string": None, "mode_count": 0, "first_read": -1})
-                continue
-            s = chr(c.head)
-            if c.indel > 0:
-                s += f"+{c.indel}" + bytes(bases[c.bases_off:c.bases_off + c.indel]).decode("ascii")
-            elif c.indel < 0:
-                s += f"-{-c.indel}" + "N" * (-c.indel)
-            out.append({"pos": c.pos, "n_entries": c.n_entries, "string": s, "mode_count": c.mode_count,
-                        "first_read": c.first_read})
-        return out
+            return self._insert_dicts(calls, n, bases)
 
 
 _default_ctx: dict[int, Context] = {}
