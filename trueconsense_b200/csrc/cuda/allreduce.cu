@@ -156,7 +156,7 @@ TC_API int tc_pileup_counts_allreduce_finish(tc_ctx_t* ctx, int32_t ticket) {
         if (prc) { memcpy(ctx->err, keep, sizeof(keep)); return prc; }
         return arc;
     }
-    return tc_pileup_finish(ctx, h.st, &sl.pend, &sl.reads, L, &sl.p, sl.counts, sl.stream);
+    return tc_pileup_settle(ctx, h.st, sl.pend, &sl.reads, L, &sl.p, sl.counts, s, nullptr);
 }
 
 TC_API int tc_pileup_counts_allreduce(tc_ctx_t* ctx, const tc_reads_t* reads, int32_t ref_len, const tc_pileup_params_t* p,

@@ -239,6 +239,21 @@ static void launch_depth_diff(const pileup_args& a, int64_t n_cigar_ops, cudaStr
     else depth_diff_kernel<<<(unsigned)((a.r.n + 255) / 256), 256, 0, s>>>(a);
 }
 
+template <bool PER_ENTRY_COV>
+static int launch_scatter(tc_ctx* ctx, const pileup_args& a, cudaStream_t s) {
+    const int n_chunks = (int)((a.r.n + SC_CHUNK - 1) / SC_CHUNK);
+    const size_t smem = sizeof(int32_t) * SC_ROWS * SC_W;
+    TC_CUDA(cudaFuncSetAttribute(pileup_scatter_kernel<PER_ENTRY_COV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    pileup_scatter_kernel<PER_ENTRY_COV><<<min(n_chunks, ctx->sm_count * 3), SC_THREADS, smem, s>>>(a, n_chunks);
+    TC_LAUNCH_CHECK();
+    return TC_OK;
+}
+
+// timing on: the events around the pileup kernel (inside a graph capture they become external event nodes)
+static cudaError_t timing_event(tc_ctx* ctx, cudaEvent_t e, cudaStream_t s) {
+    return ctx->timing ? cudaEventRecordWithFlags(e, s, ctx->in_capture ? cudaEventRecordExternal : cudaEventRecordDefault) : cudaSuccess;
+}
+
 static int fetch_status(tc_ctx* ctx, tc_status* d_status, tc_status* out, cudaStream_t s) {
     TC_D2H(ctx->host_status, d_status, sizeof(tc_status), s);
     TC_CUDA(cudaStreamSynchronize(s));
@@ -266,112 +281,110 @@ static int check_common(tc_ctx* ctx, const tc_reads_t* reads, int32_t ref_len, c
     return TC_OK;
 }
 
-// Everything of tc_pileup_counts up to (not including) the read-back of the status block: memsets, the span pass if one is
-// needed, the pileup kernel, the coverage scan.  `counts` may be a host pointer (the table is then built in a context buffer).
-int tc_pileup_enqueue(tc_ctx* ctx, const tc_reads_t* reads, int32_t ref_len, const tc_pileup_params_t* p, int32_t* counts, cudaStream_t s,
-                      tc_pileup_pending* pend) {
-    const int L = ref_len;
-    pileup_args a;
-    int rc = tc_resolve_reads(ctx, reads, &a.r, p->min_base_quality > 0 ? NEED_QUAL : 0, s);
-    if (rc) return rc;
-    const bool out_dev = tc_is_device_ptr(counts);
-    int32_t* d_counts = out_dev ? counts : (int32_t*)tc_dev_buf(ctx, SLOT_COUNTS, sizeof(int32_t) * TC_NROWS * (size_t)L);
-    // one buffer, one memset: the status block, the coverage difference array and, behind it, variant 3's packed X | I event counters
-    const size_t diff_words = ((size_t)L + 2) & ~(size_t)1;
-    const size_t head_words = 16;                   // tc_status
-    static_assert(sizeof(tc_status) == 64, "tc_status is 16 words");
-    int32_t* d_head = (int32_t*)tc_dev_buf(ctx, SLOT_DIFF, sizeof(int32_t) * (head_words + diff_words) + 8 * ((size_t)L + 1));
-    if (!d_counts || !d_head) return TC_ERR_NOMEM;
-    tc_status* d_status = (tc_status*)d_head;
-    int32_t* d_diff = d_head + head_words;
-    TC_CUDA(cudaMemsetAsync(d_counts, 0, sizeof(int32_t) * TC_NROWS * (size_t)L, s));
-    TC_CUDA(cudaMemsetAsync(d_head, 0, sizeof(int32_t) * (head_words + diff_words) + 8 * ((size_t)L + 1), s));
-    a.xi = (unsigned long long*)(d_diff + diff_words);
-    a.L = L; a.flag_filter = p->flag_filter; a.min_mapq = p->min_mapq; a.min_bq = p->min_base_quality;
-    a.ignore_orphans = p->ignore_orphans; a.counts = d_counts; a.diff = d_diff; a.status = d_status;
-    a.span_hint = reads->max_ref_span > 0 ? reads->max_ref_span : 0;
-    a.span_out = nullptr;
-    const bool per_entry = p->min_base_quality > 0;
-    int variant = p->kernel;
-    // reads longer than variant 3's widest window are cut into pieces first (variant 4, pileup_long.cu)
-    const int LONG_SPAN = 1024 - 8 - 64;
-    if (variant == 0) variant = (!per_entry && tc_pileup_warp_supported(a)) ? (a.span_hint > LONG_SPAN ? 4 : 3) : 1;
-    if (variant != 1 && variant != 3 && variant != 4) return tc_fail(ctx, TC_ERR_ARG, "unknown pileup kernel variant %d", variant);
-    if (variant != 1 && per_entry) return tc_fail(ctx, TC_ERR_ARG, "the bit-parallel kernels have no base-quality filter; use kernel=1");
-    if (variant != 1 && !tc_pileup_warp_supported(a)) return tc_fail(ctx, TC_ERR_ARG, "the bit-parallel kernels need 16-byte aligned seq4 / cigar arrays; use kernel=1");
-    const bool is_long = variant == 4;      // long reads cut into pieces, the pieces piled up by variant 3
-    const bool direct = variant == 3;
-    pend->span_hint = a.span_hint;
-    if (a.r.n > 0) {
-        if (ctx->timing) TC_CUDA(cudaEventRecordWithFlags(ctx->ev0, s, ctx->in_capture ? cudaEventRecordExternal : cudaEventRecordDefault));
-        if (variant != 1) {
-            // coverage ends, span statistics and the sortedness / range checks: one thread per read — unless the
-            // caller bounded the longest span, then variant 3 does all of that while it walks the CIGARs anyway
-            if (!direct || a.span_hint == 0 || a.span_hint > LONG_SPAN) {
-                a.span_hint = 0;
-                if (is_long) {         // the long-read split needs every read's span: one walk over the CIGARs serves both
-                    a.span_out = (int32_t*)tc_dev_buf(ctx, SLOT_SPAN_END, sizeof(int32_t) * (size_t)a.r.n);
-                    if (!a.span_out) return TC_ERR_NOMEM;
-                }
-                launch_depth_diff(a, reads->n_cigar_ops, s);
-                TC_LAUNCH_CHECK();
-            }
-            pend->span_hint = a.span_hint;
-            a.pieces = nullptr; a.piece_order = nullptr; a.n_pieces = 0;
-            rc = is_long ? tc_pileup_long_launch(ctx, a, s) : tc_pileup_warp_launch(ctx, a, s);
-            if (rc) return rc;
-        } else {
-            int n_chunks = (int)((a.r.n + SC_CHUNK - 1) / SC_CHUNK);
-            int grid = min(n_chunks, ctx->sm_count * 3);
-            size_t smem = sizeof(int32_t) * SC_ROWS * SC_W;
-            if (per_entry) {
-                TC_CUDA(cudaFuncSetAttribute(pileup_scatter_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                pileup_scatter_kernel<true><<<grid, SC_THREADS, smem, s>>>(a, n_chunks);
-            } else {
-                TC_CUDA(cudaFuncSetAttribute(pileup_scatter_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                pileup_scatter_kernel<false><<<grid, SC_THREADS, smem, s>>>(a, n_chunks);
-            }
-            TC_LAUNCH_CHECK();
-        }
-        if (ctx->timing) { TC_CUDA(cudaEventRecordWithFlags(ctx->ev1, s, ctx->in_capture ? cudaEventRecordExternal : cudaEventRecordDefault)); ctx->ev_valid = 1; }
-    }
-    if (!per_entry) {
-        rc = coverage_scan(ctx, d_diff, d_counts, L, d_status, variant != 1 ? a.xi : nullptr, s);
-        if (rc) return rc;
-    }
-    pend->d_status = d_status; pend->d_counts = d_counts; pend->variant = variant; pend->per_entry = per_entry ? 1 : 0;
-    pend->out_dev = out_dev ? 1 : 0; pend->n_reads = a.r.n;
+// A pass's filters, and its status block and coverage difference array [L + 1] in one buffer under one memset.  with_xi (the
+// pileup): behind them the packed X | I event counters of variants 3 / 4, one 64-bit word per column.
+static int init_pass(tc_ctx* ctx, const tc_pileup_params_t* p, int32_t L, bool with_xi, cudaStream_t s, pileup_args& a) {
+    const size_t diff_words = ((size_t)L + 2) & ~(size_t)1;        // keeps the X | I words 8-byte aligned
+    const size_t bytes = sizeof(tc_status) + sizeof(int32_t) * diff_words + (with_xi ? 8 * ((size_t)L + 1) : 0);
+    uint8_t* head = (uint8_t*)tc_dev_buf(ctx, SLOT_DIFF, bytes);
+    if (!head) return TC_ERR_NOMEM;
+    TC_CUDA(cudaMemsetAsync(head, 0, bytes, s));
+    a.status = (tc_status*)head;
+    a.diff = (int32_t*)(head + sizeof(tc_status));
+    a.xi = with_xi ? (unsigned long long*)(a.diff + diff_words) : nullptr;
+    a.L = L; a.flag_filter = p->flag_filter; a.min_mapq = p->min_mapq; a.min_bq = p->min_base_quality; a.ignore_orphans = p->ignore_orphans;
     return TC_OK;
 }
 
-// The host side of tc_pileup_counts once the status block has come back: errors, the depth-cap proof, and the re-run
-// through another kernel variant when the bit-parallel kernel declined the batch.
-int tc_pileup_finish(tc_ctx* ctx, const tc_status& st_in, const tc_pileup_pending* pend, const tc_reads_t* reads, int32_t ref_len,
-                     const tc_pileup_params_t* p, int32_t* counts, void* stream) {
-    tc_status st = st_in;
-    const int variant = pend->variant;
-    const int LONG_SPAN = 1024 - 8 - 64;
-    if (st.err == TC_ERR_CAPACITY && variant != 1 && p->kernel == 0) {
-        // reads spanning more than variant 3's window: cut them into pieces (variant 4); anything else the bit-parallel
-        // kernels decline (pads in long reads, a single read beyond the staging buffers): the scatter kernel
-        tc_pileup_params_t q = *p;
-        q.kernel = (variant == 3 && pend->span_hint == 0 && st.max_span > LONG_SPAN) ? 4 : 1;
-        if (q.kernel == 4) {
-            const int rc4 = tc_pileup_counts(ctx, reads, ref_len, &q, counts, stream);
-            if (rc4 != TC_ERR_CAPACITY) return rc4;
-            q.kernel = 1;
+// The plan of one attempt.  rung 0: p->kernel, and for 0 the scatter kernel under a base-quality filter or with seq4 / cigar not
+// 16-byte aligned, else variant 4 when the caller's span bound fits no window of variant 3, else variant 3.  rung 3 / 4 / 1 (the
+// fallback ladder, tc_pileup_settle): that variant.  Coverage ends, span statistics and the sortedness / range checks take a span
+// pass, one thread per read, unless variant 3 does them while it walks the CIGARs (the caller's bound fits its windows).
+static int pileup_plan_of(tc_ctx* ctx, const tc_pileup_params_t* p, const pileup_args& a, int rung, pileup_plan* plan) {
+    const bool per_entry = p->min_base_quality > 0, fits = a.span_hint > 0 && warp_geometry(a.span_hint) != 0;
+    int v = rung ? rung : p->kernel;
+    if (v == 0) v = (per_entry || !tc_pileup_warp_supported(a)) ? 1 : (a.span_hint > 0 && !fits) ? 4 : 3;
+    if (v != 1 && v != 3 && v != 4) return tc_fail(ctx, TC_ERR_ARG, "unknown pileup kernel variant %d", v);
+    if (v != 1 && per_entry) return tc_fail(ctx, TC_ERR_ARG, "the bit-parallel kernels have no base-quality filter; use kernel=1");
+    if (v != 1 && !tc_pileup_warp_supported(a)) return tc_fail(ctx, TC_ERR_ARG, "the bit-parallel kernels need 16-byte aligned seq4 / cigar arrays; use kernel=1");
+    *plan = {v, v == 4 || (v == 3 && !fits), v == 4};
+    return TC_OK;
+}
+
+// Everything of one attempt up to (not including) the read-back of the status block: memsets, the span pass if the plan has
+// one, the pileup kernel, the coverage scan.  `counts` may be a host pointer (the table is then built in a context buffer).
+int tc_pileup_enqueue(tc_ctx* ctx, const tc_reads_t* reads, int32_t L, const tc_pileup_params_t* p, int32_t* counts, cudaStream_t s,
+                      tc_pileup_pending* pend, int rung) {
+    const bool per_entry = p->min_base_quality > 0;
+    pileup_args a = {};
+    int rc = tc_resolve_reads(ctx, reads, &a.r, per_entry ? NEED_QUAL : 0, s);
+    if (rc) return rc;
+    const bool out_dev = tc_is_device_ptr(counts);
+    int32_t* d_counts = out_dev ? counts : (int32_t*)tc_dev_buf(ctx, SLOT_COUNTS, sizeof(int32_t) * TC_NROWS * (size_t)L);
+    if (!d_counts) return TC_ERR_NOMEM;
+    TC_CUDA(cudaMemsetAsync(d_counts, 0, sizeof(int32_t) * TC_NROWS * (size_t)L, s));
+    rc = init_pass(ctx, p, L, true, s, a);
+    if (rc) return rc;
+    a.counts = d_counts;
+    a.span_hint = reads->max_ref_span > 0 ? reads->max_ref_span : 0;
+    pileup_plan plan;
+    rc = pileup_plan_of(ctx, p, a, rung, &plan);
+    if (rc) return rc;
+    if (a.r.n > 0) {
+        TC_CUDA(timing_event(ctx, ctx->ev0, s));
+        if (plan.span_pass) {
+            a.span_hint = 0;        // variant 3 reads the longest span the pass leaves in the status block
+            a.span_out = plan.span_out ? (int32_t*)tc_dev_buf(ctx, SLOT_SPAN_END, sizeof(int32_t) * (size_t)a.r.n) : nullptr;
+            if (plan.span_out && !a.span_out) return TC_ERR_NOMEM;
+            launch_depth_diff(a, reads->n_cigar_ops, s);
+            TC_LAUNCH_CHECK();
         }
-        return tc_pileup_counts(ctx, reads, ref_len, &q, counts, stream);
+        rc = plan.variant == 4 ? tc_pileup_long_launch(ctx, a, s)
+           : plan.variant == 3 ? tc_pileup_warp_launch(ctx, a, s)
+           : per_entry ? launch_scatter<true>(ctx, a, s) : launch_scatter<false>(ctx, a, s);
+        if (rc) return rc;
+        TC_CUDA(timing_event(ctx, ctx->ev1, s));
+        if (ctx->timing) ctx->ev_valid = 1;
+    }
+    rc = per_entry ? TC_OK : coverage_scan(ctx, a.diff, d_counts, L, a.status, plan.variant != 1 ? a.xi : nullptr, s);
+    if (rc) return rc;
+    pend->d_status = a.status; pend->d_counts = d_counts; pend->plan = plan; pend->out_dev = out_dev ? 1 : 0; pend->n_reads = a.r.n;
+    return TC_OK;
+}
+
+// one attempt enqueued and read back: the table when the caller's is on the host, then the status block
+static int pileup_attempt(tc_ctx* ctx, const tc_reads_t* reads, int32_t ref_len, const tc_pileup_params_t* p, int32_t* counts,
+                          cudaStream_t s, int rung, tc_pileup_pending* pend, tc_status* st) {
+    int rc = tc_pileup_enqueue(ctx, reads, ref_len, p, counts, s, pend, rung);
+    if (rc) return rc;
+    if (!pend->out_dev) TC_D2H(counts, pend->d_counts, sizeof(int32_t) * TC_NROWS * (size_t)ref_len, s);
+    return fetch_status(ctx, pend->d_status, st, s);
+}
+
+// The host side of a pileup once its status block has come back.  With kernel == 0 a batch the bit-parallel kernels decline
+// (TC_ERR_CAPACITY) goes down the fallback ladder, each rung enqueued, read back and settled in turn:
+//   3 -> 4   the span pass (no bound was given) found a read too long for every window of variant 3: cut into pieces
+//   3 -> 1   anything else variant 3 declines (pads, zero-length ops, an op of 4096+ bases, a read beyond the staging buffers)
+//   4 -> 1   anything the long-read split or its pieces decline; the scatter kernel (1) carries htslib's full look-ahead state
+// Then, for the attempt that went through: errors, the depth-cap proof and the caller's span bound.
+int tc_pileup_settle(tc_ctx* ctx, tc_status st, tc_pileup_pending pend, const tc_reads_t* reads, int32_t ref_len,
+                     const tc_pileup_params_t* p, int32_t* counts, cudaStream_t s, int* redone) {
+    while (st.err == TC_ERR_CAPACITY && p->kernel == 0 && pend.plan.variant != 1) {
+        const int next = (pend.plan.variant == 3 && pend.plan.span_pass && warp_geometry(st.max_span) == 0) ? 4 : 1;
+        if (redone) *redone = 1;
+        int rc = pileup_attempt(ctx, reads, ref_len, p, counts, s, next, &pend, &st);
+        if (rc == TC_ERR_CAPACITY && next == 4) rc = pileup_attempt(ctx, reads, ref_len, p, counts, s, 1, &pend, &st);   // too many pieces
+        if (rc) return rc;
     }
     if (st.err == TC_ERR_CAPACITY)
         return tc_fail(ctx, TC_ERR_CAPACITY, "a read exceeds the bit-parallel kernels' windows or staging buffers; use kernel=1 (or 0)");
-    if (pend->per_entry) {
+    if (p->min_base_quality > 0) {
         // coverage was counted entry by entry, so max_cov is not the live depth; fall back to the
         // trivial bound (every read live at once)
         st.max_cov = 0;
-        if (p->max_depth > 0 && pend->n_reads + 1 > p->max_depth && st.err == 0)
+        if (p->max_depth > 0 && pend.n_reads + 1 > p->max_depth && st.err == 0)
             return tc_fail(ctx, TC_ERR_DEPTH_CAP, "%lld reads with a base-quality filter: the depth cap %lld may bind and is not emulated by the bulk kernel",
-                           (long long)pend->n_reads, (long long)p->max_depth);
+                           (long long)pend.n_reads, (long long)p->max_depth);
     }
     if (st.err == 0 && reads->max_ref_span > 0 && st.max_span > reads->max_ref_span)
         return tc_fail(ctx, TC_ERR_ARG, "tc_reads_t.max_ref_span = %d but a read spans %d reference columns", reads->max_ref_span, st.max_span);
@@ -390,56 +403,45 @@ TC_API int tc_pileup_counts(tc_ctx_t* ctx, const tc_reads_t* reads, int32_t ref_
     if (rc) return rc;
     cudaStream_t s = (cudaStream_t)stream;
     TC_CUDA(cudaSetDevice(ctx->device));
-    tc_pileup_pending pend;
-    rc = tc_pileup_enqueue(ctx, reads, ref_len, p, counts, s, &pend);
+    tc_pileup_pending pend; tc_status st;
+    rc = pileup_attempt(ctx, reads, ref_len, p, counts, s, 0, &pend, &st);
     if (rc) return rc;
-    tc_status st;
-    if (!pend.out_dev) TC_D2H(counts, pend.d_counts, sizeof(int32_t) * TC_NROWS * (size_t)ref_len, s);
-    rc = fetch_status(ctx, pend.d_status, &st, s);
-    if (rc) return rc;
-    return tc_pileup_finish(ctx, st, &pend, reads, ref_len, p, counts, stream);
+    return tc_pileup_settle(ctx, st, pend, reads, ref_len, p, counts, s, nullptr);
 }
 
-TC_API int tc_depth(tc_ctx_t* ctx, const tc_reads_t* reads, int32_t ref_len, const tc_pileup_params_t* p,
+TC_API int tc_depth(tc_ctx_t* ctx, const tc_reads_t* reads, int32_t L, const tc_pileup_params_t* p,
                     int32_t* depth, void* stream) {
-    int rc = check_common(ctx, reads, ref_len, p, depth);
+    int rc = check_common(ctx, reads, L, p, depth);
     if (rc) return rc;
     if (p->min_base_quality > 0) return tc_fail(ctx, TC_ERR_ARG, "tc_depth counts whole spans; it is only the coverage column when min_base_quality == 0");
     cudaStream_t s = (cudaStream_t)stream;
     TC_CUDA(cudaSetDevice(ctx->device));
-    const int L = ref_len;
-    pileup_args a;
+    pileup_args a = {};
     // the depth pass reads pos, flag, mapq and the CIGARs only
-    tc_reads_t slim = *reads;
     dreads& d = a.r;
-    memset(&d, 0, sizeof(d));
     d.n = reads->n_reads;
     if (d.n > 0) {
-        if (!slim.pos || !slim.flag || !slim.cigar_off || (!slim.cigar && slim.n_cigar_ops)) return tc_fail(ctx, TC_ERR_ARG, "tc_reads_t: a required array is NULL");
-        d.pos = (const int32_t*)tc_stage_in(ctx, SLOT_POS, slim.pos, 4 * (size_t)d.n, s, &rc); if (rc) return rc;
-        d.flag = (const uint16_t*)tc_stage_in(ctx, SLOT_FLAG, slim.flag, 2 * (size_t)d.n, s, &rc); if (rc) return rc;
-        d.cigar_off = (const uint32_t*)tc_stage_in(ctx, SLOT_CIGOFF, slim.cigar_off, 4 * (size_t)(d.n + 1), s, &rc); if (rc) return rc;
-        d.cigar = (const uint32_t*)tc_stage_in(ctx, SLOT_CIGAR, slim.cigar, 4 * (size_t)slim.n_cigar_ops, s, &rc); if (rc) return rc;
-        if (slim.mapq) { d.mapq = (const uint8_t*)tc_stage_in(ctx, SLOT_MAPQ, slim.mapq, (size_t)d.n, s, &rc); if (rc) return rc; }
+        if (!reads->pos || !reads->flag || !reads->cigar_off || (!reads->cigar && reads->n_cigar_ops)) return tc_fail(ctx, TC_ERR_ARG, "tc_reads_t: a required array is NULL");
+        d.pos = (const int32_t*)tc_stage_in(ctx, SLOT_POS, reads->pos, 4 * (size_t)d.n, s, &rc); if (rc) return rc;
+        d.flag = (const uint16_t*)tc_stage_in(ctx, SLOT_FLAG, reads->flag, 2 * (size_t)d.n, s, &rc); if (rc) return rc;
+        d.cigar_off = (const uint32_t*)tc_stage_in(ctx, SLOT_CIGOFF, reads->cigar_off, 4 * (size_t)(d.n + 1), s, &rc); if (rc) return rc;
+        d.cigar = (const uint32_t*)tc_stage_in(ctx, SLOT_CIGAR, reads->cigar, 4 * (size_t)reads->n_cigar_ops, s, &rc); if (rc) return rc;
+        if (reads->mapq) { d.mapq = (const uint8_t*)tc_stage_in(ctx, SLOT_MAPQ, reads->mapq, (size_t)d.n, s, &rc); if (rc) return rc; }
     }
     const bool out_dev = tc_is_device_ptr(depth);
     int32_t* d_depth = out_dev ? depth : (int32_t*)tc_dev_buf(ctx, SLOT_COUNTS, sizeof(int32_t) * (size_t)L);
-    int32_t* d_diff = (int32_t*)tc_dev_buf(ctx, SLOT_DIFF, sizeof(int32_t) * ((size_t)L + 1));
-    tc_status* d_status = (tc_status*)tc_dev_buf(ctx, SLOT_STATUS, sizeof(tc_status));
-    if (!d_depth || !d_diff || !d_status) return TC_ERR_NOMEM;
-    TC_CUDA(cudaMemsetAsync(d_diff, 0, sizeof(int32_t) * ((size_t)L + 1), s));
-    TC_CUDA(cudaMemsetAsync(d_status, 0, sizeof(tc_status), s));
-    a.L = L; a.flag_filter = p->flag_filter; a.min_mapq = p->min_mapq; a.min_bq = 0; a.ignore_orphans = p->ignore_orphans;
-    a.counts = nullptr; a.diff = d_diff; a.status = d_status; a.span_hint = 0; a.span_out = nullptr;
+    if (!d_depth) return TC_ERR_NOMEM;
+    rc = init_pass(ctx, p, L, false, s, a);
+    if (rc) return rc;
     if (d.n > 0) {
         launch_depth_diff(a, reads->n_cigar_ops, s);
         TC_LAUNCH_CHECK();
     }
-    rc = coverage_scan(ctx, d_diff, d_depth, L, d_status, nullptr, s);
+    rc = coverage_scan(ctx, a.diff, d_depth, L, a.status, nullptr, s);
     if (rc) return rc;
     if (!out_dev) TC_D2H(depth, d_depth, sizeof(int32_t) * (size_t)L, s);
     tc_status st;
-    rc = fetch_status(ctx, d_status, &st, s);
+    rc = fetch_status(ctx, a.status, &st, s);
     if (rc) return rc;
     return status_to_rc(ctx, st, p);
 }

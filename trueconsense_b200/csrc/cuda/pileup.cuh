@@ -19,6 +19,20 @@ struct tc_piece {
 #endif
 constexpr int PIECE_COLS = TC_PIECE_COLS;         // a multiple of 8, at most 440 (the 512-column window minus its slack)
 
+// Variant 3 keeps a read's whole alignment inside a window of 8 * WC reference columns (WC = 32, 64 or 128 words) and takes
+// reads while their starts stay within the window's first `slack` = 8 * WC - (longest span, rounded up to 8) - 8 columns; a
+// slack below MIN_SLACK is not worth a window.
+constexpr int MIN_SLACK = 64;
+
+// The narrowest window (WC) for reads spanning at most `max_span` columns; 0 when the span is too long for any window (the
+// reads are then cut into pieces, variant 4).  warp_pileup_kernel makes the same choice on the device from the span pass.
+constexpr int warp_geometry(int max_span) {
+    const int ms = (max_span + 7) & ~7;
+    for (int wc = 32; wc <= 128; wc *= 2)
+        if (((8 * wc - ms - 8) & ~7) >= MIN_SLACK) return wc;
+    return 0;
+}
+
 struct pileup_args {
     dreads r;
     int32_t L;

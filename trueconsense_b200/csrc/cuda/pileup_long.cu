@@ -20,7 +20,7 @@
 //   lr_finish_kernel  one thread per piece: its op / SEQ word counts (it ends where the next piece starts)
 //   radix sort        piece start columns -> processing order
 //   warp_pileup_kernel<64, PIECES>
-// Reads with pads, zero-length ops or no SEQ are not cut (TC_ERR_CAPACITY -> the scatter kernel takes the batch).
+// Reads with pads, zero-length ops or no SEQ are not cut: TC_ERR_CAPACITY (the fallback ladder: tc_pileup_settle, pileup.cu).
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
 

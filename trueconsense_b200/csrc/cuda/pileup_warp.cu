@@ -40,8 +40,8 @@
 //               checks sort order and range and adds the two ends of every read's span to the coverage
 //               difference array (combined inside the warp with match.any) — no separate pass over the CIGARs.
 //   declined    sub-tiles with pads, zero-length ops, or an op of 4096+ bases that matters raise
-//               TC_ERR_CAPACITY: tc_pileup_counts then runs the batch through the scatter kernel, which
-//               carries htslib's full look-ahead state (such CIGARs are legal and essentially never seen).
+//               TC_ERR_CAPACITY (such CIGARs are legal and essentially never seen); what runs next is the
+//               fallback ladder of tc_pileup_settle (pileup.cu).
 #include <limits.h>
 
 #include "pileup_smem.cuh"
@@ -49,7 +49,6 @@
 namespace {
 
 using namespace tcsm;
-constexpr int MIN_SLACK = 64;
 constexpr int HI_PLANES = 7;            // bit-sliced planes above "eights": 15 + 16*127 = 2047 reads per run
 constexpr int RUN_CAP = 2047;
 #ifndef TC_CHUNK_WORDS
@@ -186,7 +185,7 @@ __global__ void __launch_bounds__(geom<WC>::WARPS * 32, 1) warp_pileup_kernel(pi
     const int lane = threadIdx.x & 31;
     const int L = a.L;
 
-    // which geometry handles this batch: the narrowest whose slack is usable
+    // which geometry handles this batch: the narrowest whose slack is usable (warp_geometry, pileup.cuh)
     // the longest reference span: the caller's bound (tc_reads_t.max_ref_span) or what the span pass found
     // (PIECES: the "reads" are pieces of at most PIECE_COLS columns; the span pass ran over the real reads)
     const bool fold = !PIECES && a.span_hint > 0;   // no span pass ran: this kernel also does its checks and the coverage ends
@@ -733,11 +732,10 @@ static int launch_geom(tc_ctx* ctx, const pileup_args& a, cudaStream_t s) {
 // bound the host knows which one that is.
 int tc_pileup_warp_launch(tc_ctx* ctx, const pileup_args& a, cudaStream_t s) {
     if (a.span_hint > 0) {
-        const int ms = (a.span_hint + 7) & ~7;
-        const int slack32 = (256 - ms - 8) & ~7, slack64 = (512 - ms - 8) & ~7;
-        if (slack32 >= MIN_SLACK) return launch_geom<32, false>(ctx, a, s);
-        if (slack64 >= MIN_SLACK) return launch_geom<64, false>(ctx, a, s);
-        return launch_geom<128, false>(ctx, a, s);
+        const int wc = warp_geometry(a.span_hint);
+        if (wc == 32) return launch_geom<32, false>(ctx, a, s);
+        if (wc == 64) return launch_geom<64, false>(ctx, a, s);
+        return launch_geom<128, false>(ctx, a, s);      // (too long for it too: the kernel declines the batch)
     }
     int rc = launch_geom<32, false>(ctx, a, s);
     if (rc) return rc;

@@ -200,14 +200,10 @@ TC_API int tc_sample_finish(tc_ctx_t* ctx, int32_t ticket, tc_insert_call_t* cal
     int32_t n = 0; int fit = 0;
     // the pileup's verdict first: its errors win, and a batch the bit-parallel kernel declined is redone from the start
     const int ins_rc = tc_inserts_finish_dev(ctx, &sl.ipend, sl.host_block, &pst, cands, &n, tmp_calls, bases, bases_cap, &fit);
-    int rc;
-    if (pst.err == TC_ERR_CAPACITY && sl.pend.variant != 1 && sl.pp.kernel == 0) {
-        rc = tc_pileup_finish(ctx, pst, &sl.pend, reads, ref_len, &sl.pp, sl.counts, sl.stream);     // runs the other kernel variant
-        if (rc) return rc;
-        return sample_unchained(ctx, reads, ref_len, &sl.pp, &sl.cp, &sl.ip, sl.counts, &sl.table, true, calls, calls_cap, n_calls, bases, bases_cap, sl.stream);
-    }
-    rc = tc_pileup_finish(ctx, pst, &sl.pend, reads, ref_len, &sl.pp, sl.counts, sl.stream);
+    int redone = 0;
+    int rc = tc_pileup_settle(ctx, pst, sl.pend, reads, ref_len, &sl.pp, sl.counts, (cudaStream_t)sl.stream, &redone);
     if (rc) return rc;
+    if (redone) return sample_unchained(ctx, reads, ref_len, &sl.pp, &sl.cp, &sl.ip, sl.counts, &sl.table, true, calls, calls_cap, n_calls, bases, bases_cap, sl.stream);
     if (ins_rc) return ins_rc;
     *n_calls = n;
     if (n > calls_cap) return tc_fail(ctx, TC_ERR_CAPACITY, "%d insertion candidates, capacity %d", n, calls_cap);

@@ -27,8 +27,13 @@ struct tc_buf { void* p; size_t cap; };
 
 constexpr size_t TC_HOST_SCRATCH = 64 * 1024;
 struct tc_status;
-struct tc_pileup_pending {      // what tc_pileup_finish needs once the status block is on the host
-    tc_status* d_status; int32_t* d_counts; int variant; int per_entry; int out_dev; int64_t n_reads; int32_t span_hint;
+struct pileup_plan {            // one attempt at the count table (pileup_plan_of, pileup.cu)
+    int variant;                // 1 scatter, 3 warp streams, 4 long reads cut into pieces for the warp streams
+    bool span_pass;             // a pass over the CIGARs finds the spans first (else variant 3 checks them itself)
+    bool span_out;              // ... and leaves every read's span for variant 4's split
+};
+struct tc_pileup_pending {      // what tc_pileup_settle needs once the status block is on the host
+    tc_status* d_status; int32_t* d_counts; pileup_plan plan; int out_dev; int64_t n_reads;
 };
 
 struct tc_ctx {
@@ -121,10 +126,12 @@ struct dreads {
 int tc_resolve_reads(tc_ctx* ctx, const tc_reads_t* in, dreads* out, int need, cudaStream_t s);
 
 // ---- pieces of the entry points that only ENQUEUE (tc_pileup_call_inserts chains them without a host round trip)
+// rung: the variant of the fallback ladder to run; 0 the first attempt (p->kernel, or for 0 the library's choice)
 int tc_pileup_enqueue(tc_ctx* ctx, const tc_reads_t* reads, int32_t ref_len, const tc_pileup_params_t* p, int32_t* counts, cudaStream_t s,
-                      tc_pileup_pending* pend);
-int tc_pileup_finish(tc_ctx* ctx, const tc_status& st, const tc_pileup_pending* pend, const tc_reads_t* reads, int32_t ref_len,
-                     const tc_pileup_params_t* p, int32_t* counts, void* stream);
+                      tc_pileup_pending* pend, int rung = 0);
+// redone (may be NULL): set to 1 when the batch went down the fallback ladder, i.e. another variant rebuilt the table
+int tc_pileup_settle(tc_ctx* ctx, tc_status st, tc_pileup_pending pend, const tc_reads_t* reads, int32_t ref_len,
+                     const tc_pileup_params_t* p, int32_t* counts, cudaStream_t s, int* redone);
 int tc_h2d(tc_ctx* ctx, void* d, const void* p, size_t bytes, cudaStream_t s);
 bool tc_reads_all_device(const tc_reads_t* r);     // every array of the batch already in device memory
 int tc_candidates_enqueue(tc_ctx* ctx, const uint8_t* d_flags, int32_t ref_len, int32_t cap, int32_t** d_count, int32_t** d_sorted, cudaStream_t s);
