@@ -192,6 +192,9 @@ __global__ void lr_finish_kernel(pileup_args a, const uint32_t* __restrict__ pie
                                  const uint32_t* __restrict__ end_w, const uint32_t* __restrict__ end_y) {
     const int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= n_pieces) return;
+    // a read the split declined (no SEQ, a pad) has no piece records or end state: the batch is void, nothing to finish
+    // (tests/test_pileup_edges.py: reads without SEQ or with a pad in front of variant 4 once the slab held other pieces)
+    if (a.status->err) return;
     const int32_t rd = pieces[p].pad;
     const uint32_t sbeg = a.r.seq_off[rd];
     const bool last = (uint32_t)(p + 1) == piece_base[rd + 1];

@@ -184,6 +184,8 @@ __global__ void __launch_bounds__(geom<WC>::WARPS * 32, 1) warp_pileup_kernel(pi
     constexpr int ROWW = G::ROWW, RS = G::RS, NW = G::NW, NPH = G::NPH, PW = G::PW, KW = G::PW / 32;
     const int lane = threadIdx.x & 31;
     const int L = a.L;
+    // pieces of a batch the long-read split declined: some records were never written (lr_finish_kernel)
+    if (PIECES && a.status->err) return;
 
     // which geometry handles this batch: the narrowest whose slack is usable (warp_geometry, pileup.cuh)
     // the longest reference span: the caller's bound (tc_reads_t.max_ref_span) or what the span pass found
