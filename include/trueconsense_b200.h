@@ -217,6 +217,18 @@ typedef struct tc_bam_stats {
 int  tc_bam_records_to_reads(tc_ctx_t* ctx, const uint8_t* payload, int64_t n_bytes, const int64_t* rec_off, int64_t n_reads,
                              tc_reads_t* dev, tc_bam_stats_t* stats, void* stream);
 
+/* Coordinate order for a BAM's records (what `samtools sort` would give). payload / rec_off as tc_bam_records_to_reads
+ * takes them (host or device); *payload_dev and *rec_sorted_dev feed tc_bam_records_to_reads and tc_bam_contig_ranges.
+ * Records already sorted by (refID, pos) keep their order (*reordered = 0). TC_ERR_RANGE: refID outside [0, n_ref) or
+ * pos < -1. Synchronises the stream once (twice when it reorders: the sorted offsets are complete on return).
+ * The order otherwise: refID, then pos, then forward strand before reverse (FLAG 0x10), then file order (a stable radix sort
+ * over 64-bit keys).  Host inputs are staged once into the context's payload / record buffers; the sorted offsets live in a
+ * buffer of their own that neither tc_bam_records_to_reads nor tc_bam_contig_ranges writes, valid until the next call that
+ * decodes a BAM on this context.  n_reads == 0: the inputs are handed back as they are. */
+int  tc_bam_sort_records(tc_ctx_t* ctx, const uint8_t* payload, int64_t n_bytes, const int64_t* rec_off, int64_t n_reads,
+                         int32_t n_ref, const uint8_t** payload_dev, const int64_t** rec_sorted_dev, int32_t* reordered,
+                         void* stream);
+
 /* ---- the BAM file as it lies on disk: inflate and record index on the GPU ----
  * Replaces htslib's bgzf reader and bam_read1 under pysam (reference: indexing.py:6-19 `Readbam`, :96).  The host maps
  * the file and walks the BGZF member headers (tc_host.h: tc_bgzf_map — one header per member); the file's bytes travel as

@@ -3,6 +3,7 @@ validators and exit behaviour, same order of work — on top of the GPU hot path
 
     python -m trueconsense_b200.TrueConsense -i x.bam -ref ref.fasta -gff f.gff -cov 30 -name S -o cons.fasta
     python -m trueconsense_b200.TrueConsense --all-contigs -i flu.bam -ref flu.fasta -gff flu.gff -cov 30 -name S -o S.fasta
+    python -m trueconsense_b200.TrueConsense --sort-input -i aligner_out.bam -ref ref.fasta -gff f.gff -cov 30 -name S -o S.fasta
 
 ``main(args)`` is the console-script entry point of the reference (pyproject.toml:38-40).
 """
@@ -87,6 +88,9 @@ def GetArgs(givenargs):
                      help="Call every reference of a multi-contig BAM (a segmented genome, a panel of references) in one "
                           "pass: one FASTA record '{samplename}_{reference}' per reference, the GFF rows matched by seqid, "
                           "one VCF and one depth file for all references")
+    opt.add_argument("--sort-input", action="store_true",
+                     help="Accept a BAM whose records are not coordinate-sorted (e.g. straight from the aligner); they are put "
+                          "in samtools' coordinate order on the GPU. A sorted BAM is used as written")
     opt.add_argument("--version", "-v", action="version", version=__version__,
                      help="Show the TrueConsense version and exit")
     opt.add_argument("--help", "-h", action="help", default=argparse.SUPPRESS, help="Show this help message and exit")
@@ -132,7 +136,7 @@ def main(args: list[str] | None = None):
               "Use 'TrueConsense -h' to see the help document")
         sys.exit(1)
     opts = GetArgs(argv)
-    bam = Readbam(opts.input)        # one decoded copy of the BAM serves the index and the insertion columns
+    bam = Readbam(opts.input, sort=opts.sort_input)        # one decoded copy of the BAM serves the index and the insertion columns
     if opts.all_contigs:
         return _main_all_contigs(opts, bam)
     frame, gff = _index_and_features(opts, bam)

@@ -120,6 +120,8 @@ def lib() -> C.CDLL:
                                                  C.POINTER(i32), vp, i64, vp]
             l.tc_bam_records_to_reads.argtypes = [vp, vp, i64, vp, i64, C.POINTER(TcReads), C.POINTER(BamStats), vp]
             l.tc_bam_records_to_reads.restype = C.c_int
+            l.tc_bam_sort_records.argtypes = [vp, vp, i64, vp, i64, i32, C.POINTER(vp), C.POINTER(vp), C.POINTER(i32), vp]
+            l.tc_bam_sort_records.restype = C.c_int
             l.tc_bgzf_inflate.argtypes = [vp, vp, i64, vp, i64, i64, C.POINTER(vp), vp]
             l.tc_bgzf_inflate.restype = C.c_int
             l.tc_bam_index_records.argtypes = [vp, vp, i64, i64, i32, vp, C.POINTER(vp), C.POINTER(i64), C.POINTER(i64), vp]
@@ -295,30 +297,50 @@ class Context:
         self._check(self._lib.tc_bam_contig_ranges(self._h, payload_ptr, n_bytes, rec_ptr, n_reads, n_ref, _ptr(first), stream))
         return first
 
-    def bam_to_device(self, payload, stream: int = 0, contig_ranges: bool = False) -> DeviceReads:
+    def _sort_records(self, payload_ptr, n_bytes: int, rec_ptr, n_reads: int, n_ref: int, stream: int):
+        """tc_bam_sort_records: (device payload, record offsets in coordinate order, whether they moved)."""
+        p, r, moved = C.c_void_p(), C.c_void_p(), C.c_int32(0)
+        self._check(self._lib.tc_bam_sort_records(self._h, payload_ptr, n_bytes, rec_ptr, n_reads, n_ref, C.byref(p), C.byref(r),
+                                                  C.byref(moved), stream))
+        return p.value, r.value, bool(moved.value)
+
+    def bam_to_device(self, payload, stream: int = 0, contig_ranges: bool = False, sort: bool = False) -> DeviceReads:
         """GPU-side record parsing (tc_bam_records_to_reads): a ``bamio.BamPayload`` (the BAM inflated on the host, its records
         indexed) becomes the flat read arrays in the context's device buffers — the CPU never touches a record's body.
-        ``.stats`` of the result: aligned bases, longest span, sortedness, whether more than one reference occurs."""
+        ``.stats`` of the result: aligned bases, longest span, sortedness, whether more than one reference occurs.
+        ``sort``: records that are not sorted by (refID, pos) are put in samtools' coordinate order first
+        (``tc_bam_sort_records``; the payload then travels to the device once); ``.info`` says whether they moved
+        (``reordered``) and what that took (``t_sort_s``)."""
+        import time
+
+        pay, rec, n = payload.payload_ptr, payload.rec_off_ptr, payload.n_reads
+        self._generation += 1
+        t0 = time.perf_counter()
+        moved = False
+        if sort:
+            pay, rec, moved = self._sort_records(pay, payload.n_bytes, rec, n, len(payload.ref_lens), stream)
+        t1 = time.perf_counter()
         dev = TcReads()
         st = BamStats()
-        self._generation += 1
-        self._check(self._lib.tc_bam_records_to_reads(self._h, payload.payload_ptr, payload.n_bytes, payload.rec_off_ptr,
-                                                      payload.n_reads, C.byref(dev), C.byref(st), stream))
+        self._check(self._lib.tc_bam_records_to_reads(self._h, pay, payload.n_bytes, rec, n, C.byref(dev), C.byref(st), stream))
         d = DeviceReads(dev, None, self, self._generation)
         d.stats = st
+        d.info = {"reordered": moved, "t_sort_s": t1 - t0}
         if contig_ranges and payload.ref_names and not st.unsorted:
-            d.first_read = self._contig_ranges(payload.payload_ptr, payload.n_bytes, payload.rec_off_ptr, payload.n_reads,
-                                               len(payload.ref_names), stream)
+            d.first_read = self._contig_ranges(pay, payload.n_bytes, rec, n, len(payload.ref_names), stream)
         return d
 
-    def bam_file_to_device(self, path: str, stream: int = 0, contig_ranges: bool = False) -> DeviceReads:
+    def bam_file_to_device(self, path: str, stream: int = 0, contig_ranges: bool = False, sort: bool = False) -> DeviceReads:
         """A BAM file to the flat read arrays in device memory with the GPU doing all of it: the host maps the file and walks
         the BGZF member headers (``bamio.map_bgzf``); the device inflates every member and checks its CRC-32
         (``tc_bgzf_inflate``), finds and proves the record offsets (``tc_bam_index_records``) and parses the records
         (``tc_bam_records_to_reads``).  The result carries ``.ref_names``, ``.ref_lens``, ``.stats`` and ``.info``
         (records, unplaced records dropped, timings).  ``TcError`` / ``OSError`` for a file that does not decode.
         ``contig_ranges``: also ``.first_read``, where each reference's reads begin (``tc_bam_contig_ranges``, taken while the
-        payload and the record offsets are still in the context's buffers); left None for an unsorted file."""
+        payload and the record offsets are still in the context's buffers); left None for an unsorted file.
+        ``sort``: a file whose records are not sorted by (refID, pos) has its record offsets put in samtools' coordinate order
+        on the device before the parse (``tc_bam_sort_records``); a sorted file is parsed as written.  ``.info`` then tells
+        ``reordered`` and ``t_sort_s``."""
         import time
 
         from . import bamio
@@ -348,6 +370,11 @@ class Context:
         self._check(self._lib.tc_bam_index_records(self._h, payload, n_bytes, first, len(lens), ref_len.ctypes.data, C.byref(rec),
                                                    C.byref(n_placed), C.byref(n_records), stream))
         t3 = time.perf_counter()
+        moved = False
+        if sort:
+            _, rec, moved = self._sort_records(payload, n_bytes, rec, n_placed.value, len(lens), stream)
+            rec = C.c_void_p(rec)
+        t3s = time.perf_counter()
         dev = TcReads()
         st = BamStats()
         self._check(self._lib.tc_bam_records_to_reads(self._h, payload, n_bytes, rec, n_placed.value, C.byref(dev), C.byref(st), stream))
@@ -358,7 +385,7 @@ class Context:
         if contig_ranges and lens and not st.unsorted:
             d.first_read = self._contig_ranges(payload, n_bytes, rec, n_placed.value, len(lens), stream)
         info.update(n_records=int(n_records.value), n_dropped_unplaced=int(n_records.value - n_placed.value), t_map_s=t1 - t0,
-                    t_inflate_s=t2 - t1, t_index_s=t3 - t2, t_parse_s=t4 - t3)
+                    t_inflate_s=t2 - t1, t_index_s=t3 - t2, t_sort_s=t3s - t3, t_parse_s=t4 - t3s, reordered=moved)
         d.info = info
         return d
 

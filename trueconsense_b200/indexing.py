@@ -24,10 +24,17 @@ class BamHandle:
     """What ``Readbam`` returns: a BAM on its way to the device plus the attributes of ``pysam.AlignmentFile`` the reference
     touches (``references``; Events.py:63).  The file travels to the device as it is: BGZF members inflated, record offsets
     found and records parsed on the GPU (``gpu.Context.bam_file_to_device``) straight into the context's read buffers; ``reads`` (a host-side decode into numpy arrays) is
-    only made when somebody asks for it."""
+    only made when somebody asks for it.
 
-    def __init__(self, filename: str, reads: ReadBatch | None = None):
+    ``sort``: a file whose records are not sorted by (refID, pos) (aligner output, a queryname-sorted BAM) is accepted and its
+    records are put in samtools' coordinate order on the GPU (``tc_bam_sort_records``), so every pass computes what it
+    computes after ``samtools sort``; a sorted file is used as written.  Only the device reads are reordered: ``reads``, the
+    host decode, stays in file order, and a handle made from a host ``ReadBatch`` (``reads=``) that is not sorted still
+    raises ``ValueError`` (host batches are not sorted here)."""
+
+    def __init__(self, filename: str, reads: ReadBatch | None = None, sort: bool = False):
         self.filename = filename
+        self.sort = sort
         self._reads = reads
         self._payload = None
         self._hdr = None
@@ -93,13 +100,13 @@ class BamHandle:
                     d = ctx.upload(b, with_qual=False)
                 else:
                     try:
-                        d = ctx.bam_file_to_device(self.filename)      # inflate, record index and parse on the GPU
+                        d = ctx.bam_file_to_device(self.filename, sort=self.sort)      # inflate, record index (sort) and parse on the GPU
                         self._hdr = (d.ref_names, d.ref_lens)
                     except gpu.TcError:
                         # a file the device path refuses: the host reader names the broken member / record (or, should it
                         # read the file after all, feeds the device parse)
                         self._payload = bamio.read_bam_payload(self.filename)
-                        d = ctx.bam_to_device(self._payload)
+                        d = ctx.bam_to_device(self._payload, sort=self.sort)
                         self._payload.release()     # the device holds the arrays now; the header stays
                     if d.stats.multi_contig:
                         raise ValueError("multi-contig BAM: TrueConsense indexes positions of a single reference "
@@ -129,11 +136,11 @@ class BamHandle:
                 d = ctx.upload(b)       # QUAL and mate fields too: the move shifts PNEXT on the device
             else:
                 try:
-                    d = ctx.bam_file_to_device(self.filename, contig_ranges=True)
+                    d = ctx.bam_file_to_device(self.filename, contig_ranges=True, sort=self.sort)
                     self._hdr = (d.ref_names, d.ref_lens)
                 except gpu.TcError:
                     self._payload = bamio.read_bam_payload(self.filename)
-                    d = ctx.bam_to_device(self._payload, contig_ranges=True)
+                    d = ctx.bam_to_device(self._payload, contig_ranges=True, sort=self.sort)
                     self._payload.release()
                 if d.stats.unsorted:
                     raise ValueError("Unsorted input. Pileup aborts")
@@ -210,12 +217,13 @@ def gff_by_contig(df: pd.DataFrame, names) -> dict:
     return {n: df[df["seqid"] == n].reset_index(drop=True) for n in names}
 
 
-def Readbam(f):
+def Readbam(f, sort: bool = False):
     """indexing.py:6-19.  A handle passed in is returned as is, so one decoded copy of the BAM can
-    serve BuildIndex, ListInserts and WriteOutputs."""
+    serve BuildIndex, ListInserts and WriteOutputs.  ``sort``: accept records that are not coordinate-sorted and put them
+    in samtools' coordinate order on the GPU (``BamHandle``)."""
     if isinstance(f, BamHandle):
         return f
-    return BamHandle(f)
+    return BamHandle(f, sort=sort)
 
 
 class _GffHeader:
