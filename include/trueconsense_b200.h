@@ -229,6 +229,26 @@ int  tc_bam_sort_records(tc_ctx_t* ctx, const uint8_t* payload, int64_t n_bytes,
                          int32_t n_ref, const uint8_t** payload_dev, const int64_t** rec_sorted_dev, int32_t* reordered,
                          void* stream);
 
+/* ---- SAM text straight from the aligner -> BAM records on the device ----
+ * text[0 .. n_bytes): the SAM file (host or device memory); its records begin at first_line_off, which is file line
+ * first_line_no (1-based) — the caller has read the '@' header lines and hands over the @SQ names in header order:
+ * ref_names holds them concatenated, reference k is ref_names[ref_name_off[k] .. ref_name_off[k+1]).  Only the body travels
+ * to the device (large pageable sources through the staging ring).  Every line becomes the BAM record `samtools view -b`
+ * would write for it, without `bin` (0) and without optional fields; lines with RNAME '*' are dropped like
+ * tc_bam_index_records drops refID -1.  *payload_dev / *rec_off_dev: the placed records and their refID offsets in file
+ * order, as tc_bam_index_records leaves them (feed tc_bam_sort_records, tc_bam_records_to_reads, tc_bam_contig_ranges; valid
+ * until the next call that decodes a BAM or SAM on this context); *n_payload their bytes; *n_records every record,
+ * *n_placed the kept ones; *n_lines the lines of the body.
+ * A malformed line (fewer than 11 fields, a number out of range, an unknown RNAME / RNEXT, a bad CIGAR, CIGAR / SEQ or QUAL /
+ * SEQ lengths that differ, a QUAL character below '!', an empty line before the last, an '@' line, more than 65535 CIGAR
+ * ops, a CG:B placeholder CIGAR): TC_ERR_ARG, the message "line <k>: <reason>" for the first such line; err[0] = k (1-based
+ * in the file), err[1] = the reason's code.  t_steps (may be NULL): host seconds of the upload, the line index and the
+ * conversion.  Synchronises the stream. */
+int  tc_sam_to_bam_records(tc_ctx_t* ctx, const uint8_t* text, int64_t n_bytes, int64_t first_line_off, int64_t first_line_no,
+                           int32_t n_ref, const char* ref_names, const int64_t* ref_name_off, const uint8_t** payload_dev,
+                           int64_t* n_payload, const int64_t** rec_off_dev, int64_t* n_placed, int64_t* n_records,
+                           int64_t* n_lines, int64_t err[2], double* t_steps, void* stream);
+
 /* ---- the BAM file as it lies on disk: inflate and record index on the GPU ----
  * Replaces htslib's bgzf reader and bam_read1 under pysam (reference: indexing.py:6-19 `Readbam`, :96).  The host maps
  * the file and walks the BGZF member headers (tc_host.h: tc_bgzf_map — one header per member); the file's bytes travel as

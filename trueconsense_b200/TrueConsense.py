@@ -5,6 +5,9 @@ validators and exit behaviour, same order of work — on top of the GPU hot path
     python -m trueconsense_b200.TrueConsense --all-contigs -i flu.bam -ref flu.fasta -gff flu.gff -cov 30 -name S -o S.fasta
     python -m trueconsense_b200.TrueConsense --sort-input -i aligner_out.bam -ref ref.fasta -gff f.gff -cov 30 -name S -o S.fasta
 
+    minimap2 -a ref.fa r.fq > s.sam
+    python -m trueconsense_b200.TrueConsense --sort-input -i s.sam -ref ref.fa -gff f.gff -cov 30 -name S -o S.fasta
+
 ``main(args)`` is the console-script entry point of the reference (pyproject.toml:38-40).
 """
 from __future__ import annotations
@@ -58,8 +61,8 @@ def GetArgs(givenargs):
         return fname
 
     req = parser.add_argument_group("Required arguments")
-    req.add_argument("--input", "-i", type=with_suffix("BAM-file", (".bam",), -1, "Input file"), metavar="File",
-                     help="Input file in BAM format", required=True)
+    req.add_argument("--input", "-i", type=with_suffix("BAM or SAM file", (".bam", ".sam"), -1, "Input file"), metavar="File",
+                     help="Input file in BAM or SAM format (SAM: the aligner's text output, converted on the GPU)", required=True)
     req.add_argument("--output", "-o", type=str, default=os.getcwd() + "consensus.fasta", metavar="File",
                      help="Output consensus fasta", required=True)
     req.add_argument("--reference", "-ref", type=with_suffix("Fasta-file", (".fasta", ".fa"), 1, "Reference file"),
@@ -89,8 +92,8 @@ def GetArgs(givenargs):
                           "pass: one FASTA record '{samplename}_{reference}' per reference, the GFF rows matched by seqid, "
                           "one VCF and one depth file for all references")
     opt.add_argument("--sort-input", action="store_true",
-                     help="Accept a BAM whose records are not coordinate-sorted (e.g. straight from the aligner); they are put "
-                          "in samtools' coordinate order on the GPU. A sorted BAM is used as written")
+                     help="Accept a BAM or SAM whose records are not coordinate-sorted (e.g. straight from the aligner); they "
+                          "are put in samtools' coordinate order on the GPU. A sorted file is used as written")
     opt.add_argument("--version", "-v", action="version", version=__version__,
                      help="Show the TrueConsense version and exit")
     opt.add_argument("--help", "-h", action="help", default=argparse.SUPPRESS, help="Show this help message and exit")

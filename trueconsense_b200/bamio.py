@@ -187,6 +187,37 @@ def read_bam_header(path: str):
         n *= 4
 
 
+def read_sam_header(path: str):
+    """(reference names, reference lengths, byte offset of the first record, its 1-based line number) of a SAM file: the
+    ``@`` lines at its start are read, no record.  ``@SQ`` lines give the references (``SN``, ``LN``) in order; ``@HD``,
+    ``@RG``, ``@PG``, ``@CO`` and any other header line are skipped.  ``OSError`` names the line of an ``@SQ`` without
+    ``SN``, with a name seen before, or without an ``LN`` in 1..2^31-1.  Names keep their bytes (undecodable ones as
+    surrogates: ``name.encode(errors="surrogateescape")`` gives them back)."""
+    names, lens, seen = [], [], set()
+    off, line_no = 0, 1
+    with open(path, "rb") as fh:
+        while fh.peek(1)[:1] == b"@":
+            line = fh.readline()
+            if line[:4] in (b"@SQ\t", b"@SQ\n", b"@SQ"):
+                tags = {}
+                for f in line.rstrip(b"\n").split(b"\t")[1:]:
+                    tags.setdefault(f[:3], f[3:])
+                sn, ln = tags.get(b"SN:"), tags.get(b"LN:")
+                if not sn:
+                    raise OSError(f"{path}: line {line_no}: @SQ line without a reference name (SN)")
+                name = sn.decode(errors="surrogateescape")
+                if name in seen:
+                    raise OSError(f"{path}: line {line_no}: reference {name!r} is listed twice")
+                if ln is None or not ln.isdigit() or not 1 <= int(ln) <= 0x7FFFFFFF:
+                    raise OSError(f"{path}: line {line_no}: reference {name!r} needs a length (LN) in 1..2147483647")
+                seen.add(name)
+                names.append(name)
+                lens.append(int(ln))
+            off += len(line)
+            line_no += 1
+    return names, lens, off, line_no
+
+
 _lib = None
 
 

@@ -122,6 +122,9 @@ def lib() -> C.CDLL:
             l.tc_bam_records_to_reads.restype = C.c_int
             l.tc_bam_sort_records.argtypes = [vp, vp, i64, vp, i64, i32, C.POINTER(vp), C.POINTER(vp), C.POINTER(i32), vp]
             l.tc_bam_sort_records.restype = C.c_int
+            l.tc_sam_to_bam_records.argtypes = [vp, vp, i64, i64, i64, i32, vp, vp, C.POINTER(vp), C.POINTER(i64), C.POINTER(vp),
+                                                C.POINTER(i64), C.POINTER(i64), C.POINTER(i64), C.POINTER(i64), C.POINTER(C.c_double), vp]
+            l.tc_sam_to_bam_records.restype = C.c_int
             l.tc_bgzf_inflate.argtypes = [vp, vp, i64, vp, i64, i64, C.POINTER(vp), vp]
             l.tc_bgzf_inflate.restype = C.c_int
             l.tc_bam_index_records.argtypes = [vp, vp, i64, i64, i32, vp, C.POINTER(vp), C.POINTER(i64), C.POINTER(i64), vp]
@@ -370,24 +373,85 @@ class Context:
         self._check(self._lib.tc_bam_index_records(self._h, payload, n_bytes, first, len(lens), ref_len.ctypes.data, C.byref(rec),
                                                    C.byref(n_placed), C.byref(n_records), stream))
         t3 = time.perf_counter()
+        info.update(n_records=int(n_records.value), n_dropped_unplaced=int(n_records.value - n_placed.value), t_map_s=t1 - t0,
+                    t_inflate_s=t2 - t1, t_index_s=t3 - t2)
+        return self._records_to_device(payload, n_bytes, rec, n_placed.value, names, lens, info, stream, contig_ranges, sort)
+
+    def _records_to_device(self, payload, n_bytes: int, rec, n_placed: int, names, lens, info: dict, stream: int,
+                           contig_ranges: bool, sort: bool) -> DeviceReads:
+        """The tail of both file routes: BAM records in device memory (payload, offsets of the placed ones) -> sorted when
+        asked (``tc_bam_sort_records``), parsed (``tc_bam_records_to_reads``), the contig ranges -> ``DeviceReads`` with
+        ``.ref_names``, ``.ref_lens``, ``.stats`` and ``info`` plus the sort's and the parse's timings."""
+        import time
+
+        t3 = time.perf_counter()
         moved = False
         if sort:
-            _, rec, moved = self._sort_records(payload, n_bytes, rec, n_placed.value, len(lens), stream)
+            _, rec, moved = self._sort_records(payload, n_bytes, rec, n_placed, len(lens), stream)
             rec = C.c_void_p(rec)
         t3s = time.perf_counter()
         dev = TcReads()
         st = BamStats()
-        self._check(self._lib.tc_bam_records_to_reads(self._h, payload, n_bytes, rec, n_placed.value, C.byref(dev), C.byref(st), stream))
+        self._check(self._lib.tc_bam_records_to_reads(self._h, payload, n_bytes, rec, n_placed, C.byref(dev), C.byref(st), stream))
         t4 = time.perf_counter()
         d = DeviceReads(dev, None, self, self._generation)
         d.stats = st
         d.ref_names, d.ref_lens = names, lens
         if contig_ranges and lens and not st.unsorted:
-            d.first_read = self._contig_ranges(payload, n_bytes, rec, n_placed.value, len(lens), stream)
-        info.update(n_records=int(n_records.value), n_dropped_unplaced=int(n_records.value - n_placed.value), t_map_s=t1 - t0,
-                    t_inflate_s=t2 - t1, t_index_s=t3 - t2, t_sort_s=t3s - t3, t_parse_s=t4 - t3s, reordered=moved)
+            d.first_read = self._contig_ranges(payload, n_bytes, rec, n_placed, len(lens), stream)
+        info.update(t_sort_s=t3s - t3, t_parse_s=t4 - t3s, reordered=moved)
         d.info = info
         return d
+
+    def sam_file_to_device(self, path: str, stream: int = 0, contig_ranges: bool = False, sort: bool = False) -> DeviceReads:
+        """A SAM file (an aligner's text output) to the flat read arrays in device memory, with the contract of
+        :meth:`bam_file_to_device`: the host reads the ``@`` header lines (``bamio.read_sam_header``) and maps the file; the
+        device turns every line into the BAM record ``samtools view -b`` would write for it (``tc_sam_to_bam_records``)
+        and the BAM route's own steps follow (sort when asked, parse, contig ranges).  Lines with RNAME ``*`` are dropped
+        and counted.  ``.info``: ``sam_bytes``, ``n_lines``, ``n_records``, ``n_dropped_unplaced``, ``reordered`` and the
+        timings of each step (``t_map_s``, ``t_upload_s``, ``t_line_index_s``, ``t_convert_s``, ``t_sort_s``,
+        ``t_parse_s``).  A malformed line is ``OSError("<path>: line <k>: <reason>")``."""
+        import mmap
+        import time
+
+        from . import bamio
+
+        t0 = time.perf_counter()
+        names, lens, first_off, first_no = bamio.read_sam_header(path)
+        raw = [n.encode(errors="surrogateescape") for n in names]
+        name_off = np.zeros(len(raw) + 1, np.int64)
+        name_off[1:] = np.cumsum([len(n) for n in raw])
+        name_bytes = b"".join(raw) + b"\0"
+        payload, rec = C.c_void_p(), C.c_void_p()
+        n_payload, n_placed, n_records, n_lines = C.c_int64(0), C.c_int64(0), C.c_int64(0), C.c_int64(0)
+        err = (C.c_int64 * 2)()
+        steps = (C.c_double * 3)()
+        with open(path, "rb") as fh:
+            size = os.fstat(fh.fileno()).st_size
+            mm = mmap.mmap(fh.fileno(), 0, access=mmap.ACCESS_READ) if size > first_off else None
+            text = None
+            try:
+                text = np.frombuffer(mm, np.uint8) if mm is not None else None
+                t1 = time.perf_counter()
+                self._generation += 1
+                rc = self._lib.tc_sam_to_bam_records(self._h, None if text is None else text.ctypes.data, size, first_off, first_no,
+                                                     len(raw), name_bytes, name_off.ctypes.data, C.byref(payload), C.byref(n_payload),
+                                                     C.byref(rec), C.byref(n_placed), C.byref(n_records), C.byref(n_lines), err,
+                                                     steps, stream)
+            finally:
+                del text
+                if mm is not None:
+                    mm.close()
+        if rc != 0:
+            msg = self._lib.tc_last_error(self._h).decode()
+            if err[0] > 0:
+                raise OSError(f"{path}: {msg}")
+            raise TcError(rc, msg)
+        info = {"sam_bytes": size, "n_lines": int(n_lines.value), "n_records": int(n_records.value),
+                "n_dropped_unplaced": int(n_records.value - n_placed.value), "t_map_s": t1 - t0, "t_upload_s": steps[0],
+                "t_line_index_s": steps[1], "t_convert_s": steps[2]}
+        return self._records_to_device(payload, int(n_payload.value), rec, int(n_placed.value), names, lens, info, stream,
+                                       contig_ranges, sort)
 
     def reads_to_contig_coords(self, reads: DeviceReads, ref_lens, first_read, names=None, stream: int = 0) -> np.ndarray:
         """Move device-resident reads to the global columns of a multi-reference pass, in place (``tc_reads_to_contig_coords``):

@@ -8,6 +8,7 @@ BAM is inflated on the host (csrc/host/bamio.c), its records are parsed on the G
 """
 from __future__ import annotations
 
+import pathlib
 import threading
 from dataclasses import dataclass
 
@@ -30,11 +31,16 @@ class BamHandle:
     records are put in samtools' coordinate order on the GPU (``tc_bam_sort_records``), so every pass computes what it
     computes after ``samtools sort``; a sorted file is used as written.  Only the device reads are reordered: ``reads``, the
     host decode, stays in file order, and a handle made from a host ``ReadBatch`` (``reads=``) that is not sorted still
-    raises ``ValueError`` (host batches are not sorted here)."""
+    raises ``ValueError`` (host batches are not sorted here).
+
+    A path ending in ``.sam`` is an aligner's text output: its lines become BAM records on the GPU
+    (``gpu.Context.sam_file_to_device``) and take the BAM route from there, ``sort`` included.  There is no host decode of
+    SAM: ``reads`` raises ``NotImplementedError``, the device arrays are the product."""
 
     def __init__(self, filename: str, reads: ReadBatch | None = None, sort: bool = False):
         self.filename = filename
         self.sort = sort
+        self.is_sam = reads is None and pathlib.Path(filename).suffix == ".sam"
         self._reads = reads
         self._payload = None
         self._hdr = None
@@ -47,6 +53,9 @@ class BamHandle:
     def reads(self) -> ReadBatch:
         with self._lock:
             if self._reads is None:
+                if self.is_sam:
+                    raise NotImplementedError(f"{self.filename}: a SAM file is decoded on the GPU only (device_reads); "
+                                              "there are no host-side read arrays of it")
                 self._reads = bamio.read_bam(self.filename)
             return self._reads
 
@@ -57,6 +66,8 @@ class BamHandle:
                 return self._reads.ref_names, self._reads.ref_lens
             if self._payload is not None:
                 return self._payload.ref_names, self._payload.ref_lens
+            if self._hdr is None and self.is_sam:
+                self._hdr = bamio.read_sam_header(self.filename)[:2]    # the '@' lines only
             if self._hdr is None:
                 self._hdr = bamio.read_bam_header(self.filename)       # only the members holding the header are inflated
             return self._hdr
@@ -99,15 +110,7 @@ class BamHandle:
                         raise ValueError("Unsorted input. Pileup aborts")
                     d = ctx.upload(b, with_qual=False)
                 else:
-                    try:
-                        d = ctx.bam_file_to_device(self.filename, sort=self.sort)      # inflate, record index (sort) and parse on the GPU
-                        self._hdr = (d.ref_names, d.ref_lens)
-                    except gpu.TcError:
-                        # a file the device path refuses: the host reader names the broken member / record (or, should it
-                        # read the file after all, feeds the device parse)
-                        self._payload = bamio.read_bam_payload(self.filename)
-                        d = ctx.bam_to_device(self._payload, sort=self.sort)
-                        self._payload.release()     # the device holds the arrays now; the header stays
+                    d = self._file_to_device(ctx)
                     if d.stats.multi_contig:
                         raise ValueError("multi-contig BAM: TrueConsense indexes positions of a single reference "
                                          "(its DataFrame index would hold duplicate positions)")
@@ -135,13 +138,7 @@ class BamHandle:
                 first_read = contig_ranges_from_tid(b.tid, len(names), b.n_reads)
                 d = ctx.upload(b)       # QUAL and mate fields too: the move shifts PNEXT on the device
             else:
-                try:
-                    d = ctx.bam_file_to_device(self.filename, contig_ranges=True, sort=self.sort)
-                    self._hdr = (d.ref_names, d.ref_lens)
-                except gpu.TcError:
-                    self._payload = bamio.read_bam_payload(self.filename)
-                    d = ctx.bam_to_device(self._payload, contig_ranges=True, sort=self.sort)
-                    self._payload.release()
+                d = self._file_to_device(ctx, contig_ranges=True)
                 if d.stats.unsorted:
                     raise ValueError("Unsorted input. Pileup aborts")
                 first_read = d.first_read
@@ -151,6 +148,23 @@ class BamHandle:
             layout = ContigLayout(list(names), list(key[1]), start.astype(np.int64), np.asarray(first_read, np.int64))
             self._dev_contigs = (key, d, layout)
             return d, layout
+
+    def _file_to_device(self, ctx, contig_ranges: bool = False):
+        """The file's reads parsed into device memory (the caller holds the lock)."""
+        if self.is_sam:
+            d = ctx.sam_file_to_device(self.filename, contig_ranges=contig_ranges, sort=self.sort)
+            self._hdr = (d.ref_names, d.ref_lens)
+            return d
+        try:
+            d = ctx.bam_file_to_device(self.filename, contig_ranges=contig_ranges, sort=self.sort)      # inflate, record index (sort) and parse on the GPU
+            self._hdr = (d.ref_names, d.ref_lens)
+        except gpu.TcError:
+            # a file the device path refuses: the host reader names the broken member / record (or, should it
+            # read the file after all, feeds the device parse)
+            self._payload = bamio.read_bam_payload(self.filename)
+            d = ctx.bam_to_device(self._payload, contig_ranges=contig_ranges, sort=self.sort)
+            self._payload.release()     # the device holds the arrays now; the header stays
+        return d
 
     def pileup(self, *args, **kwargs):
         raise NotImplementedError("column iteration is not part of this implementation; "
@@ -220,7 +234,7 @@ def gff_by_contig(df: pd.DataFrame, names) -> dict:
 def Readbam(f, sort: bool = False):
     """indexing.py:6-19.  A handle passed in is returned as is, so one decoded copy of the BAM can
     serve BuildIndex, ListInserts and WriteOutputs.  ``sort``: accept records that are not coordinate-sorted and put them
-    in samtools' coordinate order on the GPU (``BamHandle``)."""
+    in samtools' coordinate order on the GPU (``BamHandle``).  A ``.sam`` path is read as SAM text, on the GPU."""
     if isinstance(f, BamHandle):
         return f
     return BamHandle(f, sort=sort)
