@@ -229,6 +229,28 @@ int  tc_bam_sort_records(tc_ctx_t* ctx, const uint8_t* payload, int64_t n_bytes,
                          int32_t n_ref, const uint8_t** payload_dev, const int64_t** rec_sorted_dev, int32_t* reordered,
                          void* stream);
 
+/* ---- amplicon primers soft-clipped off the aligned records (samtools ampliconclip --soft-clip; the rule: DESIGN §4) ----
+ * payload / rec_off as tc_bam_sort_records takes them (host or device).  The primers: n_primers rows of 0-based half-open
+ * [primer_start, primer_end) on reference primer_ref (host or device; 0 <= start < end, refs in [0, n_ref), else TC_ERR_ARG).
+ * tolerance >= 0; mode bit 0: check both ends of every read (else only the 5' end: left for forward, right for reverse reads).
+ * A placed, mapped record with an M / = / X op whose checked end lies under a primer loses those reference columns to a soft
+ * clip (pos, CIGAR, n_cigar_op, block_size and bin change); a record left without a match op is marked unmapped (FLAG 0x4,
+ * pos and CIGAR as they were).  Every other byte is copied.  *payload_dev / *rec_off_dev: the records in input order in a
+ * context buffer of their own (distinct from the payload, record and sorted-offset buffers; valid until the next decode on this
+ * context), *n_bytes_out their bytes; they feed tc_bam_sort_records, tc_bam_records_to_reads and tc_bam_contig_ranges as they
+ * are.  stats: records clipped on the left / on the right (that stay mapped), records fully clipped, reference columns removed.
+ * TC_ERR_ARG naming the record: a clipped CIGAR of more than 65535 ops; a mapped record with an M / = / X op whose CIGAR has
+ * an op of length 0 or an H / S op between other ops (the SAM spec allows neither).  Synchronises the stream once (twice
+ * when the primer rows are in device memory: they are read back first).
+ * n_reads == 0: the inputs are handed back as they are (*payload_dev = payload, which may be host memory, *n_bytes_out =
+ * n_bytes, *rec_off_dev = rec_off). */
+typedef struct tc_clip_stats { int64_t n_left, n_right, n_unmapped, n_columns; } tc_clip_stats_t;
+int  tc_bam_clip_primers(tc_ctx_t* ctx, const uint8_t* payload, int64_t n_bytes, const int64_t* rec_off, int64_t n_reads,
+                         int32_t n_ref, const int32_t* primer_ref, const int32_t* primer_start, const int32_t* primer_end,
+                         int32_t n_primers, int32_t tolerance, uint32_t mode /* bit 0: both ends */,
+                         const uint8_t** payload_dev, int64_t* n_bytes_out, const int64_t** rec_off_dev,
+                         tc_clip_stats_t* stats, void* stream);
+
 /* ---- SAM text straight from the aligner -> BAM records on the device ----
  * text[0 .. n_bytes): the SAM file (host or device memory); its records begin at first_line_off, which is file line
  * first_line_no (1-based) — the caller has read the '@' header lines and hands over the @SQ names in header order:

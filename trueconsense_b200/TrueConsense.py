@@ -7,6 +7,8 @@ validators and exit behaviour, same order of work — on top of the GPU hot path
 
     minimap2 -a ref.fa r.fq > s.sam
     python -m trueconsense_b200.TrueConsense --sort-input -i s.sam -ref ref.fa -gff f.gff -cov 30 -name S -o S.fasta
+    python -m trueconsense_b200.TrueConsense --primers scheme.primer.bed --primer-both-ends -i s.sam -ref ref.fa -gff f.gff \
+        -cov 30 -name S -o S.fasta
 
 ``main(args)`` is the console-script entry point of the reference (pyproject.toml:38-40).
 """
@@ -24,6 +26,7 @@ from .func import MyHelpFormatter, color
 from .indexing import (BuildIndex, BuildIndexContigs, Gffindex, Override_index_positions, Readbam, gff_by_contig,
                        read_override_index)
 from .Outputs import WriteOutputs, WriteOutputsContigs
+from .primers import read_bed
 from .version import __version__
 
 
@@ -94,12 +97,27 @@ def GetArgs(givenargs):
     opt.add_argument("--sort-input", action="store_true",
                      help="Accept a BAM or SAM whose records are not coordinate-sorted (e.g. straight from the aligner); they "
                           "are put in samtools' coordinate order on the GPU. A sorted file is used as written")
+    opt.add_argument("--primers", type=with_suffix("BED file", (".bed",), 1, "Primer file"), metavar="File",
+                     help="Amplicon primer scheme (BED: chrom, 0-based start, end). The primers are soft-clipped off the "
+                          "aligned reads on the GPU, as samtools ampliconclip --soft-clip does; implies --sort-input")
+    opt.add_argument("--primer-tolerance", type=int, default=None, metavar="N",
+                     help="Bases a read end may lie in front of a primer's start or behind its end and still match it "
+                          "(default 5; needs --primers)")
+    opt.add_argument("--primer-both-ends", action="store_true",
+                     help="Clip primers at both ends of every read (nanopore reads span the whole amplicon), not only at "
+                          "the 5' end (needs --primers)")
     opt.add_argument("--version", "-v", action="version", version=__version__,
                      help="Show the TrueConsense version and exit")
     opt.add_argument("--help", "-h", action="help", default=argparse.SUPPRESS, help="Show this help message and exit")
     opts = parser.parse_args(givenargs)
     if opts.all_contigs and opts.index_override:
         parser.error("--index-override cannot be combined with --all-contigs: its positions name no reference")
+    if opts.primers is None and (opts.primer_tolerance is not None or opts.primer_both_ends):
+        parser.error("--primer-tolerance and --primer-both-ends need --primers")
+    if opts.primer_tolerance is None:
+        opts.primer_tolerance = 5
+    elif opts.primer_tolerance < 0:
+        parser.error("--primer-tolerance must be 0 or more")
     return opts
 
 
@@ -139,7 +157,9 @@ def main(args: list[str] | None = None):
               "Use 'TrueConsense -h' to see the help document")
         sys.exit(1)
     opts = GetArgs(argv)
-    bam = Readbam(opts.input, sort=opts.sort_input)        # one decoded copy of the BAM serves the index and the insertion columns
+    primers = None if opts.primers is None else read_bed(opts.primers, opts.primer_tolerance, opts.primer_both_ends)
+    # one decoded copy of the BAM serves the index and the insertion columns
+    bam = Readbam(opts.input, sort=opts.sort_input, primers=primers)
     if opts.all_contigs:
         return _main_all_contigs(opts, bam)
     frame, gff = _index_and_features(opts, bam)

@@ -21,6 +21,7 @@ enum tc_slot {
     SLOT_CALL_E, SLOT_CALL_F, SLOT_INS_A, SLOT_INS_B, SLOT_INS_C, SLOT_INS_D, SLOT_INS_E, SLOT_INS_F, SLOT_INS_G,
     SLOT_TMP_A, SLOT_TMP_B, SLOT_TMP_C, SLOT_TILES, SLOT_SEGS, SLOT_COV_TOTALS, SLOT_BAM_PAYLOAD, SLOT_BAM_REC, SLOT_CIGAR16, SLOT_SEQ2, SLOT_SEQ_EXC_IDX, SLOT_SEQ_EXC_VAL, SLOT_BGZF_FILE, SLOT_BGZF_BLOCKS,
     SLOT_CONTIG_A, SLOT_CONTIG_B, SLOT_CONTIG_C, SLOT_BAM_REC_SORTED, SLOT_SAM_TEXT, SLOT_SAM_LINES, SLOT_SAM_META, SLOT_SAM_REFS,
+    SLOT_CLIP_PLAN, SLOT_CLIP_PAYLOAD, SLOT_CLIP_REC,
     SLOT_COUNT
 };
 

@@ -42,6 +42,10 @@ class BamStats(C.Structure):
                 ("sorted", C.c_int32), ("n_seq_words", C.c_int64), ("n_cigar_ops", C.c_int64)]
 
 
+class ClipStats(C.Structure):
+    _fields_ = [("n_left", C.c_int64), ("n_right", C.c_int64), ("n_unmapped", C.c_int64), ("n_columns", C.c_int64)]
+
+
 class CallParams(C.Structure):
     _fields_ = [("mincov", C.c_int32), ("include_ambig", C.c_int32), ("ambig_maxdist", C.c_double),
                 ("minority_del_pct", C.c_double), ("insert_pct", C.c_double)]
@@ -122,6 +126,9 @@ def lib() -> C.CDLL:
             l.tc_bam_records_to_reads.restype = C.c_int
             l.tc_bam_sort_records.argtypes = [vp, vp, i64, vp, i64, i32, C.POINTER(vp), C.POINTER(vp), C.POINTER(i32), vp]
             l.tc_bam_sort_records.restype = C.c_int
+            l.tc_bam_clip_primers.argtypes = [vp, vp, i64, vp, i64, i32, vp, vp, vp, i32, i32, C.c_uint32, C.POINTER(vp), C.POINTER(i64),
+                                              C.POINTER(vp), C.POINTER(ClipStats), vp]
+            l.tc_bam_clip_primers.restype = C.c_int
             l.tc_sam_to_bam_records.argtypes = [vp, vp, i64, i64, i64, i32, vp, vp, C.POINTER(vp), C.POINTER(i64), C.POINTER(vp),
                                                 C.POINTER(i64), C.POINTER(i64), C.POINTER(i64), C.POINTER(i64), C.POINTER(C.c_double), vp]
             l.tc_sam_to_bam_records.restype = C.c_int
@@ -307,33 +314,59 @@ class Context:
                                                   C.byref(moved), stream))
         return p.value, r.value, bool(moved.value)
 
-    def bam_to_device(self, payload, stream: int = 0, contig_ranges: bool = False, sort: bool = False) -> DeviceReads:
+    def clip_primers(self, payload_ptr, n_bytes: int, rec_ptr, n_reads: int, names, primers, stream: int = 0):
+        """``tc_bam_clip_primers``: the records (payload and refID offsets, host or device) with the primers of ``primers`` (a
+        ``primers.PrimerScheme``; its chrom names mapped to ``names``, the header's references) soft-clipped off.  Returns
+        (device payload, its bytes, device record offsets in input order, ``ClipStats``); the buffers stay valid until the next
+        decode on this context.  A chrom the header does not list is a ValueError."""
+        ref, start, end = primers.rows(names)
+        p, nb, r, st = C.c_void_p(), C.c_int64(0), C.c_void_p(), ClipStats()
+        self._check(self._lib.tc_bam_clip_primers(self._h, payload_ptr, n_bytes, rec_ptr, n_reads, len(names), ref.ctypes.data,
+                                                  start.ctypes.data, end.ctypes.data, len(primers), int(primers.tolerance),
+                                                  int(bool(primers.both_ends)), C.byref(p), C.byref(nb), C.byref(r), C.byref(st), stream))
+        return p.value, int(nb.value), r.value, st
+
+    @staticmethod
+    def _clip_info(st: "ClipStats", t: float) -> dict:
+        return {"n_clipped_left": int(st.n_left), "n_clipped_right": int(st.n_right), "n_fully_clipped": int(st.n_unmapped),
+                "clipped_columns": int(st.n_columns), "t_clip_s": t}
+
+    def bam_to_device(self, payload, stream: int = 0, contig_ranges: bool = False, sort: bool = False, primers=None) -> DeviceReads:
         """GPU-side record parsing (tc_bam_records_to_reads): a ``bamio.BamPayload`` (the BAM inflated on the host, its records
         indexed) becomes the flat read arrays in the context's device buffers — the CPU never touches a record's body.
         ``.stats`` of the result: aligned bases, longest span, sortedness, whether more than one reference occurs.
         ``sort``: records that are not sorted by (refID, pos) are put in samtools' coordinate order first
         (``tc_bam_sort_records``; the payload then travels to the device once); ``.info`` says whether they moved
-        (``reordered``) and what that took (``t_sort_s``)."""
+        (``reordered``) and what that took (``t_sort_s``).
+        ``primers`` (a ``primers.PrimerScheme``): the primers are soft-clipped off the records first (``tc_bam_clip_primers``)
+        and the clipped records are sorted (``sort`` is implied); ``.info`` then also holds the clip's counts and ``t_clip_s``."""
         import time
 
-        pay, rec, n = payload.payload_ptr, payload.rec_off_ptr, payload.n_reads
+        pay, rec, n, n_bytes = payload.payload_ptr, payload.rec_off_ptr, payload.n_reads, payload.n_bytes
         self._generation += 1
+        t0 = time.perf_counter()
+        clip = {}
+        if primers is not None:
+            pay, n_bytes, rec, cst = self.clip_primers(pay, n_bytes, rec, n, payload.ref_names, primers, stream)
+            clip = self._clip_info(cst, time.perf_counter() - t0)
+            sort = True
         t0 = time.perf_counter()
         moved = False
         if sort:
-            pay, rec, moved = self._sort_records(pay, payload.n_bytes, rec, n, len(payload.ref_lens), stream)
+            pay, rec, moved = self._sort_records(pay, n_bytes, rec, n, len(payload.ref_lens), stream)
         t1 = time.perf_counter()
         dev = TcReads()
         st = BamStats()
-        self._check(self._lib.tc_bam_records_to_reads(self._h, pay, payload.n_bytes, rec, n, C.byref(dev), C.byref(st), stream))
+        self._check(self._lib.tc_bam_records_to_reads(self._h, pay, n_bytes, rec, n, C.byref(dev), C.byref(st), stream))
         d = DeviceReads(dev, None, self, self._generation)
         d.stats = st
-        d.info = {"reordered": moved, "t_sort_s": t1 - t0}
+        d.info = {"reordered": moved, "t_sort_s": t1 - t0, **clip}
         if contig_ranges and payload.ref_names and not st.unsorted:
-            d.first_read = self._contig_ranges(pay, payload.n_bytes, rec, n, len(payload.ref_names), stream)
+            d.first_read = self._contig_ranges(pay, n_bytes, rec, n, len(payload.ref_names), stream)
         return d
 
-    def bam_file_to_device(self, path: str, stream: int = 0, contig_ranges: bool = False, sort: bool = False) -> DeviceReads:
+    def bam_file_to_device(self, path: str, stream: int = 0, contig_ranges: bool = False, sort: bool = False,
+                           primers=None) -> DeviceReads:
         """A BAM file to the flat read arrays in device memory with the GPU doing all of it: the host maps the file and walks
         the BGZF member headers (``bamio.map_bgzf``); the device inflates every member and checks its CRC-32
         (``tc_bgzf_inflate``), finds and proves the record offsets (``tc_bam_index_records``) and parses the records
@@ -343,7 +376,10 @@ class Context:
         payload and the record offsets are still in the context's buffers); left None for an unsorted file.
         ``sort``: a file whose records are not sorted by (refID, pos) has its record offsets put in samtools' coordinate order
         on the device before the parse (``tc_bam_sort_records``); a sorted file is parsed as written.  ``.info`` then tells
-        ``reordered`` and ``t_sort_s``."""
+        ``reordered`` and ``t_sort_s``.
+        ``primers`` (a ``primers.PrimerScheme``): the primers are soft-clipped off the records before the sort
+        (``tc_bam_clip_primers``), and the sort is implied: ``.info`` adds ``n_clipped_left``, ``n_clipped_right``,
+        ``n_fully_clipped``, ``clipped_columns`` and ``t_clip_s``.  A primer chrom the header does not list is a ValueError."""
         import time
 
         from . import bamio
@@ -375,15 +411,23 @@ class Context:
         t3 = time.perf_counter()
         info.update(n_records=int(n_records.value), n_dropped_unplaced=int(n_records.value - n_placed.value), t_map_s=t1 - t0,
                     t_inflate_s=t2 - t1, t_index_s=t3 - t2)
-        return self._records_to_device(payload, n_bytes, rec, n_placed.value, names, lens, info, stream, contig_ranges, sort)
+        return self._records_to_device(payload, n_bytes, rec, n_placed.value, names, lens, info, stream, contig_ranges, sort,
+                                       primers)
 
     def _records_to_device(self, payload, n_bytes: int, rec, n_placed: int, names, lens, info: dict, stream: int,
-                           contig_ranges: bool, sort: bool) -> DeviceReads:
-        """The tail of both file routes: BAM records in device memory (payload, offsets of the placed ones) -> sorted when
-        asked (``tc_bam_sort_records``), parsed (``tc_bam_records_to_reads``), the contig ranges -> ``DeviceReads`` with
-        ``.ref_names``, ``.ref_lens``, ``.stats`` and ``info`` plus the sort's and the parse's timings."""
+                           contig_ranges: bool, sort: bool, primers=None) -> DeviceReads:
+        """The tail of both file routes: BAM records in device memory (payload, offsets of the placed ones) -> primers
+        clipped when given (``tc_bam_clip_primers``, which implies the sort), sorted when asked (``tc_bam_sort_records``),
+        parsed (``tc_bam_records_to_reads``), the contig ranges -> ``DeviceReads`` with ``.ref_names``, ``.ref_lens``,
+        ``.stats`` and ``info`` plus the clip's, the sort's and the parse's timings."""
         import time
 
+        if primers is not None:
+            t = time.perf_counter()
+            payload, n_bytes, rec, cst = self.clip_primers(payload, n_bytes, rec, n_placed, names, primers, stream)
+            payload, rec = C.c_void_p(payload), C.c_void_p(rec)
+            info.update(self._clip_info(cst, time.perf_counter() - t))
+            sort = True
         t3 = time.perf_counter()
         moved = False
         if sort:
@@ -403,14 +447,16 @@ class Context:
         d.info = info
         return d
 
-    def sam_file_to_device(self, path: str, stream: int = 0, contig_ranges: bool = False, sort: bool = False) -> DeviceReads:
+    def sam_file_to_device(self, path: str, stream: int = 0, contig_ranges: bool = False, sort: bool = False,
+                           primers=None) -> DeviceReads:
         """A SAM file (an aligner's text output) to the flat read arrays in device memory, with the contract of
         :meth:`bam_file_to_device`: the host reads the ``@`` header lines (``bamio.read_sam_header``) and maps the file; the
         device turns every line into the BAM record ``samtools view -b`` would write for it (``tc_sam_to_bam_records``)
         and the BAM route's own steps follow (sort when asked, parse, contig ranges).  Lines with RNAME ``*`` are dropped
         and counted.  ``.info``: ``sam_bytes``, ``n_lines``, ``n_records``, ``n_dropped_unplaced``, ``reordered`` and the
         timings of each step (``t_map_s``, ``t_upload_s``, ``t_line_index_s``, ``t_convert_s``, ``t_sort_s``,
-        ``t_parse_s``).  A malformed line is ``OSError("<path>: line <k>: <reason>")``."""
+        ``t_parse_s``).  A malformed line is ``OSError("<path>: line <k>: <reason>")``.  ``primers``: as for
+        :meth:`bam_file_to_device`."""
         import mmap
         import time
 
@@ -451,7 +497,7 @@ class Context:
                 "n_dropped_unplaced": int(n_records.value - n_placed.value), "t_map_s": t1 - t0, "t_upload_s": steps[0],
                 "t_line_index_s": steps[1], "t_convert_s": steps[2]}
         return self._records_to_device(payload, int(n_payload.value), rec, int(n_placed.value), names, lens, info, stream,
-                                       contig_ranges, sort)
+                                       contig_ranges, sort, primers)
 
     def reads_to_contig_coords(self, reads: DeviceReads, ref_lens, first_read, names=None, stream: int = 0) -> np.ndarray:
         """Move device-resident reads to the global columns of a multi-reference pass, in place (``tc_reads_to_contig_coords``):

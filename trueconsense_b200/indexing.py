@@ -35,11 +35,19 @@ class BamHandle:
 
     A path ending in ``.sam`` is an aligner's text output: its lines become BAM records on the GPU
     (``gpu.Context.sam_file_to_device``) and take the BAM route from there, ``sort`` included.  There is no host decode of
-    SAM: ``reads`` raises ``NotImplementedError``, the device arrays are the product."""
+    SAM: ``reads`` raises ``NotImplementedError``, the device arrays are the product.
 
-    def __init__(self, filename: str, reads: ReadBatch | None = None, sort: bool = False):
+    ``primers`` (a ``primers.PrimerScheme``, ``primers.read_bed``): the amplicon primers are soft-clipped off the records on
+    the GPU before the sort (``tc_bam_clip_primers``), so every pass computes what it computes after ``samtools ampliconclip``
+    and ``samtools sort``; ``sort`` is then always on.  There is no host-side clip: ``reads`` raises
+    ``NotImplementedError``, and a handle made from a host ``ReadBatch`` cannot take primers (``ValueError``)."""
+
+    def __init__(self, filename: str, reads: ReadBatch | None = None, sort: bool = False, primers=None):
+        if primers is not None and reads is not None:
+            raise ValueError("primers are clipped on the GPU during the decode of a file; a host ReadBatch cannot take them")
         self.filename = filename
-        self.sort = sort
+        self.sort = sort or primers is not None
+        self.primers = primers
         self.is_sam = reads is None and pathlib.Path(filename).suffix == ".sam"
         self._reads = reads
         self._payload = None
@@ -56,6 +64,9 @@ class BamHandle:
                 if self.is_sam:
                     raise NotImplementedError(f"{self.filename}: a SAM file is decoded on the GPU only (device_reads); "
                                               "there are no host-side read arrays of it")
+                if self.primers is not None:
+                    raise NotImplementedError(f"{self.filename}: primers are clipped on the GPU only (device_reads); "
+                                              "there are no host-side read arrays of the clipped reads")
                 self._reads = bamio.read_bam(self.filename)
             return self._reads
 
@@ -152,17 +163,18 @@ class BamHandle:
     def _file_to_device(self, ctx, contig_ranges: bool = False):
         """The file's reads parsed into device memory (the caller holds the lock)."""
         if self.is_sam:
-            d = ctx.sam_file_to_device(self.filename, contig_ranges=contig_ranges, sort=self.sort)
+            d = ctx.sam_file_to_device(self.filename, contig_ranges=contig_ranges, sort=self.sort, primers=self.primers)
             self._hdr = (d.ref_names, d.ref_lens)
             return d
         try:
-            d = ctx.bam_file_to_device(self.filename, contig_ranges=contig_ranges, sort=self.sort)      # inflate, record index (sort) and parse on the GPU
+            # inflate, record index, (clip, sort) and parse on the GPU
+            d = ctx.bam_file_to_device(self.filename, contig_ranges=contig_ranges, sort=self.sort, primers=self.primers)
             self._hdr = (d.ref_names, d.ref_lens)
         except gpu.TcError:
             # a file the device path refuses: the host reader names the broken member / record (or, should it
             # read the file after all, feeds the device parse)
             self._payload = bamio.read_bam_payload(self.filename)
-            d = ctx.bam_to_device(self._payload, contig_ranges=contig_ranges, sort=self.sort)
+            d = ctx.bam_to_device(self._payload, contig_ranges=contig_ranges, sort=self.sort, primers=self.primers)
             self._payload.release()     # the device holds the arrays now; the header stays
         return d
 
@@ -231,13 +243,14 @@ def gff_by_contig(df: pd.DataFrame, names) -> dict:
     return {n: df[df["seqid"] == n].reset_index(drop=True) for n in names}
 
 
-def Readbam(f, sort: bool = False):
+def Readbam(f, sort: bool = False, primers=None):
     """indexing.py:6-19.  A handle passed in is returned as is, so one decoded copy of the BAM can
     serve BuildIndex, ListInserts and WriteOutputs.  ``sort``: accept records that are not coordinate-sorted and put them
-    in samtools' coordinate order on the GPU (``BamHandle``).  A ``.sam`` path is read as SAM text, on the GPU."""
+    in samtools' coordinate order on the GPU (``BamHandle``).  A ``.sam`` path is read as SAM text, on the GPU.
+    ``primers`` (``primers.read_bed``): the amplicon primers are soft-clipped off the reads on the GPU (implies ``sort``)."""
     if isinstance(f, BamHandle):
         return f
-    return BamHandle(f, sort=sort)
+    return BamHandle(f, sort=sort, primers=primers)
 
 
 class _GffHeader:
