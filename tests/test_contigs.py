@@ -2,61 +2,21 @@
 WriteOutputsContigs, tc_call_contigs): each reference's results equal what the single-reference path computes for a BAM
 holding only that reference's records (mates elsewhere still "on another reference"), the FASTA record of its name, its
 GFF rows and the sample name {sample}_{reference}.  The fixtures are built here from seeded synthetic reads."""
-import gzip
 import os
 import struct
-import zlib
 
 import numpy as np
 import pytest
 
+from bamfiles import bam_header, bgzf, split
 from conftest import GOLD
 
 
 # ---------------------------------------------------------------------------- fixture helpers (host only)
-def _bgzf(path: str, payload: bytes, member_bytes: int = 65280) -> None:
-    """Write a BAM payload as BGZF members (and the EOF member)."""
-    def member(chunk):
-        c = zlib.compressobj(1, zlib.DEFLATED, -15, 8, 0)
-        data = c.compress(chunk) + c.flush()
-        bsize = 18 + len(data) + 8
-        return (bytes([31, 139, 8, 4, 0, 0, 0, 0, 0, 255]) + struct.pack("<H", 6) + b"BC" + struct.pack("<HH", 2, bsize - 1) + data +
-                struct.pack("<II", zlib.crc32(chunk) & 0xFFFFFFFF, len(chunk)))
-
-    out = [member(payload[p:p + member_bytes]) for p in range(0, len(payload), member_bytes)]
-    out.append(member(b""))
-    with open(path, "wb") as fh:
-        fh.write(b"".join(out))
-
-
-def _records(path: str) -> list[bytes]:
-    """The records of a BAM file, each with its block_size."""
-    from trueconsense_b200 import bamio
-
-    with gzip.open(path, "rb") as fh:
-        payload = fh.read()
-    _, _, q = bamio.parse_bam_header(payload, len(payload))
-    recs = []
-    while q + 4 <= len(payload):
-        bs = struct.unpack_from("<i", payload, q)[0]
-        recs.append(payload[q:q + 4 + bs])
-        q += 4 + bs
-    return recs
-
-
 def _unplaced(k: int) -> bytes:
     name = b"unplaced%04d\0" % k
     body = struct.pack("<iiBBHHHIiii", -1, -1, len(name), 0, 4680, 0, 4, 6, -1, -1, 0) + name + bytes([0x12, 0x48, 0x21]) + bytes([30] * 6)
     return struct.pack("<i", len(body)) + body
-
-
-def _header(refs) -> bytes:
-    text = b"@HD\tVN:1.6\tSO:coordinate\n"
-    h = b"BAM\1" + struct.pack("<i", len(text)) + text + struct.pack("<i", len(refs))
-    for n, l in refs:
-        nb = n.encode() + b"\0"
-        h += struct.pack("<i", len(nb)) + nb + struct.pack("<i", l)
-    return h
 
 
 def _multi_bam(path, contigs, extra_refs=(), unplaced_every=0, order=None):
@@ -66,7 +26,7 @@ def _multi_bam(path, contigs, extra_refs=(), unplaced_every=0, order=None):
     n = len(contigs)
     body = []
     for k in (order or range(n)):
-        for r in _records(contigs[k]["bam"]):
+        for r in split(contigs[k]["bam"])[1]:
             r = bytearray(r)
             mtid = struct.unpack_from("<i", r, 24)[0]
             struct.pack_into("<i", r, 4, k)
@@ -78,7 +38,7 @@ def _multi_bam(path, contigs, extra_refs=(), unplaced_every=0, order=None):
     if unplaced_every:
         body += [_unplaced(90000 + j) for j in range(3)]
     refs = [(c["name"], c["bam_len"]) for c in contigs] + list(extra_refs)
-    _bgzf(path, _header(refs) + b"".join(body))
+    bgzf(path, bam_header([(n.encode(), l) for n, l in refs]) + b"".join(body))
 
 
 def _with_mates(b, rng, frac_other):

@@ -4,22 +4,18 @@ The CPU tests pin the rule (DESIGN §4) through ``oracle/primer_clip.py`` with h
 CIGARs, and check the BED reader and the flags.  The GPU tests compare the clip's record bytes with the oracle's, and every
 decode route with primers against the plain decode of a BAM this file writes from the oracle's clipped and sorted records —
 down to the CLI's four output files."""
-import json
 import os
 import struct
 
 import numpy as np
 import pytest
 
+from bamfiles import (assert_same_arrays, bam_header, bam_to_sam, dev_arrays, mini_argv, multi_ref_files, run_cli, sam_header,
+                      sam_line, sam_record, split, write)
 from conftest import GOLD
 from oracle import primer_clip as pc
-from test_sam_input import _sam_header, sam_line
-from test_sort_input import _multi_ref_files, _split, _write
 
 MINIS = ("quirk", "mini_illumina", "mini_ont", "mini_long", "mini_overlap")
-FIELDS = (("pos", np.int32), ("flag", np.uint16), ("mapq", np.uint8), ("l_seq", np.int32), ("seq_off", np.uint32),
-          ("cigar_off", np.uint32), ("seq4", np.uint32), ("qual", np.uint8), ("cigar", np.uint32), ("qname_hash", np.uint64),
-          ("mpos", np.int32), ("isize", np.int32))
 OPS = "MIDNSHP=X"
 
 
@@ -57,14 +53,6 @@ def kat(cigar, pos, primers, flag=0, t=5, both=False):
     return _str(f["cigar"]), f["pos"], kind
 
 
-def _bam_header(refs):
-    text = b"@HD\tVN:1.6\tSO:coordinate\n"
-    head = b"BAM\1" + struct.pack("<i", len(text)) + text + struct.pack("<i", len(refs))
-    for n, l in refs:
-        head += struct.pack("<i", len(n) + 1) + n + b"\0" + struct.pack("<i", l)
-    return head
-
-
 def _write_bed(path, rows, extra=""):
     with open(path, "w") as fh:
         fh.write("".join(f"{c}\t{s}\t{e}{extra}\n" for c, s, e in rows))
@@ -78,7 +66,7 @@ def _placed(recs):
 def _oracle_file(src_recs, head, rows, dst, tol=5, both=False):
     """The oracle's clipped and sorted records written as a BAM; returns (path, stats)."""
     out, st = pc.clip_and_sort(_placed(src_recs), rows, tol, both)
-    _write(dst, head, out)
+    write(dst, head, out)
     return dst, st
 
 
@@ -384,21 +372,6 @@ def ctx():
     return gpu.default_context()
 
 
-def _dev_arrays(ctx, d):
-    s, n = d.struct, d.n_reads
-    if n == 0:
-        return {}
-    sizes = {"seq_off": n + 1, "cigar_off": n + 1, "seq4": d.stats.n_seq_words, "qual": 8 * d.stats.n_seq_words,
-             "cigar": d.stats.n_cigar_ops}
-    return {f: ctx.download(getattr(s, f), sizes.get(f, n), t) for f, t in FIELDS}
-
-
-def _assert_same(a, b, what=""):
-    assert a.keys() == b.keys(), what
-    for f in a:
-        assert np.array_equal(a[f], b[f]), (what, f)
-
-
 def _scheme(path, rows, names, tol=5, both=False):
     from trueconsense_b200 import primers
 
@@ -426,40 +399,38 @@ def test_record_bytes(ctx, seed, both, tol, tmp_path):
     give the arrays of the oracle's clipped and sorted records, and the oracle's stats."""
     refs, recs, rows = random_records(seed)
     names = [n.decode() for n, _ in refs]
-    head = _bam_header(refs)
+    head = bam_header(refs)
     sch = _scheme(tmp_path / "s.bed", rows, names, tol, both)
     want, want_st = pc.clip_records(recs, rows, tol, both)
     got, st = _clip_host(ctx, head, recs, names, sch)
     assert st == want_st and want_st["n_left"] + want_st["n_right"] > 100
     for i, (g, w) in enumerate(zip(got, want)):
         assert g == w, (i, pc.parse(recs[i])["cigar"], pc.parse(g)["cigar"], pc.parse(w)["cigar"])
-    src = _write(str(tmp_path / "in.bam"), head, recs, (65280, 3000))
+    src = write(str(tmp_path / "in.bam"), head, recs, (65280, 3000))
     exp_bam, st2 = _oracle_file(recs, head, rows, str(tmp_path / "oracle.bam"), tol, both)
     assert st2 == want_st
-    want_arr = _dev_arrays(ctx, ctx.bam_file_to_device(exp_bam))
+    want_arr = dev_arrays(ctx, ctx.bam_file_to_device(exp_bam))
     d = ctx.bam_file_to_device(src, primers=sch)
     assert _stats(d.info) == want_st and d.info["t_clip_s"] > 0
-    _assert_same(_dev_arrays(ctx, d), want_arr, "bam")
+    assert_same_arrays(dev_arrays(ctx, d), want_arr, "bam")
     from trueconsense_b200 import bamio
 
     payload = bamio.read_bam_payload(src)
     h = ctx.bam_to_device(payload, primers=sch)
     payload.release()
     assert _stats(h.info) == want_st
-    _assert_same(_dev_arrays(ctx, h), want_arr, "host payload")
+    assert_same_arrays(dev_arrays(ctx, h), want_arr, "host payload")
     # SAM: the records the SAM route builds (bin 0, no optional fields), clipped by the oracle
-    from test_sam_input import sam_record
-
     lines = [sam_line(r, [n for n, _ in refs]) for r in recs]
     sam = str(tmp_path / "in.sam")
     with open(sam, "wb") as fh:
-        fh.write(_sam_header(refs) + b"".join(lines))
+        fh.write(sam_header(refs) + b"".join(lines))
     sam_recs = [sam_record(l, [n for n, _ in refs]) for l in lines]
     exp_sam, st3 = _oracle_file(sam_recs, head, rows, str(tmp_path / "oracle_sam.bam"), tol, both)
-    want_sam = _dev_arrays(ctx, ctx.bam_file_to_device(exp_sam))
+    want_sam = dev_arrays(ctx, ctx.bam_file_to_device(exp_sam))
     s = ctx.sam_file_to_device(sam, primers=sch)
     assert _stats(s.info) == st3 == want_st
-    _assert_same(_dev_arrays(ctx, s), want_sam, "sam")
+    assert_same_arrays(dev_arrays(ctx, s), want_sam, "sam")
 
 
 def _mini_scheme(name, tmp):
@@ -472,22 +443,6 @@ def _mini_scheme(name, tmp):
     return names, rows, _write_bed(os.path.join(tmp, f"{name}.bed"), [(names[r], s, e) for r, s, e in rows])
 
 
-def _cli(argv, out, monkeypatch):
-    from trueconsense_b200 import TrueConsense
-
-    monkeypatch.setattr("sys.argv", ["TrueConsense", "<cli>"])
-    try:
-        TrueConsense.main(argv + ["-o", out + ".fasta", "-vcf", out + ".vcf", "-ogff", out + ".gff", "-doc", out + ".tsv", "-t", "2"])
-    except Exception as e:          # the reference's own exceptions (e.g. KeyError) must match too
-        return type(e).__name__
-    return {e: open(f"{out}.{e}").read() if os.path.exists(f"{out}.{e}") else None for e in ("fasta", "vcf", "gff", "tsv")}
-
-
-def _mini_argv(name, path):
-    mincov = json.load(open(f"{GOLD}/{name}.json"))["mincov"]
-    return ["-i", path, "-ref", f"{GOLD}/{name}.fasta", "-gff", f"{GOLD}/{name}.gff", "-cov", str(mincov), "-name", name]
-
-
 @pytest.mark.gpu
 @pytest.mark.parametrize("both", [False, True])
 @pytest.mark.parametrize("name", MINIS)
@@ -498,24 +453,22 @@ def test_goldens_with_a_scheme(ctx, name, both, tmp_path, monkeypatch):
     tmp = str(tmp_path)
     names, rows, bed = _mini_scheme(name, tmp)
     src = f"{GOLD}/{name}.bam"
-    head, recs = _split(src)
+    head, recs = split(src)
     exp, st = _oracle_file(recs, head, rows, os.path.join(tmp, "oracle.bam"), 5, both)
     d = ctx.bam_file_to_device(src, primers=primers.read_bed(bed, 5, both))
     assert _stats(d.info) == st and st["n_left"] + st["n_right"] > 0
-    _assert_same(_dev_arrays(ctx, d), _dev_arrays(ctx, ctx.bam_file_to_device(exp)), name)
+    assert_same_arrays(dev_arrays(ctx, d), dev_arrays(ctx, ctx.bam_file_to_device(exp)), name)
     flags = ["--primers", bed] + (["--primer-both-ends"] if both else [])
-    got = _cli(flags + _mini_argv(name, src), os.path.join(tmp, "p"), monkeypatch)
-    want = _cli(_mini_argv(name, exp), os.path.join(tmp, "o"), monkeypatch)
+    got = run_cli(flags + mini_argv(name, src), os.path.join(tmp, "p"), monkeypatch)
+    want = run_cli(mini_argv(name, exp), os.path.join(tmp, "o"), monkeypatch)
     assert got == want
     # the same records as a shuffled SAM; the oracle clips them in that order (ties of the sort keep it)
-    from test_sam_input import bam_to_sam
-
     perm = np.random.default_rng(7).permutation(len(recs))
     sam = bam_to_sam(src, os.path.join(tmp, "shuf.sam"), aux=True, order=perm)
     exp_sam, st_sam = _oracle_file([recs[i] for i in perm], head, rows, os.path.join(tmp, "oracle_sam.bam"), 5, both)
     assert st_sam == st
-    got = _cli(flags + _mini_argv(name, sam), os.path.join(tmp, "s"), monkeypatch)
-    assert got == _cli(_mini_argv(name, exp_sam), os.path.join(tmp, "os"), monkeypatch)
+    got = run_cli(flags + mini_argv(name, sam), os.path.join(tmp, "s"), monkeypatch)
+    assert got == run_cli(mini_argv(name, exp_sam), os.path.join(tmp, "os"), monkeypatch)
 
 
 def _amplicon_pairs(tmp, L=1500, width=320, step=280, read_len=190, ins_at=None):
@@ -563,17 +516,17 @@ def test_amplicon_pairs_with_insertions_in_mate_overlaps(ctx, tmp_path, monkeypa
     tmp = str(tmp_path)
     src, rows = _amplicon_pairs(tmp)
     bed = _write_bed(os.path.join(tmp, "amp.bed"), [("ref", s, e) for _, s, e in rows], "\tamp\t1\t+")
-    head, recs = _split(src)
+    head, recs = split(src)
     for both in (False, True):
         exp, st = _oracle_file(recs, head, rows, os.path.join(tmp, f"oracle{both}.bam"), 5, both)
         assert st["n_left"] > 0 and st["n_right"] > 0
         d = ctx.bam_file_to_device(src, primers=primers.read_bed(bed, 5, both))
         assert _stats(d.info) == st
-        _assert_same(_dev_arrays(ctx, d), _dev_arrays(ctx, ctx.bam_file_to_device(exp)))
+        assert_same_arrays(dev_arrays(ctx, d), dev_arrays(ctx, ctx.bam_file_to_device(exp)))
         argv = ["-ref", os.path.join(tmp, "amp.fasta"), "-gff", os.path.join(tmp, "amp.gff"), "-cov", "10", "-name", "A"]
         flags = ["--primers", bed] + (["--primer-both-ends"] if both else [])
-        got = _cli(flags + ["-i", src] + argv, os.path.join(tmp, f"p{both}"), monkeypatch)
-        want = _cli(["-i", exp] + argv, os.path.join(tmp, f"o{both}"), monkeypatch)
+        got = run_cli(flags + ["-i", src] + argv, os.path.join(tmp, f"p{both}"), monkeypatch)
+        want = run_cli(["-i", exp] + argv, os.path.join(tmp, f"o{both}"), monkeypatch)
         assert isinstance(got, dict) and got == want
         assert sum(1 for l in got["vcf"].splitlines() if l and not l.startswith("#") and len(l.split("\t")[4]) > 1) >= 1
 
@@ -583,7 +536,7 @@ def test_all_contigs_each_reference_its_scheme(ctx, tmp_path, monkeypatch):
     from trueconsense_b200 import primers
 
     tmp = str(tmp_path)
-    head, real, slots, fasta, gff = _multi_ref_files(tmp, n_decoys=4)
+    head, real, slots, fasta, gff = multi_ref_files(tmp, n_decoys=4)
     rows, bed_rows = [], []
     for i in slots:
         L = len(real[i]["seq"])
@@ -592,15 +545,15 @@ def test_all_contigs_each_reference_its_scheme(ctx, tmp_path, monkeypatch):
             bed_rows += [(real[i]["name"], a, a + 20), (real[i]["name"], a + 180, a + 200)]
     bed = _write_bed(os.path.join(tmp, "multi.bed"), bed_rows)
     body = [r for i in slots for r in real[i]["recs"]]
-    src = _write(os.path.join(tmp, "multi.bam"), head, body)
+    src = write(os.path.join(tmp, "multi.bam"), head, body)
     exp, st = _oracle_file(body, head, rows, os.path.join(tmp, "oracle.bam"), 5, True)
     d = ctx.bam_file_to_device(src, primers=primers.read_bed(bed, 5, True), contig_ranges=True)
     assert _stats(d.info) == st
     want = ctx.bam_file_to_device(exp, contig_ranges=True)
     assert d.first_read.tolist() == want.first_read.tolist()
     base = ["-ref", fasta, "-gff", gff, "-cov", "30", "-name", "S", "--all-contigs"]
-    got = _cli(["--primers", bed, "--primer-both-ends", "-i", src] + base, os.path.join(tmp, "p"), monkeypatch)
-    exp_out = _cli(["-i", exp] + base, os.path.join(tmp, "o"), monkeypatch)
+    got = run_cli(["--primers", bed, "--primer-both-ends", "-i", src] + base, os.path.join(tmp, "p"), monkeypatch)
+    exp_out = run_cli(["-i", exp] + base, os.path.join(tmp, "o"), monkeypatch)
     assert isinstance(got, dict) and got == exp_out
     # a primer row on a chrom the header does not list
     bad = _write_bed(os.path.join(tmp, "bad.bed"), bed_rows + [("nowhere", 1, 5)])
@@ -614,14 +567,14 @@ def test_no_op_scheme_and_empty_scheme(ctx, tmp_path):
 
     src = f"{GOLD}/mini_illumina.bam"
     names, lens = bamio.read_bam_header(src)
-    plain = _dev_arrays(ctx, ctx.bam_file_to_device(src))
+    plain = dev_arrays(ctx, ctx.bam_file_to_device(src))
     far = primers.read_bed(_write_bed(tmp_path / "far.bed", [(names[0], lens[0] + 100, lens[0] + 120)]), 5, True)
     d = ctx.bam_file_to_device(src, primers=far)
     assert _stats(d.info) == dict(n_left=0, n_right=0, n_unmapped=0, n_columns=0) and d.info["reordered"] is False
-    _assert_same(_dev_arrays(ctx, d), plain)
+    assert_same_arrays(dev_arrays(ctx, d), plain)
     (tmp_path / "empty.bed").write_text("")
     d = ctx.bam_file_to_device(src, primers=primers.read_bed(str(tmp_path / "empty.bed")))
-    _assert_same(_dev_arrays(ctx, d), plain)
+    assert_same_arrays(dev_arrays(ctx, d), plain)
 
 
 @pytest.mark.gpu
@@ -642,11 +595,11 @@ def test_size_200k_config2_amplicons(ctx, tmp_path):
         st = room * a // (p.n_amplicons - 1)
         rows += [(0, st, st + 24), (0, st + p.read_len - 24, st + p.read_len)]
     bed = _write_bed(tmp_path / "cfg2.bed", [("ref", s, e) for _, s, e in rows])
-    head, recs = _split(src)
+    head, recs = split(src)
     exp, st = _oracle_file(recs, head, rows, str(tmp_path / "oracle.bam"), 5, True)
     d = ctx.bam_file_to_device(src, primers=primers.read_bed(bed, 5, True))
     assert d.n_reads == 200_000 and _stats(d.info) == st and st["n_left"] > 100_000
-    _assert_same(_dev_arrays(ctx, d), _dev_arrays(ctx, ctx.bam_file_to_device(exp)))
+    assert_same_arrays(dev_arrays(ctx, d), dev_arrays(ctx, ctx.bam_file_to_device(exp)))
 
 
 @pytest.mark.gpu
@@ -658,7 +611,7 @@ def test_too_many_ops_after_the_clip(ctx, tmp_path):
     recs = [make_rec(100, "50M", name=b"a"), make_rec(100, ops, name=b"b")]
     sch = primers.read_bed(_write_bed(tmp_path / "s.bed", [("chr1", 95, 110)]))
     with pytest.raises(gpu.TcError) as ei:
-        _clip_host(ctx, _bam_header([(b"chr1", 200000)]), recs, ["chr1"], sch)
+        _clip_host(ctx, bam_header([(b"chr1", 200000)]), recs, ["chr1"], sch)
     assert ei.value.code == -2 and "record 1 " in str(ei.value)
 
 
@@ -669,7 +622,7 @@ def test_cigars_the_rule_does_not_cover(ctx, tmp_path):
     from trueconsense_b200 import gpu, primers
 
     sch = primers.read_bed(_write_bed(tmp_path / "s.bed", [("chr1", 95, 110)]))
-    head = _bam_header([(b"chr1", 5000)])
+    head = bam_header([(b"chr1", 5000)])
     for bad in ("10M5S40M", "10M2H40M", [(0, 10), (2, 0), (0, 40)]):
         recs = [make_rec(100, "50M", name=b"a"), make_rec(100, "50M", name=b"b"), make_rec(3000, bad, name=b"c")]
         with pytest.raises(gpu.TcError) as ei:

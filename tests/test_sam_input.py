@@ -3,190 +3,43 @@ into the BAM record ``samtools view -b`` would write and the BAM route's steps f
 BAM route computes for the same records.  The SAM inputs are written here at test time: from a BAM's records as
 ``samtools view -h`` prints them (``sam_line``), or by hand; a small SAM -> BAM encoder (``sam_record``) restates the
 conversion rules for hand-written lines, so each device result is compared with the BAM route over the encoded file."""
-import gzip
 import json
 import os
 import re
 import struct
-import zlib
 
 import numpy as np
 import pytest
 
+from bamfiles import (MM2_AUX, assert_same_arrays, bam_header, bam_to_sam, bgzf, dev_arrays, mini_argv, refs_of, run_cli, sam_header,
+                      sam_line, sam_record, split)
 from conftest import GOLD, load_golden_counts
 
 MINIS = ("quirk", "mini_illumina", "mini_ont", "mini_long", "mini_overlap")
-FIELDS = (("pos", np.int32), ("flag", np.uint16), ("mapq", np.uint8), ("l_seq", np.int32), ("seq_off", np.uint32),
-          ("cigar_off", np.uint32), ("seq4", np.uint32), ("qual", np.uint8), ("cigar", np.uint32), ("qname_hash", np.uint64),
-          ("mpos", np.int32), ("isize", np.int32))
 STATS = ("aligned_bases", "max_ref_span", "unsorted", "multi_contig", "sorted", "n_seq_words", "n_cigar_ops")
-OPS = b"MIDNSHP=X"
-NT16 = b"=ACMGRSVTWYHKDBN"
-_HI = bytes(NT16[b >> 4] for b in range(256))
-_LO = bytes(NT16[b & 15] for b in range(256))
-_Q33 = bytes((b + 33) & 0xFF for b in range(256))
-MM2_AUX = b"\tNM:i:%d\tms:i:372\tAS:i:372\tnn:i:0\ttp:A:P\tcm:i:41\ts1:i:355\ts2:i:0\tde:f:0.0123\trl:i:0"
 
 
 # ---------------------------------------------------------------------------- fixture helpers (host only)
-def _bgzf(path, payload: bytes, member_bytes=(65280,)) -> None:
-    """Write a BAM payload as BGZF members of the given payload sizes (cycled), and the EOF member."""
-    def member(chunk):
-        c = zlib.compressobj(1, zlib.DEFLATED, -15, 8, 0)
-        data = c.compress(chunk) + c.flush()
-        return (bytes([31, 139, 8, 4, 0, 0, 0, 0, 0, 255]) + struct.pack("<H", 6) + b"BC" + struct.pack("<HH", 2, 18 + len(data) + 7) +
-                data + struct.pack("<II", zlib.crc32(chunk) & 0xFFFFFFFF, len(chunk)))
-
-    out, p, k = [], 0, 0
-    while p < len(payload):
-        n = member_bytes[k % len(member_bytes)]
-        out.append(member(payload[p:p + n]))
-        p, k = p + n, k + 1
-    out.append(member(b""))
-    with open(path, "wb") as fh:
-        fh.write(b"".join(out))
-
-
-def _split(path):
-    """(header bytes, reference names as bytes, [records with their block_size]) of a BAM file."""
-    from trueconsense_b200 import bamio
-
-    with gzip.open(path, "rb") as fh:
-        payload = fh.read()
-    names, _, q = bamio.parse_bam_header(payload, len(payload))
-    head, recs = payload[:q], []
-    while q + 4 <= len(payload):
-        bs = struct.unpack_from("<i", payload, q)[0]
-        recs.append(payload[q:q + 4 + bs])
-        q += 4 + bs
-    return head, [n.encode() for n in names], recs
-
-
-def _bam_header(refs, text=b"@HD\tVN:1.6\tSO:coordinate\n"):
-    head = b"BAM\1" + struct.pack("<i", len(text)) + text + struct.pack("<i", len(refs))
-    for n, l in refs:
-        head += struct.pack("<i", len(n) + 1) + n + b"\0" + struct.pack("<i", l)
-    return head
-
-
-def _sam_header(refs, text=b"@HD\tVN:1.6\tSO:coordinate\n"):
-    return text + b"".join(b"@SQ\tSN:%s\tLN:%d\n" % (n, l) for n, l in refs) + b"@PG\tID:minimap2\tPN:minimap2\tVN:2.28\n"
-
-
-def _refs_of(head):
-    from trueconsense_b200 import bamio
-
-    names, lens, _ = bamio.parse_bam_header(head, len(head))
-    return [(n.encode(), l) for n, l in zip(names, lens)]
-
-
-def sam_line(r: bytes, names, aux=b"", lower=False) -> bytes:
-    """A BAM record (block_size included) as ``samtools view`` prints it (its optional fields replaced by ``aux``)."""
-    tid, pos, l_name, mapq, _, n_cig, flag, l_seq, mtid, mpos, tlen = struct.unpack_from("<iiBBHHHiiii", r, 4)
-    p = 36
-    qname = r[p:p + l_name - 1]
-    p += l_name
-    cig = struct.unpack_from(f"<{n_cig}I", r, p)
-    p += 4 * n_cig
-    sb = (l_seq + 1) // 2
-    packed = r[p:p + sb]
-    qual = r[p + sb:p + sb + l_seq]
-    seq = bytearray(2 * sb)
-    seq[0::2] = packed.translate(_HI)
-    seq[1::2] = packed.translate(_LO)
-    seq = bytes(seq[:l_seq]) or b"*"
-    if lower:
-        seq = seq.lower()
-    q = b"*" if not l_seq or qual[0] == 0xFF else qual.translate(_Q33)
-    cigar = b"".join(b"%d%c" % (c >> 4, OPS[c & 15]) for c in cig) or b"*"
-    rnext = b"*" if mtid < 0 else b"=" if mtid == tid else names[mtid]
-    return b"\t".join([qname, b"%d" % flag, names[tid] if tid >= 0 else b"*", b"%d" % (pos + 1), b"%d" % mapq, cigar, rnext,
-                       b"%d" % (mpos + 1), b"%d" % tlen, seq, q]) + aux + b"\n"
-
-
-def sam_record(line: bytes, names):
-    """The BAM record (block_size included, ``bin`` 0, no optional fields) of a valid SAM line; None for RNAME '*'."""
-    f = line.rstrip(b"\n").split(b"\t")
-    qname, flag, rname, pos, mapq, cigar, rnext, pnext, tlen, seq, qual = f[:11]
-    index = {n: i for i, n in enumerate(names)}
-    if rname == b"*":
-        return None
-    tid = index[rname]
-    mtid = tid if rnext == b"=" else -1 if rnext == b"*" else index[rnext]
-    ops = [] if cigar == b"*" else [int(n) << 4 | OPS.index(o) for n, o in re.findall(rb"(\d+)([MIDNSHP=X])", cigar)]
-    seq = b"" if seq == b"*" else seq
-    codes = [NT16.find(bytes([c]).upper()) % 16 if bytes([c]).upper() in NT16 else 15 for c in seq] + [0]
-    packed = bytes(codes[i] << 4 | codes[i + 1] for i in range(0, len(seq), 2))
-    q = b"\xff" * len(seq) if qual == b"*" else bytes(c - 33 for c in qual)
-    body = (struct.pack("<iiBBHHHiiii", tid, int(pos) - 1, len(qname) + 1, int(mapq), 0, len(ops), int(flag), len(seq), mtid,
-                        int(pnext) - 1, int(tlen)) + qname + b"\0" + struct.pack(f"<{len(ops)}I", *ops) + packed + q)
-    return struct.pack("<i", len(body)) + body
-
-
-def bam_to_sam(bam, sam, aux=False, lower=False, order=None, newline_at_end=True):
-    """A BAM file written as SAM (header with @SQ lines, every record; ``order``: the records in that order), each line with
-    minimap2-like optional fields (``aux``) and lower-case SEQ (``lower``) when asked."""
-    head, names, recs = _split(bam)
-    lines = [sam_line(r, names, MM2_AUX % (i % 7) if aux else b"", lower) for i, r in enumerate(recs)]
-    if order is not None:
-        lines = [lines[i] for i in order]
-    body = b"".join(lines)
-    if not newline_at_end:
-        body = body[:-1]
-    with open(sam, "wb") as fh:
-        fh.write(_sam_header(_refs_of(head)) + body)
-    return sam
-
-
 def write_pair(tmp, stem, refs, lines, newline_at_end=True):
     """Hand-written SAM lines as a .sam file and, encoded by ``sam_record``, as a .bam file (RNAME '*' lines left out)."""
     names = [n for n, _ in refs]
     sam, bam = os.path.join(tmp, stem + ".sam"), os.path.join(tmp, stem + ".bam")
     body = b"".join(lines)
     with open(sam, "wb") as fh:
-        fh.write(_sam_header(refs) + (body if newline_at_end else body[:-1]))
+        fh.write(sam_header(refs) + (body if newline_at_end else body[:-1]))
     recs = [r for r in (sam_record(l, names) for l in lines) if r is not None]
-    _bgzf(bam, _bam_header(refs) + b"".join(recs))
+    bgzf(bam, bam_header(refs) + b"".join(recs))
     return sam, bam
 
 
-def _dev_arrays(ctx, d):
-    """Every array of device reads, on the host (taken before the context stages anything else)."""
-    s, n = d.struct, d.n_reads
-    if n == 0:
-        return {}
-    sizes = {"seq_off": n + 1, "cigar_off": n + 1, "seq4": d.stats.n_seq_words, "qual": 8 * d.stats.n_seq_words,
-             "cigar": d.stats.n_cigar_ops}
-    return {f: ctx.download(getattr(s, f), sizes.get(f, n), t) for f, t in FIELDS}
-
-
 def _snapshot(ctx, d):
-    return (_dev_arrays(ctx, d), {k: getattr(d.stats, k) for k in STATS}, d.ref_names, d.ref_lens,
+    return (dev_arrays(ctx, d), {k: getattr(d.stats, k) for k in STATS}, d.ref_names, d.ref_lens,
             d.info["n_records"], d.info["n_dropped_unplaced"], None if d.first_read is None else d.first_read.tolist())
 
 
 def _assert_same(a, b, what=""):
-    assert a[0].keys() == b[0].keys(), what
-    for f in a[0]:
-        assert np.array_equal(a[0][f], b[0][f]), (what, f)
+    assert_same_arrays(a[0], b[0], what)
     assert a[1:] == b[1:], what
-
-
-def _cli(argv, out, monkeypatch):
-    """main(argv) writing {out}.{ext}: the files' text, or the exception type's name."""
-    from trueconsense_b200 import TrueConsense
-
-    monkeypatch.setattr("sys.argv", ["TrueConsense", "<cli>"])
-    try:
-        TrueConsense.main(argv + ["-o", out + ".fasta", "-vcf", out + ".vcf", "-ogff", out + ".gff", "-doc", out + ".tsv", "-t", "2"])
-    except Exception as e:          # the reference's own exceptions (e.g. KeyError) must match too
-        return type(e).__name__
-    return {e: open(f"{out}.{e}").read() if os.path.exists(f"{out}.{e}") else None for e in ("fasta", "vcf", "gff", "tsv")}
-
-
-def _mini_argv(name, path):
-    mincov = json.load(open(f"{GOLD}/{name}.json"))["mincov"]
-    return ["-i", path, "-ref", f"{GOLD}/{name}.fasta", "-gff", f"{GOLD}/{name}.gff", "-cov", str(mincov), "-name", name]
 
 
 REFS = [(b"chr1", 5000), (b"chr2", 3000)]
@@ -232,7 +85,7 @@ def test_read_sam_header_6000_references(tmp_path):
 
     refs = [(b"decoy_%05d_with_a_long_name" % i, 10 + i % 23) for i in range(6000)]
     p = tmp_path / "many.sam"
-    p.write_bytes(_sam_header(refs) + b"".join(_good_lines(3, rname=refs[4321][0])))
+    p.write_bytes(sam_header(refs) + b"".join(_good_lines(3, rname=refs[4321][0])))
     names, lens, off, no = bamio.read_sam_header(str(p))
     assert names == [n.decode() for n, _ in refs] and lens == [l for _, l in refs]
     assert no == 6003 and p.read_bytes()[off:].startswith(b"g0\t")
@@ -259,7 +112,7 @@ def test_sam_handle_header_without_a_device(tmp_path):
     from trueconsense_b200 import indexing
 
     p = tmp_path / "x.sam"
-    p.write_bytes(_sam_header(REFS) + b"".join(_good_lines(2)))
+    p.write_bytes(sam_header(REFS) + b"".join(_good_lines(2)))
     h = indexing.Readbam(str(p))
     assert h.references == ("chr1", "chr2") and h.lengths == (5000, 3000) and h.ref_len == 5000
     with pytest.raises(NotImplementedError, match="SAM"):
@@ -272,7 +125,8 @@ def test_sam_helpers_round_trip(tmp_path):
 
     build.build_host()
     for name in MINIS:
-        _, names, recs = _split(f"{GOLD}/{name}.bam")
+        head, recs = split(f"{GOLD}/{name}.bam")
+        names = [n for n, _ in refs_of(head)]
         for r in recs:
             line = sam_line(r, names, MM2_AUX % 3)
             assert line.count(b"\t") == 20 and line.endswith(b"\n")
@@ -319,7 +173,7 @@ def test_cli_parity(ctx, name, tmp_path, monkeypatch):
     sam = bam_to_sam(f"{GOLD}/{name}.bam", str(tmp_path / f"{name}.sam"), aux=True)
     status = json.load(open(f"{GOLD}/cli_{name}.status.json"))
     out = str(tmp_path / f"cli_{name}")
-    argv = _mini_argv(name, sam) + ["-o", out + ".fasta", "-vcf", out + ".vcf", "-ogff", out + ".gff",
+    argv = mini_argv(name, sam) + ["-o", out + ".fasta", "-vcf", out + ".vcf", "-ogff", out + ".gff",
                                     "-doc", out + ".cov.tsv", "-t", "2"]
     monkeypatch.setattr("sys.argv", ["TrueConsense", "<golden>"])
     if status["status"] == "raise":
@@ -348,11 +202,11 @@ def test_shuffled_sam_sorted_on_device(ctx, name, tmp_path, monkeypatch):
     from trueconsense_b200 import indexing
 
     bam = f"{GOLD}/{name}.bam"
-    head, _, recs = _split(bam)
+    head, recs = split(bam)
     order = np.random.default_rng(11).permutation(len(recs))
     sam = bam_to_sam(bam, str(tmp_path / "shuf.sam"), aux=True, order=order)
     shuf_bam = str(tmp_path / "shuf.bam")
-    _bgzf(shuf_bam, head + b"".join(recs[i] for i in order), (3000, 65280))
+    bgzf(shuf_bam, head + b"".join(recs[i] for i in order), (3000, 65280))
     L = load_golden_counts(name).shape[1]
     b = ctx.bam_file_to_device(shuf_bam, sort=True)
     want = _snapshot(ctx, b)
@@ -363,8 +217,8 @@ def test_shuffled_sam_sorted_on_device(ctx, name, tmp_path, monkeypatch):
     assert ctx.extract_inserts(d, L, np.arange(1, L + 1, dtype=np.int32)) == want_cols
     with pytest.raises(ValueError, match="Unsorted input. Pileup aborts"):
         indexing.BuildIndex(sam, f"{GOLD}/{name}.fasta")
-    got = _cli(["--sort-input"] + _mini_argv(name, sam), str(tmp_path / "s"), monkeypatch)
-    exp = _cli(["--sort-input"] + _mini_argv(name, shuf_bam), str(tmp_path / "b"), monkeypatch)
+    got = run_cli(["--sort-input"] + mini_argv(name, sam), str(tmp_path / "s"), monkeypatch)
+    exp = run_cli(["--sort-input"] + mini_argv(name, shuf_bam), str(tmp_path / "b"), monkeypatch)
     assert got == exp
 
 
@@ -384,7 +238,7 @@ def _multi_ref(tmp, n_decoys=40):
         one = os.path.join(tmp, f"c{k}.bam")
         bamio.write_bam(one, synth.generate_reads(p, seq), f"c{k}", L)
         recs = []
-        for r in _split(one)[2]:
+        for r in split(one)[1]:
             r = bytearray(r)
             struct.pack_into("<i", r, 4, slots[k])
             if struct.unpack_from("<i", r, 24)[0] >= 0:
@@ -406,7 +260,7 @@ def _multi_ref(tmp, n_decoys=40):
             for f in c["feats"]:
                 attrs = f"ID=cds-{c['name']}-{f['name']};Name={f['name']};gbkey=CDS"
                 fh.write("\t".join([c["name"], "synthetic", "CDS", str(f["start"]), str(f["end"]), ".", f["strand"], "0", attrs]) + "\n")
-    return _bam_header(refs, b"@HD\tVN:1.6\tSO:unsorted\n"), refs, real, slots, fasta, gff
+    return bam_header(refs, b"@HD\tVN:1.6\tSO:unsorted\n"), refs, real, slots, fasta, gff
 
 
 @pytest.mark.gpu
@@ -426,9 +280,9 @@ def test_multi_reference_interleaved(ctx, tmp_path, monkeypatch):
     names = [n for n, _ in refs]
     for stem, rs, flags in (("shuf", body, ["--sort-input"]), ("sorted", [r for i in slots for r in real[i]["recs"]], [])):
         bam, sam = os.path.join(tmp, stem + ".bam"), os.path.join(tmp, stem + ".sam")
-        _bgzf(bam, head + b"".join(rs), (65280, 3000))
+        bgzf(bam, head + b"".join(rs), (65280, 3000))
         with open(sam, "wb") as fh:
-            fh.write(_sam_header(refs, b"@HD\tVN:1.6\tSO:unsorted\n") + b"".join(sam_line(r, names, MM2_AUX % 1) for r in rs))
+            fh.write(sam_header(refs, b"@HD\tVN:1.6\tSO:unsorted\n") + b"".join(sam_line(r, names, MM2_AUX % 1) for r in rs))
         sort = bool(flags)
         hs, hb = indexing.Readbam(sam, sort=sort), indexing.Readbam(bam, sort=sort)
         fs, fb = indexing.BuildIndexContigs(hs, fasta), indexing.BuildIndexContigs(hb, fasta)
@@ -443,8 +297,8 @@ def test_multi_reference_interleaved(ctx, tmp_path, monkeypatch):
         ins = Events.ListInsertsContigs(idx, 30, hs)
         assert ins == Events.ListInsertsContigs(idx, 30, hb) and ins["c0"][0]
         base = ["-ref", fasta, "-gff", gff, "-cov", "30", "-name", "S", "--all-contigs"] + flags
-        got = _cli(["-i", sam] + base, os.path.join(tmp, stem + "_s"), monkeypatch)
-        exp = _cli(["-i", bam] + base, os.path.join(tmp, stem + "_b"), monkeypatch)
+        got = run_cli(["-i", sam] + base, os.path.join(tmp, stem + "_s"), monkeypatch)
+        exp = run_cli(["-i", bam] + base, os.path.join(tmp, stem + "_b"), monkeypatch)
         assert isinstance(got, dict) and got == exp
         assert got["fasta"].count(">") == len(refs)
         with pytest.raises(ValueError, match="multi-contig"):
@@ -477,7 +331,7 @@ def test_dialect(ctx, tmp_path):
         _assert_same(_snapshot(ctx, d), (want[0], want[1], want[2], want[3], len(lines), 2, None))
         assert d.info["n_lines"] == len(lines) and d.n_reads == len(lines) - 2
     # an empty body, a header-only file without its last newline, a file without anything
-    for text in (_sam_header(REFS), _sam_header(REFS)[:-1], b""):
+    for text in (sam_header(REFS), sam_header(REFS)[:-1], b""):
         p = os.path.join(ctxt, "empty.sam")
         open(p, "wb").write(text)
         d = ctx.sam_file_to_device(p, contig_ranges=True, sort=True)
@@ -585,7 +439,7 @@ def test_malformed_line(ctx, case, tmp_path):
     good = _good_lines(300)
     k = 137
     path = str(tmp_path / "bad.sam")
-    header = _sam_header(REFS)
+    header = sam_header(REFS)
     with open(path, "wb") as fh:
         fh.write(header + b"".join(good[:k] + [bad] + good[k:]))
     line_no = header.count(b"\n") + k + 1
@@ -605,7 +459,7 @@ def test_first_bad_line_is_named(ctx, tmp_path):
     lines = good[:1500] + [BAD["qual_char"][0]] + good[1500:1700] + [BAD["fields"][0]] + good[1700:]
     lines[900] = BAD["cigar_op"][0]
     path = str(tmp_path / "two.sam")
-    header = _sam_header(REFS)
+    header = sam_header(REFS)
     open(path, "wb").write(header + b"".join(lines))
     line_no = header.count(b"\n") + 901
     with pytest.raises(OSError, match=f"line {line_no}: bad CIGAR"):

@@ -3,63 +3,20 @@ default coordinate order on the GPU (``tc_bam_sort_records``) and every pass the
 ``samtools sort`` would have written.  The order oracle here restates that order on the host (refID, pos + 1, forward
 before reverse, file order; a file already sorted by (refID, pos) is used as written) and writes the same record bytes in
 that order, so each device result is compared with the existing path over the oracle-ordered file."""
-import gzip
 import json
 import os
 import struct
-import zlib
 
 import numpy as np
 import pytest
 
+from bamfiles import assert_same_arrays, dev_arrays, mini_argv, multi_ref_files, run_cli, split, write
 from conftest import GOLD, load_golden_counts
 
 MINIS = ("quirk", "mini_illumina", "mini_ont", "mini_long", "mini_overlap")
-FIELDS = (("pos", np.int32), ("flag", np.uint16), ("mapq", np.uint8), ("l_seq", np.int32), ("seq_off", np.uint32),
-          ("cigar_off", np.uint32), ("seq4", np.uint32), ("qual", np.uint8), ("cigar", np.uint32), ("qname_hash", np.uint64),
-          ("mpos", np.int32), ("isize", np.int32))
 
 
 # ---------------------------------------------------------------------------- fixture helpers (host only)
-def _bgzf(path, payload: bytes, member_bytes=(65280,)) -> None:
-    """Write a BAM payload as BGZF members of the given payload sizes (cycled), and the EOF member."""
-    def member(chunk):
-        c = zlib.compressobj(1, zlib.DEFLATED, -15, 8, 0)
-        data = c.compress(chunk) + c.flush()
-        bsize = 18 + len(data) + 8
-        return (bytes([31, 139, 8, 4, 0, 0, 0, 0, 0, 255]) + struct.pack("<H", 6) + b"BC" + struct.pack("<HH", 2, bsize - 1) + data +
-                struct.pack("<II", zlib.crc32(chunk) & 0xFFFFFFFF, len(chunk)))
-
-    out, p, k = [], 0, 0
-    while p < len(payload):
-        n = member_bytes[k % len(member_bytes)]
-        out.append(member(payload[p:p + n]))
-        p, k = p + n, k + 1
-    out.append(member(b""))
-    with open(path, "wb") as fh:
-        fh.write(b"".join(out))
-
-
-def _split(path):
-    """(header bytes, [records with their block_size]) of a BAM file."""
-    from trueconsense_b200 import bamio
-
-    with gzip.open(path, "rb") as fh:
-        payload = fh.read()
-    _, _, q = bamio.parse_bam_header(payload, len(payload))
-    head, recs = payload[:q], []
-    while q + 4 <= len(payload):
-        bs = struct.unpack_from("<i", payload, q)[0]
-        recs.append(payload[q:q + 4 + bs])
-        q += 4 + bs
-    return head, recs
-
-
-def _write(path, head, recs, member_bytes=(65280,)):
-    _bgzf(path, head + b"".join(recs), member_bytes)
-    return path
-
-
 def _rec_keys(recs):
     """refID, pos, FLAG of raw records."""
     tid = np.array([struct.unpack_from("<i", r, 4)[0] for r in recs], np.int64)
@@ -70,11 +27,11 @@ def _rec_keys(recs):
 
 def _shuffle(src, dst, seed, order=None):
     """The records of ``src`` in a seeded random order (or ``order``), re-blocked into members of varying size."""
-    head, recs = _split(src)
+    head, recs = split(src)
     rng = np.random.default_rng(seed)
     perm = rng.permutation(len(recs)) if order is None else order
     sizes = tuple(int(x) for x in rng.integers(200, 65280, 7))
-    return _write(dst, head, [recs[i] for i in perm], sizes)
+    return write(dst, head, [recs[i] for i in perm], sizes)
 
 
 def oracle_order(tid, pos, flag, strand=True):
@@ -92,46 +49,18 @@ def _oracle_bam(src, dst, strand=True):
     """The placed records of ``src`` in the oracle's order, keys from the host decode (bamio.read_bam, file order)."""
     from trueconsense_b200 import bamio
 
-    head, recs = _split(src)
+    head, recs = split(src)
     recs = [r for r in recs if struct.unpack_from("<i", r, 4)[0] >= 0]
     b = bamio.read_bam(src)
     assert b.n_reads == len(recs) and np.array_equal(b.pos, _rec_keys(recs)[1])
     tid = np.zeros(b.n_reads, np.int64) if b.tid is None else b.tid
     order = oracle_order(tid, b.pos, b.flag, strand)
-    _write(dst, head, [recs[i] for i in order])
+    write(dst, head, [recs[i] for i in order])
     return dst, order
-
-
-def _dev_arrays(ctx, d):
-    """Every array of device reads, on the host (taken before the context stages anything else)."""
-    s, n = d.struct, d.n_reads
-    if n == 0:
-        return {}
-    sizes = {"seq_off": n + 1, "cigar_off": n + 1, "seq4": d.stats.n_seq_words, "qual": 8 * d.stats.n_seq_words,
-             "cigar": d.stats.n_cigar_ops}
-    return {f: ctx.download(getattr(s, f), sizes.get(f, n), t) for f, t in FIELDS}
-
-
-def _assert_same(a, b, what=""):
-    assert a.keys() == b.keys(), what
-    for f in a:
-        assert np.array_equal(a[f], b[f]), (what, f)
 
 
 def _all_columns(ctx, d, L, params=None):
     return ctx.extract_inserts(d, L, np.arange(1, L + 1, dtype=np.int32), params)
-
-
-def _cli(argv, out, monkeypatch, exts=("fasta", "vcf", "gff", "tsv")):
-    """main(argv) writing {out}.{ext}: the files' text, or the exception type's name."""
-    from trueconsense_b200 import TrueConsense
-
-    monkeypatch.setattr("sys.argv", ["TrueConsense", "<sorted>"])
-    try:
-        TrueConsense.main(argv + ["-o", out + ".fasta", "-vcf", out + ".vcf", "-ogff", out + ".gff", "-doc", out + ".tsv", "-t", "2"])
-    except Exception as e:          # the reference's own exceptions (e.g. KeyError) must match too
-        return type(e).__name__
-    return {e: open(f"{out}.{e}").read() if os.path.exists(f"{out}.{e}") else None for e in exts}
 
 
 def _golden(name):
@@ -144,11 +73,6 @@ def _as_golden(got):
     assert isinstance(got, dict), got
     vcf = "".join("##fileDate=<date>\n" if l.startswith("##fileDate=") else l for l in got["vcf"].splitlines(keepends=True))
     return dict(got, vcf=vcf.replace(GOLD + os.sep, "").replace("<sorted>", "<golden>"))
-
-
-def _mini_argv(name, bam):
-    mincov = json.load(open(f"{GOLD}/{name}.json"))["mincov"]
-    return ["-i", bam, "-ref", f"{GOLD}/{name}.fasta", "-gff", f"{GOLD}/{name}.gff", "-cov", str(mincov), "-name", name]
 
 
 # ---------------------------------------------------------------------------- CPU tests
@@ -192,11 +116,11 @@ def test_shuffle_helpers_keep_the_records(tmp_path):
     build.build_host()
     src = f"{GOLD}/mini_illumina.bam"
     shuf = _shuffle(src, str(tmp_path / "s.bam"), 3)
-    h0, r0 = _split(src)
-    h1, r1 = _split(shuf)
+    h0, r0 = split(src)
+    h1, r1 = split(shuf)
     assert h0 == h1 and sorted(r0) == sorted(r1) and r0 != r1
     dst, order = _oracle_bam(shuf, str(tmp_path / "o.bam"))
-    _, r2 = _split(dst)
+    _, r2 = split(dst)
     assert r2 == [r1[i] for i in order]
     tid, pos, flag = _rec_keys(r2)
     key = (tid << 33) | ((pos + 1) << 1) | ((flag >> 4) & 1)
@@ -220,11 +144,11 @@ def test_sorted_files_are_untouched(ctx, name, tmp_path, monkeypatch):
     """A coordinate-sorted file with sort=True: the same device arrays as without, nothing reordered, and --sort-input writes
     the reference CLI's golden files."""
     path = f"{GOLD}/{name}.bam"
-    plain = _dev_arrays(ctx, ctx.bam_file_to_device(path))
+    plain = dev_arrays(ctx, ctx.bam_file_to_device(path))
     d = ctx.bam_file_to_device(path, sort=True)
     assert d.info["reordered"] is False and not d.stats.unsorted
-    _assert_same(_dev_arrays(ctx, d), plain, name)
-    got = _cli(["--sort-input"] + _mini_argv(name, path), str(tmp_path / name), monkeypatch)
+    assert_same_arrays(dev_arrays(ctx, d), plain, name)
+    got = run_cli(["--sort-input"] + mini_argv(name, path), str(tmp_path / name), monkeypatch, argv0="<sorted>")
     assert _as_golden(got) == _golden(name)
 
 
@@ -241,10 +165,10 @@ def test_shuffled_goldens(ctx, name, seed, tmp_path, monkeypatch):
     shuf = _shuffle(src, str(tmp_path / "shuf.bam"), seed)
     ordered, _ = _oracle_bam(shuf, str(tmp_path / "ordered.bam"))
     L = load_golden_counts(name).shape[1]
-    want = _dev_arrays(ctx, ctx.bam_file_to_device(ordered))
+    want = dev_arrays(ctx, ctx.bam_file_to_device(ordered))
     d = ctx.bam_file_to_device(shuf, sort=True)
     assert d.info["reordered"] is True and not d.stats.unsorted and not d.stats.multi_contig
-    _assert_same(_dev_arrays(ctx, d), want, name)
+    assert_same_arrays(dev_arrays(ctx, d), want, name)
     cols = _all_columns(ctx, d, L)
     assert cols == _all_columns(ctx, ctx.bam_file_to_device(ordered), L)
     with pytest.raises(ValueError, match="Unsorted input. Pileup aborts"):
@@ -255,11 +179,11 @@ def test_shuffled_goldens(ctx, name, seed, tmp_path, monkeypatch):
     index = frame.to_dict("index")
     mincov = json.load(open(f"{GOLD}/{name}.json"))["mincov"]
     assert Events.ListInserts(index, mincov, h) == Events.ListInserts(index, mincov, indexing.Readbam(ordered))
-    got = _cli(["--sort-input"] + _mini_argv(name, shuf), str(tmp_path / "s"), monkeypatch)
-    exp = _cli(_mini_argv(name, ordered), str(tmp_path / "o"), monkeypatch)
+    got = run_cli(["--sort-input"] + mini_argv(name, shuf), str(tmp_path / "s"), monkeypatch, argv0="<sorted>")
+    exp = run_cli(mini_argv(name, ordered), str(tmp_path / "o"), monkeypatch, argv0="<sorted>")
     assert got == exp
-    _, golden_recs = _split(src)
-    _, ordered_recs = _split(ordered)
+    _, golden_recs = split(src)
+    _, ordered_recs = split(ordered)
     if ordered_recs == [r for r in golden_recs if struct.unpack_from("<i", r, 4)[0] >= 0]:
         # the oracle restores the golden file's own order: the reference CLI's files apply as they are
         assert _as_golden(got) == _golden(name), f"{name}: the oracle order is the golden file's own order"
@@ -287,10 +211,10 @@ def test_ties_decide_the_result(ctx, tmp_path):
     later = str(tmp_path / "later.bam")
     bamio.write_bam(later, ReadBatch.from_records([dict(pos=300, cigar="50M", seq="C" * 50, qname=f"l{j}") for j in range(3)]),
                     "ref", 1000)
-    head, recs = _split(sorted_bam)
+    head, recs = split(sorted_bam)
     perm = np.random.default_rng(8).permutation(len(recs))
-    shuffled = _split(later)[1] + [recs[i] for i in perm]          # a few later reads ahead: not sorted by (refID, pos)
-    path = _write(str(tmp_path / "shuf.bam"), head, shuffled, (40000, 9000, 65280))
+    shuffled = split(later)[1] + [recs[i] for i in perm]          # a few later reads ahead: not sorted by (refID, pos)
+    path = write(str(tmp_path / "shuf.bam"), head, shuffled, (40000, 9000, 65280))
     assert np.sum(perm[:8000] < 4500) < 4000                        # the file's own order admits more GT than AC
     col = 110                       # 1-based: the last M column before the insertion
     assert Events.ExtractInserts(indexing.Readbam(path, sort=True), col) == ("AC", "2")
@@ -310,7 +234,7 @@ def test_mates_far_apart(ctx, tmp_path):
     from trueconsense_b200 import gpu
 
     src = f"{GOLD}/mini_overlap.bam"
-    _, recs = _split(src)
+    _, recs = split(src)
     _, _, flag = _rec_keys(recs)
     rng = np.random.default_rng(4)
     first = rng.permutation(np.flatnonzero(flag & 0x40))
@@ -330,54 +254,6 @@ def test_mates_far_apart(ctx, tmp_path):
         assert any(c["n_entries"] for c in got)
 
 
-def _multi_ref_files(tmp, n_decoys=6000):
-    """Three references with reads (insertions and a deletion inside ORFs, paired reads) spread over a header of
-    n_decoys + 3 references (refIDs 0, n_decoys // 2 + 1, n_decoys + 2), the FASTA of all of them and the GFF rows of the
-    three.  Returns the paths and the records of each reference (refID patched)."""
-    from trueconsense_b200 import bamio, synth
-
-    real = {}
-    slots = [0, n_decoys // 2 + 1, n_decoys + 2]
-    for k, (L, seed) in enumerate(((2341, 1), (1565, 2), (890, 3))):
-        seq, feats = synth.make_genome(L, 300 + seed, "sars2")
-        a = feats[0]["start"] - 1
-        vs = [synth.Variant(a + 400, synth.VAR_INS, 3, 7, 0.9)] if k != 1 else [synth.Variant(a + 60, synth.VAR_DEL, 3, 0, 0.85)]
-        p = synth.SynthParams(seed=400 + seed, n_reads=L * 60 // 150, ref_len=L, read_len=150, paired=(k != 2), insert_mean=300,
-                              insert_sd=40, sub_rate=0.01, softclip_rate=0.05, softclip_max=8, variants=vs)
-        one = os.path.join(tmp, f"c{k}.bam")
-        bamio.write_bam(one, synth.generate_reads(p, seq), f"c{k}", L)
-        recs = []
-        for r in _split(one)[1]:
-            r = bytearray(r)
-            struct.pack_into("<i", r, 4, slots[k])
-            if struct.unpack_from("<i", r, 24)[0] >= 0:
-                struct.pack_into("<i", r, 24, slots[k])
-            recs.append(bytes(r))
-        real[slots[k]] = {"name": f"c{k}", "seq": seq, "feats": feats, "recs": recs}
-    refs = []
-    for i in range(n_decoys + 3):
-        refs.append((real[i]["name"], len(real[i]["seq"])) if i in real else (f"decoy_{i:05d}_with_a_long_name", 10 + i % 23))
-    text = b"@HD\tVN:1.6\tSO:unsorted\n"
-    head = b"BAM\1" + struct.pack("<i", len(text)) + text + struct.pack("<i", len(refs))
-    for n, l in refs:
-        nb = n.encode() + b"\0"
-        head += struct.pack("<i", len(nb)) + nb + struct.pack("<i", l)
-    fasta = os.path.join(tmp, "multi.fasta")
-    with open(fasta, "w") as fh:
-        for i, (n, l) in enumerate(refs):
-            s = real[i]["seq"] if i in real else "ACGT" * (l // 4) + "A" * (l % 4)
-            fh.write(f">{n}\n" + "".join(s[j:j + 60] + "\n" for j in range(0, len(s), 60)))
-    gff = os.path.join(tmp, "multi.gff")
-    with open(gff, "w") as fh:
-        fh.write("##gff-version 3\n")
-        for i in slots:
-            c = real[i]
-            for f in c["feats"]:
-                attrs = f"ID=cds-{c['name']}-{f['name']};Name={f['name']};gbkey=CDS"
-                fh.write("\t".join([c["name"], "synthetic", "CDS", str(f["start"]), str(f["end"]), ".", f["strand"], "0", attrs]) + "\n")
-    return head, real, slots, fasta, gff
-
-
 @pytest.mark.gpu
 def test_multi_reference_interleaved_long_header(ctx, tmp_path, monkeypatch):
     """References' records interleaved (refIDs decreasing, shuffled inside each reference) under a header of 6003
@@ -386,13 +262,13 @@ def test_multi_reference_interleaved_long_header(ctx, tmp_path, monkeypatch):
     from trueconsense_b200 import Events, indexing
 
     tmp = str(tmp_path)
-    head, real, slots, fasta, gff = _multi_ref_files(tmp)
+    head, real, slots, fasta, gff = multi_ref_files(tmp)
     rng = np.random.default_rng(9)
     body = []
     for i in reversed(slots):
         recs = real[i]["recs"]
         body += [recs[j] for j in rng.permutation(len(recs))]
-    shuf = _write(os.path.join(tmp, "shuf.bam"), head, body, (65280, 3000, 20000))
+    shuf = write(os.path.join(tmp, "shuf.bam"), head, body, (65280, 3000, 20000))
     ordered, _ = _oracle_bam(shuf, os.path.join(tmp, "ordered.bam"))
     hs, ho = indexing.Readbam(shuf, sort=True), indexing.Readbam(ordered)
     fs, fo = indexing.BuildIndexContigs(hs, fasta), indexing.BuildIndexContigs(ho, fasta)
@@ -409,8 +285,8 @@ def test_multi_reference_interleaved_long_header(ctx, tmp_path, monkeypatch):
     ins_s, ins_o = Events.ListInsertsContigs(idx, 30, hs), Events.ListInsertsContigs(idx, 30, ho)
     assert ins_s == ins_o and ins_s["c0"][0] and ins_s["c2"][0]
     base = ["-ref", fasta, "-gff", gff, "-cov", "30", "-name", "S", "--all-contigs"]
-    got = _cli(["--sort-input", "-i", shuf] + base, os.path.join(tmp, "s"), monkeypatch)
-    exp = _cli(["-i", ordered] + base, os.path.join(tmp, "o"), monkeypatch)
+    got = run_cli(["--sort-input", "-i", shuf] + base, os.path.join(tmp, "s"), monkeypatch, argv0="<sorted>")
+    exp = run_cli(["-i", ordered] + base, os.path.join(tmp, "o"), monkeypatch, argv0="<sorted>")
     assert isinstance(got, dict) and got == exp
     assert got["fasta"].count(">") == 6003
     with pytest.raises(ValueError, match="Unsorted input. Pileup aborts"):
@@ -425,14 +301,14 @@ def test_host_inflate_route(ctx, tmp_path):
     shuf = _shuffle(f"{GOLD}/mini_illumina.bam", str(tmp_path / "shuf.bam"), 5)
     d = ctx.bam_file_to_device(shuf, sort=True)
     assert d.info["reordered"] is True
-    want = _dev_arrays(ctx, d)
+    want = dev_arrays(ctx, d)
     payload = bamio.read_bam_payload(shuf)
     x0 = ctx.transfer_bytes()[0]
     h = ctx.bam_to_device(payload, sort=True)
     x1 = ctx.transfer_bytes()[0]
     assert h.info["reordered"] is True and not h.stats.unsorted
     assert x1 - x0 <= payload.n_bytes + 8 * payload.n_reads + 4096, (x1 - x0, payload.n_bytes)
-    _assert_same(_dev_arrays(ctx, h), want)
+    assert_same_arrays(dev_arrays(ctx, h), want)
     # and first_read from the sorted offsets
     h = ctx.bam_to_device(payload, sort=True, contig_ranges=True)
     assert h.first_read.tolist() == [0, payload.n_reads]
@@ -455,11 +331,11 @@ def test_size_200k_config2_slice(ctx, tmp_path):
     bamio.write_bam(src, b, "ref", L)
     shuf = _shuffle(src, str(tmp_path / "shuf.bam"), 6)
     ordered, _ = _oracle_bam(shuf, str(tmp_path / "ordered.bam"))
-    want = _dev_arrays(ctx, ctx.bam_file_to_device(ordered))
+    want = dev_arrays(ctx, ctx.bam_file_to_device(ordered))
     exp_counts = ctx.pileup_counts(b, L)
     d = ctx.bam_file_to_device(shuf, sort=True)
     assert d.info["reordered"] is True and d.n_reads == b.n_reads
-    _assert_same(_dev_arrays(ctx, d), want)
+    assert_same_arrays(dev_arrays(ctx, d), want)
     assert np.array_equal(ctx.pileup_counts(d, L), exp_counts)
     res = ctx.call(exp_counts, L, w.mincov, True)
     cands = ctx.list_insert_candidates(res.flags, L)
@@ -490,10 +366,10 @@ def test_edge_cases(ctx, tmp_path):
 
     one = str(tmp_path / "one.bam")
     bamio.write_bam(one, ReadBatch.from_records([dict(pos=7, cigar="5M", seq="ACGTA", flag=16)]), "ref", 100)
-    want = _dev_arrays(ctx, ctx.bam_file_to_device(one))
+    want = dev_arrays(ctx, ctx.bam_file_to_device(one))
     d = ctx.bam_file_to_device(one, sort=True)
     assert d.info["reordered"] is False
-    _assert_same(_dev_arrays(ctx, d), want)
+    assert_same_arrays(dev_arrays(ctx, d), want)
 
     rng = np.random.default_rng(2)
     recs = [dict(pos=20, cigar="30M", seq="".join(rng.choice(list("ACGT"), 30)), flag=int(16 * (j % 3 == 0)), qname=f"s{j}")
@@ -504,24 +380,24 @@ def test_edge_cases(ctx, tmp_path):
     shuf = _shuffle(same, str(tmp_path / "same_shuf.bam"), 2)
     d = ctx.bam_file_to_device(shuf, sort=True)
     assert d.info["reordered"] is False
-    _assert_same(_dev_arrays(ctx, d), _dev_arrays(ctx, ctx.bam_file_to_device(shuf)))
+    assert_same_arrays(dev_arrays(ctx, d), dev_arrays(ctx, ctx.bam_file_to_device(shuf)))
     # ... unless one record at another position makes the file unsorted: then forward before reverse, file order in each
-    head, rr = _split(shuf)
+    head, rr = split(shuf)
     before = bytearray(rr[-1])
     struct.pack_into("<i", before, 8, 25)
-    mixed = _write(str(tmp_path / "mixed.bam"), head, [bytes(before)] + rr[:-1])
+    mixed = write(str(tmp_path / "mixed.bam"), head, [bytes(before)] + rr[:-1])
     ordered, order = _oracle_bam(mixed, str(tmp_path / "mixed_ordered.bam"))
     assert order[-1] == 0
     d = ctx.bam_file_to_device(mixed, sort=True)
     assert d.info["reordered"] is True
-    _assert_same(_dev_arrays(ctx, d), _dev_arrays(ctx, ctx.bam_file_to_device(ordered)))
+    assert_same_arrays(dev_arrays(ctx, d), dev_arrays(ctx, ctx.bam_file_to_device(ordered)))
 
     # refID >= n_ref / pos < -1: the host reader passes them on, the sort refuses them and names the record
-    head, rr = _split(same)
+    head, rr = split(same)
     for off, value in ((4, 1), (8, -2)):
         bad = bytearray(rr[5])
         struct.pack_into("<i", bad, off, value)
-        path = _write(str(tmp_path / f"bad{off}.bam"), head, rr[:5] + [bytes(bad)] + rr[6:])
+        path = write(str(tmp_path / f"bad{off}.bam"), head, rr[:5] + [bytes(bad)] + rr[6:])
         p = bamio.read_bam_payload(path)
         with pytest.raises(gpu.TcError) as ei:
             ctx.bam_to_device(p, sort=True)

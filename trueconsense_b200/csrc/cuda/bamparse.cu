@@ -13,14 +13,10 @@
 // read buffers like after tc_reads_upload — the CPU never touches a record's body.
 #include <cub/device/device_scan.cuh>
 
+#include "bamrec.cuh"
 #include "tc_common.cuh"
 
 namespace {
-
-__device__ __forceinline__ uint32_t ld16(const uint8_t* p) { return (uint32_t)p[0] | ((uint32_t)p[1] << 8); }
-__device__ __forceinline__ uint32_t ld32(const uint8_t* p) {
-    return (uint32_t)p[0] | ((uint32_t)p[1] << 8) | ((uint32_t)p[2] << 16) | ((uint32_t)p[3] << 24);
-}
 
 struct bam_args {
     const uint8_t* u; const long long* rec; long long n;
@@ -36,15 +32,15 @@ __global__ void __launch_bounds__(256) bam_meta_kernel(bam_args a) {
     int bad_order = 0, other_contig = 0;
     if (i < a.n) {
         const uint8_t* r = a.u + a.rec[i];
-        const int32_t tid = (int32_t)ld32(r), pos = (int32_t)ld32(r + 4);
-        const uint32_t l_name = r[8], n_cig = ld16(r + 12), l_seq = ld32(r + 16);
-        const int32_t mtid = (int32_t)ld32(r + 20);
-        a.pos[i] = pos; a.mapq[i] = r[9]; a.flag[i] = (uint16_t)ld16(r + 14); a.l_seq[i] = (int32_t)l_seq;
+        const int32_t tid = (int32_t)ld32(r + BAM_REF_ID), pos = (int32_t)ld32(r + BAM_POS);
+        const uint32_t l_name = r[BAM_L_READ_NAME], n_cig = ld16(r + BAM_N_CIGAR_OP), l_seq = ld32(r + BAM_L_SEQ);
+        const int32_t mtid = (int32_t)ld32(r + BAM_NEXT_REF_ID);
+        a.pos[i] = pos; a.mapq[i] = r[BAM_MAPQ]; a.flag[i] = (uint16_t)ld16(r + BAM_FLAG); a.l_seq[i] = (int32_t)l_seq;
         // tc_reads_t.mpos: PNEXT, -2 when the mate maps to another reference
-        a.mpos[i] = (mtid >= 0 && mtid != tid) ? -2 : (int32_t)ld32(r + 24);
-        a.isize[i] = (int32_t)ld32(r + 28);
+        a.mpos[i] = (mtid >= 0 && mtid != tid) ? -2 : (int32_t)ld32(r + BAM_NEXT_POS);
+        a.isize[i] = (int32_t)ld32(r + BAM_TLEN);
         // low 32 bits: khash's X31 string hash (htslib keys its mate-overlap table with it), high 32: folded FNV-1a — as bamio.c
-        const uint8_t* name = r + 32;
+        const uint8_t* name = r + BAM_READ_NAME;
         uint32_t h = name[0];
         unsigned long long f = 1469598103934665603ull;
         for (uint32_t k = 0; k + 1 < l_name && name[k]; ++k) {
@@ -52,18 +48,14 @@ __global__ void __launch_bounds__(256) bam_meta_kernel(bam_args a) {
             f ^= name[k]; f *= 1099511628211ull;
         }
         a.qname_hash[i] = ((unsigned long long)((uint32_t)(f >> 32) ^ (uint32_t)f) << 32) | h;
-        const uint8_t* cg = r + 32 + l_name;
+        const uint8_t* cg = name + l_name;
         for (uint32_t k = 0; k < n_cig; ++k) {
-            const uint32_t c = ld32(cg + 4 * k), op = c & 15u;
-            if (op == 0 || op == 2 || op == 3 || op == 7 || op == 8) span += (long long)(c >> 4);
+            const uint32_t c = ld32(cg + 4 * k);
+            if (op_consumes_ref(c & 15u)) span += (long long)(c >> 4);
         }
         a.seq_n[i] = (l_seq + 7) / 8; a.cig_n[i] = n_cig;
-        if (i > 0) {
-            const uint8_t* q = a.u + a.rec[i - 1];
-            const int32_t ptid = (int32_t)ld32(q), ppos = (int32_t)ld32(q + 4);
-            bad_order = (tid < ptid) || (tid == ptid && pos < ppos);
-        }
-        other_contig = tid != (int32_t)ld32(a.u + a.rec[0]);
+        bad_order = bam_out_of_order(a.u, a.rec, i, tid, pos);
+        other_contig = tid != (int32_t)ld32(a.u + a.rec[0] + BAM_REF_ID);
     }
     const long long wspan = __reduce_max_sync(0xffffffffu, (int)min(span, (long long)0x7fffffff));
     unsigned long long wsum = (unsigned long long)span;
@@ -84,8 +76,8 @@ __global__ void __launch_bounds__(256) bam_pack_kernel(bam_args a) {
     const int lane = threadIdx.x & 31;
     if (i >= a.n) return;
     const uint8_t* r = a.u + a.rec[i];
-    const uint32_t l_name = r[8], n_cig = ld16(r + 12), l_seq = ld32(r + 16);
-    const uint8_t* cg = r + 32 + l_name;
+    const uint32_t n_cig = ld16(r + BAM_N_CIGAR_OP), l_seq = ld32(r + BAM_L_SEQ);
+    const uint8_t* cg = bam_cigar(r);
     const uint8_t* sq = cg + 4 * (size_t)n_cig;
     const uint32_t sbytes = (l_seq + 1) / 2;
     const uint8_t* ql = sq + sbytes;

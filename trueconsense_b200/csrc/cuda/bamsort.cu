@@ -10,13 +10,10 @@
 //                         header's reference count can set — skipped when the records are sorted already
 #include <cub/device/device_radix_sort.cuh>
 
+#include "bamrec.cuh"
 #include "tc_common.cuh"
 
 namespace {
-
-__device__ __forceinline__ uint32_t ld32(const uint8_t* p) {       // records start at any byte
-    return (uint32_t)p[0] | ((uint32_t)p[1] << 8) | ((uint32_t)p[2] << 16) | ((uint32_t)p[3] << 24);
-}
 
 struct sort_status {
     int unsorted;                   // some record sorts before its predecessor by (refID, pos)
@@ -30,16 +27,12 @@ __global__ void __launch_bounds__(256) bam_sort_key_kernel(const uint8_t* __rest
     int bad_order = 0;
     if (i < n) {
         const uint8_t* r = u + rec[i];
-        const int32_t tid = (int32_t)ld32(r), pos = (int32_t)ld32(r + 4);
-        const uint32_t reverse = (ld32(r + 12) >> 20) & 1u;            // FLAG (bytes 14-15) & 0x10
+        const int32_t tid = (int32_t)ld32(r + BAM_REF_ID), pos = (int32_t)ld32(r + BAM_POS);
+        const uint32_t reverse = (ld16(r + BAM_FLAG) >> 4) & 1u;      // FLAG & 0x10
         if (tid < 0 || tid >= n_ref || pos < -1) atomicMin(&st->bad, (unsigned long long)i);
         // refID < 2^31 - 1 and pos + 1 < 2^31: both fields fit (refID above bit 32, pos + 1 in bits 1..31, the strand in bit 0)
         key[i] = ((unsigned long long)(uint32_t)tid << 32) | ((unsigned long long)(uint32_t)(pos + 1) << 1) | reverse;
-        if (i > 0) {
-            const uint8_t* q = u + rec[i - 1];
-            const int32_t ptid = (int32_t)ld32(q), ppos = (int32_t)ld32(q + 4);
-            bad_order = (tid < ptid) || (tid == ptid && pos < ppos);
-        }
+        bad_order = bam_out_of_order(u, rec, i, tid, pos);
     }
     if (__ballot_sync(0xffffffffu, bad_order) && (threadIdx.x & 31) == 0) atomicExch(&st->unsorted, 1);
 }

@@ -29,17 +29,13 @@
 // tc_bam_records_to_reads — which takes device pointers as they are.
 #include <cub/device/device_scan.cuh>
 
+#include "bamrec.cuh"
 #include "inflate_core.cuh"
 #include "tc_common.cuh"
 
 namespace {
 
 using namespace tcinf;
-
-__device__ __forceinline__ uint32_t ld16(const uint8_t* p) { return (uint32_t)p[0] | ((uint32_t)p[1] << 8); }
-__device__ __forceinline__ uint32_t ld32(const uint8_t* p) {
-    return (uint32_t)p[0] | ((uint32_t)p[1] << 8) | ((uint32_t)p[2] << 16) | ((uint32_t)p[3] << 24);
-}
 
 constexpr unsigned long long NO_ERROR = ~0ull;
 
@@ -128,14 +124,15 @@ __device__ __forceinline__ bool record_valid(const uint8_t* u, long long n, long
     const uint32_t bs = ld32(u + q);
     *bs_out = bs;
     if (bs < 32u || bs > 0x7fffffffu || q + 4 + (long long)bs > n) return false;
-    const uint8_t* r = u + q + 4;
-    const uint32_t l_name = r[8], n_cig = ld16(r + 12), l_seq = ld32(r + 16);
-    const long long need = 32ll + l_name + 4ll * n_cig + ((long long)l_seq + 1) / 2 + (long long)l_seq;
+    const uint8_t* r = u + q - BAM_BLOCK_SIZE;
+    const uint32_t l_name = r[BAM_L_READ_NAME], n_cig = ld16(r + BAM_N_CIGAR_OP), l_seq = ld32(r + BAM_L_SEQ);
+    const long long need = (long long)BAM_READ_NAME + l_name + 4ll * n_cig + ((long long)l_seq + 1) / 2 + (long long)l_seq;
     if (l_seq > 0x7fffffffu || need > (long long)bs || l_name < 1u) return false;
-    if (r[32 + l_name - 1] != 0) return false;
-    const int32_t refid = (int32_t)ld32(r);
+    if (r[BAM_READ_NAME + l_name - 1] != 0) return false;
+    const int32_t refid = (int32_t)ld32(r + BAM_REF_ID);
     if (refid >= 0 && n_cig == 2) {             // the CG-tag placeholder of a CIGAR with more than 65535 operations: not expanded
-        const uint32_t c0 = ld32(r + 32 + l_name), c1 = ld32(r + 32 + l_name + 4);
+        const uint8_t* cg = bam_cigar(r);
+        const uint32_t c0 = ld32(cg), c1 = ld32(cg + 4);
         if ((c0 & 15u) == 4u && (c0 >> 4) == l_seq && (c1 & 15u) == 3u && l_seq > 0) return false;
     }
     return true;
@@ -146,15 +143,16 @@ __device__ bool record_plausible(const chain_args& a, long long q) {
     if (q + 36 > a.n) return false;
     uint32_t bs;
     if (!record_valid(a.u, a.n, q, &bs)) return false;
-    const uint8_t* r = a.u + q + 4;
-    const int32_t refid = (int32_t)ld32(r), pos = (int32_t)ld32(r + 4), mrefid = (int32_t)ld32(r + 20), mpos = (int32_t)ld32(r + 24);
+    const uint8_t* r = a.u + q - BAM_BLOCK_SIZE;
+    const int32_t refid = (int32_t)ld32(r + BAM_REF_ID), pos = (int32_t)ld32(r + BAM_POS);
+    const int32_t mrefid = (int32_t)ld32(r + BAM_NEXT_REF_ID), mpos = (int32_t)ld32(r + BAM_NEXT_POS);
     if (refid < -1 || refid >= a.n_ref || mrefid < -1 || mrefid >= a.n_ref || pos < -1 || mpos < -1) return false;
     if (refid >= 0 && pos > a.ref_len[refid]) return false;
-    const uint32_t l_name = r[8], n_cig = ld16(r + 12);
+    const uint32_t l_name = r[BAM_L_READ_NAME], n_cig = ld16(r + BAM_N_CIGAR_OP);
     for (uint32_t k = 0; k + 1 < l_name; ++k)
-        if (r[32 + k] < 33 || r[32 + k] > 126) return false;
+        if (r[BAM_READ_NAME + k] < 33 || r[BAM_READ_NAME + k] > 126) return false;
     for (uint32_t k = 0; k < n_cig; ++k)
-        if ((r[32 + l_name + 4 * k] & 15u) > 8u) return false;
+        if ((r[BAM_READ_NAME + l_name + 4 * k] & 15u) > 8u) return false;
     return true;
 }
 
@@ -248,10 +246,10 @@ __global__ void __launch_bounds__(128) bam_chain_walk_kernel(chain_args a) {
             uint32_t bs;
             if (!WRITE && !record_valid(a.u, a.n, q, &bs)) { atomicMin(&a.totals[4], (unsigned long long)q + 1ull); break; }
             if (WRITE) bs = ld32(a.u + q);
-            const uint8_t* r = a.u + q + 4;
-            if ((int32_t)ld32(r) >= 0) {
-                if (WRITE) out[kept] = q + 4;
-                else { words += (ld32(r + 16) + 7u) / 8u; ops += ld16(r + 12); }
+            const uint8_t* r = a.u + q - BAM_BLOCK_SIZE;
+            if ((int32_t)ld32(r + BAM_REF_ID) >= 0) {
+                if (WRITE) out[kept] = q - BAM_BLOCK_SIZE;
+                else { words += (ld32(r + BAM_L_SEQ) + 7u) / 8u; ops += ld16(r + BAM_N_CIGAR_OP); }
                 ++kept;
             }
             ++total;

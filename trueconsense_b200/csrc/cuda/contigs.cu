@@ -13,20 +13,17 @@
 #include <algorithm>
 #include <vector>
 
+#include "bamrec.cuh"
 #include "tc_common.cuh"
 
 namespace {
-
-__device__ __forceinline__ int32_t ld_i32(const uint8_t* p) {     // records start at any byte
-    return (int32_t)((uint32_t)p[0] | ((uint32_t)p[1] << 8) | ((uint32_t)p[2] << 16) | ((uint32_t)p[3] << 24));
-}
 
 __global__ void __launch_bounds__(256) contig_ranges_kernel(const uint8_t* __restrict__ u, const long long* __restrict__ rec, long long n,
                                                             int n_ref, int32_t* __restrict__ first_read, int* __restrict__ err) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    const int tid = ld_i32(u + rec[i]);
-    const int prev = i > 0 ? ld_i32(u + rec[i - 1]) : -1;
+    const int tid = (int32_t)ld32(u + rec[i] + BAM_REF_ID);
+    const int prev = i > 0 ? (int32_t)ld32(u + rec[i - 1] + BAM_REF_ID) : -1;
     if (tid < 0 || tid >= n_ref) { atomicCAS(err, 0, TC_ERR_RANGE); return; }
     if (tid < prev) { atomicCAS(err, 0, TC_ERR_UNSORTED); return; }
     for (int k = max(prev, -1) + 1; k <= tid; ++k) first_read[k] = (int32_t)i;        // references tid and the empty ones before it
@@ -50,9 +47,11 @@ __global__ void __launch_bounds__(256) contig_shift_kernel(shift_args a) {
     }
     const int b = __ldg(a.base + lo), len = __ldg(a.base + lo + 1) - b;
     long long span = 0;
+    // (unrolled twice: nvcc's own four-fold unroll of op_consumes_ref's bit test takes four more registers)
+#pragma unroll 2
     for (uint32_t k = a.cigar_off[r]; k < a.cigar_off[r + 1]; ++k) {
-        const uint32_t c = a.cigar[k], op = c & 15u;
-        if (op == OP_M || op == OP_D || op == OP_N || op == OP_EQ || op == OP_X) span += (long long)(c >> 4);
+        const uint32_t c = a.cigar[k];
+        if (op_consumes_ref(c & 15u)) span += (long long)(c >> 4);
     }
     int p = a.pos[r];
     if (!(a.flag[r] & 4u)) {

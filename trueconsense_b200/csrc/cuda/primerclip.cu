@@ -17,6 +17,7 @@
 #include <algorithm>
 #include <vector>
 
+#include "bamrec.cuh"
 #include "tc_common.cuh"
 
 namespace {
@@ -24,12 +25,6 @@ namespace {
 constexpr unsigned FULL = 0xffffffffu;
 constexpr int REC_WARPS = 8;            // records per 256-thread block
 
-__device__ __forceinline__ uint32_t ld32(const uint8_t* p) {       // records start at any byte
-    return (uint32_t)p[0] | ((uint32_t)p[1] << 8) | ((uint32_t)p[2] << 16) | ((uint32_t)p[3] << 24);
-}
-__device__ __forceinline__ void st32(uint8_t* p, uint32_t v) {
-    p[0] = (uint8_t)v; p[1] = (uint8_t)(v >> 8); p[2] = (uint8_t)(v >> 16); p[3] = (uint8_t)(v >> 24);
-}
 __device__ __forceinline__ bool is_clip(uint32_t op) { return op == OP_S || op == OP_H; }
 __device__ __forceinline__ uint32_t query_len(uint32_t c) {          // M, I, S, =, X
     const uint32_t op = c & 15u;
@@ -95,15 +90,14 @@ __device__ __forceinline__ long long warp_scan(long long v, int lane) {
 }
 
 __device__ void plan_record(const clip_args& a, long long i, int lane, unsigned long long* acc) {
-    const uint8_t* r = a.u + a.rec[i] - 4;
-    const int32_t tid = (int32_t)ld32(r + 4);
-    const long long p = (int32_t)ld32(r + 8);
-    const uint32_t w3 = ld32(r + 12), w4 = ld32(r + 16);
-    const uint32_t l_name = w3 & 0xffu, n_cig = w4 & 0xffffu, flag = w4 >> 16;
-    const uint8_t* cig = r + 36 + l_name;
-    const unsigned long long size = 4ull + ld32(r);
+    const uint8_t* r = a.u + a.rec[i];
+    const int32_t tid = (int32_t)ld32(r + BAM_REF_ID);
+    const long long p = (int32_t)ld32(r + BAM_POS);
+    const uint32_t n_cig = ld16(r + BAM_N_CIGAR_OP), flag = ld16(r + BAM_FLAG);
+    const uint8_t* cig = bam_cigar(r);
+    const unsigned long long size = 4ull + ld32(r + BAM_BLOCK_SIZE);
     clip_plan pl;
-    pl.pos = (int32_t)p; pl.flag_bin = flag | (w3 & 0xffff0000u); pl.n_cig = n_cig; pl.edit = 0;
+    pl.pos = (int32_t)p; pl.flag_bin = flag | (ld16(r + BAM_BIN) << 16); pl.n_cig = n_cig; pl.edit = 0;
     // the span, whether a match op occurs, where the body begins and ends, whether an op has length 0, how many H / S ops
     long long span = 0;
     bool any_match = false, zero_len = false;
@@ -268,33 +262,33 @@ __global__ void __launch_bounds__(256) clip_pack_kernel(clip_args a) {
     const long long i = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
     if (i >= a.n) return;
-    const uint8_t* r = a.u + a.rec[i] - 4;
-    const unsigned long long o = a.off[i];
-    uint8_t* w = a.out + o;
+    const uint8_t* r = a.u + a.rec[i];
+    const unsigned long long o = a.off[i];     // the output record's block_size
+    uint8_t* w = a.out + o - BAM_BLOCK_SIZE;
     const clip_plan pl = a.plan[i];
-    const uint32_t old_size = 4u + ld32(r);
-    if (lane == 0) a.rec_out[i] = (long long)o + 4;
+    const uint32_t old_size = 4u + ld32(r + BAM_BLOCK_SIZE);
+    if (lane == 0) a.rec_out[i] = (long long)o - BAM_BLOCK_SIZE;
     if (!pl.edit) {
-        warp_copy(w, r, old_size, lane);
+        warp_copy(w + BAM_BLOCK_SIZE, r + BAM_BLOCK_SIZE, old_size, lane);
         __syncwarp();
-        if (lane == 0) { w[18] = (uint8_t)pl.flag_bin; w[19] = (uint8_t)(pl.flag_bin >> 8); }
+        if (lane == 0) { w[BAM_FLAG] = (uint8_t)pl.flag_bin; w[BAM_FLAG + 1] = (uint8_t)(pl.flag_bin >> 8); }
         return;
     }
-    const uint32_t l_name = r[12], n_old = ld32(r + 16) & 0xffffu;
-    const uint8_t* cig = r + 36 + l_name;
+    const uint32_t l_name = r[BAM_L_READ_NAME], n_old = ld16(r + BAM_N_CIGAR_OP);
+    const uint8_t* cig = bam_cigar(r);
     const uint32_t new_size = old_size + 4u * pl.n_cig - 4u * n_old;
-    // fixed fields: block_size, pos, bin, n_cigar_op patched; refID, l_read_name, MAPQ, FLAG, l_seq, mate fields and the name as
-    // they were
+    // the fixed fields one 32-bit word per lane: 0 block_size, 1 refID, 2 pos, 3 l_read_name | MAPQ | bin, 4 n_cigar_op | FLAG,
+    // 5 l_seq, 6 next refID, 7 next pos, 8 tlen.  block_size, pos, bin and n_cigar_op are patched; the rest and the name stay
     if (lane < 9) {
-        uint32_t x = ld32(r + 4 * lane);
+        uint32_t x = ld32(r + BAM_BLOCK_SIZE + 4 * lane);
         if (lane == 0) x = new_size - 4u;
         else if (lane == 2) x = (uint32_t)pl.pos;
         else if (lane == 3) x = (x & 0xffffu) | (pl.flag_bin & 0xffff0000u);
         else if (lane == 4) x = pl.n_cig | (x & 0xffff0000u);
-        st32(w + 4 * lane, x);
+        st32(w + BAM_BLOCK_SIZE + 4 * lane, x);
     }
-    for (uint32_t j = lane; j < l_name; j += 32) w[36 + j] = r[36 + j];
-    uint8_t* nc = w + 36 + l_name;
+    for (uint32_t j = lane; j < l_name; j += 32) w[BAM_READ_NAME + j] = r[BAM_READ_NAME + j];
+    uint8_t* nc = w + BAM_READ_NAME + l_name;
     // leading section, then the body ops kl..kr (kl cut at its front, kr at its back), then the trailing section
     uint32_t at = 0;
     if (pl.edit & 1u) {
@@ -329,8 +323,8 @@ __global__ void __launch_bounds__(256) clip_pack_kernel(clip_args a) {
         for (uint32_t k = (uint32_t)pl.trail + lane; k < n_old_i; k += 32) st32(nc + 4ull * (at + k - (uint32_t)pl.trail), ld32(cig + 4ull * k));
     }
     // SEQ, QUAL and the optional fields as they are
-    const uint32_t tail_off = 36u + l_name + 4u * n_old;
-    warp_copy(nc + 4ull * pl.n_cig, r + tail_off, old_size - tail_off, lane);
+    const uint32_t tail_off = BAM_READ_NAME + l_name + 4u * n_old;
+    warp_copy(nc + 4ull * pl.n_cig, r + tail_off, old_size - 4u - tail_off, lane);
 }
 
 }  // namespace

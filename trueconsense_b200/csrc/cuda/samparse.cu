@@ -20,6 +20,7 @@
 #include <utility>
 #include <vector>
 
+#include "bamrec.cuh"
 #include "tc_common.cuh"
 
 namespace {
@@ -338,10 +339,6 @@ __global__ void __launch_bounds__(256) sam_meta_kernel(sam_args a) {
     if (threadIdx.x < 3 && acc[threadIdx.x]) atomicAdd(&a.status[1 + threadIdx.x], acc[threadIdx.x]);
 }
 
-__device__ __forceinline__ void st32(uint8_t* p, uint32_t v) {      // records start at any byte
-    p[0] = (uint8_t)v; p[1] = (uint8_t)(v >> 8); p[2] = (uint8_t)(v >> 16); p[3] = (uint8_t)(v >> 24);
-}
-
 // htslib's seq_nt16 rule: "=ACMGRSVTWYHKDBN" in either case -> 0..15, anything else 15
 __device__ uint8_t nt16_of(unsigned c) {
     if (c >= 'a' && c <= 'z') c -= 32;
@@ -363,10 +360,12 @@ __global__ void __launch_bounds__(256) sam_pack_kernel(sam_args a) {
     const uint8_t* u = a.u;
     const sam_meta& m = a.meta[k];
     const long long b = a.ls[k];
-    const unsigned long long o = a.off[k];
-    uint8_t* r = a.out + o;
+    const unsigned long long o = a.off[k];     // the record's block_size
+    uint8_t* r = a.out + o - BAM_BLOCK_SIZE;
     const uint32_t l_name = (uint32_t)m.tab[0] + 1, n_cig = m.n_cig, l_seq = (uint32_t)m.l_seq;
-    if (lane == 0) a.rec[a.rank[k]] = (long long)o + 4;
+    if (lane == 0) a.rec[a.rank[k]] = (long long)o - BAM_BLOCK_SIZE;
+    // the fixed fields one 32-bit word per lane: 0 block_size, 1 refID, 2 pos, 3 l_read_name | MAPQ | bin, 4 n_cigar_op | FLAG,
+    // 5 l_seq, 6 next refID, 7 next pos, 8 tlen
     if (lane < 9) {
         const unsigned long long size = a.off[k + 1] - o;       // placed: the next offset is this record's end
         uint32_t x;
@@ -381,9 +380,9 @@ __global__ void __launch_bounds__(256) sam_pack_kernel(sam_args a) {
             case 7: x = (uint32_t)m.mpos; break;
             default: x = (uint32_t)m.tlen; break;
         }
-        st32(r + 4 * lane, x);
+        st32(r + BAM_BLOCK_SIZE + 4 * lane, x);
     }
-    uint8_t* nm = r + 36;
+    uint8_t* nm = r + BAM_READ_NAME;
     for (uint32_t j = lane; j < l_name; j += 32) nm[j] = j + 1 < l_name ? u[b + j] : 0;
     uint8_t* cg = nm + l_name;
     if (n_cig) {

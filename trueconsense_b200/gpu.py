@@ -208,6 +208,9 @@ class DeviceReads:
         self.ctx = ctx
         self.generation = generation
         self.stats = None
+        self.info = {}              # what the decode counted and how long each step took (the *_to_device routes)
+        self.ref_names = None       # the header's references (the *_to_device routes)
+        self.ref_lens = None
         self.first_read = None      # [n_ref + 1]: where each reference's reads begin (bam_file_to_device(contig_ranges=True))
         self.contig_start = None    # set once the reads sit in the global columns of a multi-reference pass
 
@@ -302,18 +305,6 @@ class Context:
         self._check(self._lib.tc_download(self._h, _ptr(out), dev_ptr, out.nbytes, stream))
         return out
 
-    def _contig_ranges(self, payload_ptr, n_bytes: int, rec_ptr, n_reads: int, n_ref: int, stream: int) -> np.ndarray:
-        first = np.zeros(n_ref + 1, np.int32)
-        self._check(self._lib.tc_bam_contig_ranges(self._h, payload_ptr, n_bytes, rec_ptr, n_reads, n_ref, _ptr(first), stream))
-        return first
-
-    def _sort_records(self, payload_ptr, n_bytes: int, rec_ptr, n_reads: int, n_ref: int, stream: int):
-        """tc_bam_sort_records: (device payload, record offsets in coordinate order, whether they moved)."""
-        p, r, moved = C.c_void_p(), C.c_void_p(), C.c_int32(0)
-        self._check(self._lib.tc_bam_sort_records(self._h, payload_ptr, n_bytes, rec_ptr, n_reads, n_ref, C.byref(p), C.byref(r),
-                                                  C.byref(moved), stream))
-        return p.value, r.value, bool(moved.value)
-
     def clip_primers(self, payload_ptr, n_bytes: int, rec_ptr, n_reads: int, names, primers, stream: int = 0):
         """``tc_bam_clip_primers``: the records (payload and refID offsets, host or device) with the primers of ``primers`` (a
         ``primers.PrimerScheme``; its chrom names mapped to ``names``, the header's references) soft-clipped off.  Returns
@@ -326,11 +317,6 @@ class Context:
                                                   int(bool(primers.both_ends)), C.byref(p), C.byref(nb), C.byref(r), C.byref(st), stream))
         return p.value, int(nb.value), r.value, st
 
-    @staticmethod
-    def _clip_info(st: "ClipStats", t: float) -> dict:
-        return {"n_clipped_left": int(st.n_left), "n_clipped_right": int(st.n_right), "n_fully_clipped": int(st.n_unmapped),
-                "clipped_columns": int(st.n_columns), "t_clip_s": t}
-
     def bam_to_device(self, payload, stream: int = 0, contig_ranges: bool = False, sort: bool = False, primers=None) -> DeviceReads:
         """GPU-side record parsing (tc_bam_records_to_reads): a ``bamio.BamPayload`` (the BAM inflated on the host, its records
         indexed) becomes the flat read arrays in the context's device buffers — the CPU never touches a record's body.
@@ -339,31 +325,12 @@ class Context:
         (``tc_bam_sort_records``; the payload then travels to the device once); ``.info`` says whether they moved
         (``reordered``) and what that took (``t_sort_s``).
         ``primers`` (a ``primers.PrimerScheme``): the primers are soft-clipped off the records first (``tc_bam_clip_primers``)
-        and the clipped records are sorted (``sort`` is implied); ``.info`` then also holds the clip's counts and ``t_clip_s``."""
-        import time
-
-        pay, rec, n, n_bytes = payload.payload_ptr, payload.rec_off_ptr, payload.n_reads, payload.n_bytes
+        and the clipped records are sorted (``sort`` is implied); ``.info`` then also holds the clip's counts and ``t_clip_s``.
+        The result carries ``.ref_names`` and ``.ref_lens`` (the payload's header), and ``contig_ranges`` adds ``.first_read``
+        as for :meth:`bam_file_to_device`."""
         self._generation += 1
-        t0 = time.perf_counter()
-        clip = {}
-        if primers is not None:
-            pay, n_bytes, rec, cst = self.clip_primers(pay, n_bytes, rec, n, payload.ref_names, primers, stream)
-            clip = self._clip_info(cst, time.perf_counter() - t0)
-            sort = True
-        t0 = time.perf_counter()
-        moved = False
-        if sort:
-            pay, rec, moved = self._sort_records(pay, n_bytes, rec, n, len(payload.ref_lens), stream)
-        t1 = time.perf_counter()
-        dev = TcReads()
-        st = BamStats()
-        self._check(self._lib.tc_bam_records_to_reads(self._h, pay, n_bytes, rec, n, C.byref(dev), C.byref(st), stream))
-        d = DeviceReads(dev, None, self, self._generation)
-        d.stats = st
-        d.info = {"reordered": moved, "t_sort_s": t1 - t0, **clip}
-        if contig_ranges and payload.ref_names and not st.unsorted:
-            d.first_read = self._contig_ranges(pay, n_bytes, rec, n, len(payload.ref_names), stream)
-        return d
+        return self._records_to_device(payload.payload_ptr, payload.n_bytes, payload.rec_off_ptr, payload.n_reads,
+                                       payload.ref_names, payload.ref_lens, {}, stream, contig_ranges, sort, primers)
 
     def bam_file_to_device(self, path: str, stream: int = 0, contig_ranges: bool = False, sort: bool = False,
                            primers=None) -> DeviceReads:
@@ -411,39 +378,45 @@ class Context:
         t3 = time.perf_counter()
         info.update(n_records=int(n_records.value), n_dropped_unplaced=int(n_records.value - n_placed.value), t_map_s=t1 - t0,
                     t_inflate_s=t2 - t1, t_index_s=t3 - t2)
-        return self._records_to_device(payload, n_bytes, rec, n_placed.value, names, lens, info, stream, contig_ranges, sort,
-                                       primers)
+        return self._records_to_device(payload.value, n_bytes, rec.value, n_placed.value, names, lens, info, stream, contig_ranges,
+                                       sort, primers)
 
-    def _records_to_device(self, payload, n_bytes: int, rec, n_placed: int, names, lens, info: dict, stream: int,
+    def _records_to_device(self, payload, n_bytes: int, rec, n_reads: int, names, lens, info: dict, stream: int,
                            contig_ranges: bool, sort: bool, primers=None) -> DeviceReads:
-        """The tail of both file routes: BAM records in device memory (payload, offsets of the placed ones) -> primers
+        """The tail every route shares: BAM records (payload and the offsets of the placed ones, host or device) -> primers
         clipped when given (``tc_bam_clip_primers``, which implies the sort), sorted when asked (``tc_bam_sort_records``),
-        parsed (``tc_bam_records_to_reads``), the contig ranges -> ``DeviceReads`` with ``.ref_names``, ``.ref_lens``,
-        ``.stats`` and ``info`` plus the clip's, the sort's and the parse's timings."""
+        parsed (``tc_bam_records_to_reads``), the contig ranges when asked (``tc_bam_contig_ranges``) -> ``DeviceReads``
+        with ``.ref_names``, ``.ref_lens``, ``.stats`` and ``info`` plus the clip's, the sort's and the parse's timings.
+        The caller has bumped ``_generation``."""
         import time
 
+        payload, rec = C.c_void_p(payload), C.c_void_p(rec)
         if primers is not None:
             t = time.perf_counter()
-            payload, n_bytes, rec, cst = self.clip_primers(payload, n_bytes, rec, n_placed, names, primers, stream)
-            payload, rec = C.c_void_p(payload), C.c_void_p(rec)
-            info.update(self._clip_info(cst, time.perf_counter() - t))
+            p, n_bytes, r, st = self.clip_primers(payload, n_bytes, rec, n_reads, names, primers, stream)
+            payload, rec = C.c_void_p(p), C.c_void_p(r)
+            info.update(n_clipped_left=int(st.n_left), n_clipped_right=int(st.n_right), n_fully_clipped=int(st.n_unmapped),
+                        clipped_columns=int(st.n_columns), t_clip_s=time.perf_counter() - t)
             sort = True
-        t3 = time.perf_counter()
-        moved = False
+        t0 = time.perf_counter()
+        moved = C.c_int32(0)
         if sort:
-            _, rec, moved = self._sort_records(payload, n_bytes, rec, n_placed, len(lens), stream)
-            rec = C.c_void_p(rec)
-        t3s = time.perf_counter()
+            # a host payload is staged once here: the parse and the contig ranges go on from the device copy
+            self._check(self._lib.tc_bam_sort_records(self._h, payload, n_bytes, rec, n_reads, len(lens), C.byref(payload),
+                                                      C.byref(rec), C.byref(moved), stream))
+        t1 = time.perf_counter()
         dev = TcReads()
         st = BamStats()
-        self._check(self._lib.tc_bam_records_to_reads(self._h, payload, n_bytes, rec, n_placed, C.byref(dev), C.byref(st), stream))
-        t4 = time.perf_counter()
+        self._check(self._lib.tc_bam_records_to_reads(self._h, payload, n_bytes, rec, n_reads, C.byref(dev), C.byref(st), stream))
+        t2 = time.perf_counter()
         d = DeviceReads(dev, None, self, self._generation)
         d.stats = st
         d.ref_names, d.ref_lens = names, lens
         if contig_ranges and lens and not st.unsorted:
-            d.first_read = self._contig_ranges(payload, n_bytes, rec, n_placed, len(lens), stream)
-        info.update(t_sort_s=t3s - t3, t_parse_s=t4 - t3s, reordered=moved)
+            d.first_read = np.zeros(len(lens) + 1, np.int32)
+            self._check(self._lib.tc_bam_contig_ranges(self._h, payload, n_bytes, rec, n_reads, len(lens), _ptr(d.first_read),
+                                                       stream))
+        info.update(reordered=bool(moved.value), t_sort_s=t1 - t0, t_parse_s=t2 - t1)
         d.info = info
         return d
 
@@ -496,8 +469,8 @@ class Context:
         info = {"sam_bytes": size, "n_lines": int(n_lines.value), "n_records": int(n_records.value),
                 "n_dropped_unplaced": int(n_records.value - n_placed.value), "t_map_s": t1 - t0, "t_upload_s": steps[0],
                 "t_line_index_s": steps[1], "t_convert_s": steps[2]}
-        return self._records_to_device(payload, int(n_payload.value), rec, int(n_placed.value), names, lens, info, stream,
-                                       contig_ranges, sort, primers)
+        return self._records_to_device(payload.value, int(n_payload.value), rec.value, int(n_placed.value), names, lens, info,
+                                       stream, contig_ranges, sort, primers)
 
     def reads_to_contig_coords(self, reads: DeviceReads, ref_lens, first_read, names=None, stream: int = 0) -> np.ndarray:
         """Move device-resident reads to the global columns of a multi-reference pass, in place (``tc_reads_to_contig_coords``):

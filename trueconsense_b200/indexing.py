@@ -20,6 +20,23 @@ from .reads import ReadBatch
 
 COLUMNS = ["coverage", "A", "T", "C", "G", "X", "I"]
 
+# the refusals of a pass over one reference: pysam's pileup message for reads out of order, and ours for a second reference
+UNSORTED = "Unsorted input. Pileup aborts"
+MULTI_CONTIG = ("multi-contig BAM: TrueConsense indexes positions of a single reference "
+                "(its DataFrame index would hold duplicate positions)")
+
+
+def _refuse(multi_contig: bool, unsorted: bool) -> None:
+    if multi_contig:
+        raise ValueError(MULTI_CONTIG)
+    if unsorted:
+        raise ValueError(UNSORTED)
+
+
+def _fresh(d, ctx) -> bool:
+    """Whether device reads made earlier still sit in ``ctx``'s buffers (the context has staged nothing since)."""
+    return d is not None and d.ctx is ctx and d.generation == ctx._generation
+
 
 class BamHandle:
     """What ``Readbam`` returns: a BAM on its way to the device plus the attributes of ``pysam.AlignmentFile`` the reference
@@ -50,7 +67,6 @@ class BamHandle:
         self.primers = primers
         self.is_sam = reads is None and pathlib.Path(filename).suffix == ".sam"
         self._reads = reads
-        self._payload = None
         self._hdr = None
         self._dev = None
         self._dev_contigs = None        # (key, DeviceReads, ContigLayout): the reads moved to a multi-reference layout
@@ -75,8 +91,6 @@ class BamHandle:
         with self._lock:
             if self._reads is not None:
                 return self._reads.ref_names, self._reads.ref_lens
-            if self._payload is not None:
-                return self._payload.ref_names, self._payload.ref_lens
             if self._hdr is None and self.is_sam:
                 self._hdr = bamio.read_sam_header(self.filename)[:2]    # the '@' lines only
             if self._hdr is None:
@@ -99,9 +113,7 @@ class BamHandle:
         """Host-side reads placed on the first reference (the only one the reference implementation is
         meaningful for: indexing.py:98,139 and Events.py:63 use lengths[0] / references[0])."""
         b = self.reads
-        if b.tid is not None and b.n_reads and np.any(b.tid != 0):
-            raise ValueError("multi-contig BAM: TrueConsense indexes positions of a single reference "
-                             "(its DataFrame index would hold duplicate positions)")
+        _refuse(b.tid is not None and b.n_reads and np.any(b.tid != 0), False)
         return b
 
     def device_reads(self, with_host_qual: bool = False):
@@ -112,21 +124,13 @@ class BamHandle:
         ctx = gpu.default_context()
         with self._lock:
             d = self._dev
-            if d is None or d.ctx is not ctx or d.generation != ctx._generation:
-                if self._reads is not None:
-                    b = self._reads
-                    if b.tid is not None and b.n_reads and np.any(b.tid != 0):
-                        raise ValueError("multi-contig BAM: TrueConsense indexes positions of a single reference")
-                    if not b.sorted:
-                        raise ValueError("Unsorted input. Pileup aborts")
-                    d = ctx.upload(b, with_qual=False)
-                else:
-                    d = self._file_to_device(ctx)
-                    if d.stats.multi_contig:
-                        raise ValueError("multi-contig BAM: TrueConsense indexes positions of a single reference "
-                                         "(its DataFrame index would hold duplicate positions)")
-                    if d.stats.unsorted:
-                        raise ValueError("Unsorted input. Pileup aborts")
+            if not _fresh(d, ctx):
+                b = self._reads
+                if b is not None:       # refused before anything is staged
+                    _refuse(b.tid is not None and b.n_reads and np.any(b.tid != 0), not b.sorted)
+                d = self._to_device(ctx)
+                if b is None:
+                    _refuse(d.stats.multi_contig, d.stats.unsorted)
                 self._dev = d
             return d.with_host_qual() if with_host_qual else d
 
@@ -139,19 +143,16 @@ class BamHandle:
         key = (tuple(names), tuple(int(x) for x in lens))
         with self._lock:
             c = self._dev_contigs
-            if c is not None and c[0] == key and c[1].ctx is ctx and c[1].generation == ctx._generation:
+            if c is not None and c[0] == key and _fresh(c[1], ctx):
                 return c[1], c[2]
             self._dev_contigs = None
-            if self._reads is not None:
-                b = self._reads
-                if not b.sorted:
-                    raise ValueError("Unsorted input. Pileup aborts")
+            b = self._reads
+            if b is not None:           # refused before anything is staged
+                _refuse(False, not b.sorted)
                 first_read = contig_ranges_from_tid(b.tid, len(names), b.n_reads)
-                d = ctx.upload(b)       # QUAL and mate fields too: the move shifts PNEXT on the device
-            else:
-                d = self._file_to_device(ctx, contig_ranges=True)
-                if d.stats.unsorted:
-                    raise ValueError("Unsorted input. Pileup aborts")
+            d = self._to_device(ctx, contig_ranges=True)
+            if b is None:
+                _refuse(False, d.stats.unsorted)
                 first_read = d.first_read
             if len(first_read) != len(names) + 1:
                 raise ValueError(f"the BAM header holds {len(first_read) - 1} references, {len(names)} were given")
@@ -160,22 +161,26 @@ class BamHandle:
             self._dev_contigs = (key, d, layout)
             return d, layout
 
-    def _file_to_device(self, ctx, contig_ranges: bool = False):
-        """The file's reads parsed into device memory (the caller holds the lock)."""
+    def _to_device(self, ctx, contig_ranges: bool = False):
+        """The reads in device memory, not yet checked (the caller holds the lock).  A host batch is uploaded: for a pass
+        over one reference without QUAL and the mate fields (see :meth:`device_reads`), for a multi-reference pass
+        (``contig_ranges``) with them, as the move shifts PNEXT on the device.  A file is decoded on the GPU."""
+        if self._reads is not None:
+            return ctx.upload(self._reads, with_qual=contig_ranges)
+        kw = dict(contig_ranges=contig_ranges, sort=self.sort, primers=self.primers)
         if self.is_sam:
-            d = ctx.sam_file_to_device(self.filename, contig_ranges=contig_ranges, sort=self.sort, primers=self.primers)
-            self._hdr = (d.ref_names, d.ref_lens)
-            return d
-        try:
-            # inflate, record index, (clip, sort) and parse on the GPU
-            d = ctx.bam_file_to_device(self.filename, contig_ranges=contig_ranges, sort=self.sort, primers=self.primers)
-            self._hdr = (d.ref_names, d.ref_lens)
-        except gpu.TcError:
-            # a file the device path refuses: the host reader names the broken member / record (or, should it
-            # read the file after all, feeds the device parse)
-            self._payload = bamio.read_bam_payload(self.filename)
-            d = ctx.bam_to_device(self._payload, contig_ranges=contig_ranges, sort=self.sort, primers=self.primers)
-            self._payload.release()     # the device holds the arrays now; the header stays
+            d = ctx.sam_file_to_device(self.filename, **kw)
+        else:
+            try:
+                # inflate, record index, (clip, sort) and parse on the GPU
+                d = ctx.bam_file_to_device(self.filename, **kw)
+            except gpu.TcError:
+                # a file the device path refuses: the host reader names the broken member / record (or, should it
+                # read the file after all, feeds the device parse)
+                payload = bamio.read_bam_payload(self.filename)
+                d = ctx.bam_to_device(payload, **kw)
+                payload.release()       # the device holds the arrays now
+        self._hdr = (d.ref_names, d.ref_lens)
         return d
 
     def pileup(self, *args, **kwargs):
@@ -214,7 +219,7 @@ def contig_ranges_from_tid(tid, n_ref: int, n_reads: int) -> np.ndarray:
     if t.size and (int(t.min()) < 0 or int(t.max()) >= n_ref):
         raise ValueError(f"a read's reference index lies outside the header's {n_ref} references")
     if t.size and np.any(np.diff(t.astype(np.int64)) < 0):
-        raise ValueError("Unsorted input. Pileup aborts")
+        raise ValueError(UNSORTED)
     return np.searchsorted(t, np.arange(n_ref + 1), side="left").astype(np.int32)
 
 
