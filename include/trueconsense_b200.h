@@ -251,6 +251,20 @@ int  tc_bam_clip_primers(tc_ctx_t* ctx, const uint8_t* payload, int64_t n_bytes,
                          const uint8_t** payload_dev, int64_t* n_bytes_out, const int64_t** rec_off_dev,
                          tc_clip_stats_t* stats, void* stream);
 
+/* ---- the decoded records written back as a BAM file image, BGZF members compressed on the device ----
+ * header[0 .. n_header): the BAM header to write (magic to the last reference, host memory).  payload / rec_off: records as
+ * tc_bam_records_to_reads takes them (host or device), written in rec_off's order, byte for byte except bin, which becomes
+ * reg2bin(pos, end) (end = pos + the CIGAR's reference length, pos + 1 without one).  The uncompressed stream is the header
+ * in members of its own, then the records from a fresh member on, cut every 0xff00 bytes; every member is one raw DEFLATE
+ * stream (dynamic Huffman, or stored when that is smaller) in a gzip member with the BC subfield, CRC-32 and ISIZE, as
+ * htslib writes them; the 28-byte EOF member ends the image.  *image_dev: the file's bytes in a context buffer of its own
+ * (valid until the next tc_bam_write_records on this context), *image_bytes their count, *n_members the members before the
+ * EOF member.  Writes no buffer a decode's read arrays, payload or record offsets live in.  t_ms (may be NULL): CUDA-event
+ * milliseconds of the gather, the compression and the compaction.  Synchronises the stream twice. */
+int  tc_bam_write_records(tc_ctx_t* ctx, const uint8_t* header, int64_t n_header, const uint8_t* payload, int64_t n_bytes,
+                          const int64_t* rec_off, int64_t n_reads, const uint8_t** image_dev, int64_t* image_bytes,
+                          int64_t* n_members, float t_ms[3], void* stream);
+
 /* ---- SAM text straight from the aligner -> BAM records on the device ----
  * text[0 .. n_bytes): the SAM file (host or device memory); its records begin at first_line_off, which is file line
  * first_line_no (1-based) — the caller has read the '@' header lines and hands over the @SQ names in header order:

@@ -9,6 +9,8 @@ validators and exit behaviour, same order of work — on top of the GPU hot path
     python -m trueconsense_b200.TrueConsense --sort-input -i s.sam -ref ref.fa -gff f.gff -cov 30 -name S -o S.fasta
     python -m trueconsense_b200.TrueConsense --primers scheme.primer.bed --primer-both-ends -i s.sam -ref ref.fa -gff f.gff \
         -cov 30 -name S -o S.fasta
+    python -m trueconsense_b200.TrueConsense --primers scheme.primer.bed -i s.sam -ref ref.fa -gff f.gff -cov 30 -name S \
+        -o S.fasta --output-bam S.clipped.sorted.bam
 
 ``main(args)`` is the console-script entry point of the reference (pyproject.toml:38-40).
 """
@@ -82,6 +84,9 @@ def GetArgs(givenargs):
     opt.add_argument("--depth-of-coverage", "-doc", type=str, metavar="File",
                      help="Output TSV file listing the coverage per position")
     opt.add_argument("--output-gff", "-ogff", type=str, metavar="File", help="Ouput location a corrected GFF file")
+    opt.add_argument("--output-bam", "-obam", type=str, metavar="File",
+                     help="Output BAM of the reads the consensus was called from (primers clipped, coordinate-sorted), "
+                          "compressed on the GPU; unplaced reads are left out")
     opt.add_argument("--threads", "-t", default=min(multiprocessing.cpu_count(), 128), metavar="N", type=int,
                      help="Number of threads that can be used by TrueConsense")
     opt.add_argument("--noambiguity", "-noambig", action="store_true",
@@ -114,6 +119,8 @@ def GetArgs(givenargs):
         parser.error("--index-override cannot be combined with --all-contigs: its positions name no reference")
     if opts.primers is None and (opts.primer_tolerance is not None or opts.primer_both_ends):
         parser.error("--primer-tolerance and --primer-both-ends need --primers")
+    if opts.output_bam is not None and pathlib.Path(opts.output_bam).suffix != ".bam":
+        parser.error(f"Output BAM {color.YELLOW}({opts.output_bam}){color.END} doesn't seem to be a BAM file.")
     if opts.primer_tolerance is None:
         opts.primer_tolerance = 5
     elif opts.primer_tolerance < 0:
@@ -159,7 +166,7 @@ def main(args: list[str] | None = None):
     opts = GetArgs(argv)
     primers = None if opts.primers is None else read_bed(opts.primers, opts.primer_tolerance, opts.primer_both_ends)
     # one decoded copy of the BAM serves the index and the insertion columns
-    bam = Readbam(opts.input, sort=opts.sort_input, primers=primers)
+    bam = Readbam(opts.input, sort=opts.sort_input, primers=primers, output_bam=opts.output_bam)
     if opts.all_contigs:
         return _main_all_contigs(opts, bam)
     frame, gff = _index_and_features(opts, bam)

@@ -218,6 +218,46 @@ def read_sam_header(path: str):
     return names, lens, off, line_no
 
 
+def sam_bam_header(path: str, names, lens, first_off: int) -> bytes:
+    """The BAM header of a SAM file: its ``@`` lines (the file's first ``first_off`` bytes) as the text, then the ``@SQ``
+    references ``names`` / ``lens`` (``read_sam_header``)."""
+    import struct
+
+    with open(path, "rb") as fh:
+        text = fh.read(first_off)
+    refs = b"".join(struct.pack("<i", len(r) + 1) + r + b"\0" + struct.pack("<i", ln)
+                    for r, ln in zip((n.encode(errors="surrogateescape") for n in names), lens))
+    return b"BAM\1" + struct.pack("<i", len(text)) + text + struct.pack("<i", len(names)) + refs
+
+
+HD_COORDINATE = b"@HD\tVN:1.6\tSO:coordinate"
+
+
+def coordinate_header(header: bytes) -> bytes:
+    """A BAM header (magic to the last reference) whose text says the records are in coordinate order: a first ``@HD``
+    line has its ``SO:`` value replaced (or ``\\tSO:coordinate`` added); without one, ``@HD\\tVN:1.6\\tSO:coordinate`` is
+    inserted as the first line.  A header that says ``SO:coordinate`` already comes back as it is."""
+    import struct
+
+    l_text = struct.unpack_from("<i", header, 4)[0]
+    text, rest = header[8:8 + l_text], header[8 + l_text:]
+    if text.startswith(b"@HD\t") or text.startswith(b"@HD\n") or text == b"@HD":
+        end = text.find(b"\n")
+        end = len(text) if end < 0 else end
+        fields = text[:end].split(b"\t")
+        so = [k for k, f in enumerate(fields) if f.startswith(b"SO:")]
+        if so:
+            if fields[so[0]] == b"SO:coordinate":
+                return header
+            fields[so[0]] = b"SO:coordinate"
+        else:
+            fields.append(b"SO:coordinate")
+        text = b"\t".join(fields) + text[end:]
+    else:
+        text = HD_COORDINATE + b"\n" + text
+    return b"BAM\1" + struct.pack("<i", len(text)) + text + rest
+
+
 _lib = None
 
 

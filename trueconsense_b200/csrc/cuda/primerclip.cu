@@ -32,17 +32,6 @@ __device__ __forceinline__ uint32_t query_len(uint32_t c) {          // M, I, S,
 }
 __device__ __forceinline__ uint32_t ref_len(uint32_t c) { return op_consumes_ref(c & 15u) ? (c >> 4) : 0u; }
 
-// htslib's hts_reg2bin(beg, end, 14, 5)
-__device__ __forceinline__ uint32_t reg2bin(long long beg, long long end) {
-    --end;
-    if (beg >> 14 == end >> 14) return (uint32_t)(4681 + (beg >> 14));
-    if (beg >> 17 == end >> 17) return (uint32_t)(585 + (beg >> 17));
-    if (beg >> 20 == end >> 20) return (uint32_t)(73 + (beg >> 20));
-    if (beg >> 23 == end >> 23) return (uint32_t)(9 + (beg >> 23));
-    if (beg >> 26 == end >> 26) return (uint32_t)(1 + (beg >> 26));
-    return 0;
-}
-
 // per reference r the primers [first[r], first[r + 1]): starts ascending with the running max of the ends, ends ascending with
 // the running min of the starts from the right
 struct primer_tables {
@@ -239,23 +228,6 @@ __global__ void __launch_bounds__(256) clip_plan_kernel(clip_args a) {
     if (i < a.n) plan_record(a, i, threadIdx.x & 31, acc);
     __syncthreads();
     if (threadIdx.x < 4 && acc[threadIdx.x]) atomicAdd(&a.status[1 + threadIdx.x], acc[threadIdx.x]);
-}
-
-// n bytes from s to d, the lanes sharing them: 4-byte stores wherever d is aligned (s may lie at any byte: two aligned
-// loads and a funnel shift; every word loaded holds at least one byte of the source)
-__device__ void warp_copy(uint8_t* d, const uint8_t* s, uint32_t n, int lane) {
-    const uint32_t head = (uint32_t)((4u - ((uintptr_t)d & 3u)) & 3u) < n ? (uint32_t)((4u - ((uintptr_t)d & 3u)) & 3u) : n;
-    if ((uint32_t)lane < head) d[lane] = s[lane];
-    d += head; s += head; n -= head;
-    const uint32_t words = n >> 2, sh = (uint32_t)((uintptr_t)s & 3u);
-    uint32_t* dw = reinterpret_cast<uint32_t*>(d);
-    const uint32_t* sw = reinterpret_cast<const uint32_t*>(s - sh);
-    if (sh == 0) {
-        for (uint32_t j = lane; j < words; j += 32) dw[j] = sw[j];
-    } else {
-        for (uint32_t j = lane; j < words; j += 32) dw[j] = __funnelshift_r(sw[j], sw[j + 1], 8 * sh);
-    }
-    for (uint32_t j = 4 * words + lane; j < n; j += 32) d[j] = s[j];
 }
 
 __global__ void __launch_bounds__(256) clip_pack_kernel(clip_args a) {

@@ -22,6 +22,7 @@ enum tc_slot {
     SLOT_TMP_A, SLOT_TMP_B, SLOT_TMP_C, SLOT_TILES, SLOT_SEGS, SLOT_COV_TOTALS, SLOT_BAM_PAYLOAD, SLOT_BAM_REC, SLOT_CIGAR16, SLOT_SEQ2, SLOT_SEQ_EXC_IDX, SLOT_SEQ_EXC_VAL, SLOT_BGZF_FILE, SLOT_BGZF_BLOCKS,
     SLOT_CONTIG_A, SLOT_CONTIG_B, SLOT_CONTIG_C, SLOT_BAM_REC_SORTED, SLOT_SAM_TEXT, SLOT_SAM_LINES, SLOT_SAM_META, SLOT_SAM_REFS,
     SLOT_CLIP_PLAN, SLOT_CLIP_PAYLOAD, SLOT_CLIP_REC,
+    SLOT_BAMW_PAYLOAD, SLOT_BAMW_REC, SLOT_BAMW_WORK, SLOT_BAMW_TMP, SLOT_BAMW_RAW, SLOT_BAMW_MEMBERS, SLOT_BAMW_IMAGE,
     SLOT_COUNT
 };
 

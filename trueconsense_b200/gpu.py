@@ -136,6 +136,9 @@ def lib() -> C.CDLL:
             l.tc_bgzf_inflate.restype = C.c_int
             l.tc_bam_index_records.argtypes = [vp, vp, i64, i64, i32, vp, C.POINTER(vp), C.POINTER(i64), C.POINTER(i64), vp]
             l.tc_bam_index_records.restype = C.c_int
+            l.tc_bam_write_records.argtypes = [vp, vp, i64, vp, i64, vp, i64, C.POINTER(vp), C.POINTER(i64), C.POINTER(i64),
+                                               C.POINTER(C.c_float), vp]
+            l.tc_bam_write_records.restype = C.c_int
             l.tc_download.argtypes = [vp, vp, vp, i64, vp]
             l.tc_download.restype = C.c_int
             l.tc_sample_enqueue.argtypes = [vp, C.POINTER(TcReads), i32, C.POINTER(PileupParams), C.POINTER(CallParams),
@@ -213,6 +216,7 @@ class DeviceReads:
         self.ref_lens = None
         self.first_read = None      # [n_ref + 1]: where each reference's reads begin (bam_file_to_device(contig_ranges=True))
         self.contig_start = None    # set once the reads sit in the global columns of a multi-reference pass
+        self.records = None         # (BAM header bytes, payload, bytes, record offsets, count) the reads were parsed from
 
     def with_host_qual(self) -> "DeviceReads":
         """The same device arrays plus the batch's HOST quality and mate arrays (QNAME hash, PNEXT, TLEN):
@@ -328,9 +332,15 @@ class Context:
         and the clipped records are sorted (``sort`` is implied); ``.info`` then also holds the clip's counts and ``t_clip_s``.
         The result carries ``.ref_names`` and ``.ref_lens`` (the payload's header), and ``contig_ranges`` adds ``.first_read``
         as for :meth:`bam_file_to_device`."""
+        from . import bamio
+
+        n = 1 << 16
+        while (hdr := bamio.parse_bam_header(C.string_at(payload.payload_ptr, min(n, payload.n_bytes)), payload.n_bytes)) is None:
+            n *= 4
+        header = C.string_at(payload.payload_ptr, hdr[2])
         self._generation += 1
         return self._records_to_device(payload.payload_ptr, payload.n_bytes, payload.rec_off_ptr, payload.n_reads,
-                                       payload.ref_names, payload.ref_lens, {}, stream, contig_ranges, sort, primers)
+                                       payload.ref_names, payload.ref_lens, {}, stream, contig_ranges, sort, primers, header)
 
     def bam_file_to_device(self, path: str, stream: int = 0, contig_ranges: bool = False, sort: bool = False,
                            primers=None) -> DeviceReads:
@@ -379,15 +389,16 @@ class Context:
         info.update(n_records=int(n_records.value), n_dropped_unplaced=int(n_records.value - n_placed.value), t_map_s=t1 - t0,
                     t_inflate_s=t2 - t1, t_index_s=t3 - t2)
         return self._records_to_device(payload.value, n_bytes, rec.value, n_placed.value, names, lens, info, stream, contig_ranges,
-                                       sort, primers)
+                                       sort, primers, head[:first])
 
     def _records_to_device(self, payload, n_bytes: int, rec, n_reads: int, names, lens, info: dict, stream: int,
-                           contig_ranges: bool, sort: bool, primers=None) -> DeviceReads:
+                           contig_ranges: bool, sort: bool, primers=None, header: bytes = b"") -> DeviceReads:
         """The tail every route shares: BAM records (payload and the offsets of the placed ones, host or device) -> primers
         clipped when given (``tc_bam_clip_primers``, which implies the sort), sorted when asked (``tc_bam_sort_records``),
         parsed (``tc_bam_records_to_reads``), the contig ranges when asked (``tc_bam_contig_ranges``) -> ``DeviceReads``
-        with ``.ref_names``, ``.ref_lens``, ``.stats`` and ``info`` plus the clip's, the sort's and the parse's timings.
-        The caller has bumped ``_generation``."""
+        with ``.ref_names``, ``.ref_lens``, ``.stats`` and ``info`` plus the clip's, the sort's and the parse's timings, and
+        ``.records``: the BAM header (``header``) and the final records, what :meth:`write_bam` writes.  The caller has bumped
+        ``_generation``."""
         import time
 
         payload, rec = C.c_void_p(payload), C.c_void_p(rec)
@@ -412,6 +423,7 @@ class Context:
         d = DeviceReads(dev, None, self, self._generation)
         d.stats = st
         d.ref_names, d.ref_lens = names, lens
+        d.records = (header, payload.value, n_bytes, rec.value, n_reads)
         if contig_ranges and lens and not st.unsorted:
             d.first_read = np.zeros(len(lens) + 1, np.int32)
             self._check(self._lib.tc_bam_contig_ranges(self._h, payload, n_bytes, rec, n_reads, len(lens), _ptr(d.first_read),
@@ -470,7 +482,48 @@ class Context:
                 "n_dropped_unplaced": int(n_records.value - n_placed.value), "t_map_s": t1 - t0, "t_upload_s": steps[0],
                 "t_line_index_s": steps[1], "t_convert_s": steps[2]}
         return self._records_to_device(payload.value, int(n_payload.value), rec.value, int(n_placed.value), names, lens, info,
-                                       stream, contig_ranges, sort, primers)
+                                       stream, contig_ranges, sort, primers, bamio.sam_bam_header(path, names, lens, first_off))
+
+    def write_bam(self, reads: DeviceReads, path: str, stream: int = 0) -> dict:
+        """Write the records ``reads`` were parsed from as a BAM file (``tc_bam_write_records``: BGZF members compressed on the
+        GPU).  The file holds the decode's placed records in the order the passes read them (clipped, sorted), byte for byte
+        except ``bin``, which is recomputed; the header is the input's with ``@HD ... SO:coordinate`` (DESIGN §4).  The file is
+        written beside ``path`` and renamed onto it, so a failure leaves no partial file there.  ``reads`` stay valid.
+        Returns, and adds to ``reads.info``: ``bam_out_bytes``, ``n_out_members``, ``n_written``, ``t_write_s`` and
+        ``t_device_ms`` (CUDA-event milliseconds of the gather, the compression and the compaction)."""
+        import time
+
+        from . import bamio
+
+        if not isinstance(reads, DeviceReads) or reads.ctx is not self:
+            raise TypeError("write_bam writes the device reads of this context")
+        if reads.records is None:
+            raise ValueError("these device reads were uploaded from a host ReadBatch, which holds no BAM records: only reads "
+                             "decoded from a file or payload (bam_file_to_device, sam_file_to_device, bam_to_device) can be written")
+        if reads.generation != self._generation:
+            raise RuntimeError("these device reads are stale: the context has decoded or staged another batch since, and their "
+                               "records are gone")
+        t0 = time.perf_counter()
+        header, payload, n_bytes, rec, n = reads.records
+        header = bamio.coordinate_header(header)
+        img, nb, nm = C.c_void_p(), C.c_int64(0), C.c_int64(0)
+        t_ms = (C.c_float * 3)()
+        self._check(self._lib.tc_bam_write_records(self._h, header, len(header), payload, n_bytes, rec, n, C.byref(img), C.byref(nb),
+                                                   C.byref(nm), t_ms, stream))
+        data = self.download(img.value, nb.value, np.uint8, stream)
+        tmp = f"{path}.{os.getpid()}.{threading.get_ident()}.tmp"
+        try:
+            with open(tmp, "xb") as fh:
+                fh.write(data.data)
+            os.replace(tmp, path)
+        except BaseException:
+            if os.path.exists(tmp):
+                os.unlink(tmp)
+            raise
+        out = {"bam_out_bytes": int(nb.value), "n_out_members": int(nm.value), "n_written": int(n),
+               "t_write_s": time.perf_counter() - t0, "t_device_ms": float(t_ms[0] + t_ms[1] + t_ms[2])}
+        reads.info.update(out)
+        return out
 
     def reads_to_contig_coords(self, reads: DeviceReads, ref_lens, first_read, names=None, stream: int = 0) -> np.ndarray:
         """Move device-resident reads to the global columns of a multi-reference pass, in place (``tc_reads_to_contig_coords``):

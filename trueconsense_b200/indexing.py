@@ -57,11 +57,20 @@ class BamHandle:
     ``primers`` (a ``primers.PrimerScheme``, ``primers.read_bed``): the amplicon primers are soft-clipped off the records on
     the GPU before the sort (``tc_bam_clip_primers``), so every pass computes what it computes after ``samtools ampliconclip``
     and ``samtools sort``; ``sort`` is then always on.  There is no host-side clip: ``reads`` raises
-    ``NotImplementedError``, and a handle made from a host ``ReadBatch`` cannot take primers (``ValueError``)."""
+    ``NotImplementedError``, and a handle made from a host ``ReadBatch`` cannot take primers (``ValueError``).
 
-    def __init__(self, filename: str, reads: ReadBatch | None = None, sort: bool = False, primers=None):
+    ``output_bam`` (a path): the records the device reads were parsed from (clipped and sorted when asked) are written there
+    as a BAM (``gpu.Context.write_bam``), once, at the first device decode and after its checks pass: an input the decode
+    refuses leaves no file.  A handle made from a host ``ReadBatch`` cannot take it (``ValueError``)."""
+
+    def __init__(self, filename: str, reads: ReadBatch | None = None, sort: bool = False, primers=None, output_bam=None):
         if primers is not None and reads is not None:
             raise ValueError("primers are clipped on the GPU during the decode of a file; a host ReadBatch cannot take them")
+        if output_bam is not None and reads is not None:
+            raise ValueError("output_bam writes the records of a file decoded on the GPU; a host ReadBatch holds none")
+        self.output_bam = output_bam
+        self._written = output_bam is None
+        self._payload = None            # the host payload of the fallback route, kept until the BAM is written
         self.filename = filename
         self.sort = sort or primers is not None
         self.primers = primers
@@ -131,6 +140,7 @@ class BamHandle:
                 d = self._to_device(ctx)
                 if b is None:
                     _refuse(d.stats.multi_contig, d.stats.unsorted)
+                self._write_once(ctx, d)
                 self._dev = d
             return d.with_host_qual() if with_host_qual else d
 
@@ -156,6 +166,7 @@ class BamHandle:
                 first_read = d.first_read
             if len(first_read) != len(names) + 1:
                 raise ValueError(f"the BAM header holds {len(first_read) - 1} references, {len(names)} were given")
+            self._write_once(ctx, d)
             start = ctx.reads_to_contig_coords(d, key[1], first_read, names)
             layout = ContigLayout(list(names), list(key[1]), start.astype(np.int64), np.asarray(first_read, np.int64))
             self._dev_contigs = (key, d, layout)
@@ -179,9 +190,22 @@ class BamHandle:
                 # read the file after all, feeds the device parse)
                 payload = bamio.read_bam_payload(self.filename)
                 d = ctx.bam_to_device(payload, **kw)
-                payload.release()       # the device holds the arrays now
+                if self._written:
+                    payload.release()       # the device holds the arrays now
+                else:
+                    self._payload = payload     # unsorted, unclipped records stay in the host payload until written
         self._hdr = (d.ref_names, d.ref_lens)
         return d
+
+    def _write_once(self, ctx, d) -> None:
+        """``output_bam`` from the first device decode that passed its checks (the caller holds the lock)."""
+        if self._written:
+            return
+        ctx.write_bam(d, self.output_bam)
+        self._written = True
+        if self._payload is not None:
+            self._payload.release()
+            self._payload = None
 
     def pileup(self, *args, **kwargs):
         raise NotImplementedError("column iteration is not part of this implementation; "
@@ -248,14 +272,15 @@ def gff_by_contig(df: pd.DataFrame, names) -> dict:
     return {n: df[df["seqid"] == n].reset_index(drop=True) for n in names}
 
 
-def Readbam(f, sort: bool = False, primers=None):
+def Readbam(f, sort: bool = False, primers=None, output_bam=None):
     """indexing.py:6-19.  A handle passed in is returned as is, so one decoded copy of the BAM can
     serve BuildIndex, ListInserts and WriteOutputs.  ``sort``: accept records that are not coordinate-sorted and put them
     in samtools' coordinate order on the GPU (``BamHandle``).  A ``.sam`` path is read as SAM text, on the GPU.
-    ``primers`` (``primers.read_bed``): the amplicon primers are soft-clipped off the reads on the GPU (implies ``sort``)."""
+    ``primers`` (``primers.read_bed``): the amplicon primers are soft-clipped off the reads on the GPU (implies ``sort``).
+    ``output_bam``: the decoded (clipped, sorted) records are also written to this path as a BAM (``BamHandle``)."""
     if isinstance(f, BamHandle):
         return f
-    return BamHandle(f, sort=sort, primers=primers)
+    return BamHandle(f, sort=sort, primers=primers, output_bam=output_bam)
 
 
 class _GffHeader:
