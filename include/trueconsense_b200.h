@@ -398,7 +398,10 @@ int  tc_pileup_call_inserts(tc_ctx_t* ctx, const tc_reads_t* reads, int32_t ref_
 /* The same in two halves, so that the host's share of one sample (unpacking the results, preparing the next call) hides
  * behind the device's work on the next: tc_sample_enqueue returns as soon as everything is enqueued, tc_sample_finish
  * waits for that sample only.  At most two samples may be in flight on a context, enqueued on the same stream; the reads,
- * counts and table buffers of a sample must stay valid (and untouched by the caller) until its tc_sample_finish returns. */
+ * counts and table buffers of a sample must stay valid (and untouched by the caller) until its tc_sample_finish returns.
+ * The count table is ready in stream order on `stream`.  The call table and the insertion calls are ready once
+ * tc_sample_finish returns: they are computed on a stream of the context's own, where they may run beside the next
+ * sample's pileup. */
 int  tc_sample_enqueue(tc_ctx_t* ctx, const tc_reads_t* reads, int32_t ref_len, const tc_pileup_params_t* pileup,
                        const tc_call_params_t* call, const tc_pileup_params_t* inserts, int32_t* counts,
                        const tc_call_table_t* table, void* stream, int32_t* ticket);

@@ -314,7 +314,7 @@ static int pileup_plan_of(tc_ctx* ctx, const tc_pileup_params_t* p, const pileup
 // Everything of one attempt up to (not including) the read-back of the status block: memsets, the span pass if the plan has
 // one, the pileup kernel, the coverage scan.  `counts` may be a host pointer (the table is then built in a context buffer).
 int tc_pileup_enqueue(tc_ctx* ctx, const tc_reads_t* reads, int32_t L, const tc_pileup_params_t* p, int32_t* counts, cudaStream_t s,
-                      tc_pileup_pending* pend, int rung) {
+                      tc_pileup_pending* pend, int rung, int grid) {
     const bool per_entry = p->min_base_quality > 0;
     pileup_args a = {};
     int rc = tc_resolve_reads(ctx, reads, &a.r, per_entry ? NEED_QUAL : 0, s);
@@ -340,7 +340,7 @@ int tc_pileup_enqueue(tc_ctx* ctx, const tc_reads_t* reads, int32_t L, const tc_
             TC_LAUNCH_CHECK();
         }
         rc = plan.variant == 4 ? tc_pileup_long_launch(ctx, a, s)
-           : plan.variant == 3 ? tc_pileup_warp_launch(ctx, a, s)
+           : plan.variant == 3 ? tc_pileup_warp_launch(ctx, a, s, grid)
            : per_entry ? launch_scatter<true>(ctx, a, s) : launch_scatter<false>(ctx, a, s);
         if (rc) return rc;
         TC_CUDA(timing_event(ctx, ctx->ev1, s));

@@ -59,8 +59,9 @@ __device__ __forceinline__ bool read_passes(const pileup_args& a, int64_t r) {
 }
 
 
-// variant 3 (pileup_warp.cu): barrier-free warp-per-read-stream SWAR kernel; fills every row except coverage
-int tc_pileup_warp_launch(tc_ctx* ctx, const pileup_args& a, cudaStream_t s);
+// variant 3 (pileup_warp.cu): barrier-free warp-per-read-stream SWAR kernel; fills every row except coverage.  grid: its CTAs
+// (0: one per SM; the reads are shared out over whatever grid it gets)
+int tc_pileup_warp_launch(tc_ctx* ctx, const pileup_args& a, cudaStream_t s, int grid = 0);
 bool tc_pileup_warp_supported(const pileup_args& a);
 
 // long reads (pileup_long.cu): cut every read into pieces of <= PIECE_COLS columns and run variant 3 over the pieces

@@ -716,7 +716,7 @@ bool tc_pileup_warp_supported(const pileup_args& a) {
 }
 
 template <int WC, bool PIECES>
-static int launch_geom(tc_ctx* ctx, const pileup_args& a, cudaStream_t s) {
+static int launch_geom(tc_ctx* ctx, const pileup_args& a, cudaStream_t s, int grid = 0) {
     using G = geom<WC>;
     const size_t smem = sizeof(uint32_t) * (size_t)(G::WARP_WORDS + 2) * G::WARPS;
     const uint32_t bit = 1u << ((WC == 32 ? 0 : WC == 64 ? 1 : 2) + (PIECES ? 3 : 0));
@@ -724,7 +724,7 @@ static int launch_geom(tc_ctx* ctx, const pileup_args& a, cudaStream_t s) {
         TC_CUDA(cudaFuncSetAttribute(warp_pileup_kernel<WC, PIECES>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         ctx->warp_attr_set |= bit;
     }
-    warp_pileup_kernel<WC, PIECES><<<ctx->sm_count, G::WARPS * 32, smem, s>>>(a);
+    warp_pileup_kernel<WC, PIECES><<<grid > 0 ? grid : ctx->sm_count, G::WARPS * 32, smem, s>>>(a);
     TC_LAUNCH_CHECK();
     return TC_OK;
 }
@@ -732,18 +732,18 @@ static int launch_geom(tc_ctx* ctx, const pileup_args& a, cudaStream_t s) {
 // Without a span bound all geometries are enqueued: each reads the longest reference span the span pass left in
 // a.status and returns at once unless it is the one that fits (no host round trip in between).  With the caller's
 // bound the host knows which one that is.
-int tc_pileup_warp_launch(tc_ctx* ctx, const pileup_args& a, cudaStream_t s) {
+int tc_pileup_warp_launch(tc_ctx* ctx, const pileup_args& a, cudaStream_t s, int grid) {
     if (a.span_hint > 0) {
         const int wc = warp_geometry(a.span_hint);
-        if (wc == 32) return launch_geom<32, false>(ctx, a, s);
-        if (wc == 64) return launch_geom<64, false>(ctx, a, s);
-        return launch_geom<128, false>(ctx, a, s);      // (too long for it too: the kernel declines the batch)
+        if (wc == 32) return launch_geom<32, false>(ctx, a, s, grid);
+        if (wc == 64) return launch_geom<64, false>(ctx, a, s, grid);
+        return launch_geom<128, false>(ctx, a, s, grid);      // (too long for it too: the kernel declines the batch)
     }
-    int rc = launch_geom<32, false>(ctx, a, s);
+    int rc = launch_geom<32, false>(ctx, a, s, grid);
     if (rc) return rc;
-    rc = launch_geom<64, false>(ctx, a, s);
+    rc = launch_geom<64, false>(ctx, a, s, grid);
     if (rc) return rc;
-    return launch_geom<128, false>(ctx, a, s);
+    return launch_geom<128, false>(ctx, a, s, grid);
 }
 
 // pieces of long reads (pileup_long.cu): always the 512-column geometry

@@ -87,17 +87,35 @@ static int sample_unchained(tc_ctx* ctx, const tc_reads_t* reads, int32_t L, con
     return rc;
 }
 
+// SMs the pileup kernel leaves free while the other sample's tail may still be running.  The kernel holds one CTA of 227 KiB
+// of shared memory on every SM it gets, so no tail kernel fits beside it: with a full grid the tail of sample i waits for the
+// whole pileup of sample i + 1.  With k SMs left to it, the tail runs under that pileup, which takes about
+// sm_count / (sm_count - k) times as long.  k from a sweep on one B200 (scripts/overlap_sweep.py, profiles/overlap_sweep.json).
+// TC_OVERLAP_SMS overrides it for such measurements; a negative value runs every tail behind its head on the caller's stream.
+constexpr int TC_OVERLAP_SMS = 4;
+
+static int overlap_sms() {
+    const char* e = getenv("TC_OVERLAP_SMS");
+    return e && *e ? atoi(e) : TC_OVERLAP_SMS;
+}
+
 static int sample_slots(tc_ctx* ctx) {
     if (ctx->samples) return TC_OK;
     tc_sample_slot* sl = (tc_sample_slot*)calloc(2, sizeof(tc_sample_slot));
     if (!sl) return tc_fail(ctx, TC_ERR_NOMEM, "out of host memory");
-    for (int i = 0; i < 2; ++i) {
-        cudaError_t e = cudaMallocHost(&sl[i].host_block, TC_HOST_SCRATCH);
+    int least = 0, greatest = 0;
+    cudaError_t e = cudaDeviceGetStreamPriorityRange(&least, &greatest);
+    for (int i = 0; i < 2 && e == cudaSuccess; ++i) {
+        e = cudaMallocHost(&sl[i].host_block, TC_HOST_SCRATCH);
         if (e == cudaSuccess) e = cudaEventCreateWithFlags(&sl[i].done, cudaEventDisableTiming);
+        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&sl[i].head_done, cudaEventDisableTiming);
         if (e == cudaSuccess) e = cudaEventCreate(&sl[i].t0);
         if (e == cudaSuccess) e = cudaEventCreate(&sl[i].t1);
-        if (e != cudaSuccess) { free(sl); return tc_cuda_fail(ctx, e, "sample slot"); }
+        // non-blocking: a caller on the legacy default stream would otherwise serialise the tail with the next head again;
+        // the highest priority: the tail's CTAs go to the SMs the next pileup leaves free ahead of anything pending
+        if (e == cudaSuccess) e = cudaStreamCreateWithPriority(&sl[i].tail_stream, cudaStreamNonBlocking, greatest);
     }
+    if (e != cudaSuccess) { free(sl); return tc_cuda_fail(ctx, e, "sample slot"); }
     ctx->samples = sl;
     return TC_OK;
 }
@@ -105,9 +123,14 @@ static int sample_slots(tc_ctx* ctx) {
 void tc_sample_slots_free(tc_ctx* ctx) {
     if (!ctx->samples) return;
     for (int i = 0; i < 2; ++i) {
-        if (ctx->samples[i].host_block) cudaFreeHost(ctx->samples[i].host_block);
-        if (ctx->samples[i].done) { cudaEventDestroy(ctx->samples[i].done); cudaEventDestroy(ctx->samples[i].t0); cudaEventDestroy(ctx->samples[i].t1); }
-        tc_graph_destroy(ctx->samples[i].graph);
+        tc_sample_slot& sl = ctx->samples[i];
+        if (sl.tail_stream) { cudaStreamSynchronize(sl.tail_stream); cudaStreamDestroy(sl.tail_stream); }
+        if (sl.host_block) cudaFreeHost(sl.host_block);
+        if (sl.done) { cudaEventDestroy(sl.done); cudaEventDestroy(sl.head_done); cudaEventDestroy(sl.t0); cudaEventDestroy(sl.t1); }
+        tc_graph_destroy(sl.head);
+        tc_graph_destroy(sl.tail);
+        for (int b = 0; b < SLOT_COUNT; ++b)
+            if (sl.bufs[b].p) cudaFree(sl.bufs[b].p);
     }
     free(ctx->samples);
     ctx->samples = nullptr;
@@ -116,30 +139,53 @@ void tc_sample_slots_free(tc_ctx* ctx) {
 
 // everything the enqueued work depends on: the same key means the same kernels with the same arguments
 static int sample_key(const tc_ctx* ctx, const tc_reads_t* reads, int32_t ref_len, const tc_pileup_params_t* pp, const tc_call_params_t* cp,
-                      const tc_pileup_params_t* ip, const int32_t* counts, const tc_call_table_t* table, unsigned char* key) {
+                      const tc_pileup_params_t* ip, const int32_t* counts, const tc_call_table_t* table, int grid, unsigned char* key) {
     int n = 0;
     auto put = [&](const void* p, size_t bytes) { memcpy(key + n, p, bytes); n += (int)bytes; };
     put(reads, sizeof(*reads)); put(&ref_len, 4); put(pp, sizeof(*pp)); put(cp, sizeof(*cp)); put(ip, sizeof(*ip));
     put(&counts, sizeof(counts)); put(table, sizeof(*table));
-    put(&ctx->buf_epoch, 8); put(&ctx->ins_slot_cap, 8); put(&ctx->pair_cap, 8); put(&ctx->timing, 4);
+    put(&ctx->buf_epoch, 8); put(&ctx->ins_slot_cap, 8); put(&ctx->pair_cap, 8); put(&ctx->timing, 4); put(&grid, 4);
     return n;
 }
-static_assert(sizeof(tc_reads_t) + 4 + 2 * sizeof(tc_pileup_params_t) + sizeof(tc_call_params_t) + 8 + sizeof(tc_call_table_t) + 28 <= 512, "sample key");
+static_assert(sizeof(tc_reads_t) + 4 + 2 * sizeof(tc_pileup_params_t) + sizeof(tc_call_params_t) + 8 + sizeof(tc_call_table_t) + 32 <= 512, "sample key");
 
-static int sample_enqueue_chain(tc_ctx* ctx, tc_sample_slot& sl, cudaStream_t s) {
+// head: the pileup and the coverage scan (grid: the pileup kernel's CTAs, 0 for one per SM)
+static int sample_head(tc_ctx* ctx, tc_sample_slot& sl, int grid, cudaStream_t s) {
     // timing on: the events around the pileup kernel are this sample's own (two samples may be in flight)
     const cudaEvent_t e0 = ctx->ev0, e1 = ctx->ev1;
     sl.timed = ctx->timing;
     if (ctx->timing) { ctx->ev0 = sl.t0; ctx->ev1 = sl.t1; }
-    int rc = tc_pileup_enqueue(ctx, &sl.reads, sl.ref_len, &sl.pp, sl.counts, s, &sl.pend);
+    const int rc = tc_pileup_enqueue(ctx, &sl.reads, sl.ref_len, &sl.pp, sl.counts, s, &sl.pend, 0, grid);
     ctx->ev0 = e0; ctx->ev1 = e1;
-    if (rc) return rc;
-    rc = tc_call(ctx, sl.counts, sl.ref_len, &sl.cp, &sl.table, (void*)s);       // device outputs only: enqueues and returns
+    return rc;
+}
+
+// tail: everything behind the count table, up to the results block's copy to the host
+static int sample_tail(tc_ctx* ctx, tc_sample_slot& sl, cudaStream_t s) {
+    int rc = tc_call(ctx, sl.counts, sl.ref_len, &sl.cp, &sl.table, (void*)s);       // device outputs only: enqueues and returns
     if (rc) return rc;
     int32_t *d_ncand, *d_cand;
     rc = tc_candidates_enqueue(ctx, sl.table.flags, sl.ref_len, TC_SAMPLE_MAX_CAND, &d_ncand, &d_cand, s);
     if (rc) return rc;
     return tc_inserts_enqueue_dev(ctx, &sl.reads, d_cand, d_ncand, TC_SAMPLE_MAX_CAND, &sl.ip, sl.pend.d_status, sl.host_block, s, &sl.ipend);
+}
+
+// Whether two samples' device outputs (count table, call-table columns) share a byte.  The tail of one and the head (or the
+// fallback calls on the caller's stream) of the other then must not overlap.
+static bool outputs_overlap(const tc_sample_slot& a, const int32_t* counts, const tc_call_table_t& t, int32_t L) {
+    auto ranges = [](const int32_t* c, const tc_call_table_t& u, size_t n, const char** lo, size_t* len) {
+        const void* p[7] = {c, u.call_char, u.flags, u.xrun, u.rank_letter, u.rank_count, u.ambig_char};
+        const size_t b[7] = {4 * TC_NROWS * n, n, n, 4 * n, 4 * n, 16 * n, n};
+        for (int i = 0; i < 7; ++i) { lo[i] = (const char*)p[i]; len[i] = p[i] ? b[i] : 0; }
+    };
+    const char *alo[7], *blo[7];
+    size_t alen[7], blen[7];
+    ranges(a.counts, a.table, (size_t)a.ref_len, alo, alen);
+    ranges(counts, t, (size_t)L, blo, blen);
+    for (int i = 0; i < 7; ++i)
+        for (int j = 0; j < 7; ++j)
+            if (alen[i] && blen[j] && alo[i] < blo[j] + blen[j] && blo[j] < alo[i] + alen[i]) return true;
+    return false;
 }
 
 TC_API int tc_sample_enqueue(tc_ctx_t* ctx, const tc_reads_t* reads, int32_t ref_len, const tc_pileup_params_t* pp,
@@ -155,7 +201,11 @@ TC_API int tc_sample_enqueue(tc_ctx_t* ctx, const tc_reads_t* reads, int32_t ref
     if (rc) return rc;
     const int slot = ctx->sample_next;
     tc_sample_slot& sl = ctx->samples[slot];
+    const tc_sample_slot& other = ctx->samples[slot ^ 1];
     if (sl.state != 0) return tc_fail(ctx, TC_ERR_ARG, "two samples are in flight on this context already: finish one first");
+    // the other sample's tail may still be running beside this sample's work: with shared outputs, everything of this one waits for it
+    const bool shares = other.state != 0 && outputs_overlap(other, counts, *table, ref_len);
+    if (shares && other.state == 1) TC_CUDA(cudaStreamWaitEvent(s, other.done, 0));
     sl.reads = *reads; sl.ref_len = ref_len; sl.pp = *pp; sl.cp = *cp; sl.ip = *ip; sl.counts = counts; sl.table = *table; sl.stream = stream;
     const tc_call_table_t& t = *table;
     const bool table_dev = (!t.call_char || tc_is_device_ptr(t.call_char)) && (!t.xrun || tc_is_device_ptr(t.xrun)) &&
@@ -164,11 +214,31 @@ TC_API int tc_sample_enqueue(tc_ctx_t* ctx, const tc_reads_t* reads, int32_t ref
     if (!tc_reads_all_device(reads) || !table_dev || pp->min_base_quality > 0) {
         sl.state = 2;           // inputs the chained form does not take: the separate calls, at finish time
     } else {
+        // The tail goes to the slot's own stream, where it can run under the next sample's pileup, unless the other sample
+        // runs its separate calls at finish time (state 2) or shares outputs with this one: then it stays in stream order.
+        // This head leaves k SMs to the other sample's tail when that one is on its own stream.
+        const int k = overlap_sms();
+        const bool side = k >= 0 && !shares && other.state != 2;
+        const int grid = other.state == 1 && other.side && side && k > 0 && k < ctx->sm_count ? ctx->sm_count - k : 0;
         unsigned char key[512];
-        const int key_len = sample_key(ctx, reads, ref_len, pp, cp, ip, counts, table, key);
-        rc = tc_graph_run(ctx, sl.graph, key, key_len, true, [&](cudaStream_t cs) { return sample_enqueue_chain(ctx, sl, cs); }, s);
+        ctx->bank = sl.bufs;
+        int key_len = sample_key(ctx, reads, ref_len, pp, cp, ip, counts, table, grid, key);
+        rc = tc_graph_run(ctx, sl.head, key, key_len, true, [&](cudaStream_t cs) { return sample_head(ctx, sl, grid, cs); }, s);
+        cudaStream_t ts = s;
+        if (rc == TC_OK && side) {
+            ts = sl.tail_stream;
+            cudaError_t e = cudaEventRecord(sl.head_done, s);
+            if (e == cudaSuccess) e = cudaStreamWaitEvent(ts, sl.head_done, 0);
+            if (e != cudaSuccess) rc = tc_cuda_fail(ctx, e, "tail stream");
+        }
+        if (rc == TC_OK) {
+            key_len = sample_key(ctx, reads, ref_len, pp, cp, ip, counts, table, 0, key);
+            rc = tc_graph_run(ctx, sl.tail, key, key_len, true, [&](cudaStream_t cs) { return sample_tail(ctx, sl, cs); }, ts);
+        }
+        ctx->bank = nullptr;
         if (rc) return rc;
-        TC_CUDA(cudaEventRecord(sl.done, s));
+        TC_CUDA(cudaEventRecord(sl.done, ts));
+        sl.side = side ? 1 : 0;
         sl.state = 1;
     }
     ctx->sample_next = slot ^ 1;

@@ -46,6 +46,7 @@ struct tc_ctx {
     int64_t launches;
     int64_t h2d_bytes, d2h_bytes;
     tc_buf bufs[SLOT_COUNT];
+    tc_buf* bank;           // non-NULL while a chained sample is enqueued: its slot's buffers, which tc_dev_buf hands out instead
     int ins_attr_set;       // ins_count_kernel's shared-memory attribute has been set
     uint32_t warp_attr_set; // ... and those of the warp_pileup_kernel instances (one bit each)
     void* host_status;      // pinned, 256 bytes
@@ -130,8 +131,9 @@ int tc_resolve_reads(tc_ctx* ctx, const tc_reads_t* in, dreads* out, int need, c
 
 // ---- pieces of the entry points that only ENQUEUE (tc_pileup_call_inserts chains them without a host round trip)
 // rung: the variant of the fallback ladder to run; 0 the first attempt (p->kernel, or for 0 the library's choice)
+// grid: CTAs of the bit-parallel pileup kernel (0: one per SM)
 int tc_pileup_enqueue(tc_ctx* ctx, const tc_reads_t* reads, int32_t ref_len, const tc_pileup_params_t* p, int32_t* counts, cudaStream_t s,
-                      tc_pileup_pending* pend, int rung = 0);
+                      tc_pileup_pending* pend, int rung = 0, int grid = 0);
 // redone (may be NULL): set to 1 when the batch went down the fallback ladder, i.e. another variant rebuilt the table
 int tc_pileup_settle(tc_ctx* ctx, tc_status st, tc_pileup_pending pend, const tc_reads_t* reads, int32_t ref_len,
                      const tc_pileup_params_t* p, int32_t* counts, cudaStream_t s, int* redone);
@@ -166,15 +168,20 @@ struct tc_graph_cache {
 int tc_graph_run(tc_ctx* ctx, tc_graph_cache& g, const unsigned char* key, int key_len, bool can_capture,
                  const std::function<int(cudaStream_t)>& chain, cudaStream_t s);
 void tc_graph_destroy(tc_graph_cache& g);
-// a sample in flight
+// a sample in flight: a head on the caller's stream (pileup and coverage scan) and a tail behind it (call, candidates,
+// ExtractInserts, the results copy), on the slot's own stream when it may overlap the next sample's head
 struct tc_sample_slot {
     int state;                      // 0 free, 1 chained and enqueued, 2 to be run through the separate calls at finish time
+    int side;                       // state 1: the tail went to tail_stream (else it follows the head on the caller's stream)
     void* host_block;               // pinned, TC_HOST_SCRATCH bytes: this sample's results block
     cudaEvent_t done, t0, t1;       // t0 / t1: around this sample's pileup kernel when the context's timing is on
+    cudaEvent_t head_done;          // the tail's start
+    cudaStream_t tail_stream;       // non-blocking, high priority
     int timed;
     tc_reads_t reads; int32_t ref_len; tc_pileup_params_t pp, ip; tc_call_params_t cp; int32_t* counts; tc_call_table_t table; void* stream;
     tc_pileup_pending pend; tc_ins_pending ipend;
-    tc_graph_cache graph;           // one launch per sample instead of ~25 (kernels, memsets, the results copy)
+    tc_graph_cache head, tail;      // two launches per sample instead of ~25 (kernels, memsets, the results copy)
+    tc_buf bufs[SLOT_COUNT];        // every context buffer the chained form uses, this sample's own (ctx->bank)
 };
 
 // ---------------------------------------------------------------- device helpers

@@ -24,7 +24,7 @@ int tc_cuda_fail(tc_ctx* ctx, cudaError_t e, const char* what) {
 }
 
 void* tc_dev_buf(tc_ctx* ctx, int slot, size_t bytes) {
-    tc_buf* b = &ctx->bufs[slot];
+    tc_buf* b = ctx->bank ? &ctx->bank[slot] : &ctx->bufs[slot];
     if (bytes == 0) bytes = 16;
     if (b->cap >= bytes) return b->p;
     if (b->p) { cudaFree(b->p); b->p = NULL; b->cap = 0; }
