@@ -122,8 +122,8 @@ typedef struct tc_pileup_params {
     int64_t  max_depth;         /* BuildIndex: 10000000; ExtractInserts: 8000 */
     int32_t  kernel;            /* 0 = library's choice; 1 = scatter (smem atomics); 3 = bit-parallel, one warp per read stream;
                                    4 = long reads: cut into pieces, then 3 */
-    int32_t  reserved;          /* bit 0: used by the library when it re-enters itself (pass 0).  Bits 8-9, only read with a base-quality
-                                   filter: mate-overlap quality rewriting — 0 = as htslib >= 1.13 does it (pysam 0.23.3 bundles 1.21),
+    int32_t  reserved;          /* bits 8-9, only read with a base-quality filter:
+                                   mate-overlap quality rewriting — 0 = as htslib >= 1.13 does it (pysam 0.23.3 bundles 1.21),
                                    1 = off (pysam's ignore_overlaps=False), 2 = as htslib <= 1.12 did (the first mate keeps its quality) */
 } tc_pileup_params_t;
 

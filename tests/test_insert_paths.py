@@ -69,6 +69,24 @@ def test_column_with_more_distinct_strings_than_the_hash_table(orc):
     assert exp[0][1] == 5000
 
 
+def test_more_candidates_than_a_64_kib_results_block(orc):
+    """720 candidate columns: the results the separate call copies back (96 bytes per candidate) outgrow 64 KiB, and the
+    chained sample's list outgrows its 256 candidates."""
+    from trueconsense_b200.reads import ReadBatch
+
+    rng = np.random.default_rng(14)
+    n_sites = 720
+    sites = [("".join(rng.choice(list("ACGT"), 2)), ["".join(rng.choice(list("ACGT"), 1 + k % 3)) for _ in range(2)])
+             for k in range(n_sites)]
+    recs = []
+    for i in range(12):
+        ins = [v[1] if i % 3 == 0 else v[0] for _, v in sites]
+        recs.append(dict(pos=0, cigar="".join(f"2M{len(s)}I" for s in ins) + "2M",
+                         seq="".join(m + s for (m, _), s in zip(sites, ins)) + "AC"))
+    exp = _all_routes(orc, ReadBatch.from_records(recs), 2 * n_sites + 2, 2 * np.arange(n_sites) + 2)
+    assert exp == [(m[1] + f"+{len(v[0])}" + v[0], 12) for m, v in sites]
+
+
 def test_overlapping_mates_beyond_the_initial_pair_scratch(orc):
     """4,000 overlapping pairs of 1,000-base mates over one column: their rewritten qualities take 8 MB, more than the first
     pair scratch (4 MB)."""

@@ -730,20 +730,44 @@ __global__ void ins_bases_kernel(ins_args a, const tc_insert_call_t* __restrict_
     for (int j = threadIdx.x; j < c.indel; j += blockDim.x) bases[c.bases_off + j] = (uint8_t)ins_char(a, r, a.ent_qpos[e], j + 1, rev);
 }
 
-// ---------------------------------------------------------------- host side, shared by both drivers
-// The results block: status, device-built layout, overflow flags, pair-scratch bump; with_extra (the chained form) the
-// candidate count, the pileup's status and the candidates; then seg_count / pair_any, the calls and their inserted
-// characters.  n_cand: the candidates, or the capacity the chained form enqueues for.
+// ---------------------------------------------------------------- host side
+// Two drivers, each chosen from what the input is:
+//   D, the device layout: the reads are resident on the device and the hash form of the count runs.  The slot / tile layout
+//      is built on the device into buffers sized from earlier calls, so nothing comes back before the results block.  The
+//      chained sample (sample.cu) runs it with the candidate list and its count on the device, tc_extract_inserts with the list
+//      uploaded from the host.
+//   H, the host layout (tc_extract_inserts only): some arrays are host-resident and staged range by range, or the sorted form
+//      is asked for, or D could not hold the input.  The candidates' read ranges come back first and the host lays the slots out.
+// Every pass ends in one copy of its results block, which ins_unpack reads.
+
+// The results block: the calls and their inserted characters; the status, whose reserved words hold the device-built layout
+// and the pair-scratch bump; the overflow flags; with_extra (the chained form) the extra section 128 bytes behind the status
+// (candidate count, the pileup's status, the candidates); then seg_count / pair_any.  The host copies back everything up to
+// the overflow flags, the chained form the whole block.  n_cand: the candidates, or the capacity the chained form enqueues for.
 static ins_block ins_block_of(int n_cand, bool with_extra) {
-    static_assert(sizeof(tc_status) <= 64, "tc_status outgrew its place in the results block");
+    static_assert(sizeof(tc_status) <= 64 && offsetof(tc_status, reserved) == 24 && sizeof(tc_status::reserved) >= 24,
+                  "the results block's layout words and pair bump no longer fit the status block's reserved words");
+    const size_t n = (size_t)n_cand;
     ins_block b;
-    b.layout = 64; b.over = 80; b.bump = 88;
-    b.extra = with_extra ? 128 : 0;
-    b.seg = with_extra ? b.extra + 4 * (TC_RB_EXTRA_CAND + (size_t)n_cand) : 96;
-    b.calls = b.seg + ((4 * (2 * (size_t)n_cand + 2) + 15) & ~(size_t)15);
-    b.fixed = b.calls + sizeof(tc_insert_call_t) * (size_t)n_cand;
-    b.bytes = b.fixed + (size_t)n_cand * INS_BASES_FIXED;
+    b.calls = 0; b.fixed = sizeof(tc_insert_call_t) * n; b.status = b.fixed + n * INS_BASES_FIXED;
+    b.layout = b.status + 24; b.bump = b.status + 40; b.over = b.status + 64;
+    b.extra = with_extra ? b.status + 128 : 0;
+    b.seg = with_extra ? b.extra + 4 * (TC_RB_EXTRA_CAND + n) : (b.over + 4 + 15) & ~(size_t)15;
+    b.bytes = b.seg + ((4 * (2 * n + 2) + 15) & ~(size_t)15);
+    b.host = with_extra ? b.bytes : b.over + 4;
     return b;
+}
+
+// What every results block holds ahead of the calls.  ins_unpack also copies its first n calls to `calls`; the inserted
+// characters stay in the block (blk + rb.fixed).
+struct ins_result { tc_status st; int32_t layout[3]; int32_t over; unsigned long long bump; };
+
+static ins_result ins_unpack(const uint8_t* blk, const ins_block& rb, int n, tc_insert_call_t* calls) {
+    ins_result res;
+    memcpy(&res.st, blk + rb.status, sizeof(res.st));
+    memcpy(res.layout, blk + rb.layout, sizeof(res.layout)); memcpy(&res.over, blk + rb.over, 4); memcpy(&res.bump, blk + rb.bump, 8);
+    memcpy(calls, blk + rb.calls, sizeof(tc_insert_call_t) * (size_t)n);
+    return res;
 }
 
 // One slab (SLOT_INS_D) for T entry slots and NT tiles: keys, indel, qpos, head, sel, quality per slot; tile tables;
@@ -772,13 +796,21 @@ static int ins_bind(tc_ctx* ctx, ins_args& a, uint8_t* d_rb, const ins_block& rb
     return TC_OK;
 }
 
-// the slot / tile layout built on the device into the bound buffers (T slots, NT tiles); rb.extra: the chained form's extra section
-static int ins_layout_dev(tc_ctx* ctx, ins_args& a, uint8_t* d_rb, const ins_block& rb, size_t T, size_t NT, const tc_status* pileup_status,
-                          cudaStream_t s) {
-    int32_t* d_layout = (int32_t*)(d_rb + rb.layout);
-    a.layout = d_layout;
-    ins_layout_kernel<<<1, 256, 0, s>>>(a, const_cast<int64_t*>(a.seg_off), const_cast<int32_t*>(a.tile_first), const_cast<int32_t*>(a.tile_cand),
-                                        d_layout, (int64_t)T, (int)NT, pileup_status, rb.extra ? (int32_t*)(d_rb + rb.extra) : nullptr);
+// The results block (SLOT_INS_E, zeroed from its status on) and the read range of each of up to `cap` candidates; without the
+// caller's span bound (a.span_hint == 0) the longest span is found first.
+static int ins_ranges(tc_ctx* ctx, ins_args& a, const ins_block& rb, const int32_t* d_cand, int cap, const int32_t* d_ncand, uint8_t** d_rb,
+                      cudaStream_t s) {
+    *d_rb = (uint8_t*)tc_dev_buf(ctx, SLOT_INS_E, rb.bytes + 16);
+    int32_t* d_range = (int32_t*)tc_dev_buf(ctx, SLOT_INS_B, 24 * (size_t)cap);       // [cap][2] ranges, then [cap][4] offsets
+    if (!*d_rb || !d_range) return TC_ERR_NOMEM;
+    TC_CUDA(cudaMemsetAsync(*d_rb + rb.status, 0, rb.bytes - rb.status, s));
+    a.status = (tc_status*)(*d_rb + rb.status);
+    if (a.span_hint == 0 && a.r.n > 0) {
+        max_span_kernel<<<(unsigned)((a.r.n + 255) / 256), 256, 0, s>>>(a.r, a.status);
+        TC_LAUNCH_CHECK();
+    }
+    a.cand = d_cand; a.n_cand = cap; a.n_cand_dev = d_ncand; a.range = d_range; a.range_off = (uint32_t*)(d_range + 2 * (size_t)cap);
+    cand_range_kernel<<<(cap + 3) / 4, 128, 0, s>>>(a);
     TC_LAUNCH_CHECK();
     return TC_OK;
 }
@@ -820,15 +852,12 @@ static int ins_check_status(tc_ctx* ctx, const tc_status& st) {
 }
 
 // Every call's offset into the caller's `bases` (-1 without inserted characters), and the winners' inserted characters
-// placed there from `fixed` ([n][INS_BASES_FIXED]); an insertion longer than INS_BASES_FIXED gets its offset only.  *need_out:
-// the bytes all insertions take.
-static int ins_place_bases(tc_ctx* ctx, tc_insert_call_t* calls, int n, const uint8_t* fixed, uint8_t* bases, int64_t bases_cap,
-                           int64_t* need_out = nullptr) {
+// placed there from `fixed` ([n][INS_BASES_FIXED]); an insertion longer than INS_BASES_FIXED gets its offset only.
+static int ins_place_bases(tc_ctx* ctx, tc_insert_call_t* calls, int n, const uint8_t* fixed, uint8_t* bases, int64_t bases_cap) {
     int64_t need = 0;
     for (int i = 0; i < n; ++i) {
         if (calls[i].indel > 0) { calls[i].bases_off = need; need += calls[i].indel; } else calls[i].bases_off = -1;
     }
-    if (need_out) *need_out = need;
     if (need > 0 && (!bases || need > bases_cap)) return tc_fail(ctx, TC_ERR_CAPACITY, "bases buffer too small: need %lld bytes", (long long)need);
     for (int i = 0; i < n; ++i)
         if (calls[i].indel > 0 && calls[i].indel <= INS_BASES_FIXED)
@@ -855,18 +884,74 @@ static int ins_stage_merged(const T* r, int stride, int n, F copy) {
     return TC_OK;
 }
 
-static int ins_copy(tc_ctx* ctx, const void* dst, const void* src, size_t bytes, cudaMemcpyKind kind, cudaStream_t s, const char* what) {
-    const cudaError_t e = cudaMemcpyAsync(const_cast<void*>(dst), src, bytes, kind, s);
-    return e == cudaSuccess ? TC_OK : tc_cuda_fail(ctx, e, what);
-}
-
-static int ins_sync(tc_ctx* ctx, cudaStream_t s, const char* what) {
-    const cudaError_t e = cudaStreamSynchronize(s);
-    return e == cudaSuccess ? TC_OK : tc_cuda_fail(ctx, e, what);
-}
-
 template <class T>
 static std::unique_ptr<T[]> host_array(size_t n) { return std::unique_ptr<T[]>(new (std::nothrow) T[n > 0 ? n : 1]); }
+
+// The pinned buffer the separate call's blocks come back to (a copy into pageable memory waits for the stream), grow-only.
+// Nothing else uses it, and every copy into it has completed when tc_extract_inserts returns.
+static uint8_t* ins_host_block(tc_ctx* ctx, size_t bytes) {
+    if (ctx->host_scratch_cap < bytes) {
+        if (ctx->host_scratch) cudaFreeHost(ctx->host_scratch);
+        ctx->host_scratch_cap = (bytes + 0xffff) & ~(size_t)0xffff;
+        const cudaError_t e = cudaMallocHost(&ctx->host_scratch, ctx->host_scratch_cap);
+        if (e != cudaSuccess) {
+            tc_fail(ctx, TC_ERR_NOMEM, "cudaMallocHost(%zu) failed: %s", ctx->host_scratch_cap, cudaGetErrorString(e));
+            cudaGetLastError();
+            ctx->host_scratch = nullptr; ctx->host_scratch_cap = 0;
+        }
+    }
+    return (uint8_t*)ctx->host_scratch;
+}
+
+// Insertions longer than INS_BASES_FIXED (rare), after ins_place_bases gave them their place in `bases`: one more small kernel
+// fetches their characters.  The calls in the block (blk) still hold the winners' entry ids in bases_off.
+static int ins_fetch_long(tc_ctx* ctx, const ins_args& a, const uint8_t* blk, const ins_block& rb, const tc_insert_call_t* calls, int n,
+                          uint8_t* bases, cudaStream_t s) {
+    int64_t need = 0, n_long = 0;
+    for (int i = 0; i < n; ++i) { need += calls[i].indel > 0 ? calls[i].indel : 0; n_long += calls[i].indel > INS_BASES_FIXED; }
+    if (n_long == 0) return TC_OK;
+    uint8_t* d_bases = (uint8_t*)tc_dev_buf(ctx, SLOT_TMP_A, (size_t)need);
+    tc_insert_call_t* d_calls = (tc_insert_call_t*)tc_dev_buf(ctx, SLOT_TMP_B, (sizeof(tc_insert_call_t) + 8) * (size_t)n);
+    if (!d_bases || !d_calls) return TC_ERR_NOMEM;
+    int64_t* d_entry = (int64_t*)(d_calls + n);
+    auto h_entry = host_array<int64_t>((size_t)n);
+    auto h_long = host_array<uint8_t>((size_t)need);
+    if (!h_entry || !h_long) return tc_fail(ctx, TC_ERR_NOMEM, "out of host memory");
+    const tc_insert_call_t* found = (const tc_insert_call_t*)(blk + rb.calls);
+    for (int i = 0; i < n; ++i) h_entry[i] = found[i].bases_off;
+    TC_CUDA(cudaMemcpyAsync(d_entry, h_entry.get(), 8 * (size_t)n, cudaMemcpyHostToDevice, s));
+    TC_CUDA(cudaMemcpyAsync(d_calls, calls, sizeof(tc_insert_call_t) * (size_t)n, cudaMemcpyHostToDevice, s));
+    ins_bases_kernel<<<n, 128, 0, s>>>(a, d_calls, d_entry, d_bases);
+    TC_LAUNCH_CHECK();
+    TC_D2H(h_long.get(), d_bases, (size_t)need, s);
+    TC_CUDA(cudaStreamSynchronize(s));
+    for (int i = 0; i < n; ++i)
+        if (calls[i].indel > INS_BASES_FIXED) memcpy(bases + calls[i].bases_off, h_long.get() + calls[i].bases_off, (size_t)calls[i].indel);
+    return TC_OK;
+}
+
+// D: the ranges, the layout built on the device into ins_slot_cap slots, select -> admit -> pair -> count for up to `cap`
+// candidates (d_ncand not NULL: their number is on the device, and the block gets the extra section), and the block's copy to
+// host_block.  a.r and a.span_hint are set.
+static int ins_enqueue_dev(tc_ctx* ctx, ins_args& a, const int32_t* d_cand, int cap, const int32_t* d_ncand, const tc_pileup_params_t* p,
+                           const tc_status* d_pileup_status, void* host_block, cudaStream_t s, tc_ins_pending* pend) {
+    const ins_block rb = ins_block_of(cap, d_ncand != nullptr);
+    uint8_t* d_rb = nullptr;
+    int rc = ins_ranges(ctx, a, rb, d_cand, cap, d_ncand, &d_rb, s);
+    if (rc) return rc;
+    if (ctx->ins_slot_cap <= 0) ctx->ins_slot_cap = 1 << 16;     // grows to twice the largest layout seen
+    const size_t T = (size_t)ctx->ins_slot_cap, NT = T / INS_TILE + (size_t)cap + 1;
+    if ((rc = ins_bind(ctx, a, d_rb, rb, T, NT, cap, p))) return rc;
+    int32_t* d_layout = (int32_t*)(d_rb + rb.layout);
+    a.layout = d_layout;
+    ins_layout_kernel<<<1, 256, 0, s>>>(a, const_cast<int64_t*>(a.seg_off), const_cast<int32_t*>(a.tile_first), const_cast<int32_t*>(a.tile_cand),
+                                        d_layout, (int64_t)T, (int)NT, d_pileup_status, rb.extra ? (int32_t*)(d_rb + rb.extra) : nullptr);
+    TC_LAUNCH_CHECK();
+    if (a.r.n > 0 && (rc = ins_enqueue_count(ctx, a, (unsigned)NT, cap, (tc_insert_call_t*)(d_rb + rb.calls), s))) return rc;
+    TC_D2H(host_block, d_rb, rb.host, s);
+    pend->rb = rb; pend->cap = cap; pend->n_reads = a.r.n;
+    return TC_OK;
+}
 
 TC_API int tc_extract_inserts(tc_ctx_t* ctx, const tc_reads_t* reads, int32_t ref_len, const int32_t* cand_pos, int32_t n_cand,
                               const tc_pileup_params_t* p, tc_insert_call_t* calls, uint8_t* bases, int64_t bases_cap, void* stream) {
@@ -879,15 +964,14 @@ TC_API int tc_extract_inserts(tc_ctx_t* ctx, const tc_reads_t* reads, int32_t re
         if (cand_pos[i] < 1 || cand_pos[i] > ref_len) return tc_fail(ctx, TC_ERR_ARG, "candidate position %d outside 1..%d", cand_pos[i], ref_len);
     cudaStream_t s = (cudaStream_t)stream;
     TC_CUDA(cudaSetDevice(ctx->device));
-    auto upload = [&](const void* d, const void* h, size_t bytes, const char* what) {
-        const int rc = ins_copy(ctx, d, h, bytes, cudaMemcpyHostToDevice, s, what);
-        if (rc == TC_OK) ctx->h2d_bytes += (int64_t)bytes;
-        return rc;
+    auto upload = [&](const void* d, const void* h, size_t bytes) {
+        TC_CUDA(cudaMemcpyAsync(const_cast<void*>(d), h, bytes, cudaMemcpyHostToDevice, s));
+        ctx->h2d_bytes += (int64_t)bytes;
+        return TC_OK;
     };
-    // Every pass runs from the start.  A pass runs again when the pair scratch overflowed (sized from its bump), or when the
-    // speculative layout did not fit (sized for next time) or a column needs the sorted form: then with the layout built on
-    // the host (reserved bit 0).
-    tc_pileup_params_t q = *p;
+    // D unless some array is staged range by range or the sorted form is asked for.  Every pass runs from the start: again
+    // after a pair-scratch overflow (the scratch sized from its bump), and as H when D could not hold the input.
+    bool dev = p->kernel != 2;
     for (;;) {
         ins_args a;
         memset(&a, 0, sizeof(a));
@@ -903,132 +987,75 @@ TC_API int tc_extract_inserts(tc_ctx_t* ctx, const tc_reads_t* reads, int32_t re
         const bool host_qual = reads->qual && !tc_is_device_ptr(reads->qual);
         const bool host_cig = bounded && reads->cigar && !tc_is_device_ptr(reads->cigar);
         const bool host_mate = reads->qname_hash && reads->mpos && reads->isize && !tc_is_device_ptr(reads->qname_hash);
+        dev = dev && !(host_seq || host_qual || host_cig || host_mate);
         int rc = tc_resolve_reads(ctx, reads, &a.r, stage, s);
         if (rc) return rc;
-        const int64_t n = a.r.n;
         for (int i = 0; i < n_cand; ++i) { calls[i].pos = cand_pos[i]; calls[i].n_entries = 0; calls[i].mode_count = 0; calls[i].first_read = -1; calls[i].head = 0; calls[i].indel = 0; calls[i].bases_off = -1; }
-        if (n == 0) return TC_OK;
-        const ins_block rb = ins_block_of(n_cand, false);
-        uint8_t* d_rb = (uint8_t*)tc_dev_buf(ctx, SLOT_INS_E, rb.bytes + 16);
-        int32_t* d_cand = (int32_t*)tc_dev_buf(ctx, SLOT_INS_A, 4 * (size_t)n_cand);
-        int32_t* d_range = (int32_t*)tc_dev_buf(ctx, SLOT_INS_B, 24 * (size_t)n_cand);       // [n_cand][2] ranges, then [n_cand][4] offsets
-        if (!d_rb || !d_cand || !d_range) return TC_ERR_NOMEM;
-        a.status = (tc_status*)d_rb;
-        TC_CUDA(cudaMemsetAsync(d_rb, 0, rb.calls, s));
-        TC_CUDA(cudaMemcpyAsync(d_cand, cand_pos, 4 * (size_t)n_cand, cudaMemcpyHostToDevice, s));
-        ctx->h2d_bytes += 4 * (int64_t)n_cand;
+        if (a.r.n == 0) return TC_OK;
         a.span_hint = bounded ? reads->max_ref_span : 0;
-        if (a.span_hint == 0) {
-            max_span_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(a.r, a.status);
-            TC_LAUNCH_CHECK();
+        const ins_block rb = ins_block_of(n_cand, false);
+        int32_t* d_cand = (int32_t*)tc_dev_buf(ctx, SLOT_INS_A, 4 * (size_t)n_cand);
+        uint8_t* blk = ins_host_block(ctx, rb.host);
+        if (!d_cand || !blk) return TC_ERR_NOMEM;
+        if ((rc = upload(d_cand, cand_pos, 4 * (size_t)n_cand))) return rc;
+        if (dev) {
+            tc_ins_pending pend;
+            int fit = 0;
+            if ((rc = ins_enqueue_dev(ctx, a, d_cand, n_cand, nullptr, p, nullptr, blk, s, &pend))) return rc;
+            TC_CUDA(cudaStreamSynchronize(s));
+            rc = tc_inserts_finish_dev(ctx, &pend, blk, nullptr, nullptr, nullptr, calls, bases, bases_cap, &fit);
+            if (fit == 0) dev = false;
+            if (fit <= 0) continue;
+            return rc ? rc : ins_fetch_long(ctx, a, blk, rb, calls, n_cand, bases, s);
         }
-        a.cand = d_cand; a.n_cand = n_cand; a.range = d_range; a.range_off = (uint32_t*)(d_range + 2 * (size_t)n_cand);
-        cand_range_kernel<<<(n_cand + 3) / 4, 128, 0, s>>>(a);
-        TC_LAUNCH_CHECK();
-        // Layout of the entry slots.  With everything resident on the device and the hash count, the layout is built
-        // on the device into buffers sized from the last calls (no read-back of the ranges, one synchronisation per
-        // call); otherwise — host arrays to stage range by range, the sorted form, or a layout that did not fit — on
-        // the host from the ranges.
-        const bool spec = !(host_seq || host_qual || host_cig || host_mate) && q.kernel != 2 && !(q.reserved & 1);
-        if (ctx->ins_slot_cap <= 0) ctx->ins_slot_cap = 1 << 16;     // grows to twice the largest layout seen
-        std::unique_ptr<int64_t[]> h_off;
-        std::unique_ptr<int32_t[]> h_tfirst, h_tcand;
-        int64_t total = ctx->ins_slot_cap;
-        int n_tiles = (int)(total / INS_TILE) + n_cand + 1;
-        if (!spec) {
-            auto h_range = host_array<int32_t>(6 * (size_t)n_cand);
-            h_off = host_array<int64_t>((size_t)n_cand + 1);
-            h_tfirst = host_array<int32_t>((size_t)n_cand + 1);
-            if (!h_range || !h_off || !h_tfirst) return tc_fail(ctx, TC_ERR_NOMEM, "out of host memory");
-            if ((rc = ins_copy(ctx, h_range.get(), d_range, 24 * (size_t)n_cand, cudaMemcpyDeviceToHost, s, "range readback")) ||
-                (rc = ins_sync(ctx, s, "range readback")))
-                return rc;
-            ctx->d2h_bytes += 24 * (int64_t)n_cand;
-            // QNAME hash, PNEXT, TLEN of the reads over the candidate columns (read index ranges); SEQ + QUAL word ranges; CIGAR op ranges
-            if (host_mate)
-                rc = ins_stage_merged(h_range.get(), 2, n_cand, [&](size_t b0, size_t len) {
-                    int e = upload(a.r.qname_hash + b0, reads->qname_hash + b0, 8 * len, "QNAME hash range upload");
-                    if (!e) e = upload(a.r.mpos + b0, reads->mpos + b0, 4 * len, "PNEXT range upload");
-                    if (!e) e = upload(a.r.isize + b0, reads->isize + b0, 4 * len, "TLEN range upload");
-                    return e;
-                });
-            const uint32_t* ho = (const uint32_t*)(h_range.get() + 2 * (size_t)n_cand);
-            if (!rc && (host_seq || host_qual))
-                rc = ins_stage_merged(ho, 4, n_cand, [&](size_t b0, size_t len) {
-                    int e = host_seq ? upload(a.r.seq4 + b0, reads->seq4 + b0, 4 * len, "SEQ range upload") : TC_OK;
-                    if (!e && host_qual) e = upload(a.r.qual + 8 * b0, reads->qual + 8 * b0, 8 * len, "QUAL range upload");
-                    return e;
-                });
-            if (!rc && host_cig)
-                rc = ins_stage_merged(ho + 2, 4, n_cand,
-                                      [&](size_t b0, size_t len) { return upload(a.r.cigar + b0, reads->cigar + b0, 4 * len, "CIGAR range upload"); });
-            if (rc) return rc;
-            h_off[0] = 0; h_tfirst[0] = 0;
-            for (int i = 0; i < n_cand; ++i) {
-                const int64_t len = h_range[2 * i + 1] - h_range[2 * i];
-                h_off[i + 1] = h_off[i] + len;
-                h_tfirst[i + 1] = h_tfirst[i] + (int32_t)((len + INS_TILE - 1) / INS_TILE);
-            }
-            total = h_off[n_cand];
-            n_tiles = h_tfirst[n_cand];
-            if (total >= 0x7fffffffll) return tc_fail(ctx, TC_ERR_CAPACITY, "too many candidate column entries (%lld)", (long long)total);
-            h_tcand = host_array<int32_t>((size_t)n_tiles);
-            if (!h_tcand) return tc_fail(ctx, TC_ERR_NOMEM, "out of host memory");
-            for (int i = 0; i < n_cand; ++i) for (int t = h_tfirst[i]; t < h_tfirst[i + 1]; ++t) h_tcand[t] = i;
-        }
-        const size_t T = (size_t)(total > 0 ? total : 1), NT = (size_t)(n_tiles > 0 ? n_tiles : 1);
-        if ((rc = ins_bind(ctx, a, d_rb, rb, T, NT, n_cand, &q))) return rc;
-        tc_insert_call_t* d_calls = (tc_insert_call_t*)(d_rb + rb.calls);
-        if (spec) rc = ins_layout_dev(ctx, a, d_rb, rb, T, NT, nullptr, s);
-        else if (!(rc = upload(a.seg_off, h_off.get(), 8 * ((size_t)n_cand + 1), "offset upload")) &&
-                 !(rc = upload(a.tile_first, h_tfirst.get(), 4 * ((size_t)n_cand + 1), "tile table upload")) && n_tiles)
-            rc = upload(a.tile_cand, h_tcand.get(), 4 * (size_t)n_tiles, "tile table upload");
+        // H
+        uint8_t* d_rb = nullptr;
+        if ((rc = ins_ranges(ctx, a, rb, d_cand, n_cand, nullptr, &d_rb, s))) return rc;
+        auto h_range = host_array<int32_t>(6 * (size_t)n_cand);
+        auto h_off = host_array<int64_t>((size_t)n_cand + 1);
+        auto h_tfirst = host_array<int32_t>((size_t)n_cand + 1);
+        if (!h_range || !h_off || !h_tfirst) return tc_fail(ctx, TC_ERR_NOMEM, "out of host memory");
+        TC_D2H(h_range.get(), a.range, 24 * (size_t)n_cand, s);
+        TC_CUDA(cudaStreamSynchronize(s));
+        // QNAME hash, PNEXT, TLEN of the reads over the candidate columns (read index ranges); SEQ + QUAL word ranges; CIGAR op ranges
+        if (host_mate)
+            rc = ins_stage_merged(h_range.get(), 2, n_cand, [&](size_t b0, size_t len) {
+                int e = upload(a.r.qname_hash + b0, reads->qname_hash + b0, 8 * len);
+                if (!e) e = upload(a.r.mpos + b0, reads->mpos + b0, 4 * len);
+                if (!e) e = upload(a.r.isize + b0, reads->isize + b0, 4 * len);
+                return e;
+            });
+        const uint32_t* ho = (const uint32_t*)(h_range.get() + 2 * (size_t)n_cand);
+        if (!rc && (host_seq || host_qual))
+            rc = ins_stage_merged(ho, 4, n_cand, [&](size_t b0, size_t len) {
+                int e = host_seq ? upload(a.r.seq4 + b0, reads->seq4 + b0, 4 * len) : TC_OK;
+                if (!e && host_qual) e = upload(a.r.qual + 8 * b0, reads->qual + 8 * b0, 8 * len);
+                return e;
+            });
+        if (!rc && host_cig)
+            rc = ins_stage_merged(ho + 2, 4, n_cand, [&](size_t b0, size_t len) { return upload(a.r.cigar + b0, reads->cigar + b0, 4 * len); });
         if (rc) return rc;
-        const bool sorted_form = q.kernel == 2;
-        if ((rc = ins_enqueue_count(ctx, a, (unsigned)n_tiles, n_cand, sorted_form ? nullptr : d_calls, s))) return rc;
-        int32_t h_over = 0;
-        unsigned long long h_bump = 0;
-        int32_t h_layout[3] = {0, 0, 0};
-        const size_t calls_bytes = sizeof(tc_insert_call_t) * (size_t)n_cand, fixed_bytes = (size_t)n_cand * INS_BASES_FIXED;
-        auto h_fixed = host_array<uint8_t>(fixed_bytes);
-        if (!h_fixed) return tc_fail(ctx, TC_ERR_NOMEM, "out of host memory");
-        // the results block comes back in one copy through pinned memory (copies into the caller's pageable buffers
-        // would each wait for the stream)
-        if (rb.bytes <= TC_HOST_SCRATCH) {
-            const uint8_t* pin = (const uint8_t*)ctx->host_scratch;
-            if ((rc = ins_copy(ctx, pin, d_rb, rb.bytes, cudaMemcpyDeviceToHost, s, "results readback")) || (rc = ins_sync(ctx, s, "results readback")))
-                return rc;
-            memcpy(ctx->host_status, pin, sizeof(tc_status));
-            memcpy(h_layout, pin + rb.layout, 12); memcpy(&h_over, pin + rb.over, 4); memcpy(&h_bump, pin + rb.bump, 8);
-            memcpy(calls, pin + rb.calls, calls_bytes); memcpy(h_fixed.get(), pin + rb.fixed, fixed_bytes);
-        } else if ((rc = ins_copy(ctx, &h_over, a.overflow, 4, cudaMemcpyDeviceToHost, s, "overflow readback")) ||
-                   (rc = ins_copy(ctx, &h_bump, a.pair_bump, 8, cudaMemcpyDeviceToHost, s, "overflow readback")) ||
-                   (spec && (rc = ins_copy(ctx, h_layout, a.layout, 12, cudaMemcpyDeviceToHost, s, "layout readback"))) ||
-                   (rc = ins_copy(ctx, calls, d_calls, calls_bytes, cudaMemcpyDeviceToHost, s, "insert calls readback")) ||
-                   (rc = ins_copy(ctx, h_fixed.get(), a.bases_fixed, fixed_bytes, cudaMemcpyDeviceToHost, s, "inserted bases readback")) ||
-                   (rc = ins_copy(ctx, ctx->host_status, a.status, sizeof(tc_status), cudaMemcpyDeviceToHost, s, "status readback")) ||
-                   (rc = ins_sync(ctx, s, "insert calls readback"))) {
+        h_off[0] = 0; h_tfirst[0] = 0;
+        for (int i = 0; i < n_cand; ++i) {
+            const int64_t len = h_range[2 * i + 1] - h_range[2 * i];
+            h_off[i + 1] = h_off[i] + len;
+            h_tfirst[i + 1] = h_tfirst[i] + (int32_t)((len + INS_TILE - 1) / INS_TILE);
+        }
+        const int64_t total = h_off[n_cand];
+        const int n_tiles = h_tfirst[n_cand];
+        if (total >= 0x7fffffffll) return tc_fail(ctx, TC_ERR_CAPACITY, "too many candidate column entries (%lld)", (long long)total);
+        auto h_tcand = host_array<int32_t>((size_t)n_tiles);
+        if (!h_tcand) return tc_fail(ctx, TC_ERR_NOMEM, "out of host memory");
+        for (int i = 0; i < n_cand; ++i) for (int t = h_tfirst[i]; t < h_tfirst[i + 1]; ++t) h_tcand[t] = i;
+        const size_t T = (size_t)(total > 0 ? total : 1), NT = (size_t)(n_tiles > 0 ? n_tiles : 1);
+        if ((rc = ins_bind(ctx, a, d_rb, rb, T, NT, n_cand, p))) return rc;
+        if ((rc = upload(a.seg_off, h_off.get(), 8 * ((size_t)n_cand + 1))) || (rc = upload(a.tile_first, h_tfirst.get(), 4 * ((size_t)n_cand + 1))) ||
+            (n_tiles && (rc = upload(a.tile_cand, h_tcand.get(), 4 * (size_t)n_tiles))))
             return rc;
-        }
-        ctx->d2h_bytes += (int64_t)(sizeof(tc_insert_call_t) + INS_BASES_FIXED) * n_cand + (int64_t)sizeof(tc_status) + 4;
-        if (sorted_form) h_over &= 2;
-        if (h_over & 2) {
-            // the scratch for the rewritten quality strings of overlapping mates was too small: size it and run again
-            ctx->pair_cap = 2 * (int64_t)h_bump + 4096;
-            continue;
-        }
-        if (spec) {
-            if (h_layout[2] || h_over) {
-                // the layout did not fit the speculative buffers (size them for next time), or a column needs the sorted
-                // form: run again with the layout built on the host
-                if (h_layout[2]) ctx->ins_slot_cap = 2 * (int64_t)h_layout[1] + 4096;
-                q.reserved |= 1;
-                continue;
-            }
-            total = h_layout[1];
-        }
-        if (sorted_form || h_over) {
-            // radix sort + run-length encoding over the same slots
+        const bool sorted_form = p->kernel == 2;
+        tc_insert_call_t* d_calls = (tc_insert_call_t*)(d_rb + rb.calls);
+        // the sorted form of the count: radix sort + run-length encoding over the same slots
+        auto sorted_count = [&]() {
             uint8_t* slab2 = (uint8_t*)tc_dev_buf(ctx, SLOT_INS_C, T * (8 + 4 + 4) + 64);
             if (!slab2) return TC_ERR_NOMEM;
             uint64_t* d_skey = (uint64_t*)slab2; uint32_t* d_idx = (uint32_t*)(d_skey + T); uint32_t* d_sidx = d_idx + T;
@@ -1047,106 +1074,70 @@ TC_API int tc_extract_inserts(tc_ctx_t* ctx, const tc_reads_t* reads, int32_t re
             ctx->launches++;
             ins_mode_kernel<<<n_cand, 1024, 0, s>>>(a, d_skey, d_sidx, d_calls);
             TC_LAUNCH_CHECK();
-            if ((rc = ins_copy(ctx, calls, d_calls, calls_bytes, cudaMemcpyDeviceToHost, s, "insert calls readback")) ||
-                (rc = ins_copy(ctx, h_fixed.get(), a.bases_fixed, fixed_bytes, cudaMemcpyDeviceToHost, s, "inserted bases readback")) ||
-                (rc = ins_copy(ctx, ctx->host_status, a.status, sizeof(tc_status), cudaMemcpyDeviceToHost, s, "status readback")) ||
-                (rc = ins_sync(ctx, s, "insert calls readback")))
-                return rc;
-        }
-        tc_status st; memcpy(&st, ctx->host_status, sizeof(st));
-        if ((rc = ins_check_status(ctx, st))) return rc;
-        // lay the winners' inserted characters out in the caller's buffer: up to INS_BASES_FIXED characters came back
-        // with the call; longer insertions (rare) are fetched by one more small kernel
-        auto h_entry = host_array<int64_t>((size_t)n_cand);
-        if (!h_entry) return tc_fail(ctx, TC_ERR_NOMEM, "out of host memory");
-        int64_t n_long = 0;
-        for (int i = 0; i < n_cand; ++i) { h_entry[i] = calls[i].bases_off; n_long += calls[i].indel > INS_BASES_FIXED; }
-        int64_t need = 0;
-        if ((rc = ins_place_bases(ctx, calls, n_cand, h_fixed.get(), bases, bases_cap, &need)) || n_long == 0) return rc;
-        uint8_t* d_bases = (uint8_t*)tc_dev_buf(ctx, SLOT_TMP_A, (size_t)need);
-        int64_t* d_entry = (int64_t*)tc_dev_buf(ctx, SLOT_TMP_B, 8 * (size_t)n_cand);
-        auto h_long = host_array<uint8_t>((size_t)need);
-        if (!d_bases || !d_entry || !h_long) return TC_ERR_NOMEM;
-        const char* what = "inserted bases readback";
-        if ((rc = ins_copy(ctx, d_entry, h_entry.get(), 8 * (size_t)n_cand, cudaMemcpyHostToDevice, s, what)) ||
-            (rc = ins_copy(ctx, d_calls, calls, calls_bytes, cudaMemcpyHostToDevice, s, what)))
+            return TC_OK;
+        };
+        if ((rc = ins_enqueue_count(ctx, a, (unsigned)n_tiles, n_cand, sorted_form ? nullptr : d_calls, s)) || (sorted_form && (rc = sorted_count())))
             return rc;
-        ins_bases_kernel<<<n_cand, 128, 0, s>>>(a, d_calls, d_entry, d_bases);
-        TC_LAUNCH_CHECK();
-        if (!(rc = ins_copy(ctx, h_long.get(), d_bases, (size_t)need, cudaMemcpyDeviceToHost, s, what))) rc = ins_sync(ctx, s, what);
-        ctx->d2h_bytes += need;
-        if (rc) return rc;
-        for (int i = 0; i < n_cand; ++i)
-            if (calls[i].indel > INS_BASES_FIXED) memcpy(bases + calls[i].bases_off, h_long.get() + calls[i].bases_off, (size_t)calls[i].indel);
-        return TC_OK;
+        TC_D2H(blk, d_rb, rb.host, s);
+        TC_CUDA(cudaStreamSynchronize(s));
+        ins_result res = ins_unpack(blk, rb, n_cand, calls);
+        if (res.over & 2) {
+            // the scratch for the rewritten quality strings of overlapping mates was too small: size it and run again
+            ctx->pair_cap = 2 * (int64_t)res.bump + 4096;
+            continue;
+        }
+        if (res.over) {
+            // a column has more distinct strings than the hash count's table holds: the sorted form, and its block
+            if ((rc = sorted_count())) return rc;
+            TC_D2H(blk, d_rb, rb.host, s);
+            TC_CUDA(cudaStreamSynchronize(s));
+            res = ins_unpack(blk, rb, n_cand, calls);
+        }
+        if ((rc = ins_check_status(ctx, res.st)) || (rc = ins_place_bases(ctx, calls, n_cand, blk + rb.fixed, bases, bases_cap))) return rc;
+        return ins_fetch_long(ctx, a, blk, rb, calls, n_cand, bases, s);
     }
 }
 
-
-// ---------------------------------------------------------------- candidates that never leave the device
-// tc_pileup_call_inserts (sample.cu): the candidate list is what the call kernel flagged; its length is only known on
-// the device.  Everything is enqueued for up to `cap` candidates into buffers sized from earlier calls, and ONE block
-// of results travels back: the insertion calls, the candidate list, and the pileup's status.  Whatever does not fit this
-// speculative layout (more candidates than cap, more entry slots than the buffers hold, a column with thousands of
-// distinct strings, an insertion longer than INS_BASES_FIXED characters) is reported as TC_ERR_CAPACITY in `fit` and the
-// caller runs tc_extract_inserts with the list it got back.
+// The chained sample's D (tc_pileup_call_inserts): the candidate list is what the call kernel flagged, its length known only on
+// the device.  The block comes back to the slot's pinned host_block of TC_HOST_SCRATCH bytes.
 int tc_inserts_enqueue_dev(tc_ctx* ctx, const tc_reads_t* reads, const int32_t* d_cand, const int32_t* d_ncand, int cap,
                            const tc_pileup_params_t* p, const tc_status* d_pileup_status, void* host_block, cudaStream_t s, tc_ins_pending* pend) {
+    if (ins_block_of(cap, true).bytes > TC_HOST_SCRATCH) return tc_fail(ctx, TC_ERR_ARG, "candidate capacity %d too large for the pinned results block", cap);
     ins_args a;
     memset(&a, 0, sizeof(a));
-    memset(pend, 0, sizeof(*pend));
-    int rc = tc_resolve_reads(ctx, reads, &a.r, NEED_QUAL | NEED_MATE, s);       // every array is a device pointer already: nothing is copied
+    const int rc = tc_resolve_reads(ctx, reads, &a.r, NEED_QUAL | NEED_MATE, s);     // every array is a device pointer already: nothing is copied
     if (rc) return rc;
-    const int64_t n = a.r.n;
-    const ins_block rb = ins_block_of(cap, true);
-    if (rb.bytes > TC_HOST_SCRATCH) return tc_fail(ctx, TC_ERR_ARG, "candidate capacity %d too large for the pinned results block", cap);
-    uint8_t* d_rb = (uint8_t*)tc_dev_buf(ctx, SLOT_INS_E, rb.bytes + 16);
-    int32_t* d_range = (int32_t*)tc_dev_buf(ctx, SLOT_INS_B, 24 * (size_t)cap);
-    if (!d_rb || !d_range) return TC_ERR_NOMEM;
-    TC_CUDA(cudaMemsetAsync(d_rb, 0, rb.calls, s));
     a.span_hint = reads->max_ref_span > 0 ? reads->max_ref_span : 0;
-    a.status = (tc_status*)d_rb;
-    if (a.span_hint == 0 && n > 0) {
-        max_span_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(a.r, a.status);
-        TC_LAUNCH_CHECK();
-    }
-    a.cand = d_cand; a.n_cand = cap; a.n_cand_dev = d_ncand; a.range = d_range; a.range_off = (uint32_t*)(d_range + 2 * (size_t)cap);
-    cand_range_kernel<<<(cap + 3) / 4, 128, 0, s>>>(a);
-    TC_LAUNCH_CHECK();
-    if (ctx->ins_slot_cap <= 0) ctx->ins_slot_cap = 1 << 16;
-    const size_t T = (size_t)ctx->ins_slot_cap, NT = T / INS_TILE + (size_t)cap + 1;
-    if ((rc = ins_bind(ctx, a, d_rb, rb, T, NT, cap, p)) || (rc = ins_layout_dev(ctx, a, d_rb, rb, T, NT, d_pileup_status, s))) return rc;
-    if (n > 0 && (rc = ins_enqueue_count(ctx, a, (unsigned)NT, cap, (tc_insert_call_t*)(d_rb + rb.calls), s))) return rc;
-    TC_CUDA(cudaMemcpyAsync(host_block, d_rb, rb.bytes, cudaMemcpyDeviceToHost, s));
-    ctx->d2h_bytes += (int64_t)rb.bytes;
-    pend->rb = rb; pend->cap = cap; pend->n_reads = n;
-    return TC_OK;
+    return ins_enqueue_dev(ctx, a, d_cand, cap, d_ncand, p, d_pileup_status, host_block, s, pend);
 }
 
-// After the sample's event has completed: unpack its results block.  *fit = 0 when the speculative layout
-// did not hold everything (cands / n_cand are valid all the same whenever n_cand <= cap).
+// A D pass's block, back on the host.  *fit = 1: the calls are final.  0: D could not hold the input (more candidates than cap,
+// more entry slots than the buffers hold — sized for next time —, or a column with more distinct strings than the count's
+// table), H runs.  -1: the pair scratch was too small (sized now), D runs again.  With the chained form's extra section the
+// pileup's status, the candidate count and (when it is at most cap) the candidates come back too, and an insertion longer than
+// INS_BASES_FIXED does not fit either; the separate call fetches those (ins_fetch_long).
 int tc_inserts_finish_dev(tc_ctx* ctx, const tc_ins_pending* pend, const void* host_block, tc_status* pileup_status, int32_t* cands, int32_t* n_cand,
                           tc_insert_call_t* calls, uint8_t* bases, int64_t bases_cap, int* fit) {
-    const uint8_t* pin = (const uint8_t*)host_block;
+    const uint8_t* blk = (const uint8_t*)host_block;
     const ins_block& rb = pend->rb;
-    const int32_t* extra = (const int32_t*)(pin + rb.extra);
-    tc_status st; memcpy(&st, pin, sizeof(st));
-    memcpy(pileup_status, extra + TC_RB_EXTRA_STATUS, sizeof(tc_status));
-    int32_t layout[3]; memcpy(layout, pin + rb.layout, 12);
-    int32_t over; memcpy(&over, pin + rb.over, 4);
-    const int n = extra[TC_RB_EXTRA_NCAND];
-    *n_cand = n;
+    int n = pend->cap;
+    *fit = 0;
+    if (rb.extra) {
+        const int32_t* extra = (const int32_t*)(blk + rb.extra);
+        memcpy(pileup_status, extra + TC_RB_EXTRA_STATUS, sizeof(tc_status));
+        n = *n_cand = extra[TC_RB_EXTRA_NCAND];
+        if (n > pend->cap) return TC_OK;
+        memcpy(cands, extra + TC_RB_EXTRA_CAND, 4 * (size_t)n);
+    }
+    const ins_result res = ins_unpack(blk, rb, n, calls);
+    if (res.layout[2]) { ctx->ins_slot_cap = 2 * (int64_t)res.layout[1] + 4096; return TC_OK; }
+    if (res.over & 2) { ctx->pair_cap = 2 * (int64_t)res.bump + 4096; *fit = -1; return TC_OK; }
+    if (res.over) return TC_OK;
     *fit = 1;
-    if (n > pend->cap) { *fit = 0; return TC_OK; }
-    memcpy(cands, extra + TC_RB_EXTRA_CAND, 4 * (size_t)n);
-    if (layout[2]) { ctx->ins_slot_cap = 2 * (int64_t)layout[1] + 4096; *fit = 0; return TC_OK; }
-    if (over & 2) { unsigned long long bump; memcpy(&bump, pin + rb.bump, 8); ctx->pair_cap = 2 * (int64_t)bump + 4096; }
-    if (over) { *fit = 0; return TC_OK; }
-    if (const int rc = ins_check_status(ctx, st)) return rc;
-    memcpy(calls, pin + rb.calls, sizeof(tc_insert_call_t) * (size_t)n);
+    if (const int rc = ins_check_status(ctx, res.st)) return rc;
     for (int i = 0; i < n; ++i) {
         if (pend->n_reads == 0) { calls[i].pos = cands[i]; calls[i].n_entries = 0; calls[i].mode_count = 0; calls[i].first_read = -1; calls[i].head = 0; calls[i].indel = 0; }
-        if (calls[i].indel > INS_BASES_FIXED) { *fit = 0; return TC_OK; }       // rare: the separate call fetches long insertions
+        if (rb.extra && calls[i].indel > INS_BASES_FIXED) { *fit = 0; return TC_OK; }
     }
-    return ins_place_bases(ctx, calls, n, pin + rb.fixed, bases, bases_cap);
+    return ins_place_bases(ctx, calls, n, blk + rb.fixed, bases, bases_cap);
 }

@@ -5,11 +5,12 @@
 // library mirror them — each returning host-visible results, i.e. each ending in a synchronisation: the pileup's status
 // block, the candidate list, the insertion calls.  On a sample whose pileup takes half a millisecond those three round
 // trips were a quarter of the step (VERDICT r1: 0.195 ms of 0.715).  Here nothing is read back in between: the
-// candidate list and its length stay on the device, the insertion kernels run for up to TC_SAMPLE_MAX_CAND candidates
-// into buffers sized from earlier calls, and ONE block of results comes back — insertion calls, candidate positions,
-// pileup status — behind one synchronisation.  Whatever the speculative layout cannot hold (more candidates, more entry
-// slots, a column with thousands of distinct strings, an insertion of more than 64 characters, a batch the bit-parallel
-// pileup kernel declines) falls back to the separate entry points, with identical results.
+// candidate list and its length stay on the device, ExtractInserts runs its device-layout driver (D, inserts.cu) for up
+// to TC_SAMPLE_MAX_CAND candidates, and ONE block of results comes back — insertion calls, candidate positions, pileup
+// status — behind one synchronisation.  Whatever D cannot hold here (more candidates, more entry slots, a column with
+// thousands of distinct strings, a pair scratch too small, an insertion of more than 64 characters) goes to
+// tc_extract_inserts with the candidate list that came back, and a batch the bit-parallel pileup kernel declines to the
+// separate entry points, with identical results.
 #include "tc_common.cuh"
 
 constexpr int TC_SAMPLE_MAX_CAND = 256;
@@ -278,9 +279,9 @@ TC_API int tc_sample_finish(tc_ctx_t* ctx, int32_t ticket, tc_insert_call_t* cal
     *n_calls = n;
     if (n > calls_cap) return tc_fail(ctx, TC_ERR_CAPACITY, "%d insertion candidates, capacity %d", n, calls_cap);
     if (n == 0) return TC_OK;
-    if (!fit) {
-        // the speculative layout did not hold it: the separate call, with the candidate list that came back (or, beyond
-        // the chained form's capacity, with a fresh one)
+    if (fit != 1) {
+        // D did not hold it here: the separate call, with the candidate list that came back (or, beyond the chained form's
+        // capacity, with a fresh one)
         if (n > TC_SAMPLE_MAX_CAND) {
             int32_t* cand = (int32_t*)malloc(4 * (size_t)n);
             if (!cand) return tc_fail(ctx, TC_ERR_NOMEM, "out of host memory");

@@ -28,7 +28,7 @@ enum tc_slot {
 
 struct tc_buf { void* p; size_t cap; };
 
-constexpr size_t TC_HOST_SCRATCH = 64 * 1024;
+constexpr size_t TC_HOST_SCRATCH = 64 * 1024;       // a chained sample slot's pinned results block
 struct tc_status;
 struct pileup_plan {            // one attempt at the count table (pileup_plan_of, pileup.cu)
     int variant;                // 1 scatter, 3 warp streams, 4 long reads cut into pieces for the warp streams
@@ -50,8 +50,8 @@ struct tc_ctx {
     int ins_attr_set;       // ins_count_kernel's shared-memory attribute has been set
     uint32_t warp_attr_set; // ... and those of the warp_pileup_kernel instances (one bit each)
     void* host_status;      // pinned, 256 bytes
-    void* host_scratch;     // pinned, TC_HOST_SCRATCH bytes: small results come back here in truly asynchronous copies
-                            // (a cudaMemcpyAsync into pageable memory waits for the stream)
+    void* host_scratch;     // pinned, host_scratch_cap bytes, grow-only: tc_extract_inserts' results blocks (inserts.cu)
+    size_t host_scratch_cap;
     int timing;             // bracket the pileup kernel with events
     cudaEvent_t ev0, ev1;
     int ev_valid;
@@ -59,7 +59,7 @@ struct tc_ctx {
     // trusts a bound only when it is this one — otherwise it finds the longest span itself
     const void* span_ok_cigar; const void* span_ok_off; int64_t span_ok_n, span_ok_ops; int32_t span_ok_bound;
     int64_t pair_cap;       // tc_extract_inserts: bytes of scratch for the rewritten quality strings of overlapping mates; grows on demand
-    int64_t ins_slot_cap;   // tc_extract_inserts: entry slots its speculative (no read-back) layout may use; grows on demand
+    int64_t ins_slot_cap;   // ExtractInserts: entry slots its device-built layout (no read-back) may use; grows on demand
     struct tc_sample_slot* samples;     // [2] samples in flight (tc_sample_enqueue / tc_sample_finish), allocated on first use
     int sample_next;
     int64_t buf_epoch;      // bumped whenever a context buffer is (re)allocated: captured graphs hold the old addresses
@@ -140,8 +140,11 @@ int tc_pileup_settle(tc_ctx* ctx, tc_status st, tc_pileup_pending pend, const tc
 int tc_h2d(tc_ctx* ctx, void* d, const void* p, size_t bytes, cudaStream_t s);
 bool tc_reads_all_device(const tc_reads_t* r);     // every array of the batch already in device memory
 int tc_candidates_enqueue(tc_ctx* ctx, const uint8_t* d_flags, int32_t ref_len, int32_t cap, int32_t** d_count, int32_t** d_sorted, cudaStream_t s);
-// ExtractInserts' results block: one memset in front, one copy back.  Offsets in bytes; ins_block_of (inserts.cu) lays it out.
+// ExtractInserts' results block: one memset in front, one copy back at the end of every pass of either driver (D, the
+// device-built layout; H, the host-built one: inserts.cu).  Offsets in bytes; ins_block_of lays it out.
 struct ins_block {
+    size_t status;      // tc_status of the pass; the memset zeroes the block from here on
+    size_t host;        // the bytes [0, host) the host copies back
     size_t layout;      // int32[3] device-built layout: tiles, slots, 1 = did not fit
     size_t over;        // int32 overflow flags: 1 a column needs the sorted form, 2 the pair scratch was too small
     size_t bump;        // uint64 pair-scratch bump
@@ -153,6 +156,7 @@ struct ins_block {
 };
 // int32 words of the chained form's extra section
 constexpr int TC_RB_EXTRA_NCAND = 0, TC_RB_EXTRA_STATUS = 16, TC_RB_EXTRA_CAND = 32;
+// A D pass enqueued and not yet finished: its block's layout, the candidate capacity, the reads (*fit: tc_inserts_finish_dev).
 struct tc_ins_pending { ins_block rb; int cap; int64_t n_reads; };
 int tc_inserts_enqueue_dev(tc_ctx* ctx, const tc_reads_t* reads, const int32_t* d_cand, const int32_t* d_ncand, int cap,
                            const tc_pileup_params_t* p, const tc_status* d_pileup_status, void* host_block, cudaStream_t s, tc_ins_pending* pend);

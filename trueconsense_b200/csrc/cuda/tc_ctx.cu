@@ -301,8 +301,6 @@ TC_API int tc_ctx_create(int device, tc_ctx_t** out) {
     }
     e = cudaMallocHost(&ctx->host_status, 256);
     if (e != cudaSuccess) { free(ctx); return tc_cuda_fail(NULL, e, "cudaMallocHost"); }
-    e = cudaMallocHost(&ctx->host_scratch, TC_HOST_SCRATCH);
-    if (e != cudaSuccess) { cudaFreeHost(ctx->host_status); free(ctx); return tc_cuda_fail(NULL, e, "cudaMallocHost"); }
     *out = ctx;
     return TC_OK;
 }
